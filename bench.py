@@ -11,6 +11,7 @@ inputs; outputs go to one reused device buffer set (1e9 steps x 160 B does not f
 anything else in 180 GB).  Every launch reads/writes >> 126 MB (L2), so no explicit flush.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--series S] [--T T]
+                  [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -30,6 +31,8 @@ sys.path.insert(0, ROOT)
 N_STATE, N_OBS = 2, 1
 ALGO_BYTES_PER_STEP = 8 * (N_OBS + (2 * N_STATE + 2 * N_STATE ** 2 + N_OBS + N_OBS ** 2)
                            + (N_STATE + N_STATE ** 2) + (N_STATE + N_STATE ** 2))  # 216 (SURVEY 8d)
+# --dump-outputs sample: 256 series at T = 1000 are 41 MB; fewer when one series' outputs are larger
+DUMP_SERIES, DUMP_BYTES, DUMP_SEED = 256, 60_000_000, 20260109
 
 
 def parse():
@@ -48,7 +51,16 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-ffbs", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed for a fixed "
+                         "sample of series as DIR/<field>.npy (float64, rank 0's series; f and Q "
+                         "without the initial row, which holds no forecast)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
+    return args
 
 
 class ClockSampler(threading.Thread):
@@ -143,9 +155,10 @@ def timed_cpu(run, min_seconds=2.0, max_reps=100000):
             return reps, dt
 
 
-def cpu_reference_leg(series, T, seconds_target=15.0, threads=None, warm_passes=1):
+def cpu_reference_leg(series, T, seconds_target=15.0, threads=None, warm_passes=1, passes=None):
     """Time the CPU restatement of the reference (oracle, all host cores) on a bounded sample of
-    the same workload.  The JVM reference itself cannot run here (no JDK): kind = "port"."""
+    the same workload.  The JVM reference itself cannot run here (no JDK): kind = "port".
+    `passes` fixes the number of timed passes; without it they fill ~seconds_target."""
     import oracle
     from bayesian_dlms_b200 import dlm
     oracle.build()
@@ -172,8 +185,10 @@ def cpu_reference_leg(series, T, seconds_target=15.0, threads=None, warm_passes=
     _, out = run()          # warm: page-faults the output arrays, spins up the OpenMP team
     for _ in range(max(0, warm_passes - 1)):
         run(out)
-    dt1, out = run(out)
-    reps = int(max(1, min(200, round(seconds_target / max(dt1, 1e-6)))))
+    reps = passes
+    if reps is None:
+        dt1, out = run(out)
+        reps = int(max(1, min(200, round(seconds_target / max(dt1, 1e-6)))))
     t0 = time.perf_counter()
     for _ in range(reps):
         run(out)
@@ -834,8 +849,7 @@ def main():
         if rank != 0:
             return
         # K timed steps, each one pass over the bounded sample (W untimed passes first)
-        base, nser, dt = cpu_reference_leg(B, T, seconds_target=min(30.0, 3.0 * max(1, args.steps)),
-                                           warm_passes=max(1, args.warmup))
+        base, nser, dt = cpu_reference_leg(B, T, passes=args.steps, warm_passes=max(1, args.warmup))
         v = base["value"]
         print(json.dumps({
             "impl": "reference", "metric": "filter+smoother series-steps/s", "value": v,
@@ -886,24 +900,27 @@ def main():
     geometry["series_per_launch"] = bounds[1] - bounds[0]
     Bc_max = max(bounds[i + 1] - bounds[i] for i in range(nch))
     rows = T + 1
+    # The rank's whole batch is drawn first and then cut into launches, so that a series gets the
+    # same data whatever the launch geometry (which follows the kernel's occupancy): two builds of
+    # the library then see identical inputs and their outputs compare series for series.
     g = torch.Generator(device=dev).manual_seed(20260101 + rank)
-    ys, pars = [], []
     Vs_all, Ws_all = synth_params(B, 20260101 + 1000 * rank, np)
+    Vd, Wd = torch.from_numpy(Vs_all).to(dev), torch.from_numpy(Ws_all).to(dev)
+    x0 = 10.0 * torch.randn((B,), generator=g, device=dev, dtype=torch.float64)
+    x1 = 10.0 * torch.randn((B,), generator=g, device=dev, dtype=torch.float64)
+    yall = torch.empty((T, 1, B), device=dev, dtype=torch.float64)
+    sw0, sw1, sv = Wd[0].sqrt(), Wd[3].sqrt(), Vd[0].sqrt()
+    for t in range(T):
+        x0 = x0 + x1 + sw0 * torch.randn((B,), generator=g, device=dev, dtype=torch.float64)
+        x1 = x1 + sw1 * torch.randn((B,), generator=g, device=dev, dtype=torch.float64)
+        yall[t, 0] = x0 + sv * torch.randn((B,), generator=g, device=dev, dtype=torch.float64)
+    ys, pars = [], []
     for i in range(nch):
         b0, b1 = bounds[i], bounds[i + 1]
-        Bc = b1 - b0
-        Vs = torch.from_numpy(Vs_all[:, b0:b1].copy()).to(dev)
-        Ws = torch.from_numpy(Ws_all[:, b0:b1].copy()).to(dev)
-        x0 = 10.0 * torch.randn((Bc,), generator=g, device=dev, dtype=torch.float64)
-        x1 = 10.0 * torch.randn((Bc,), generator=g, device=dev, dtype=torch.float64)
-        y = torch.empty((T, 1, Bc), device=dev, dtype=torch.float64)
-        sw0, sw1, sv = Ws[0].sqrt(), Ws[3].sqrt(), Vs[0].sqrt()
-        for t in range(T):
-            x0 = x0 + x1 + sw0 * torch.randn((Bc,), generator=g, device=dev, dtype=torch.float64)
-            x1 = x1 + sw1 * torch.randn((Bc,), generator=g, device=dev, dtype=torch.float64)
-            y[t, 0] = x0 + sv * torch.randn((Bc,), generator=g, device=dev, dtype=torch.float64)
-        ys.append(y)
-        pars.append(dict(V=Vs, W=Ws, m0=np.zeros(2), C0=100.0 * np.eye(2), per_series=("V", "W")))
+        ys.append(yall[:, :, b0:b1].contiguous())
+        pars.append(dict(V=Vd[:, b0:b1].contiguous(), W=Wd[:, b0:b1].contiguous(), m0=np.zeros(2),
+                         C0=100.0 * np.eye(2), per_series=("V", "W")))
+    del yall, x0, x1
     model = Model.build(dlm.polynomial(2), T=T)
     dims = dict(m=2, C=4, a=2, R=4, f=1, Q=1, s=2, S=4)
     outbuf = {k: torch.empty((rows, d, Bc_max), device=dev, dtype=torch.float64)
@@ -919,7 +936,26 @@ def main():
 
     chk = torch.zeros(4, device=dev, dtype=torch.float64)
 
-    def step(timers=None):
+    # --dump-outputs: the full outputs of a step (160 B per series-step) never coexist -- every
+    # launch overwrites the buffers -- so the last timed step keeps a fixed, seeded sample of series
+    # right after each launch (a gather of at most DUMP_BYTES, small next to a launch's traffic)
+    picks = kept = None
+    if args.dump_outputs and rank == 0:
+        per_series = 8 * (rows * sum(dims.values()) + 1)
+        ns = min(B, DUMP_SERIES, DUMP_BYTES // per_series)
+        if ns < 1:
+            sys.exit("--dump-outputs: the outputs of one series exceed %d bytes" % DUMP_BYTES)
+        pick = np.sort(np.random.default_rng(DUMP_SEED).choice(B, size=ns, replace=False))
+        picks = [torch.from_numpy(pick[(pick >= b0) & (pick < b1)] - b0).to(dev)
+                 for b0, b1 in zip(bounds[:-1], bounds[1:])]
+        kept = [{k: v.new_empty(v.shape[:-1] + (len(p),)) for k, v in views(b1 - b0).items()}
+                for p, b0, b1 in zip(picks, bounds[:-1], bounds[1:])]
+
+    def keep_sample(i, o):
+        for k, v in o.items():
+            torch.index_select(v, -1, picks[i], out=kept[i][k])
+
+    def step(timers=None, keep=False):
         for i in range(nch):
             Bc = bounds[i + 1] - bounds[i]
             if timers is not None:
@@ -929,6 +965,8 @@ def main():
             if timers is not None:
                 e1.record()
                 timers.append((e0, e1, Bc))
+            if keep:
+                keep_sample(i, o)
         chk[0] = o["s"][0, 0, 0]; chk[1] = o["S"][0, 0, 0]; chk[2] = o["m"][-1, 0, 0]
         chk[3] = o["status"].max().double()
         if world > 1:
@@ -943,6 +981,9 @@ def main():
 
     for _ in range(args.warmup):
         step()
+    if picks is not None:  # untimed first gather: a kernel's first launch loads its module
+        for i in range(nch):
+            keep_sample(i, views(bounds[i + 1] - bounds[i]))
     barrier()
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
@@ -952,11 +993,19 @@ def main():
     barrier()
     t0 = torch.cuda.Event(enable_timing=True); t1 = torch.cuda.Event(enable_timing=True)
     t0.record()
-    for _ in range(args.steps):
-        step(timers)
+    for it in range(args.steps):
+        step(timers, keep=picks is not None and it == args.steps - 1)
     t1.record()
     barrier()
     ms = t0.elapsed_time(t1)
+    if kept:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k in kept[0]:   # [rows][k][sampled series] as the launches return them; status [series]
+            a = torch.cat([c[k] for c in kept], dim=-1).cpu().numpy().astype(np.float64)
+            if k in ("f", "Q"):  # row 0 is the initial state's placeholder (NaN: no forecast yet)
+                a = a[1:]        # so only the T one-step forecasts are written
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), a)
+        kept.clear()
     launches = eng.ctx.launch_count() - launches0
     clocks = sampler.stop() if sampler else None
     tt = torch.tensor([ms], device=dev, dtype=torch.float64)

@@ -116,5 +116,6 @@ def test_reference_arm_prints_the_contract_line():
     assert d["config"]["workload"].startswith("config2: polynomial(2)")
     assert d["cpu_baseline"]["kind"] in ("port", "reference") and d["cpu_baseline"]["cores"] >= 1
     assert d["cpu_baseline"]["value"] == d["value"]
+    assert " x 1 passes " in d["cpu_baseline"]["sample"]     # --steps 1: one timed pass
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0,
                         "d2h_bytes_per_step": 0}
