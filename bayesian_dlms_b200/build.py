@@ -53,8 +53,7 @@ def build_lib(force: bool = False, verbose: bool = False) -> str:
         obj = os.path.join(objdir, src.replace(".cu", ".o"))
         path = os.path.join(CSRC, src)
         if force or _stale(obj, [path] + headers):
-            extra = os.environ.get("BDLM_NVCC_EXTRA", "").split()  # tuning builds only
-            cmd = ([nvcc] + NVCC_FLAGS + extra + [FMAD.get(src, "-fmad=false")] +
+            cmd = ([nvcc] + NVCC_FLAGS + [FMAD.get(src, "-fmad=false")] +
                    (["-Xptxas", "-v"] if verbose else []) + ["-c", path, "-o", obj])
             r = subprocess.run(cmd, capture_output=True, text=True)
             if verbose or r.returncode:

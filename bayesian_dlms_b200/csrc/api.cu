@@ -11,7 +11,6 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -40,7 +39,6 @@ struct bdlm_ctx {
   long long rng_first = 0;                         // global index of a call's first series
   void *scan_table = nullptr;          // scan.cu forward table of the model in scan_key
   std::vector<double> scan_key, scan_key_pending;
-  bool use_group = std::getenv("BDLM_NO_GROUP_KERNEL") == nullptr;  // A/B switch for profiling
   int64_t range_lo = -1, range_hi = -1;  // ctx_set_range: sub-batch of the next call (comm.cu)
   // Pinned staging for small transfers: the model upload of every call (F, G, dt, shared
   // parameters: a pageable source would make cudaMemcpyAsync stage it synchronously) goes through
@@ -590,7 +588,7 @@ int run_dev(bdlm_ctx *c, DevCall d, Bump bump) {
   // ---- warp-per-series path ----
   int rc = upload_model(c, d, bump, bt, hG0, hF0);
   if (rc) return rc;
-  if (d.op == A_FFBS && ffbs_small_supported(bt) && std::getenv("BDLM_NO_SMALL_FFBS") == nullptr) {
+  if (d.op == A_FFBS && ffbs_small_supported(bt)) {
     // one thread per chain (ffbs_small.cu); (m, C) spill in the caller's arrays when they are
     // wanted, else dense time-major workspace
     const int L = p.layout;
@@ -613,7 +611,7 @@ int run_dev(bdlm_ctx *c, DevCall d, Bump bump) {
     ++c->launches;
     return 0;
   }
-  if (d.op == A_LOGLIK && loglik_small_supported(bt) && std::getenv("BDLM_NO_SMALL_LOGLIK") == nullptr) {
+  if (d.op == A_LOGLIK && loglik_small_supported(bt)) {
     // thread-per-series log-likelihoods (scalar_filters.cu): strided views serve both layouts
     CU(launch_loglik_small(bt, hG0.data(), hF0.data(), d.ll_tr ? d.ll_tr + d.b0 : nullptr,
                            d.ll_in ? d.ll_in + d.b0 : nullptr,
@@ -655,7 +653,7 @@ int run_dev(bdlm_ctx *c, DevCall d, Bump bump) {
   const int wop = warp_op(d.op);
   wa.spill_k = (int64_t)warp_spill_doubles_per_row(wop, p.n, p.p);
   wa.spill = wa.spill_k ? bump.take<double>((size_t)wa.spill_k * R * d.Bc) : nullptr;
-  if (c->use_group && !p.v_tv && !p.w_tv && !bt.ps_model && bt.dt_sb == 0 &&
+  if (!p.v_tv && !p.w_tv && !bt.ps_model && bt.dt_sb == 0 &&
       group_supported(wop, p.n, p.p, p.keep_init ? 1 : 0)) {
     CU(launch_group(wop, wa, c->stream));  // two series per warp, compile-time n (kf_group.cu)
     ++c->launches;

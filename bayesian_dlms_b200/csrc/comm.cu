@@ -24,7 +24,6 @@
 
 #include <algorithm>
 #include <condition_variable>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <functional>
@@ -101,12 +100,6 @@ struct Local {
   double *agg = nullptr;     // device [2][kMaxElem]: this rank's scan aggregates (fwd, bwd)
   double *aggs = nullptr;    // device [2][world][kMaxElem]: gathered aggregates / peer mailbox
   unsigned long long *flags = nullptr;  // device [2][world] mailbox flags, then [1]: this rank's call counter
-  // CUDA graph of one time-sharded scan call on this device: the ~20 dependent launches of a rank
-  // are launch-latency bound at 8 GPUs (0.24 ms of kernels inside 0.45-0.49 ms), so the second
-  // call with the same arguments is captured and later ones replay the graph.
-  std::vector<unsigned long long> graph_key;
-  int graph_seen = 0;
-  cudaGraphExec_t graph_exec = nullptr;
 };
 
 // One persistent host thread per local device: a single thread enqueuing ~20 launches per device
@@ -157,11 +150,6 @@ struct bdlm_comm {
   std::vector<std::unique_ptr<Worker>> workers;  // one per local device when there are several
   std::string err;
   bool peer = false;               // every local device can store into every other's mailbox
-  // CUDA-graph replay of the time-sharded scan is OPT-IN (BDLM_COMM_GRAPH=1) and only used with the
-  // NCCL transport: at 2 GPUs it takes the call from 0.897 to 0.865 ms (host enqueue 0.105 ->
-  // 0.026 ms); with the peer-mailbox transport a replayed graph did not complete on the test box
-  // (unresolved), so that combination stays on direct launches.
-  bool use_graph = std::getenv("BDLM_COMM_GRAPH") != nullptr;
   ScanPeers peers[2]{};            // [forward, backward] mailbox tables for scan.cu
 };
 
@@ -334,7 +322,6 @@ void bdlm_comm_destroy(bdlm_comm *m) {
     if (L.agg) cudaFree(L.agg);
     if (L.aggs) cudaFree(L.aggs);
     if (L.flags) cudaFree(L.flags);
-    if (L.graph_exec) cudaGraphExecDestroy(L.graph_exec);
     if (L.ctx) bdlm_destroy(L.ctx);
   }
   delete m;
@@ -606,72 +593,7 @@ int bdlm_comm_scan_filter_smooth(bdlm_comm *m, const bdlm_problem *probs, const 
     }
     return 0;
   };
-  return for_each_local(m, [&](int i) -> int {
-    Local &L = m->loc[i];
-    static const bool graph_with_peers = std::getenv("BDLM_COMM_GRAPH_PEER") != nullptr;  // experiment
-    static const bool dbg = std::getenv("BDLM_COMM_DEBUG") != nullptr;
-    if (!m->use_graph || (m->peer && !graph_with_peers)) return enqueue(i);
-#define DBG(msg) do { if (dbg) { fprintf(stderr, "[comm dev %d] %s\n", L.device, msg); fflush(stderr); } } while (0)
-    // the graph bakes in every pointer and scalar of the call: replay only an identical call
-    const bdlm_problem &p = probs[i];
-    std::vector<unsigned long long> key = {
-        (unsigned long long)p.T, (unsigned long long)p.n, (unsigned long long)p.keep_init,
-        (unsigned long long)(uintptr_t)p.y, (unsigned long long)(uintptr_t)kfs[i].m,
-        (unsigned long long)(uintptr_t)kfs[i].C, (unsigned long long)(uintptr_t)kfs[i].a,
-        (unsigned long long)(uintptr_t)kfs[i].R, (unsigned long long)(uintptr_t)kfs[i].f,
-        (unsigned long long)(uintptr_t)kfs[i].Q, (unsigned long long)(uintptr_t)sms[i].s,
-        (unsigned long long)(uintptr_t)sms[i].S, (unsigned long long)(uintptr_t)(status ? status[i] : nullptr),
-        (unsigned long long)(uintptr_t)ctx_stream(L.ctx), (unsigned long long)p.layout};
-    auto bits = [&](const double *x, int cnt) {
-      for (int k = 0; k < cnt; ++k) { unsigned long long u; std::memcpy(&u, x + k, 8); key.push_back(u); }
-    };
-    bits(p.G, p.n * p.n); bits(p.F, p.n); bits(p.W, p.n * p.n); bits(p.V, 1); bits(p.m0, p.n); bits(p.C0, p.n * p.n);
-    if (key != L.graph_key) {
-      if (L.graph_exec) { cudaGraphExecDestroy(L.graph_exec); L.graph_exec = nullptr; }
-      L.graph_key = key;
-      L.graph_seen = 0;
-    }
-    if (L.graph_exec) {
-      if (cudaSetDevice(L.device) != cudaSuccess) return BDLM_E_CUDA;
-      DBG("replay");
-      const cudaError_t le = cudaGraphLaunch(L.graph_exec, ctx_stream(L.ctx));
-      DBG(le == cudaSuccess ? "replay launched" : cudaGetErrorString(le));
-      return le == cudaSuccess ? 0 : BDLM_E_CUDA;
-    }
-    if (L.graph_seen++ == 0 || L.graph_seen < 0) { DBG("direct"); return enqueue(i); }  // first call: sizes workspaces, uploads tables
-    // second identical call: capture it, instantiate, launch
-    cudaStream_t stc = ctx_stream(L.ctx);
-    if (cudaSetDevice(L.device) != cudaSuccess) return BDLM_E_CUDA;
-    if (cudaStreamBeginCapture(stc, cudaStreamCaptureModeRelaxed) != cudaSuccess) {
-      cudaGetLastError();
-      L.graph_seen = -1000000;  // capture not available on this stream: stay on direct launches
-      return enqueue(i);
-    }
-    DBG("capture begin");
-    const int rc = enqueue(i);
-    cudaGraph_t graph = nullptr;
-    const cudaError_t ee = cudaStreamEndCapture(stc, &graph);
-    DBG(ee == cudaSuccess ? "capture end ok" : cudaGetErrorString(ee));
-    if (rc != 0 || ee != cudaSuccess || !graph) {
-      cudaGetLastError();
-      if (graph) cudaGraphDestroy(graph);
-      L.graph_seen = -1000000;
-      return rc ? rc : enqueue(i);
-    }
-    cudaGraphExec_t exec = nullptr;
-    if (cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) {
-      cudaGetLastError();
-      cudaGraphDestroy(graph);
-      L.graph_seen = -1000000;
-      return enqueue(i);
-    }
-    cudaGraphDestroy(graph);
-    L.graph_exec = exec;
-    DBG("instantiated, first launch");
-    const cudaError_t fe = cudaGraphLaunch(exec, stc);
-    DBG(fe == cudaSuccess ? "first launch ok" : cudaGetErrorString(fe));
-    return fe == cudaSuccess ? 0 : BDLM_E_CUDA;
-  });
+  return for_each_local(m, enqueue);
 }
 
 int bdlm_comm_sync(bdlm_comm *m) {

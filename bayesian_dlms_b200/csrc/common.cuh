@@ -70,35 +70,10 @@ __host__ __device__ inline int64_t vidx(int64_t sb, int64_t sr, int64_t sk, int6
 }
 
 // Streaming (evict-first) store: outputs are written once and never re-read by the
-// same kernel except the (m, C) spill, which is stored with default policy.
-// BDLM_ST_POLICY / BDLM_LD_POLICY: 0 = streaming (.cs, default), 1 = default caching,
-// 2 = .cg (L2 only), 3 = write-through (.wt).  Tuning knobs, see profiles/r1_tuning.txt.
-#ifndef BDLM_ST_POLICY
-#define BDLM_ST_POLICY 0
-#endif
-#ifndef BDLM_LD_POLICY
-#define BDLM_LD_POLICY 0
-#endif
-__device__ __forceinline__ void st_stream(double *p, double v) {
-#if BDLM_ST_POLICY == 0
-  __stcs(p, v);
-#elif BDLM_ST_POLICY == 1
-  *p = v;
-#elif BDLM_ST_POLICY == 2
-  __stcg(p, v);
-#else
-  __stwt(p, v);
-#endif
-}
-__device__ __forceinline__ double ld_stream(const double *p) {
-#if BDLM_LD_POLICY == 0
-  return __ldcs(p);
-#elif BDLM_LD_POLICY == 1
-  return *p;
-#else
-  return __ldcg(p);
-#endif
-}
+// same kernel except the (m, C) spill, which is stored with default policy.  Other cache
+// policies measured no different (profiles/r1_tuning.txt, "store / load cache policy").
+__device__ __forceinline__ void st_stream(double *p, double v) { __stcs(p, v); }
+__device__ __forceinline__ double ld_stream(const double *p) { return __ldcs(p); }
 
 constexpr double kJacobiThr2 = 1e-30; // rotate iff a_pq^2 > (1e-15)^2 |a_pp a_qq|
 constexpr int kJacobiMaxSweeps = 30;

@@ -274,11 +274,8 @@ __device__ __forceinline__ int lu_cols(const Ctx<N> &cx, double (&A)[N], double 
 
 // 14 warps per SM (7 blocks): 148 x 14 x 2 = 4144 chains resident, so BASELINE config 3 (4096
 // chains) is ONE wave; ptxas gets 65536 / (14 x 32) = 146 registers per thread.
-#ifndef BDLM_GROUP_MINB
-#define BDLM_GROUP_MINB 7
-#endif
 template <int N, int OP>
-__global__ void __launch_bounds__(kWpb * 32, BDLM_GROUP_MINB)
+__global__ void __launch_bounds__(kWpb * 32, 7)
 group_kernel(const WarpArgs wa) {
   extern __shared__ double smem[];
   constexpr int LD = GSmem<N>::LD, MAT = GSmem<N>::MAT, VEC = GSmem<N>::VEC, NN = N * N;

@@ -100,20 +100,13 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 constexpr int kDoFilter = 1, kDoSmooth = 2;
 
 // Minimum resident blocks per SM asked of ptxas (register cap = 65536 / (128 * blocks)).
+// n = 2: profiles/r1_tuning.txt, kf_small_kernel table ("minBlocks=5 ... chosen"); n = 3, 4:
+// profiles/r2_tuning.txt, "register kernels away from n = 2".
 template <int N> struct Occ { static constexpr int kMinBlocks = 1; };
 template <> struct Occ<1> { static constexpr int kMinBlocks = 6; };
-#ifndef BDLM_OCC2
-#define BDLM_OCC2 5
-#endif
-template <> struct Occ<2> { static constexpr int kMinBlocks = BDLM_OCC2; };
-#ifndef BDLM_OCC3
-#define BDLM_OCC3 3
-#endif
-#ifndef BDLM_OCC4
-#define BDLM_OCC4 1
-#endif
-template <> struct Occ<3> { static constexpr int kMinBlocks = BDLM_OCC3; };
-template <> struct Occ<4> { static constexpr int kMinBlocks = BDLM_OCC4; };
+template <> struct Occ<2> { static constexpr int kMinBlocks = 5; };
+template <> struct Occ<3> { static constexpr int kMinBlocks = 3; };
+template <> struct Occ<4> { static constexpr int kMinBlocks = 1; };
 
 template <int N, bool REG, int MODE, bool RELOAD>
 __global__ void __launch_bounds__(128, Occ<N>::kMinBlocks)

@@ -11,8 +11,6 @@
 // series) so every spill access of a warp is a run of full 128-byte lines.
 //
 // Arithmetic mirrors oracle/bdlm_oracle.c operation for operation; citations there.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "launch.h"
 #include "rng.cuh"
@@ -1268,8 +1266,7 @@ cudaError_t launch_svd4_np(const WarpArgs &wa, cudaStream_t stream) {
 }
 template <int OP>
 cudaError_t launch_svd4(const WarpArgs &wa, cudaStream_t stream) {
-  static const bool fixed8 = std::getenv("BDLM_SVD4_GENERIC") == nullptr;  // A/B switch
-  if (fixed8 && wa.bt.n == 8 && wa.bt.p == 8) return launch_svd4_np<OP, 8>(wa, stream);
+  if (wa.bt.n == 8 && wa.bt.p == 8) return launch_svd4_np<OP, 8>(wa, stream);
   return launch_svd4_np<OP, 0>(wa, stream);
 }
 
@@ -1316,9 +1313,7 @@ size_t warp_smem_bytes(int op, int n, int p) {
 }
 
 cudaError_t launch_warp(int op, const WarpArgs &wa, cudaStream_t stream) {
-  // BDLM_NO_SVD4=1: A/B switch back to one warp per series for the SVD path
-  static const bool use_svd4 = std::getenv("BDLM_NO_SVD4") == nullptr;
-  if (use_svd4 && svd4_supported(op, wa.bt))
+  if (svd4_supported(op, wa.bt))
     return op == kOpSvdFilter ? launch_svd4<kOpSvdFilter>(wa, stream)
                               : launch_svd4<kOpSvdFfbs>(wa, stream);
   switch (op) {

@@ -12,8 +12,6 @@
 // Same arithmetic contract as the other bit-exact kernels (common.cuh): the reference's
 // operations in the reference's order, no FMA.  OU needs exp(): device exp() and the JVM's
 // differ in the last place, so OU parity is 1e-9 relative, AR(1) is bit exact.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "launch.h"
 #include "small_steps.cuh"
@@ -43,8 +41,11 @@ __device__ __forceinline__ void ar_predict(double phi, double mu, double sigma, 
   }
 }
 
-template <bool OU, bool FFBS, int kAhead, int MINB>
-__global__ void __launch_bounds__(128, MINB)
+// 8 resident blocks per SM and one step of y, v (and m, C, z on the way back) in flight per
+// thread: occupancy beats per-thread prefetch depth (profiles/r1_tuning.txt, "AR(1) filter /
+// FFBS": FFBS 13.1 ms at depth 1 with 8 blocks/SM asked of ptxas, 21.5 ms at depth 8 with 1).
+template <bool OU, bool FFBS>
+__global__ void __launch_bounds__(128, 8)
 ar_kernel(const ArArgs a) {
   const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (b >= a.B) return;
@@ -58,79 +59,59 @@ ar_kernel(const ArArgs a) {
   double C = OU ? sigma * sigma / phi * phi : sigma * sigma / (1 - phi * phi);
   const View &om = FFBS ? a.sm : a.m, &oC = FFBS ? a.sC : a.C;
   stv(om, b, 0, m); stv(oC, b, 0, C); stv(a.a, b, 0, m); stv(a.R, b, 0, C);
-  // y (and v) do not depend on the recursion: keep kAhead steps of them in flight
-  double yq[kAhead], vq[kAhead];
-#pragma unroll
-  for (int i = 0; i < kAhead; ++i) {
-    yq[i] = (i < T) ? ld_stream(a.y.ptr + b * a.y.sb + i * a.y.sr) : 0.0;
-    vq[i] = (i < T && a.v.ptr) ? ld_stream(a.v.ptr + b * a.v.sb + i * a.v.sr) : 0.0;
-  }
-  for (int t0 = 0; t0 < T; t0 += kAhead) {
-#pragma unroll
-    for (int i = 0; i < kAhead; ++i) {
-      const int t = t0 + i;
-      if (t < T) {
-        const double y = yq[i];
-        const double v = a.v.ptr ? vq[i] : (a.v_shared ? a.v_shared[t] : a.v_s);
-        const int tn = t + kAhead;
-        if (tn < T) {
-          yq[i] = ld_stream(a.y.ptr + b * a.y.sb + tn * a.y.sr);
-          if (a.v.ptr) vq[i] = ld_stream(a.v.ptr + b * a.v.sb + tn * a.v.sr);
-        }
-        double at, rt;
-        ar_predict<OU>(phi, mu, sigma, OU ? a.dt[t] : 1.0, m, C, at, rt);
-        if (isnan(y)) {  // None: (at, rt, at, rt)
-          m = at; C = rt;
-        } else {
-          const double kt = rt / (rt + v);
-          const double et = y - at;
-          m = at + kt * et;
-          C = kt * v;
-        }
-        if (FFBS) {
-          // spill with default policy: re-read by this thread on the way back
-          a.sm.ptr[b * a.sm.sb + (t + 1) * a.sm.sr] = m;
-          a.sC.ptr[b * a.sC.sb + (t + 1) * a.sC.sr] = C;
-        } else {
-          stv(a.m, b, t + 1, m); stv(a.C, b, t + 1, C);
-        }
-        stv(a.a, b, t + 1, at); stv(a.R, b, t + 1, rt);
-      }
+  // y (and v) do not depend on the recursion: load step t + 1 before computing step t
+  double ynext = (0 < T) ? ld_stream(a.y.ptr + b * a.y.sb) : 0.0;
+  double vnext = (0 < T && a.v.ptr) ? ld_stream(a.v.ptr + b * a.v.sb) : 0.0;
+  for (int t = 0; t < T; ++t) {
+    const double y = ynext;
+    const double v = a.v.ptr ? vnext : (a.v_shared ? a.v_shared[t] : a.v_s);
+    const int tn = t + 1;
+    if (tn < T) {
+      ynext = ld_stream(a.y.ptr + b * a.y.sb + tn * a.y.sr);
+      if (a.v.ptr) vnext = ld_stream(a.v.ptr + b * a.v.sb + tn * a.v.sr);
     }
+    double at, rt;
+    ar_predict<OU>(phi, mu, sigma, OU ? a.dt[t] : 1.0, m, C, at, rt);
+    if (isnan(y)) {  // None: (at, rt, at, rt)
+      m = at; C = rt;
+    } else {
+      const double kt = rt / (rt + v);
+      const double et = y - at;
+      m = at + kt * et;
+      C = kt * v;
+    }
+    if (FFBS) {
+      // spill with default policy: re-read by this thread on the way back
+      a.sm.ptr[b * a.sm.sb + (t + 1) * a.sm.sr] = m;
+      a.sC.ptr[b * a.sC.sb + (t + 1) * a.sC.sr] = C;
+    } else {
+      stv(a.m, b, t + 1, m); stv(a.C, b, t + 1, C);
+    }
+    stv(a.a, b, t + 1, at); stv(a.R, b, t + 1, rt);
   }
   if (!FFBS) return;
   // univariateSample: theta_T ~ N(m_T, C_T), then backStepUni down to row 0
   double th = m + sqrt(C) * ld_stream(a.z.ptr + b * a.z.sb + (int64_t)T * a.z.sr);
   stv(a.theta, b, T, th);
-  double mq[kAhead], cq[kAhead], zq[kAhead];
-#pragma unroll
-  for (int i = 0; i < kAhead; ++i) {
-    const int t = T - 1 - i;
-    mq[i] = t >= 0 ? ldv(a.sm, b, t) : 0.0;
-    cq[i] = t >= 0 ? ldv(a.sC, b, t) : 0.0;
-    zq[i] = t >= 0 ? ld_stream(a.z.ptr + b * a.z.sb + t * a.z.sr) : 0.0;
-  }
-  for (int t0 = T - 1; t0 >= 0; t0 -= kAhead) {
-#pragma unroll
-    for (int i = 0; i < kAhead; ++i) {
-      const int t = t0 - i;
-      if (t >= 0) {
-        const double mt = mq[i], ct = cq[i], z = zq[i];
-        const int tn = t - kAhead;
-        if (tn >= 0) {
-          mq[i] = ldv(a.sm, b, tn); cq[i] = ldv(a.sC, b, tn);
-          zq[i] = ld_stream(a.z.ptr + b * a.z.sb + tn * a.z.sr);
-        }
-        const double dt = OU ? a.dt[t] : 1.0;
-        double a1, r1;
-        ar_predict<OU>(phi, mu, sigma, dt, mt, ct, a1, r1);  // == the forward (a, R) of row t + 1
-        const double ph = OU ? exp(-phi * dt) : phi;
-        const double mean = mt + (ct * ph / r1) * (th - a1);
-        const double cov = ct - ((ct * ct) * (ph * ph)) / r1;
-        th = mean + sqrt(cov) * z;
-        stv(a.theta, b, t, th);
-      }
+  const int tl = T - 1;
+  double mnext = tl >= 0 ? ldv(a.sm, b, tl) : 0.0;
+  double cnext = tl >= 0 ? ldv(a.sC, b, tl) : 0.0;
+  double znext = tl >= 0 ? ld_stream(a.z.ptr + b * a.z.sb + tl * a.z.sr) : 0.0;
+  for (int t = tl; t >= 0; --t) {
+    const double mt = mnext, ct = cnext, z = znext;
+    const int tn = t - 1;
+    if (tn >= 0) {
+      mnext = ldv(a.sm, b, tn); cnext = ldv(a.sC, b, tn);
+      znext = ld_stream(a.z.ptr + b * a.z.sb + tn * a.z.sr);
     }
+    const double dt = OU ? a.dt[t] : 1.0;
+    double a1, r1;
+    ar_predict<OU>(phi, mu, sigma, dt, mt, ct, a1, r1);  // == the forward (a, R) of row t + 1
+    const double ph = OU ? exp(-phi * dt) : phi;
+    const double mean = mt + (ct * ph / r1) * (th - a1);
+    const double cov = ct - ((ct * ct) * (ph * ph)) / r1;
+    th = mean + sqrt(cov) * z;
+    stv(a.theta, b, t, th);
   }
 }
 
@@ -419,36 +400,16 @@ cudaError_t launch_conj(const ConjArgs &a, const double *hG, const double *hF, c
 
 }  // namespace
 
-template <int AHEAD, int MINB>
-static void launch_ar_ahead(const ArArgs &a, unsigned blocks, int threads, cudaStream_t stream) {
-  if (a.ou) {
-    if (a.ffbs) ar_kernel<true, true, AHEAD, MINB><<<blocks, threads, 0, stream>>>(a);
-    else ar_kernel<true, false, AHEAD, MINB><<<blocks, threads, 0, stream>>>(a);
-  } else {
-    if (a.ffbs) ar_kernel<false, true, AHEAD, MINB><<<blocks, threads, 0, stream>>>(a);
-    else ar_kernel<false, false, AHEAD, MINB><<<blocks, threads, 0, stream>>>(a);
-  }
-}
-
 cudaError_t launch_ar(const ArArgs &a, cudaStream_t stream) {
   if (a.B == 0) return cudaSuccess;
-  // tuning knobs (profiles/r1_tuning.txt): BDLM_AR_AHEAD = 1 | 2 | 4 | 8 prefetch depth,
-  // BDLM_AR_MINB = 1 | 8 resident blocks per SM asked of ptxas.  Measured: occupancy beats
-  // per-thread prefetch depth (depth 1 at 8 blocks/SM: 13.1 ms; depth 8 at 4 blocks: 21.5 ms).
-  static const int ahead = std::getenv("BDLM_AR_AHEAD") ? std::atoi(std::getenv("BDLM_AR_AHEAD")) : 1;
-  static const int minb = std::getenv("BDLM_AR_MINB") ? std::atoi(std::getenv("BDLM_AR_MINB")) : 8;
-  const int th = 128;
-  const unsigned blocks = (unsigned)((a.B + th - 1) / th);
-#define BDLM_AR_CASE(A_)                                              \
-  if (ahead == A_) {                                                  \
-    if (minb >= 8) launch_ar_ahead<A_, 8>(a, blocks, th, stream);     \
-    else launch_ar_ahead<A_, 1>(a, blocks, th, stream);               \
-    return cudaGetLastError();                                        \
+  const unsigned blocks = (unsigned)((a.B + 127) / 128);
+  if (a.ou) {
+    if (a.ffbs) ar_kernel<true, true><<<blocks, 128, 0, stream>>>(a);
+    else ar_kernel<true, false><<<blocks, 128, 0, stream>>>(a);
+  } else {
+    if (a.ffbs) ar_kernel<false, true><<<blocks, 128, 0, stream>>>(a);
+    else ar_kernel<false, false><<<blocks, 128, 0, stream>>>(a);
   }
-  BDLM_AR_CASE(2) BDLM_AR_CASE(4) BDLM_AR_CASE(8)
-#undef BDLM_AR_CASE
-  if (minb >= 8) launch_ar_ahead<1, 8>(a, blocks, th, stream);
-  else launch_ar_ahead<1, 1>(a, blocks, th, stream);
   return cudaGetLastError();
 }
 

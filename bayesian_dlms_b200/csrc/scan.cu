@@ -24,7 +24,6 @@
 // that is the reference itself); the apply phases reuse the sequential step code, so the
 // only difference is the rounding of the scanned start states.
 #include <cmath>
-#include <cstdlib>
 #include <vector>
 
 #include "common.cuh"
@@ -223,13 +222,13 @@ __host__ __device__ __forceinline__ void s_element_pred(const double *G, const d
 
 namespace {
 
-#ifndef BDLM_SCAN_SUB
-#define BDLM_SCAN_SUB 64
-#endif
-constexpr int kSub = BDLM_SCAN_SUB;  // ROWS per thread (level 1); multiple of kGrp
+// Most ROWS per thread (level 1; a multiple of kGrp); scan_rows_per_thread picks at most this many
+// per call.  64 beat 32 and 16, and 128 gained nothing (profiles/r2_tuning.txt, "scan level-1
+// granularity" and "kSub = 128").
+constexpr int kSub = 64;
 constexpr int kGrp = 4;        // rows per vector group: 4 rows x K doubles = K 32-byte sectors
 constexpr int kScanBlock = 256;
-constexpr size_t kScanTableBytes = (size_t)(kSub > 64 ? 128 : 64) << 10;
+constexpr size_t kScanTableBytes = (size_t)64 << 10;
 
 template <int N>
 struct ScanModel {
@@ -248,16 +247,9 @@ __device__ __forceinline__ int64_t first_step(int64_t c, int keep_init, int sub)
   return t < 0 ? 0 : t;
 }
 
-// BDLM_SCAN_ST=1 (environment, read per launch): default write-back policy instead of
-// evict-first, an A/B knob for profiles/r1_tuning.txt.
-__device__ int g_scan_st_default = 0;
 __device__ __forceinline__ void st_v4(double *p, double a, double b, double c, double d) {
-  if (g_scan_st_default)
-    asm volatile("st.global.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(p), "d"(a), "d"(b), "d"(c), "d"(d)
-                 : "memory");
-  else
-    asm volatile("st.global.cs.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(p), "d"(a), "d"(b), "d"(c), "d"(d)
-                 : "memory");
+  asm volatile("st.global.cs.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(p), "d"(a), "d"(b), "d"(c), "d"(d)
+               : "memory");
 }
 __device__ __forceinline__ void ld_v4(const double *p, double *x) {
   asm volatile("ld.global.v4.f64 {%0, %1, %2, %3}, [%4];"
@@ -682,13 +674,10 @@ __device__ __forceinline__ void fwd_row(const ScanModel<N> &md, const double (&W
   }
 }
 
-// BDLM_SCAN_MINB: resident blocks per SM asked of ptxas for the two apply sweeps (tuning knob,
-// profiles/r1_tuning.txt)
-#ifndef BDLM_SCAN_MINB
-#define BDLM_SCAN_MINB 1
-#endif
+// The two apply sweeps ask ptxas for one resident block per SM: asking for more makes them spill,
+// which costs more than the occupancy gains (profiles/r1_tuning.txt, "scan apply sweeps").
 template <int N, bool VEC, bool FUSE>
-__global__ void __launch_bounds__(128, BDLM_SCAN_MINB)
+__global__ void __launch_bounds__(128, 1)
 fwd_apply_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T, int64_t M,
                  const FElem<N> *pre /* [M+1] inclusive scan with slot 0 = start */,
                  int keep_init, KfViews kf, int32_t *status,
@@ -843,7 +832,7 @@ __device__ __forceinline__ void bwd_row(const ScanModel<N> &md, const double (&W
 }
 
 template <int N, bool VEC>
-__global__ void __launch_bounds__(128, BDLM_SCAN_MINB)
+__global__ void __launch_bounds__(128, 1)
 bwd_apply_kernel(const ScanModel<N> md, View fm, View fC, int64_t nrows, int64_t M,
                  const SElem<N> *suf /* [M+1] suffix-inclusive scan, slot M = terminal */,
                  View sv, View Sv, int32_t *status,
@@ -1050,12 +1039,6 @@ int apply_slots() {
 }
 
 int scan_rows_per_thread(int n, int64_t T) {
-  static const int forced = [] {
-    const char *e = std::getenv("BDLM_SCAN_ROWS");  // A/B knob: fixed rows per thread
-    const int v = e ? std::atoi(e) : 0;
-    return (v >= kGrp && v <= kSub && v % kGrp == 0) ? v : 0;
-  }();
-  if (forced) return forced;
   int slots = 444;
   switch (n) {
     case 1: slots = apply_slots<1>(); break;
@@ -1260,13 +1243,6 @@ int scan_forward_elem_doubles(int n) { return 3 * n * n + 2 * n; }
 int scan_backward_elem_doubles(int n) { return 2 * n * n + n; }
 
 cudaError_t launch_scan(const ScanArgs &a, cudaStream_t stream, int64_t *launches) {
-  static int st_default = -1;
-  if (st_default < 0) {
-    const char *e = std::getenv("BDLM_SCAN_ST");
-    st_default = (e && e[0] == '1') ? 1 : 0;
-    cudaError_t err = cudaMemcpyToSymbol(g_scan_st_default, &st_default, sizeof(int));
-    if (err != cudaSuccess) return err;
-  }
   switch (a.n) {
 #define BDLM_SCAN_CASE(N_)                                                         \
   case N_:                                                                         \
