@@ -2,19 +2,21 @@
 // dimension (n <= 4, p = 1): ONE THREAD PER SERIES.
 //
 // This is the HBM-bound headline kernel (BASELINE.json config 2: polynomial(2), 1e6
-// series x T = 1000).  Per series-step it moves 8*(p + 2n + 2n^2 + p + p^2) bytes in the
-// forward pass and 8*(2n + 2n^2) in the backward pass (216 B for n = 2, p = 1) against
-// ~130 flops, so everything is organised around HBM:
+// series x T = 1000).  Per series-step the forward pass moves 8*(p + 2n + 2n^2 + p + p^2)
+// bytes and the backward pass writes 8*(n + n^2) (s, S) and reads back what it needs of the
+// forward pass: 8*(n + n^2) of (m_t, C_t), or, fused with the filter for n <= 2 on a regular grid, one
+// checkpoint row of (m, C) in kSeg plus y again (186 B in all for n = 2, p = 1, against 216 B
+// with the full re-read) against ~130 flops, so everything is organised around HBM:
 //   * device-native layout is time-major SoA [rows][k][B]: the 32 threads of a warp read
 //     or write 256 contiguous bytes per scalar field per step (two full 128 B lines),
 //   * the whole state (m, C, a, R, W, s, S) lives in registers, the shared model (F, G)
 //     in the kernel-parameter constant bank,
-//   * y is prefetched one 4-step chunk ahead and the backward pass's (m_t, C_t) one row
-//     ahead, so every thread always has independent loads in flight while it walks its
-//     strictly sequential recursion,
-//   * outputs are written once with streaming stores (evict-first) and a_{t+1}, R_{t+1}
-//     are recomputed in the backward pass (bit-identical to the forward values) instead
-//     of being re-read.
+//   * y is prefetched one 4-step chunk ahead and the backward pass's rows are staged by
+//     cp.async ahead of use, so every thread always has independent loads in flight while it
+//     walks its strictly sequential recursion,
+//   * outputs are written once with streaming stores (evict-first); the backward pass
+//     recomputes a_{t+1}, R_{t+1} and, fused for n <= 2, the filtered (m_t, C_t) between
+//     checkpoints (bit-identical to the forward values) instead of re-reading them.
 //
 // Arithmetic mirrors oracle/bdlm_oracle.c operation for operation (see common.cuh);
 // reference citations: KalmanFilter.scala:64-107,273-321 and Smoothing.scala:31-64.
@@ -28,18 +30,31 @@ namespace {
 
 using namespace small;
 
-template <int K>
-__device__ __forceinline__ void store_vec(const View &v, int64_t b, int64_t row,
-                                          const double *x) {
-  if (v.ptr == nullptr) return;
-  double *p = v.ptr + b * v.sb + row * v.sr;
+// The time loops keep one address per field for the current row (row_ptr once, then a step of
+// v.sr per row) and store at p + k * sk: a 64-bit add of a uniform offset per element instead of
+// recomputing ptr + b * sb + row * sr + k * sk in 64-bit multiplies for every store.
+__device__ __forceinline__ double *row_ptr(const View &v, int64_t b, int64_t row) {
+  return v.ptr + b * v.sb + row * v.sr;
+}
+
+// p = row_ptr(v, b, row); a field the caller did not ask for (v.ptr == nullptr, a kernel
+// parameter) costs one uniform branch per store, unless DENSE: every field is known to be wanted
+template <bool DENSE, int K>
+__device__ __forceinline__ void store_at(const View &v, double *p, const double *x) {
+  if (!DENSE && v.ptr == nullptr) return;
 #pragma unroll
   for (int k = 0; k < K; ++k) st_stream(p + k * v.sk, x[k]);
 }
 
 template <int K>
+__device__ __forceinline__ void store_vec(const View &v, int64_t b, int64_t row,
+                                          const double *x) {
+  store_at<false, K>(v, row_ptr(v, b, row), x);
+}
+
+template <int K>
 __device__ __forceinline__ void load_vec(const View &v, int64_t b, int64_t row, double *x) {
-  const double *p = v.ptr + b * v.sb + row * v.sr;
+  const double *p = row_ptr(v, b, row);
 #pragma unroll
   for (int k = 0; k < K; ++k) x[k] = ld_stream(p + k * v.sk);
 }
@@ -98,6 +113,9 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // ptxas put the prefetch loads and the reload loads on one scoreboard slot and wait for it
 // at the merge point, which serialised the (m, C) prefetch with the recursion)
 constexpr int kDoFilter = 1, kDoSmooth = 2;
+// with kDoFilter | kDoSmooth: the caller wants all eight outputs, so the time loops store
+// without testing each field's pointer (the benchmark's and the dense device path's call)
+constexpr int kAllOut = 4;
 
 // Minimum resident blocks per SM asked of ptxas (register cap = 65536 / (128 * blocks)).
 // n = 2: profiles/r1_tuning.txt, kf_small_kernel table ("minBlocks=5 ... chosen"); n = 3, 4:
@@ -108,10 +126,36 @@ template <> struct Occ<2> { static constexpr int kMinBlocks = 5; };
 template <> struct Occ<3> { static constexpr int kMinBlocks = 3; };
 template <> struct Occ<4> { static constexpr int kMinBlocks = 1; };
 
+// Fused filter + smoother, n <= 2, regular grid and time-invariant model: the backward pass
+// rebuilds (m_t, C_t) on chip from every kSeg-th stored row instead of re-reading every row
+// (DESIGN.md §3).  The smooth-only modes have no y to re-filter with; n = 3, 4 are FP64-bound
+// (profiles/r2_tuning.txt, "which roof?"); off the REG path the re-filtering loads dt, F, G a
+// second time and per-series G measured 3.6 % slower with it (profiles/r3_recompute.txt): all of
+// those keep re-reading through the kRing ring.  kSeg: profiles/r3_recompute.txt.
+constexpr int kSeg = 4;
+template <int N, bool REG, int MODE>
+constexpr bool recompute() {
+  return (MODE & (kDoFilter | kDoSmooth)) == (kDoFilter | kDoSmooth) && N <= 2 && REG;
+}
+
+// Shared memory per thread, in doubles: the re-read ring, or kSeg recomputed rows plus a staging
+// slot for the next segment's checkpoint row and its kSeg - 1 y values.
+template <int N, bool REG, int MODE>
+constexpr int smem_doubles() {
+  return !(MODE & kDoSmooth) ? 0
+         : recompute<N, REG, MODE>() ? (kSeg + 1) * (N + N * N) + kSeg - 1
+                                 : kRing * (N + N * N);
+}
+
+// Threads per block.  The shared-memory slots are indexed with it as a compile-time stride, so
+// every slot of a thread is its base address plus an immediate offset.
+constexpr int kThreads = 128;
+
 template <int N, bool REG, int MODE, bool RELOAD>
-__global__ void __launch_bounds__(128, Occ<N>::kMinBlocks)
+__global__ void __launch_bounds__(kThreads, Occ<N>::kMinBlocks)
 kf_small_kernel(const Batch bt, const SmallModel<N> mdl, const KfViews kf, const View sv,
                 const View Sv) {
+  constexpr bool kDense = (MODE & kAllOut) != 0;
   const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (b >= bt.B) return;
   const int T = bt.T, ki = bt.keep_init, rows = T + ki;
@@ -135,15 +179,15 @@ kf_small_kernel(const Batch bt, const SmallModel<N> mdl, const KfViews kf, const
       store_vec<1>(kf.Q, b, 0, &nanv);
     }
     const double *yp = bt.y.ptr + b * bt.y.sb;
+    double *pm = row_ptr(kf.m, b, ki), *pC = row_ptr(kf.C, b, ki), *pa = row_ptr(kf.a, b, ki),
+           *pR = row_ptr(kf.R, b, ki), *pf = row_ptr(kf.f, b, ki), *pQ = row_ptr(kf.Q, b, ki);
     double ycur[kChunk], ynxt[kChunk];
 #pragma unroll
     for (int u = 0; u < kChunk; ++u) ycur[u] = (u < T) ? ld_stream(yp + u * bt.y.sr) : 0.0;
     for (int t0 = 0; t0 < T; t0 += kChunk) {
+      yp += kChunk * bt.y.sr;
 #pragma unroll
-      for (int u = 0; u < kChunk; ++u) {
-        const int t = t0 + kChunk + u;
-        ynxt[u] = (t < T) ? ld_stream(yp + (int64_t)t * bt.y.sr) : 0.0;
-      }
+      for (int u = 0; u < kChunk; ++u) ynxt[u] = (t0 + kChunk + u < T) ? ld_stream(yp + u * bt.y.sr) : 0.0;
 #pragma unroll
       for (int u = 0; u < kChunk; ++u) {
         const int t = t0 + u;
@@ -154,13 +198,13 @@ kf_small_kernel(const Batch bt, const SmallModel<N> mdl, const KfViews kf, const
           load_model<N, REG>(bt, mdl, b, t, G, F);
           advance<N, REG>(G, W, dt, m, C, a, R);
           update<N>(F, V, ycur[u], a, R, f, Q, m, C, st);
-          const int64_t row = t + ki;
-          store_vec<N>(kf.a, b, row, a);
-          store_vec<N * N>(kf.R, b, row, R);
-          store_vec<1>(kf.f, b, row, &f);
-          store_vec<1>(kf.Q, b, row, &Q);
-          store_vec<N>(kf.m, b, row, m);
-          store_vec<N * N>(kf.C, b, row, C);
+          store_at<kDense, N>(kf.a, pa, a);
+          store_at<kDense, N * N>(kf.R, pR, R);
+          store_at<kDense, 1>(kf.f, pf, &f);
+          store_at<kDense, 1>(kf.Q, pQ, &Q);
+          store_at<kDense, N>(kf.m, pm, m);
+          store_at<kDense, N * N>(kf.C, pC, C);
+          pa += kf.a.sr; pR += kf.R.sr; pf += kf.f.sr; pQ += kf.Q.sr; pm += kf.m.sr; pC += kf.C.sr;
         }
       }
 #pragma unroll
@@ -178,62 +222,137 @@ kf_small_kernel(const Batch bt, const SmallModel<N> mdl, const KfViews kf, const
     for (int i = 0; i < N; ++i) s[i] = m[i];
 #pragma unroll
     for (int k = 0; k < N * N; ++k) S[k] = C[k];
-    store_vec<N>(sv, b, rows - 1, s);
-    store_vec<N * N>(Sv, b, rows - 1, S);
+    double *ps = row_ptr(sv, b, rows - 1), *pS = row_ptr(Sv, b, rows - 1);
+    store_at<kDense, N>(sv, ps, s);
+    store_at<kDense, N * N>(Sv, pS, S);
     const bool textbook = (bt.compat & BDLM_TEXTBOOK_SMOOTHER) != 0;
-    // (m_t, C_t) spill rows are staged through a per-thread shared-memory ring by cp.async
-    // (LDGSTS), kRing rows deep: the loads bypass the register file and the scoreboard, so
-    // they stay in flight across several iterations of the recursion.  (One row of register
-    // prefetch was not enough: ncu showed 25 % of all stall samples on its first use; DRAM
-    // latency under this kernel's write-heavy load exceeds one backward iteration.)
     extern __shared__ double ring[];
     constexpr int kRow = N + N * N;
-    const int nthr = blockDim.x;
-    auto slot = [&](int r, int k) { return ring + ((size_t)(r & (kRing - 1)) * kRow + k) * nthr + threadIdx.x; };
-    auto issue = [&](int r) {
-      if (r >= 0) {
-        const double *pm = kf.m.ptr + b * kf.m.sb + (int64_t)r * kf.m.sr;
-        const double *pc = kf.C.ptr + b * kf.C.sb + (int64_t)r * kf.C.sr;
-#pragma unroll
-        for (int k = 0; k < N; ++k) cp_async8(slot(r, k), pm + k * kf.m.sk);
-#pragma unroll
-        for (int k = 0; k < N * N; ++k) cp_async8(slot(r, N + k), pc + k * kf.C.sk);
-      }
-      cp_async_commit();
-    };
-    double an[N], Rn[N * N];
-#pragma unroll
-    for (int d = 0; d < kRing - 1; ++d) issue(rows - 2 - d);
-    if (RELOAD && rows >= 2) {
-      load_vec<N>(kf.a, b, rows - 1, an);
-      load_vec<N * N>(kf.R, b, rows - 1, Rn);
-    }
-    for (int r = rows - 2; r >= 0; --r) {
-      double a1[N], R1[N * N];
-      issue(r - (kRing - 1));
-      cp_async_wait<kRing - 1>();  // the group of row r has landed
-#pragma unroll
-      for (int i = 0; i < N; ++i) m[i] = *slot(r, i);
-#pragma unroll
-      for (int k = 0; k < N * N; ++k) C[k] = *slot(r, N + k);
-      if (RELOAD) {
-#pragma unroll
-        for (int i = 0; i < N; ++i) a1[i] = an[i];
-#pragma unroll
-        for (int k = 0; k < N * N; ++k) R1[k] = Rn[k];
-        if (r > 0) {
-          load_vec<N>(kf.a, b, r, an);
-          load_vec<N * N>(kf.R, b, r, Rn);
-        }
-      }
+    // Smoothing.smoothStep for row r from its filtered (mr, Cr): a_{r+1}, R_{r+1} are recomputed
+    // (bit-identical to the forward values) unless the caller passed them (a1, R1 preset).
+    auto smooth_row = [&](int r, const double (&mr)[N], const double (&Cr)[N * N], double (&a1)[N],
+                          double (&R1)[N * N]) {
       const int tobs = r + 1 - ki;  // observation index of row r + 1
       const double dt = REG ? 1.0 : dt_at(bt, b, tobs);
       double G[N * N], F[N];
       load_model<N, REG>(bt, mdl, b, tobs, G, F);
-      if (!RELOAD) advance<N, REG>(G, W, dt, m, C, a1, R1);  // bit-identical to the forward a, R
-      rts_step<N>(G, m, C, a1, R1, textbook, s, S, st);
-      store_vec<N>(sv, b, r, s);
-      store_vec<N * N>(Sv, b, r, S);
+      if (!RELOAD) advance<N, REG>(G, W, dt, mr, Cr, a1, R1);
+      rts_step<N>(G, mr, Cr, a1, R1, textbook, s, S, st);
+      ps -= sv.sr; pS -= Sv.sr;
+      store_at<kDense, N>(sv, ps, s);
+      store_at<kDense, N * N>(Sv, pS, S);
+    };
+    if constexpr (recompute<N, REG, MODE>()) {
+      // Rows 0 .. rows - 2 in segments [r0, r0 + len), r0 a multiple of kSeg, top segment first
+      // (the only one that may be short).  The stored row r0 is the segment's checkpoint; rows
+      // r0 + 1 .. r0 + len - 1 are filtered again from it with the forward pass's operations on
+      // the same inputs, so they come out bit for bit as stored, and nothing is stored.  They are
+      // kept in shared memory as [j][k][thread] (no bank conflicts) and smoothed in descending
+      // order.  The next segment's checkpoint and y values are staged by cp.async a segment
+      // ahead, into slot kSeg: kRow doubles of (m, C), then kSeg - 1 y values.
+      auto seg = [&](int j, int k) { return ring + ((size_t)j * kRow + k) * kThreads + threadIdx.x; };
+      auto issue = [&](int r0, int len) {
+        if (r0 >= 0) {
+          const double *pcm = row_ptr(kf.m, b, r0), *pcC = row_ptr(kf.C, b, r0);
+#pragma unroll
+          for (int k = 0; k < N; ++k) cp_async8(seg(kSeg, k), pcm + k * kf.m.sk);
+#pragma unroll
+          for (int k = 0; k < N * N; ++k) cp_async8(seg(kSeg, N + k), pcC + k * kf.C.sk);
+          const double *py = bt.y.ptr + b * bt.y.sb + (int64_t)(r0 + 1 - ki) * bt.y.sr;
+#pragma unroll
+          for (int j = 0; j < kSeg - 1; ++j)
+            if (j < len - 1) cp_async8(seg(kSeg, kRow + j), py + j * bt.y.sr);
+        }
+        cp_async_commit();
+      };
+      if (rows >= 2) {
+        int r0 = (rows - 2) / kSeg * kSeg;
+        issue(r0, rows - 1 - r0);
+        for (; r0 >= 0; r0 -= kSeg) {
+          const int len = min(kSeg, rows - 1 - r0);
+          double yv[kSeg - 1];
+          cp_async_wait<0>();
+#pragma unroll
+          for (int i = 0; i < N; ++i) m[i] = *seg(kSeg, i);
+#pragma unroll
+          for (int k = 0; k < N * N; ++k) C[k] = *seg(kSeg, N + k);
+#pragma unroll
+          for (int j = 0; j < kSeg - 1; ++j) yv[j] = (j < len - 1) ? *seg(kSeg, kRow + j) : 0.0;
+          issue(r0 - kSeg, kSeg);  // the staging slot is free again
+#pragma unroll
+          for (int j = 0; j < kSeg; ++j) {
+            if (j >= len) break;
+            if (j > 0) {  // filter row r0 + j (observation r0 + j - ki) from row r0 + j - 1
+              const int t = r0 + j - ki;
+              double a[N], R[N * N], f, Q;
+              const double dt = REG ? 1.0 : dt_at(bt, b, t);
+              double G[N * N], F[N];
+              load_model<N, REG>(bt, mdl, b, t, G, F);
+              advance<N, REG>(G, W, dt, m, C, a, R);
+              update<N>(F, V, yv[j - 1], a, R, f, Q, m, C, st);
+            }
+#pragma unroll
+            for (int i = 0; i < N; ++i) *seg(j, i) = m[i];
+#pragma unroll
+            for (int k = 0; k < N * N; ++k) *seg(j, N + k) = C[k];
+          }
+#pragma unroll
+          for (int j = kSeg - 1; j >= 0; --j) {
+            if (j < len) {
+              double a1[N], R1[N * N];
+#pragma unroll
+              for (int i = 0; i < N; ++i) m[i] = *seg(j, i);
+#pragma unroll
+              for (int k = 0; k < N * N; ++k) C[k] = *seg(j, N + k);
+              smooth_row(r0 + j, m, C, a1, R1);
+            }
+          }
+        }
+      }
+    } else {
+      // (m_t, C_t) rows are staged through a per-thread shared-memory ring by cp.async
+      // (LDGSTS), kRing rows deep: the loads bypass the register file and the scoreboard, so
+      // they stay in flight across several iterations of the recursion.  (One row of register
+      // prefetch was not enough: ncu showed 25 % of all stall samples on its first use; DRAM
+      // latency under this kernel's write-heavy load exceeds one backward iteration.)
+      auto slot = [&](int r, int k) { return ring + ((size_t)(r & (kRing - 1)) * kRow + k) * kThreads + threadIdx.x; };
+      auto issue = [&](int r) {
+        if (r >= 0) {
+          const double *pcm = row_ptr(kf.m, b, r), *pcC = row_ptr(kf.C, b, r);
+#pragma unroll
+          for (int k = 0; k < N; ++k) cp_async8(slot(r, k), pcm + k * kf.m.sk);
+#pragma unroll
+          for (int k = 0; k < N * N; ++k) cp_async8(slot(r, N + k), pcC + k * kf.C.sk);
+        }
+        cp_async_commit();
+      };
+      double an[N], Rn[N * N];
+#pragma unroll
+      for (int d = 0; d < kRing - 1; ++d) issue(rows - 2 - d);
+      if (RELOAD && rows >= 2) {
+        load_vec<N>(kf.a, b, rows - 1, an);
+        load_vec<N * N>(kf.R, b, rows - 1, Rn);
+      }
+      for (int r = rows - 2; r >= 0; --r) {
+        double a1[N], R1[N * N];
+        issue(r - (kRing - 1));
+        cp_async_wait<kRing - 1>();  // the group of row r has landed
+#pragma unroll
+        for (int i = 0; i < N; ++i) m[i] = *slot(r, i);
+#pragma unroll
+        for (int k = 0; k < N * N; ++k) C[k] = *slot(r, N + k);
+        if (RELOAD) {
+#pragma unroll
+          for (int i = 0; i < N; ++i) a1[i] = an[i];
+#pragma unroll
+          for (int k = 0; k < N * N; ++k) R1[k] = Rn[k];
+          if (r > 0) {
+            load_vec<N>(kf.a, b, r, an);
+            load_vec<N * N>(kf.R, b, r, Rn);
+          }
+        }
+        smooth_row(r, m, C, a1, R1);
+      }
     }
 #pragma unroll
     for (int i = 0; i < N; ++i) m[i] = s[i];
@@ -252,14 +371,12 @@ kf_small_kernel(const Batch bt, const SmallModel<N> mdl, const KfViews kf, const
   }
 }
 
-constexpr int kThreads = 128;
-
 template <int N, bool REG, int MODE, bool RELOAD>
 cudaError_t launch_t(const Batch &bt, const SmallModel<N> &mdl, const KfViews &kf, const View &sv,
                      const View &Sv, cudaStream_t stream, int *wave_series) {
   if (wave_series) {  // occupancy query only
     int blocks = 0, dev = 0, sms = 0;
-    const size_t qsmem = (MODE & kDoSmooth) ? sizeof(double) * kRing * (N + N * N) * kThreads : 0;
+    const size_t qsmem = sizeof(double) * smem_doubles<N, REG, MODE>() * kThreads;
     if (qsmem > 48 * 1024) {  // n = 4: 80 KB ring -- the query needs the opt-in limit raised first
       cudaError_t ea = cudaFuncSetAttribute(kf_small_kernel<N, REG, MODE, RELOAD>,
                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qsmem);
@@ -275,7 +392,7 @@ cudaError_t launch_t(const Batch &bt, const SmallModel<N> &mdl, const KfViews &k
   }
   const int64_t blocks = (bt.B + kThreads - 1) / kThreads;
   if (blocks <= 0) return cudaSuccess;
-  const size_t smem = (MODE & kDoSmooth) ? sizeof(double) * kRing * (N + N * N) * kThreads : 0;
+  const size_t smem = sizeof(double) * smem_doubles<N, REG, MODE>() * kThreads;
   if (smem > 48 * 1024) {
     cudaError_t e = cudaFuncSetAttribute(kf_small_kernel<N, REG, MODE, RELOAD>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -297,8 +414,11 @@ cudaError_t launch_n(const Batch &bt, const double *hG, const double *hF, const 
 #define BDLM_GO(REG_, MODE_, RELOAD_) \
   return launch_t<N, REG_, MODE_, RELOAD_>(bt, mdl, kf, sv, Sv, stream, wave_series)
   if (mode == kDoFilter) { if (reg) BDLM_GO(true, kDoFilter, false); else BDLM_GO(false, kDoFilter, false); }
-  if (mode == (kDoFilter | kDoSmooth)) {
-    if (reg) BDLM_GO(true, kDoFilter | kDoSmooth, false); else BDLM_GO(false, kDoFilter | kDoSmooth, false);
+  if (mode == (kDoFilter | kDoSmooth)) {  // m, C are always given (the library's workspace if not wanted)
+    const bool all = kf.a.ptr && kf.R.ptr && kf.f.ptr && kf.Q.ptr && sv.ptr && Sv.ptr;
+    constexpr int kFS = kDoFilter | kDoSmooth;
+    if (all) { if (reg) BDLM_GO(true, kFS | kAllOut, false); else BDLM_GO(false, kFS | kAllOut, false); }
+    if (reg) BDLM_GO(true, kFS, false); else BDLM_GO(false, kFS, false);
   }
   if (reload) { if (reg) BDLM_GO(true, kDoSmooth, true); else BDLM_GO(false, kDoSmooth, true); }
   if (reg) BDLM_GO(true, kDoSmooth, false); else BDLM_GO(false, kDoSmooth, false);
