@@ -204,7 +204,7 @@ class Comm:
         """One entry per LOCAL device: the Model of that rank's chunk length and its CUDA slice of
         the series.  Returns a handle for ``scan_run`` (buffers are allocated once)."""
         import torch
-        from .scan import _alloc, _problem
+        from .scan import _outputs, _problem
         nl = len(self.engines)
         assert len(models) == nl and len(y_chunks) == nl
         n = models[0].n
@@ -218,13 +218,7 @@ class Comm:
                 pr, kp = _problem(model, params, y, keep_init=(rank == 0))
             probs[i] = pr
             keep.append((kp, model, y))
-            rows = model.T + int(rank == 0)
-            o = {k: _alloc(y, rows, d) for k, d in
-                 dict(m=n, C=n * n, a=n, R=n * n, f=1, Q=1, s=n, S=n * n).items()}
-            for k in ("m", "C", "a", "R", "f", "Q"):
-                setattr(kfs[i], k, o[k].data_ptr())
-            for k in ("s", "S"):
-                setattr(sms[i], k, o[k].data_ptr())
+            o, kfs[i], sms[i] = _outputs(y, model.T + int(rank == 0), n)
             st = torch.zeros(1, dtype=torch.int32, device=y.device)
             sts[i] = st.data_ptr()
             outs.append(o)

@@ -1231,88 +1231,6 @@ int bdlm_scan_combine(int32_t n, int32_t backward, const double *earlier, const 
   return 0;
 }
 
-int bdlm_scan_forward_reduce(bdlm_ctx *c, const bdlm_problem *p, double *agg_host) {
-  NvtxRange nvtx_("bdlm_scan_forward_reduce");
-  int rc = scan_validate(c, p);
-  if (rc) return rc;
-  if (!agg_host) return fail(c, BDLM_E_ARG, "null aggregate pointer");
-  CU(cudaSetDevice(c->device));
-  rc = ensure_arena(c, scan_workspace_bytes(p->n, p->T) + 4096);
-  if (rc) return rc;
-  ScanArgs a;
-  rc = scan_fill(c, p, a, true);
-  if (rc) return rc;
-  a.phase = kScanReduce; a.agg_out = agg_host; a.workspace = c->arena;
-  { rc = scan_launch_fwd(c, a); if (rc) return rc; }
-  return 0;
-}
-
-int bdlm_scan_forward_apply(bdlm_ctx *c, const bdlm_problem *p, const double *start_mC_host,
-                            const bdlm_kf_out *kf, int32_t *status) {
-  NvtxRange nvtx_("bdlm_scan_forward_apply");
-  int rc = scan_validate(c, p);
-  if (rc) return rc;
-  if (!kf) return fail(c, BDLM_E_ARG, "null output struct");
-  CU(cudaSetDevice(c->device));
-  rc = ensure_arena(c, scan_workspace_bytes(p->n, p->T) + 4096);
-  if (rc) return rc;
-  std::vector<double> prior((size_t)p->n + p->n * p->n);
-  if (!start_mC_host) {
-    std::copy(p->m0, p->m0 + p->n, prior.begin());
-    std::copy(p->C0, p->C0 + p->n * p->n, prior.begin() + p->n);
-  }
-  ScanArgs a;
-  rc = scan_fill(c, p, a, true);
-  if (rc) return rc;
-  a.phase = kScanApply; a.start = start_mC_host ? start_mC_host : prior.data();
-  a.kf = scan_kf_views(p, kf); a.status = status; a.workspace = c->arena;
-  if (status) CU(cudaMemsetAsync(status, 0, sizeof(int32_t), c->stream));
-  { rc = scan_launch_fwd(c, a); if (rc) return rc; }  // start state travels by value: no sync needed
-  return 0;
-}
-
-int bdlm_scan_backward_reduce(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *filt,
-                              int32_t has_successor, double *agg_host) {
-  NvtxRange nvtx_("bdlm_scan_backward_reduce");
-  int rc = scan_validate(c, p);
-  if (rc) return rc;
-  if (!filt || !filt->m || !filt->C || !agg_host)
-    return fail(c, BDLM_E_ARG, "backward scan needs filtered m, C and an aggregate pointer");
-  CU(cudaSetDevice(c->device));
-  rc = ensure_arena(c, scan_workspace_bytes(p->n, p->T) + 4096);
-  if (rc) return rc;
-  ScanArgs a;
-  rc = scan_fill(c, p, a);
-  if (rc) return rc;
-  a.backward = 1; a.phase = kScanReduce; a.has_successor = has_successor ? 1 : 0;
-  a.agg_out = agg_host; a.kf = scan_kf_views(p, filt); a.workspace = c->arena;
-  CU(launch_scan(a, c->stream, &c->launches));
-  return 0;
-}
-
-int bdlm_scan_backward_apply(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *filt,
-                             const double *next_sS_host, const bdlm_smooth_out *sm,
-                             int32_t *status) {
-  NvtxRange nvtx_("bdlm_scan_backward_apply");
-  int rc = scan_validate(c, p);
-  if (rc) return rc;
-  if (!filt || !filt->m || !filt->C || !sm)
-    return fail(c, BDLM_E_ARG, "backward scan needs filtered m, C and an output struct");
-  CU(cudaSetDevice(c->device));
-  rc = ensure_arena(c, scan_workspace_bytes(p->n, p->T) + 4096);
-  if (rc) return rc;
-  const int64_t n = p->n, R = rows_of(*p);
-  ScanArgs a;
-  rc = scan_fill(c, p, a);
-  if (rc) return rc;
-  a.backward = 1; a.phase = kScanApply; a.has_successor = next_sS_host ? 1 : 0;
-  a.start = next_sS_host; a.kf = scan_kf_views(p, filt);
-  a.s = mk_view(sm->s, p->layout, 0, 1, R, n); a.S = mk_view(sm->S, p->layout, 0, 1, R, n * n);
-  a.status = status; a.workspace = c->arena;
-  CU(launch_scan(a, c->stream, &c->launches));
-  return 0;
-}
-
 int bdlm_scan_filter_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *kf,
                             const bdlm_smooth_out *sm, int32_t *status) {
   NvtxRange nvtx_("bdlm_scan_filter_smooth");
@@ -1347,7 +1265,7 @@ int bdlm_scan_filter_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_ou
   // backward: scan the aggregates, apply
   rc = scan_fill(c, p, a);
   if (rc) return rc;
-  a.backward = 1; a.phase = kScanApply; a.has_successor = 0; a.pre_reduced = R > 1 ? 1 : 0;
+  a.backward = 1; a.phase = kScanApply; a.has_successor = 0;
   a.kf = scan_kf_views(p, &k);
   a.s = mk_view(sm->s, p->layout, 0, 1, R, n); a.S = mk_view(sm->S, p->layout, 0, 1, R, n * n);
   a.status = status; a.workspace = c->arena + ws;
@@ -1429,7 +1347,6 @@ int bdlm_scan_dist_backward_local(bdlm_ctx *c, const bdlm_problem *p, int32_t ra
   rc = scan_fill(c, p, a);
   if (rc) return rc;
   a.backward = 1; a.phase = kScanDistLocal; a.has_successor = rank < world - 1;
-  a.pre_reduced = 1;  // written by bdlm_scan_dist_forward_finish
   a.kf = scan_kf_views(p, filt);
   a.s = mk_view(sm->s, p->layout, 0, 1, R, n); a.S = mk_view(sm->S, p->layout, 0, 1, R, n * n);
   a.agg_dev = agg_dev; a.rank = rank; a.world = world; a.workspace = c->arena + ws;

@@ -77,11 +77,11 @@ cudaError_t launch_dt_from_times(const double *times, int64_t tsb, int64_t tsr, 
 
 // scan.cu: parallel-in-time filter / smoother for one long series (n <= 4, p = 1, regular
 // grid, time-invariant model).
-enum { kScanReduce = 0, kScanApply = 1,
-       // device-side multi-GPU protocol (no host round trip): local = level-1 + scan with an
-       // identity carry, chunk aggregate left in DEVICE memory for the all-gather; finish = fold
-       // the gathered aggregates of the other ranks on the device and apply
-       kScanDistLocal = 2, kScanDistFinish = 3 };
+enum { kScanApply = 0,
+       // time-sharded run over several GPUs: local = level-1 + scan with an identity carry, chunk
+       // aggregate left in DEVICE memory for the all-gather; finish = fold the gathered aggregates
+       // of the other ranks on the device and apply
+       kScanDistLocal = 1, kScanDistFinish = 2 };
 // Peer mailboxes of a single-process communicator (comm.cu): box[r] / flag[r] live in rank r's
 // device memory and are mapped into every other device (cudaDeviceEnablePeerAccess).  A rank
 // PUBLISHES its chunk aggregate by storing it into slot [its rank] of every peer's box over
@@ -98,21 +98,19 @@ struct ScanArgs {
   int64_t T;           // observations in this chunk
   int keep_init;       // rows = T + keep_init
   int backward;        // 0 = filter pass, 1 = smoother pass
-  int phase;           // kScanReduce: chunk aggregate only; kScanApply: write outputs
+  int phase;           // kScanApply: whole series on one GPU; kScanDist*: one rank's chunk
   int has_successor;   // backward: another chunk follows this one in time
   const double *G, *F, *W;  // host, column-major
   double V;
   const double *y;     // device [T]
-  const double *start; // host [n + n*n]: (m, C) before the chunk (forward apply) or (s, S)
-                       // of the first row of the next chunk (backward apply, has_successor)
-  double *agg_out;     // host: chunk aggregate (reduce phase)
+  const double *start; // host [n + n*n]: the prior (m0, C0) of the series (forward apply / finish)
   KfViews kf;          // forward: outputs; backward: filtered (m, C) inputs
   View s, S;           // backward outputs
   int32_t *status;     // device, one int, OR-ed
   void *workspace;     // device, scan_workspace_bytes(n, T)
-  void *fuse_sagg;     // forward apply: also write the smoother's level-1 aggregates here (the
-                       // backward workspace of the call that follows), or nullptr
-  int pre_reduced;     // backward apply: workspace already holds those aggregates
+  void *fuse_sagg;     // forward apply / finish: also write the smoother's level-1 aggregates
+                       // here (the backward workspace of the call that follows, which has no
+                       // other source of them), or nullptr
   double *agg_dev;     // dist local: device [elem doubles], this rank's chunk aggregate (out)
   const double *aggs_dev;  // dist finish: device [world][elem doubles], all ranks' aggregates
   int rank, world;     // dist phases

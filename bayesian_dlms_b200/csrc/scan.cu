@@ -186,23 +186,8 @@ __host__ __device__ __forceinline__ void s_combine(const SElem<N> &ei, const SEl
   for (int k = 0; k < N * N; ++k) out.L[k] = t2[k] + ei.L[k];
 }
 
-template <int N>
-__host__ __device__ __forceinline__ void s_element_pred(const double *G, const double (&m)[N],
-                                                        const double (&C)[N * N], const double (&a1)[N],
-                                                        const double (&R1)[N * N], SElem<N> &e);
-
 // Smoothing element of a filtered row that has a successor: E = C G^T R1^-1 (the RTS gain),
-// g = m - E a1, L = C - E R1 E^T, with (a1, R1) the prediction from (m, C).
-template <int N>
-__host__ __device__ __forceinline__ void s_element(const double *G, const double (&W)[N * N],
-                                                   const double (&m)[N], const double (&C)[N * N],
-                                                   SElem<N> &e) {
-  double a1[N], R1[N * N];
-  advance<N, true>(G, W, 1.0, m, C, a1, R1);
-  s_element_pred<N>(G, m, C, a1, R1, e);
-}
-
-// Same, with the one-step prediction (a1, R1) from (m, C) already at hand.
+// g = m - E a1, L = C - E R1 E^T, with (a1, R1) the one-step prediction from (m, C).
 template <int N>
 __host__ __device__ __forceinline__ void s_element_pred(const double *G, const double (&m)[N],
                                                         const double (&C)[N * N], const double (&a1)[N],
@@ -753,50 +738,6 @@ fwd_apply_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T,
   if (status && st) atomicOr(status, st);
 }
 
-// ---- level 1, backward: per-thread aggregate of smoothing elements over rows
-// [c*kSub, (c+1)*kSub) of the `nrows` rows that HAVE a successor.
-template <int N, bool VEC>
-__global__ void __launch_bounds__(128)
-bwd_reduce_kernel(const ScanModel<N> md, View fm, View fC, int64_t nrows, int64_t M,
-                  SElem<N> *agg /* [M + 1], slot M reserved for the terminal element */, int sub) {
-  const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (c >= M) return;
-  const int64_t r0 = c * (int64_t)sub, r1 = (r0 + sub < nrows) ? r0 + sub : nrows;
-  double W[N * N];
-#pragma unroll
-  for (int k = 0; k < N * N; ++k) W[k] = md.W[k];
-  SElem<N> acc, e, tmp;
-  auto row = [&](int64_t r, const double (&m)[N], const double (&C)[N * N]) {
-    s_element<N>(md.G, W, m, C, e);
-    if (r == r0) acc = e;
-    else { s_combine<N>(acc, e, tmp); acc = tmp; }
-  };
-  int64_t r = r0;
-  if (VEC && N <= 2) {  // whole-line loads of kGrp rows (register budget allows it for n <= 2)
-    for (; r + kGrp <= r1; r += kGrp) {
-      double gm[kGrp * N], gC[kGrp * N * N];
-      load_group<N>(fm, r, gm);
-      load_group<N * N>(fC, r, gC);
-#pragma unroll
-      for (int i = 0; i < kGrp; ++i) {
-        double m[N], C[N * N];
-#pragma unroll
-        for (int k = 0; k < N; ++k) m[k] = gm[i * N + k];
-#pragma unroll
-        for (int k = 0; k < N * N; ++k) C[k] = gC[i * N * N + k];
-        row(r + i, m, C);
-      }
-    }
-  }
-  for (; r < r1; ++r) {
-    double m[N], C[N * N];
-    load_row<N, VEC>(fm, r, m);
-    load_row<N * N, VEC>(fC, r, C);
-    row(r, m, C);
-  }
-  agg[c] = acc;
-}
-
 // ---- apply, backward: sequential (textbook) RTS recursion from the scanned successor state
 template <int N>
 __device__ __forceinline__ void bwd_step(const ScanModel<N> &md, const double (&W)[N * N],
@@ -908,13 +849,12 @@ bwd_apply_kernel(const ScanModel<N> md, View fm, View fC, int64_t nrows, int64_t
   if (status && st) atomicOr(status, st);
 }
 
+// terminal slot of a chunk that others follow: the identity, so that the chunk's aggregate leaves
+// them out (the finish phase brings them in through the carry)
 template <int N>
-__global__ void set_s_terminal(SElem<N> *slot, const StateArg<N> sS, const double *sS_dev,
-                               bool identity) {
+__global__ void set_s_identity(SElem<N> *slot) {
   SElem<N> e;
-  if (identity) s_identity<N>(e);
-  else if (sS_dev) s_state<N>(e, sS_dev, sS_dev + N);
-  else s_state<N>(e, sS.v, sS.v + N);
+  s_identity<N>(e);
   *slot = e;
 }
 // last chunk: s_T = m_T, S_T = C_T go to the outputs and become the terminal element of the scan
@@ -1098,27 +1038,21 @@ cudaError_t scan_forward(const ScanArgs &a, cudaStream_t stream, int64_t *launch
     // pageable source: staged by the driver before the call returns
     CK(cudaMemcpyAsync(tb, &host, sizeof(host), cudaMemcpyHostToDevice, stream));
   }
-  const bool reduce = a.phase == kScanReduce, local = a.phase == kScanDistLocal,
-             finish = a.phase == kScanDistFinish;
+  const bool local = a.phase == kScanDistLocal, finish = a.phase == kScanDistFinish;
   FElem<N> *carry = reinterpret_cast<FElem<N> *>(scratch + (M + 1) / kScanBlock * 2 + 8);
   if (!finish) {
-    // reduce / dist local: chunk aggregate only (identity start); apply: prefix of
+    // dist local: chunk aggregate only (identity start); apply: prefix of
     // (start (x) aggregates), a.start = host (m, C) of the state before t = 0
-    const bool ident = reduce || local;
-    const StateArg<N> st0 = state_arg<N>(ident ? nullptr : a.start);
+    const StateArg<N> st0 = state_arg<N>(local ? nullptr : a.start);
     if ((reinterpret_cast<uintptr_t>(a.y) & 31) == 0)
-      fwd_reduce_kernel<N, true><<<blocks, 128, 0, stream>>>(md, tb, a.y, T, M, a.keep_init, X, st0, ident, sub);
+      fwd_reduce_kernel<N, true><<<blocks, 128, 0, stream>>>(md, tb, a.y, T, M, a.keep_init, X, st0, local, sub);
     else
-      fwd_reduce_kernel<N, false><<<blocks, 128, 0, stream>>>(md, tb, a.y, T, M, a.keep_init, X, st0, ident, sub);
+      fwd_reduce_kernel<N, false><<<blocks, 128, 0, stream>>>(md, tb, a.y, T, M, a.keep_init, X, st0, local, sub);
     ++*launches;
     CK(cudaGetLastError());
     CK((device_scan<FElem<N>, false, false>(X, M + 1, scratch, stream, launches, /*defer_top=*/true)));
     // the whole chunk: last element of a one-block scan, else the last scanned block total
     const FElem<N> *whole = nb > 1 ? scratch + (nb - 1) : X + M;
-    if (reduce) {
-      CK(cudaMemcpyAsync(a.agg_out, whole, sizeof(FElem<N>), cudaMemcpyDeviceToHost, stream));
-      return cudaStreamSynchronize(stream);
-    }
     if (local) {
       if (a.peers.world > 0) {  // straight into every peer's mailbox over NVLink
         publish_kernel<FElem<N>><<<a.peers.world, 64, 0, stream>>>(whole, a.peers, a.rank, a.epoch_dev);
@@ -1171,33 +1105,21 @@ cudaError_t scan_backward(const ScanArgs &a, cudaStream_t stream, int64_t *launc
   double *term_dev = reinterpret_cast<double *>(scratch + (M + 1) / kScanBlock * 2 + 8);
   const unsigned blocks = (unsigned)((M + 127) / 128);
   const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);  // level-2 blocks over X
-  const bool reduce = a.phase == kScanReduce, local = a.phase == kScanDistLocal,
-             finish = a.phase == kScanDistFinish;
-  const StateArg<N> none = state_arg<N>(nullptr);
+  const bool local = a.phase == kScanDistLocal, finish = a.phase == kScanDistFinish;
   const bool vec = dense_aligned(a.kf.m, N) && dense_aligned(a.kf.C, N * N) &&
                    dense_aligned(a.s, N) && dense_aligned(a.S, N * N);
   SElem<N> *carry = reinterpret_cast<SElem<N> *>(term_dev + 64);
   if (!finish) {
-    if (reduce || (local && a.has_successor)) {
-      set_s_terminal<N><<<1, 1, 0, stream>>>(X + M, none, nullptr, true);
-    } else if (a.has_successor) {
-      set_s_terminal<N><<<1, 1, 0, stream>>>(X + M, state_arg<N>(a.start), nullptr, false);
+    // X[0, M) already holds the level-1 aggregates, written by the forward apply sweep (fuse_sagg)
+    if (a.has_successor) {  // dist local of a chunk followed by others
+      set_s_identity<N><<<1, 1, 0, stream>>>(X + M);
     } else {  // last chunk: s_T = m_T, S_T = C_T (Smoothing.scala:59-61)
       terminal_from_last_row<N><<<1, 1, 0, stream>>>(a.kf.m, a.kf.C, rows - 1, a.s, a.S, X + M);
     }
     ++*launches;
-    if (M > 0 && !a.pre_reduced) {
-      if (vec) bwd_reduce_kernel<N, true><<<blocks, 128, 0, stream>>>(md, a.kf.m, a.kf.C, nrows, M, X, sub);
-      else bwd_reduce_kernel<N, false><<<blocks, 128, 0, stream>>>(md, a.kf.m, a.kf.C, nrows, M, X, sub);
-      ++*launches;
-    }
     CK(cudaGetLastError());
     CK((device_scan<SElem<N>, true, true>(X, M + 1, scratch, stream, launches, /*defer_top=*/true)));
     const SElem<N> *whole = nb > 1 ? scratch + (nb - 1) : X;  // the whole chunk (suffix scan ends at index 0)
-    if (reduce) {
-      CK(cudaMemcpyAsync(a.agg_out, whole, sizeof(SElem<N>), cudaMemcpyDeviceToHost, stream));
-      return cudaStreamSynchronize(stream);
-    }
     if (local) {
       if (a.peers.world > 0) {
         publish_kernel<SElem<N>><<<a.peers.world, 64, 0, stream>>>(whole, a.peers, a.rank, a.epoch_dev);
@@ -1256,7 +1178,7 @@ cudaError_t launch_scan(const ScanArgs &a, cudaStream_t stream, int64_t *launche
   }
 }
 
-// Host-side carry composition for multi-GPU runs: out = ei (x) ej (ei earlier in time).
+// Host build of the combine the kernels inline: out = ei (x) ej (ei earlier in time).
 void scan_combine_host(int n, bool backward, const double *ei, const double *ej, double *out) {
   switch (n) {
 #define BDLM_COMB_CASE(N_)                                                                  \

@@ -2,14 +2,13 @@
 
 Not in the reference (strictly sequential recursion, Filter.scala:41-62); temporal
 parallelisation by associative scan (Sarkka & Garcia-Fernandez 2021), kernels in csrc/scan.cu.
-``scan_filter_smooth`` is the single-GPU call; ``ScanChunk`` exposes the reduce / apply phases
-a rank runs on its time chunk, and ``fold_*`` the host-side carry composition, so that
-``scan_filter_smooth_sharded`` can run over ``torch.distributed`` (one all-gather of a
-3n^2+2n-double aggregate per rank for the filter, 2n^2+n for the smoother).
+``scan_filter_smooth`` is the single-GPU call; ``DistScan`` runs one rank's time chunk of a
+sharded series with the device-side phases (one all-gather of a 3n^2+2n-double aggregate per rank
+for the filter, 2n^2+n for the smoother).
 """
 from __future__ import annotations
 
-from typing import Dict, List, Optional
+from typing import Dict
 
 import numpy as np
 
@@ -32,25 +31,29 @@ def _problem(model: Model, params: Dict, y, keep_init: bool):
     return pr, keep
 
 
-def _alloc(like, rows, k):
-    import torch
-    return torch.empty((rows, k), dtype=torch.float64, device=like.device)
+_FIELDS = ("m", "C", "a", "R", "f", "Q", "s", "S")
 
 
-def scan_filter_smooth(eng: Engine, model: Model, params: Dict, y, *, keep_init=True,
-                       want=("m", "C", "a", "R", "f", "Q", "s", "S")):
-    """y: CUDA tensor [T] (or [T, 1]).  Returns [rows, k] tensors (+ int status)."""
+def _outputs(like, rows: int, n: int, want=_FIELDS):
+    """[rows, k] float64 tensors on ``like``'s device for the fields in ``want``, and the
+    ``KfOut`` / ``SmoothOut`` structs that point at them (NULL for the fields left out)."""
     import torch
-    n, rows = model.n, model.T + int(keep_init)
-    with bound_engine(eng):
-        pr, keep = _problem(model, params, y, keep_init)
     dims = dict(m=n, C=n * n, a=n, R=n * n, f=1, Q=1, s=n, S=n * n)
-    out = {k: _alloc(y, rows, dims[k]) for k in want}
+    out = {k: torch.empty((rows, dims[k]), dtype=torch.float64, device=like.device) for k in want}
     ko, so = capi.KfOut(), capi.SmoothOut()
     for k in ("m", "C", "a", "R", "f", "Q"):
         setattr(ko, k, out[k].data_ptr() if k in out else None)
     for k in ("s", "S"):
         setattr(so, k, out[k].data_ptr() if k in out else None)
+    return out, ko, so
+
+
+def scan_filter_smooth(eng: Engine, model: Model, params: Dict, y, *, keep_init=True, want=_FIELDS):
+    """y: CUDA tensor [T] (or [T, 1]).  Returns [rows, k] tensors (+ int status)."""
+    import torch
+    with bound_engine(eng):
+        pr, keep = _problem(model, params, y, keep_init)
+    out, ko, so = _outputs(y, model.T + int(keep_init), model.n, want)
     st = torch.zeros((1,), dtype=torch.int32, device=y.device)
     eng.ctx.check(capi.load().bdlm_scan_filter_smooth(eng.ctx.handle, pr, ko, so, st.data_ptr()))
     out["status"] = st
@@ -59,120 +62,6 @@ def scan_filter_smooth(eng: Engine, model: Model, params: Dict, y, *, keep_init=
 
 def elem_doubles(n: int, backward: bool) -> int:
     return int(capi.load().bdlm_scan_elem_doubles(n, int(backward)))
-
-
-def combine(n: int, backward: bool, earlier: np.ndarray, later: np.ndarray) -> np.ndarray:
-    out = np.empty_like(earlier)
-    rc = capi.load().bdlm_scan_combine(n, int(backward), earlier.ctypes.data, later.ctypes.data,
-                                       out.ctypes.data)
-    assert rc == 0
-    return out
-
-
-def fold_forward_start(n: int, m0, C0, aggs: List[np.ndarray], rank: int) -> np.ndarray:
-    """(m, C) just before rank's chunk = [prior state] (x) agg_0 (x) ... (x) agg_{rank-1}."""
-    e = np.zeros(elem_doubles(n, False))
-    e[n * n: n * n + n] = np.asarray(m0, float).ravel()           # b
-    e[n * n + n: 2 * n * n + n] = _dlm.cm(np.atleast_2d(C0))      # C   (A = eta = J = 0)
-    for r in range(rank):
-        e = combine(n, False, e, aggs[r])
-    return np.concatenate([e[n * n: n * n + n], e[n * n + n: 2 * n * n + n]])
-
-
-def fold_backward_next(n: int, aggs: List[np.ndarray], rank: int, last_sS: np.ndarray) -> np.ndarray:
-    """(s, S) of the first row after rank's chunk = agg_{rank+1} (x) ... (x) agg_{last-1} (x)
-    [terminal state of the last rank], the last rank contributing its own first-row (s, S)."""
-    world = len(aggs)
-    # terminal element of the chain: the LAST rank's whole chunk folded with its terminal
-    # state is exactly its first-row smoothed state, which that rank computes itself.
-    e = np.zeros(elem_doubles(n, True))
-    e[n * n: n * n + n] = last_sS[:n]
-    e[n * n + n:] = last_sS[n:]
-    for r in range(world - 2, rank, -1):
-        e = combine(n, True, aggs[r], e)
-    return np.concatenate([e[n * n: n * n + n], e[n * n + n:]])
-
-
-class ScanChunk:
-    """One rank's time chunk: the four device phases."""
-
-    def __init__(self, eng: Engine, model: Model, params: Dict, y, keep_init: bool):
-        self.eng, self.model, self.n = eng, model, model.n
-        self.keep_init = keep_init
-        self.rows = model.T + int(keep_init)
-        self.y = y
-        with bound_engine(eng):
-            self.pr, self._keep = _problem(model, params, y, keep_init)
-        n = self.n
-        self.out = {k: _alloc(y, self.rows, d) for k, d in
-                    dict(m=n, C=n * n, a=n, R=n * n, f=1, Q=1, s=n, S=n * n).items()}
-        self.ko, self.so = capi.KfOut(), capi.SmoothOut()
-        for k in ("m", "C", "a", "R", "f", "Q"):
-            setattr(self.ko, k, self.out[k].data_ptr())
-        for k in ("s", "S"):
-            setattr(self.so, k, self.out[k].data_ptr())
-
-    def forward_reduce(self) -> np.ndarray:
-        agg = np.empty(elem_doubles(self.n, False))
-        self.eng.ctx.check(capi.load().bdlm_scan_forward_reduce(self.eng.ctx.handle, self.pr,
-                                                                agg.ctypes.data))
-        return agg
-
-    def forward_apply(self, start_mC: Optional[np.ndarray]):
-        ptr = None if start_mC is None else np.ascontiguousarray(start_mC).ctypes.data
-        self._start = start_mC
-        self.eng.ctx.check(capi.load().bdlm_scan_forward_apply(self.eng.ctx.handle, self.pr, ptr,
-                                                               self.ko, None))
-
-    def backward_reduce(self, has_successor: bool) -> np.ndarray:
-        agg = np.empty(elem_doubles(self.n, True))
-        self.eng.ctx.check(capi.load().bdlm_scan_backward_reduce(
-            self.eng.ctx.handle, self.pr, self.ko, int(has_successor), agg.ctypes.data))
-        return agg
-
-    def backward_apply(self, next_sS: Optional[np.ndarray]):
-        ptr = None if next_sS is None else np.ascontiguousarray(next_sS).ctypes.data
-        self._next = next_sS
-        self.eng.ctx.check(capi.load().bdlm_scan_backward_apply(self.eng.ctx.handle, self.pr,
-                                                                self.ko, ptr, self.so, None))
-
-    def first_row_sS(self) -> np.ndarray:
-        return np.concatenate([self.out["s"][0].cpu().numpy(), self.out["S"][0].cpu().numpy()])
-
-
-def scan_filter_smooth_sharded(eng: Engine, mod, params: Dict, y_chunk, rank: int, world: int,
-                               all_gather=None):
-    """One rank's part of a time-sharded run.  ``y_chunk``: this rank's CUDA slice of the series;
-    ``mod``: the ``Dlm`` or a prebuilt ``Model`` for the chunk length.
-    ``all_gather(np.ndarray) -> List[np.ndarray]`` exchanges the per-rank aggregates (defaults
-    to torch.distributed.all_gather_object).  Returns the rank's output dict."""
-    if all_gather is None:
-        import torch
-        import torch.distributed as dist
-
-        def all_gather(x):
-            # a few dozen doubles per rank: one tensor all-gather (NCCL on GPUs, gloo on CPU)
-            dev = y_chunk.device if dist.get_backend() == "nccl" else "cpu"
-            t = torch.from_numpy(np.ascontiguousarray(x, dtype=np.float64)).to(dev)
-            out = [torch.empty_like(t) for _ in range(dist.get_world_size())]
-            dist.all_gather(out, t)
-            return [o.cpu().numpy() for o in out]
-
-    n = len(np.asarray(params["m0"]).ravel())
-    model = mod if isinstance(mod, Model) else Model.build(mod, T=int(y_chunk.shape[0]))
-    ch = ScanChunk(eng, model, params, y_chunk, keep_init=(rank == 0))
-    aggs = all_gather(ch.forward_reduce())
-    ch.forward_apply(None if rank == 0 else fold_forward_start(n, params["m0"], params["C0"], aggs, rank))
-    # smoother: the last rank can run immediately; the others need its first-row state and
-    # the aggregates of the ranks in between
-    has_succ = rank < world - 1
-    sagg = all_gather(ch.backward_reduce(has_succ) if has_succ else np.zeros(elem_doubles(n, True)))
-    if not has_succ:
-        ch.backward_apply(None)
-    last = all_gather(ch.first_row_sS() if not has_succ else np.zeros(n + n * n))[world - 1]
-    if has_succ:
-        ch.backward_apply(fold_backward_next(n, sagg, rank, last))
-    return ch.out
 
 
 class DistScan:
@@ -191,13 +80,7 @@ class DistScan:
         with bound_engine(eng):
             self.pr, self._keep = _problem(model, params, y_chunk, self.keep_init)
         n = self.n
-        self.out = {k: _alloc(y_chunk, self.rows, d) for k, d in
-                    dict(m=n, C=n * n, a=n, R=n * n, f=1, Q=1, s=n, S=n * n).items()}
-        self.ko, self.so = capi.KfOut(), capi.SmoothOut()
-        for k in ("m", "C", "a", "R", "f", "Q"):
-            setattr(self.ko, k, self.out[k].data_ptr())
-        for k in ("s", "S"):
-            setattr(self.so, k, self.out[k].data_ptr())
+        self.out, self.ko, self.so = _outputs(y_chunk, self.rows, n)
         ef, eb = elem_doubles(n, False), elem_doubles(n, True)
         z = lambda k: torch.zeros(k, dtype=torch.float64, device=y_chunk.device)  # noqa: E731
         self.agg_f, self.aggs_f = z(ef), z(world * ef)

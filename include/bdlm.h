@@ -305,39 +305,21 @@ BDLM_API int bdlm_gibbs_suffstats(bdlm_ctx *ctx, const bdlm_problem *prob, const
  * shared parameters, mem = BDLM_DEVICE.  Results equal bdlm_kf_filter_smooth with
  * BDLM_TEXTBOOK_SMOOTHER to 1e-9 relative (for n = 1 that is the reference itself).
  *
- * Single GPU: bdlm_scan_filter_smooth.  Several GPUs, each owning a contiguous time chunk
- * (prob describes the chunk; keep_init = 1 only on the first rank):
- *   1. every rank: bdlm_scan_forward_reduce  -> agg (bdlm_scan_elem_doubles(n, 0) doubles)
- *   2. all-gather agg; rank r folds start = (prior state) (x) agg_0 (x) ... (x) agg_{r-1} with
- *      bdlm_scan_combine and reads (m, C) before its chunk from it (bdlm_scan_state_*)
- *   3. every rank: bdlm_scan_forward_apply(start_mC)           -> KfState rows of its chunk
- *   4. every rank: bdlm_scan_backward_reduce(has_successor)    -> agg (.. (n, 1) doubles)
- *   5. all-gather; rank r folds agg_{r+1} (x) ... (x) agg_last; its (g, L) part is (s, S) of
- *      the first row after its chunk
- *   6. every rank: bdlm_scan_backward_apply(next_sS)           -> (s, S) rows of its chunk
+ * Single GPU: bdlm_scan_filter_smooth.  Several GPUs, each owning a contiguous time chunk:
+ * bdlm_comm_scan_filter_smooth, or, for hosts that bring their own transport, the bdlm_scan_dist_*
+ * sequence.  There the chunk aggregate stays in device memory, the caller all-gathers it (NCCL,
+ * or a copy through the host and back) on the context's stream (aggs_dev =
+ * [world][bdlm_scan_elem_doubles] doubles), and the carry is folded by a one-thread kernel inside
+ * the finish call.  Per rank: forward_local -> all-gather -> forward_finish -> backward_local ->
+ * all-gather -> backward_finish; nothing synchronises with the host.  prob describes the rank's
+ * chunk (keep_init = 1 on rank 0 only); kf->m and kf->C are required; the context's workspace
+ * must not be used by other calls between a local and its finish phase.
  * Elements are laid out [A | b | C | eta | J] (forward) and [E | g | L] (backward), matrices
  * column-major. */
 BDLM_API int bdlm_scan_filter_smooth(bdlm_ctx *ctx, const bdlm_problem *prob,
                                      const bdlm_kf_out *kf, const bdlm_smooth_out *sm,
                                      int32_t *status);
 BDLM_API int bdlm_scan_elem_doubles(int32_t n, int32_t backward);
-BDLM_API int bdlm_scan_forward_reduce(bdlm_ctx *ctx, const bdlm_problem *prob, double *agg_host);
-BDLM_API int bdlm_scan_forward_apply(bdlm_ctx *ctx, const bdlm_problem *prob,
-                                     const double *start_mC_host, const bdlm_kf_out *kf,
-                                     int32_t *status);
-BDLM_API int bdlm_scan_backward_reduce(bdlm_ctx *ctx, const bdlm_problem *prob,
-                                       const bdlm_kf_out *filt, int32_t has_successor,
-                                       double *agg_host);
-BDLM_API int bdlm_scan_backward_apply(bdlm_ctx *ctx, const bdlm_problem *prob,
-                                      const bdlm_kf_out *filt, const double *next_sS_host,
-                                      const bdlm_smooth_out *sm, int32_t *status);
-/* The same protocol WITHOUT host round trips (what a multi-GPU run should use): the chunk
- * aggregate stays in device memory, the caller all-gathers it with NCCL on the context's stream
- * (aggs_dev = [world][bdlm_scan_elem_doubles] doubles), and the carry is folded by a one-thread
- * kernel inside the finish call.  Per rank: forward_local -> all-gather -> forward_finish ->
- * backward_local -> all-gather -> backward_finish; nothing synchronises with the host.  prob
- * describes the rank's chunk (keep_init = 1 on rank 0 only); kf->m and kf->C are required; the
- * context's workspace must not be used by other calls between a local and its finish phase. */
 BDLM_API int bdlm_scan_dist_forward_local(bdlm_ctx *ctx, const bdlm_problem *prob, int32_t rank,
                                           int32_t world, double *agg_dev);
 BDLM_API int bdlm_scan_dist_forward_finish(bdlm_ctx *ctx, const bdlm_problem *prob, int32_t rank,
@@ -350,7 +332,7 @@ BDLM_API int bdlm_scan_dist_backward_finish(bdlm_ctx *ctx, const bdlm_problem *p
                                             int32_t world, const double *aggs_dev,
                                             const bdlm_kf_out *filt, const bdlm_smooth_out *sm,
                                             int32_t *status);
-/* out = earlier (x) later on the host (carry folding between ranks; a few dozen flops). */
+/* out = earlier (x) later on the host: the host build of the combine the scan kernels inline. */
 BDLM_API int bdlm_scan_combine(int32_t n, int32_t backward, const double *earlier,
                                const double *later, double *out);
 

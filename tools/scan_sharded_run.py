@@ -3,20 +3,19 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port 29517 tools/scan_sharded_run.py --logT 24
 
-Each rank owns a contiguous time chunk; the only inter-GPU traffic is the all-gather of one
-scan aggregate per rank and pass (3n^2+2n / 2n^2+n doubles) plus the last rank's first-row
-smoothed state.  Checks the sharded result against the single-GPU scan and prints one JSON line
+Each rank owns a contiguous time chunk and runs the device-side phases (DistScan); the only
+inter-GPU traffic is the all-gather of one scan aggregate per rank and pass (3n^2+2n / 2n^2+n
+doubles).  Checks the sharded result against the single-GPU scan and prints one JSON line
 (time = max over ranks, device events).
 """
 import argparse, json, os, sys
 import numpy as np, torch, torch.distributed as dist
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from bayesian_dlms_b200 import Engine, Model, dlm
-from bayesian_dlms_b200.scan import DistScan, scan_filter_smooth, scan_filter_smooth_sharded
+from bayesian_dlms_b200.scan import DistScan, scan_filter_smooth
 from bayesian_dlms_b200.sharding import shard_range
 
 ap = argparse.ArgumentParser(); ap.add_argument("--logT", type=int, default=24); ap.add_argument("--reps", type=int, default=5)
-ap.add_argument("--host-protocol", action="store_true", help="the older host-folded protocol (bdlm_scan_*_reduce/apply)")
 a = ap.parse_args()
 rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
 torch.cuda.set_device(local)
@@ -31,8 +30,7 @@ y = torch.randn(T, generator=g, device=dev, dtype=torch.float64).cumsum(0) * 0.1
 lo, hi = shard_range(T, rank, world)
 yc = y[lo:hi].contiguous()
 cmodel = Model.build(mod, T=hi - lo)     # flattened once, outside the timed region
-ds = None if a.host_protocol else DistScan(eng, cmodel, params, yc, rank, world)
-run = (lambda: scan_filter_smooth_sharded(eng, cmodel, params, yc, rank, world)) if a.host_protocol else ds.run
+run = DistScan(eng, cmodel, params, yc, rank, world).run
 out = run()   # warm-up (NCCL communicator, arena, table)
 out = run()
 torch.cuda.synchronize(); dist.barrier()
@@ -59,7 +57,5 @@ if rank == 0:
     med = float(np.median(ms))
     print(json.dumps({"config": "config5 sharded: one series T=2^%d over %d GPUs (time chunks)" % (a.logT, world),
                       "n_gpus": world, "ms": med, "steps_per_s": T / med * 1e3,
-                      "max_rel_err_vs_single_gpu": float(e.item()),
-                      "protocol": "host-folded (3 all-gathers + host syncs)" if a.host_protocol else
-                                  "device-side (2 NCCL all-gathers of <= 16 doubles per rank, no host sync)"}))
+                      "max_rel_err_vs_single_gpu": float(e.item())}))
 dist.barrier(); dist.destroy_process_group()
