@@ -740,6 +740,16 @@ fwd_apply_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T,
 
 // ---- apply, backward: sequential (textbook) RTS recursion from the scanned successor state
 template <int N>
+__device__ __forceinline__ bool state_finite(const double *s, const double *S) {
+  bool finite = true;
+#pragma unroll
+  for (int i = 0; i < N; ++i) finite = finite && isfinite(s[i]);
+#pragma unroll
+  for (int k = 0; k < N * N; ++k) finite = finite && isfinite(S[k]);
+  return finite;
+}
+
+template <int N>
 __device__ __forceinline__ void bwd_step(const ScanModel<N> &md, const double (&W)[N * N],
                                          const double (&m)[N], const double (&C)[N * N],
                                          double (&s)[N], double (&S)[N * N], int &st) {
@@ -846,6 +856,9 @@ bwd_apply_kernel(const ScanModel<N> md, View fm, View fC, int64_t nrows, int64_t
     }
   }
   for (; r > r0; --r) scalar_row(r - 1);
+  // (s, S) now hold row 0 of the chunk.  For the whole series that is the smoothed initial state,
+  // the final state of the sequential kernels, which flag it when it is not finite.
+  if (c == 0 && !state_finite<N>(s, S)) st |= BDLM_ST_NONFINITE;
   if (status && st) atomicOr(status, st);
 }
 
@@ -857,9 +870,11 @@ __global__ void set_s_identity(SElem<N> *slot) {
   s_identity<N>(e);
   *slot = e;
 }
-// last chunk: s_T = m_T, S_T = C_T go to the outputs and become the terminal element of the scan
+// last chunk: s_T = m_T, S_T = C_T go to the outputs and become the terminal element of the scan.
+// status: the row is also row 0 (a single row, no backward sweep follows): flag it as that sweep would.
 template <int N>
-__global__ void terminal_from_last_row(View fm, View fC, int64_t row, View sv, View Sv, SElem<N> *slot) {
+__global__ void terminal_from_last_row(View fm, View fC, int64_t row, View sv, View Sv, SElem<N> *slot,
+                                       int32_t *status) {
   double sS[N + N * N];
   for (int k = 0; k < N; ++k) {
     const double v = fm.ptr[row * fm.sr + k * fm.sk];
@@ -871,6 +886,7 @@ __global__ void terminal_from_last_row(View fm, View fC, int64_t row, View sv, V
     if (Sv.ptr) Sv.ptr[row * Sv.sr + k * Sv.sk] = v;
     sS[N + k] = v;
   }
+  if (status && !state_finite<N>(sS, sS + N)) atomicOr(status, BDLM_ST_NONFINITE);
   SElem<N> e;
   s_state<N>(e, sS, sS + N);
   *slot = e;
@@ -1114,7 +1130,8 @@ cudaError_t scan_backward(const ScanArgs &a, cudaStream_t stream, int64_t *launc
     if (a.has_successor) {  // dist local of a chunk followed by others
       set_s_identity<N><<<1, 1, 0, stream>>>(X + M);
     } else {  // last chunk: s_T = m_T, S_T = C_T (Smoothing.scala:59-61)
-      terminal_from_last_row<N><<<1, 1, 0, stream>>>(a.kf.m, a.kf.C, rows - 1, a.s, a.S, X + M);
+      terminal_from_last_row<N><<<1, 1, 0, stream>>>(a.kf.m, a.kf.C, rows - 1, a.s, a.S, X + M,
+                                                     M == 0 ? a.status : nullptr);
     }
     ++*launches;
     CK(cudaGetLastError());
