@@ -355,12 +355,16 @@ class Engine:
         return res
 
     @_on_engine_stream
-    def loglik(self, model: Model, params: Dict, y, *, layout=TIME_MAJOR, status=True):
+    def loglik(self, model: Model, params: Dict, y, *, layout=TIME_MAJOR, status=True,
+               parallel_in_time=False):
         """KalmanFilter.likelihood (transition form, KalmanFilter.scala:299-306) and the
-        innovations form (conditionalLikelihood, :138-153) per series."""
+        innovations form (conditionalLikelihood, :138-153) per series.  ``parallel_in_time``: ONE
+        long eligible series may run through the scan's forward pass (1e-9 instead of bit-for-bit;
+        include/bdlm.h BDLM_PARALLEL_IN_TIME)."""
         mem, _ = _mem_and_ptr(y)
         B = self._batch_of(model, y, layout)
-        pr, keep = self._problem(model, params, y, layout, True, 0, B, mem)
+        pr, keep = self._problem(model, params, y, layout, True,
+                                 capi.PARALLEL_IN_TIME if parallel_in_time else 0, B, mem)
         tr, inn = self._alloc(y, (B,)), self._alloc(y, (B,))
         st, stp = self._status(y, B, status)
         self.ctx.check(capi.load().bdlm_loglik(self.ctx.handle, pr, _mem_and_ptr(tr)[1],
@@ -372,13 +376,14 @@ class Engine:
 
     @_on_engine_stream
     def filter_last(self, model: Model, params: Dict, y, *, layout=TIME_MAJOR, loglik=False,
-                    status=True):
+                    status=True, parallel_in_time=False):
         """``ys.foldLeft(init)(kf.step(mod, p))`` batched (NoModel.scala:153-155): only the state
         after the last observation, nothing stored per step.  Returns m (n, B) / (B, n) and
-        C (n*n, B) / (B, n*n) [+ both log-likelihoods]."""
+        C (n*n, B) / (B, n*n) [+ both log-likelihoods].  ``parallel_in_time`` as in ``loglik``."""
         mem, _ = _mem_and_ptr(y)
         B = self._batch_of(model, y, layout)
-        pr, keep = self._problem(model, params, y, layout, True, 0, B, mem)
+        pr, keep = self._problem(model, params, y, layout, True,
+                                 capi.PARALLEL_IN_TIME if parallel_in_time else 0, B, mem)
         n = model.n
         row = (lambda k: (k, B)) if layout == TIME_MAJOR else (lambda k: (B, k))
         out = dict(m=self._alloc(y, row(n)), C=self._alloc(y, row(n * n)))

@@ -1044,11 +1044,30 @@ int bdlm_rts_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *filt,
   return dispatch(c, d);
 }
 
-// BDLM_PARALLEL_IN_TIME: one long eligible series goes to the associative-scan kernels
-static bool pit_eligible(const bdlm_problem *p) {
+// BDLM_PARALLEL_IN_TIME: one long eligible series goes to the associative-scan kernels.  The
+// forward pass alone (log-likelihoods, last state) runs any n <= 4; the smoother needs n = 1 or the
+// textbook smoother, which is what its backward sweep computes.
+static bool pit_eligible_forward(const bdlm_problem *p) {
   return (p->compat & BDLM_PARALLEL_IN_TIME) && p->B == 1 && p->T >= 4096 && p->p == 1 && p->n <= 4 &&
-         !p->times && !p->f_tv && !p->g_tv && !p->per_series && !p->v_tv && !p->w_tv &&
-         (p->n == 1 || (p->compat & BDLM_TEXTBOOK_SMOOTHER));
+         !p->times && !p->f_tv && !p->g_tv && !p->per_series && !p->v_tv && !p->w_tv;
+}
+static bool pit_eligible(const bdlm_problem *p) {
+  return pit_eligible_forward(p) && (p->n == 1 || (p->compat & BDLM_TEXTBOOK_SMOOTHER));
+}
+
+// Staging buffer of the host-buffer BDLM_PARALLEL_IN_TIME calls (the scan owns the arena); y is
+// copied to its start.
+static int pit_stage_y(bdlm_ctx *c, const bdlm_problem *p, size_t bytes) {
+  CU(cudaSetDevice(c->device));
+  if (bytes > c->pit_bytes) {
+    CU(cudaStreamSynchronize(c->stream));
+    if (c->pit_buf) CU(cudaFree(c->pit_buf));
+    c->pit_buf = nullptr; c->pit_bytes = 0;
+    CU(cudaMalloc(&c->pit_buf, bytes));
+    c->pit_bytes = bytes;
+  }
+  CU(cudaMemcpyAsync(c->pit_buf, p->y, sizeof(double) * (size_t)p->T, cudaMemcpyHostToDevice, c->stream));
+  return 0;
 }
 
 static int pit_host(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *kf,
@@ -1061,15 +1080,8 @@ static int pit_host(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *kf,
   size_t off[9], pos = align_up(sizeof(double) * (size_t)p->T);
   for (int i = 0; i < 8; ++i) { off[i] = pos; if (host[i]) pos = align_up(pos + sizeof(double) * (size_t)R * ks[i]); }
   off[8] = pos; pos += 256;
-  CU(cudaSetDevice(c->device));
-  if (pos > c->pit_bytes) {
-    CU(cudaStreamSynchronize(c->stream));
-    if (c->pit_buf) CU(cudaFree(c->pit_buf));
-    c->pit_buf = nullptr; c->pit_bytes = 0;
-    CU(cudaMalloc(&c->pit_buf, pos));
-    c->pit_bytes = pos;
-  }
-  CU(cudaMemcpyAsync(c->pit_buf, p->y, sizeof(double) * (size_t)p->T, cudaMemcpyHostToDevice, c->stream));
+  int rc0 = pit_stage_y(c, p, pos);
+  if (rc0) return rc0;
   bdlm_problem q = *p;
   q.mem = BDLM_DEVICE;
   q.y = reinterpret_cast<const double *>(c->pit_buf);
@@ -1105,12 +1117,43 @@ int bdlm_kf_filter_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out 
   return dispatch(c, d);
 }
 
+// BDLM_PARALLEL_IN_TIME on bdlm_loglik / bdlm_kf_filter_last: bdlm_scan_loglik, with host buffers
+// staged through pit_buf ([y | m_last | C_last | transition | innovations | status]).
+static int pit_loglik(bdlm_ctx *c, const bdlm_problem *p, double *m_last, double *C_last,
+                      double *transition, double *innovations, int32_t *status) {
+  bdlm_problem q = *p;
+  q.compat &= ~BDLM_PARALLEL_IN_TIME;
+  if (p->mem == BDLM_DEVICE) return bdlm_scan_loglik(c, &q, m_last, C_last, transition, innovations, status);
+  const int64_t n = p->n;
+  const int64_t ks[4] = {n, n * n, 1, 1};
+  double *host[4] = {m_last, C_last, transition, innovations};
+  size_t off[5], pos = align_up(sizeof(double) * (size_t)p->T);
+  for (int i = 0; i < 4; ++i) { off[i] = pos; if (host[i]) pos = align_up(pos + sizeof(double) * (size_t)ks[i]); }
+  off[4] = pos; pos += 256;
+  int rc = pit_stage_y(c, p, pos);
+  if (rc) return rc;
+  q.mem = BDLM_DEVICE;
+  q.y = reinterpret_cast<const double *>(c->pit_buf);
+  double *dev[4];
+  for (int i = 0; i < 4; ++i) dev[i] = host[i] ? reinterpret_cast<double *>(c->pit_buf + off[i]) : nullptr;
+  int32_t *dst = status ? reinterpret_cast<int32_t *>(c->pit_buf + off[4]) : nullptr;
+  rc = bdlm_scan_loglik(c, &q, dev[0], dev[1], dev[2], dev[3], dst);
+  if (rc) return rc;
+  for (int i = 0; i < 4; ++i)
+    if (host[i])
+      CU(cudaMemcpyAsync(host[i], dev[i], sizeof(double) * (size_t)ks[i], cudaMemcpyDeviceToHost, c->stream));
+  if (status) CU(cudaMemcpyAsync(status, dst, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return 0;
+}
+
 int bdlm_loglik(bdlm_ctx *c, const bdlm_problem *p, double *transition, double *innovations,
                 int32_t *status) {
   NvtxRange nvtx_("bdlm_loglik");
   int rc = validate(c, A_LOGLIK, p);
   if (rc) return rc;
   if (!transition && !innovations) return fail(c, BDLM_E_ARG, "no log-likelihood requested");
+  if (pit_eligible_forward(p)) return pit_loglik(c, p, nullptr, nullptr, transition, innovations, status);
   DevCall d{}; d.op = A_LOGLIK; d.pr = *p; d.pr.keep_init = 1;
   d.ll_tr = transition; d.ll_in = innovations; d.status = status;
   return dispatch(c, d);
@@ -1123,6 +1166,7 @@ int bdlm_kf_filter_last(bdlm_ctx *c, const bdlm_problem *p, double *m_last, doub
   if (rc) return rc;
   if (!m_last && !C_last && !transition && !innovations)
     return fail(c, BDLM_E_ARG, "nothing requested");
+  if (pit_eligible_forward(p)) return pit_loglik(c, p, m_last, C_last, transition, innovations, status);
   DevCall d{}; d.op = A_LOGLIK; d.pr = *p; d.pr.keep_init = 1;
   d.last_m = m_last; d.last_C = C_last;
   d.ll_tr = transition; d.ll_in = innovations; d.status = status;
@@ -1202,8 +1246,8 @@ static int scan_fill(bdlm_ctx *c, const bdlm_problem *p, ScanArgs &a, bool forwa
 // launch_scan for a forward pass: the table key is committed only once the upload is enqueued, so
 // a failed launch (or a finish phase without its local phase) can never leave a stale table that
 // a later call would trust.
-static int scan_launch_fwd(bdlm_ctx *c, ScanArgs &a) {
-  CU(launch_scan(a, c->stream, &c->launches));
+static int scan_launch_fwd(bdlm_ctx *c, ScanArgs &a, const ScanLoglikOut *ll = nullptr) {
+  CU(ll ? launch_scan_loglik(a, *ll, c->stream, &c->launches) : launch_scan(a, c->stream, &c->launches));
   if (a.table_upload) c->scan_key.swap(c->scan_key_pending);
   c->scan_key_pending.clear();
   return 0;
@@ -1271,6 +1315,32 @@ int bdlm_scan_filter_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_ou
   a.status = status; a.workspace = c->arena + ws;
   CU(launch_scan(a, c->stream, &c->launches));
   return 0;
+}
+
+int bdlm_scan_loglik(bdlm_ctx *c, const bdlm_problem *p, double *m_last, double *C_last,
+                     double *transition, double *innovations, int32_t *status) {
+  NvtxRange nvtx_("bdlm_scan_loglik");
+  int rc = scan_validate(c, p);
+  if (rc) return rc;
+  if (p->v_tv || p->w_tv) return fail(c, BDLM_E_ARG, "scan path: time-invariant model (v_tv = w_tv = 0)");
+  if (!m_last && !C_last && !transition && !innovations) return fail(c, BDLM_E_ARG, "nothing requested");
+  CU(cudaSetDevice(c->device));
+  const int64_t n = p->n;
+  // arena: [forward scan workspace | block partials + last state]
+  const size_t ws = align_up(scan_workspace_bytes(p->n, p->T) + 4096);
+  rc = ensure_arena(c, ws + align_up(scan_loglik_bytes(p->n, p->T)) + 4096);
+  if (rc) return rc;
+  bdlm_problem q = *p;
+  q.keep_init = 1;  // as bdlm_loglik: the state (m0, C0) is row 0, every observation a step
+  std::vector<double> prior((size_t)n + n * n);
+  std::copy(p->m0, p->m0 + n, prior.begin());
+  std::copy(p->C0, p->C0 + n * n, prior.begin() + n);
+  ScanArgs a;
+  rc = scan_fill(c, &q, a, true);
+  if (rc) return rc;
+  a.phase = kScanApply; a.start = prior.data(); a.workspace = c->arena;
+  const ScanLoglikOut o{transition, innovations, m_last, C_last, status, c->arena + ws};
+  return scan_launch_fwd(c, a, &o);
 }
 
 // ---- device-side multi-GPU protocol for the scan (no host round trip) --------------------

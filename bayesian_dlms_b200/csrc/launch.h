@@ -125,6 +125,18 @@ size_t scan_workspace_bytes(int n, int64_t T);
 int scan_forward_elem_doubles(int n);
 int scan_backward_elem_doubles(int n);
 cudaError_t launch_scan(const ScanArgs &a, cudaStream_t stream, int64_t *launches);
+// Log-likelihoods + last filtered state of one series (forward pass only, nothing stored per row):
+// a = a forward kScanApply pass with keep_init = 1 (a.kf unused).  Outputs are device pointers,
+// any may be null; status (one int) is written, not OR-ed.
+struct ScanLoglikOut {
+  double *transition, *innovations;  // [1]
+  double *m_last, *C_last;           // [n], [n*n]
+  int32_t *status;
+  void *parts;                       // device, scan_loglik_bytes(n, T): block partials
+};
+size_t scan_loglik_bytes(int n, int64_t T);
+cudaError_t launch_scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream,
+                               int64_t *launches);
 void scan_combine_host(int n, bool backward, const double *ei, const double *ej, double *out);
 
 // scalar_filters.cu: scalar AR(1) / OU filter + backward sampler (FilterAr.scala, FilterOu.scala)

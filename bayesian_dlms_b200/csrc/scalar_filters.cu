@@ -197,116 +197,8 @@ conjugate_kernel(const ConjModel<N> md, const ConjArgs a) {
 // (MetropolisHastings.scala:126-137,199-209).  Nothing is stored per step: the kernel reads y
 // (8 B / series-step) and is bound by FP64 issue; the warp-per-series kernel it replaces for
 // these shapes needs a whole warp and shared-memory round trips per series.
-// Operation order = oracle_loglik / mvn_logpdf / chol_logdet (dgesv solve, dpotrf log-determinant).
-// breeze MultivariateGaussian(mu, S).logPdf(x) (oracle mvn_logpdf), split so that the part that
-// depends on S alone -- the dgesv factorisation (dgetf2) and sum(log(diag(cholesky(S)))) -- can be
-// hoisted out of the time loop when S = W dt is the same at every step (regular grid).  prepare()
-// followed by eval() performs exactly the operations of lu_solve + chol_logdet in the oracle's
-// order, so hoisting does not change a bit.
-template <int N>
-struct MvnPrepared {
-  double LU[N * N];  // unit-lower multipliers below the diagonal, U on and above it
-  int piv[N];        // row exchanged with row j at step j (j = no exchange)
-  bool singular[N];  // zero pivot at step j: dgetf2 skips the scaling (info > 0)
-  double ld;         // sum log diag chol(S)
-  int st;
-
-  __device__ __forceinline__ void prepare(const double (&S)[N * N]) {
-    st = 0;
-#pragma unroll
-    for (int k = 0; k < N * N; ++k) LU[k] = S[k];
-#pragma unroll
-    for (int j = 0; j < N; ++j) {
-      int jp = j;
-      double best = fabs(LU[j + j * N]);
-#pragma unroll
-      for (int i = j + 1; i < N; ++i) {
-        const double v = fabs(LU[i + j * N]);
-        if (v > best) { best = v; jp = i; }
-      }
-      double pv = LU[j + j * N];
-#pragma unroll
-      for (int i = j + 1; i < N; ++i)
-        if (jp == i) pv = LU[i + j * N];
-      piv[j] = j;
-      singular[j] = !(pv != 0.0);
-      if (pv != 0.0) {
-#pragma unroll
-        for (int i = j + 1; i < N; ++i)
-          if (jp == i) {
-            piv[j] = i;
-#pragma unroll
-            for (int c = 0; c < N; ++c) {
-              const double t = LU[j + c * N]; LU[j + c * N] = LU[i + c * N]; LU[i + c * N] = t;
-            }
-          }
-        const double r = 1.0 / LU[j + j * N];
-#pragma unroll
-        for (int i = j + 1; i < N; ++i) LU[i + j * N] = LU[i + j * N] * r;
-      } else {
-        st = BDLM_ST_SINGULAR;
-      }
-#pragma unroll
-      for (int c = j + 1; c < N; ++c)
-#pragma unroll
-        for (int i = j + 1; i < N; ++i)
-          LU[i + c * N] = LU[i + c * N] - LU[i + j * N] * LU[j + c * N];
-    }
-    double L[N * N];
-#pragma unroll
-    for (int k = 0; k < N * N; ++k) L[k] = S[k];
-    ld = 0.0;
-#pragma unroll
-    for (int j = 0; j < N; ++j) {
-      double d = L[j + j * N];
-#pragma unroll
-      for (int k = 0; k < j; ++k) d = d - L[j + k * N] * L[j + k * N];
-      if (!(d > 0.0)) st |= BDLM_ST_NOTPD;
-      d = sqrt(d);
-      L[j + j * N] = d;
-#pragma unroll
-      for (int i = j + 1; i < N; ++i) {
-        double v = L[i + j * N];
-#pragma unroll
-        for (int k = 0; k < j; ++k) v = v - L[i + k * N] * L[j + k * N];
-        L[i + j * N] = v / d;
-      }
-      ld = ld + log(d);
-    }
-  }
-
-  __device__ __forceinline__ double eval(const double (&x)[N], const double (&mu)[N]) const {
-    double c[N], slv[N];
-#pragma unroll
-    for (int i = 0; i < N; ++i) { c[i] = x[i] - mu[i]; slv[i] = c[i]; }
-    // the row exchanges dgetf2 applied to the right-hand side as it went (same order)
-#pragma unroll
-    for (int j = 0; j < N; ++j)
-      if (!singular[j]) {
-#pragma unroll
-        for (int i = j + 1; i < N; ++i)
-          if (piv[j] == i) { const double t = slv[j]; slv[j] = slv[i]; slv[i] = t; }
-      }
-#pragma unroll
-    for (int k = 0; k < N; ++k)
-#pragma unroll
-      for (int i = k + 1; i < N; ++i) slv[i] = slv[i] - slv[k] * LU[i + k * N];
-#pragma unroll
-    for (int k = N - 1; k >= 0; --k) {
-      slv[k] = slv[k] / LU[k + k * N];
-#pragma unroll
-      for (int i = 0; i < k; ++i) slv[i] = slv[i] - slv[k] * LU[i + k * N];
-    }
-    double dot = 0.0;
-#pragma unroll
-    for (int i = 0; i < N; ++i) {
-      const double prod = slv[i] * c[i];
-      dot = (i == 0) ? prod : dot + prod;
-    }
-    return -dot / 2.0 - (N / 2.0 * 1.8378770664093453 + ld);
-  }
-};
-
+// Operation order = oracle_loglik / mvn_logpdf / chol_logdet (dgesv solve, dpotrf log-determinant);
+// the transition density goes through small::MvnPrepared (small_steps.cuh).
 template <int N>
 __global__ void __launch_bounds__(128)
 loglik_small_kernel(const ConjModel<N> md, const Batch bt, double *ll_transition, double *ll_innov,

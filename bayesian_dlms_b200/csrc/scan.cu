@@ -659,6 +659,29 @@ __device__ __forceinline__ void fwd_row(const ScanModel<N> &md, const double (&W
   }
 }
 
+// Filtered (m, C) of the row before thread c's first row on one GPU: (b, C) of its exclusive prefix
+// pre[c], composed with the top-level block prefix that device_scan left unapplied (defer_top).
+// fwd_apply_kernel inlines the same composition (plus the multi-GPU carry) by hand: calling this
+// function from it reorders its SASS.
+template <int N>
+__device__ __forceinline__ void fwd_start_state(const FElem<N> *pre, int64_t c, const FElem<N> *tot,
+                                                double (&m)[N], double (&C)[N * N]) {
+  const int64_t blk = c / (kScanBlock * kPer);  // level-2 block of scan position c
+  if (tot && blk > 0) {
+    FElem<N> o;  // only (b, C) is live, the rest folds away
+    f_combine<N>(tot[blk - 1], pre[c], o);
+#pragma unroll
+    for (int k = 0; k < N; ++k) m[k] = o.b[k];
+#pragma unroll
+    for (int k = 0; k < N * N; ++k) C[k] = o.C[k];
+  } else {
+#pragma unroll
+    for (int k = 0; k < N; ++k) m[k] = pre[c].b[k];
+#pragma unroll
+    for (int k = 0; k < N * N; ++k) C[k] = pre[c].C[k];
+  }
+}
+
 // The two apply sweeps ask ptxas for one resident block per SM: asking for more makes them spill,
 // which costs more than the occupancy gains (profiles/r1_tuning.txt, "scan apply sweeps").
 template <int N, bool VEC, bool FUSE>
@@ -736,6 +759,131 @@ fwd_apply_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T,
   }
   if (FUSE && shave) sagg[c] = sacc;
   if (status && st) atomicOr(status, st);
+}
+
+// ---- log-likelihoods + last filtered state (bdlm_scan_loglik): the forward apply recursion of
+// one thread's rows with nothing stored per row.  keep_init = 1: row 0 is the prior, row r holds
+// step t = r - 1.  Per row (after the update) the thread adds, in row order,
+//   TR:          log N(m_t; a_t, W), a_t = G m_{t-1} being the prediction fwd_row carries in;
+//   innovations: -dd^2/2 - log(sqrt(2 pi) sd), sd = sqrt(Q_t), dd = (y_t - f_t) / sd, y_t observed
+// (scalar_filters.cu loglik_small_kernel's terms).  The block's thread sums then go through a
+// fixed-order tree in shared memory to one LoglikPart per block, which loglik_finish_kernel sums in
+// a fixed order: no atomics, so a call gives the same bits on any stream or context.
+struct LoglikPart {
+  double tr, in;
+  int st;
+};
+constexpr int kLlBlock = 128, kLlFinish = 256;
+
+template <int N, bool VEC, bool TR>
+__global__ void __launch_bounds__(kLlBlock)
+fwd_loglik_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T, int64_t M,
+                  const FElem<N> *pre /* [M+1] inclusive scan with slot 0 = the prior */,
+                  const FElem<N> *tot /* scanned level-2 block totals `pre` still lacks, or nullptr */,
+                  int sub, LoglikPart *part /* [gridDim.x] */, double *last /* [N + N*N]: (m_T, C_T) */) {
+  __shared__ double s_tr[kLlBlock], s_in[kLlBlock];
+  __shared__ int s_st[kLlBlock];
+  const int tid = threadIdx.x;
+  const int64_t c = blockIdx.x * (int64_t)blockDim.x + tid;
+  double tr = 0.0, li = 0.0;
+  int st = 0;
+  if (c < M) {
+    const int64_t rows = T + 1;
+    const int64_t r0 = c * (int64_t)sub, r1 = (r0 + sub < rows) ? r0 + sub : rows;
+    double m[N], C[N * N], W[N * N], an[N], Rn[N * N];
+    fwd_start_state<N>(pre, c, tot, m, C);
+#pragma unroll
+    for (int k = 0; k < N * N; ++k) W[k] = md.W[k];
+    MvnPrepared<N> mvn;  // S = W * 1.0 at every step: factorised once per thread
+    if (TR) {
+      mvn.prepare(W);
+      st |= mvn.st;
+    }
+    advance<N, true>(md.G, W, 1.0, m, C, an, Rn);
+    SElem<N> sacc;  // unused (no smoother fold)
+    bool shave = false;
+    auto row = [&](int64_t r, double yv) {
+      FwdRow<N> o;
+      fwd_row<N, false>(md, W, r == 0, yv, m, C, an, Rn, o, st, false, sacc, shave);
+      if (r == 0) return;
+      if (TR) tr += mvn.eval(o.m, o.a);
+      if (!isnan(yv)) {
+        const double sd = sqrt(o.Q);
+        const double dd = (yv - o.f) / sd;
+        li += -dd * dd / 2.0 - log(sqrt(2.0 * 3.141592653589793) * sd);
+      }
+    };
+    int64_t r = r0;
+    if (VEC) {
+      YGroup<true> yg;
+      yg.start(y, r0, 1);
+      for (; r + kGrp <= r1; r += kGrp) {
+        double yv[kGrp];
+        yg.load(y, r, T, 1, yv);
+#pragma unroll
+        for (int i = 0; i < kGrp; ++i) row(r + i, yv[i]);
+      }
+    }
+    for (; r < r1; ++r) row(r, r > 0 ? y[r - 1] : 0.0);
+    if (r1 == rows) {  // this thread owns row T: its state is the final filtered state
+#pragma unroll
+      for (int k = 0; k < N; ++k) last[k] = m[k];
+#pragma unroll
+      for (int k = 0; k < N * N; ++k) last[N + k] = C[k];
+    }
+  }
+  s_tr[tid] = tr; s_in[tid] = li; s_st[tid] = st;
+  __syncthreads();
+#pragma unroll
+  for (int off = kLlBlock / 2; off > 0; off >>= 1) {
+    if (tid < off) {
+      s_tr[tid] = s_tr[tid] + s_tr[tid + off];
+      s_in[tid] = s_in[tid] + s_in[tid + off];
+      s_st[tid] |= s_st[tid + off];
+    }
+    __syncthreads();
+  }
+  if (tid == 0) part[blockIdx.x] = LoglikPart{s_tr[0], s_in[0], s_st[0]};
+}
+
+// One block: thread i sums parts i, i + kLlFinish, ... in order, then the same fixed-order tree.
+// Status as the sequential kernel: the bits the sweep raised, plus BDLM_ST_NONFINITE when the final
+// filtered mean is not finite (C is not checked).
+__global__ void __launch_bounds__(kLlFinish)
+loglik_finish_kernel(const LoglikPart *part, int64_t nparts, const double *last, int n, double *transition,
+                     double *innovations, double *m_last, double *C_last, int32_t *status) {
+  __shared__ double s_tr[kLlFinish], s_in[kLlFinish];
+  __shared__ int s_st[kLlFinish];
+  const int tid = threadIdx.x;
+  double tr = 0.0, li = 0.0;
+  int st = 0;
+  for (int64_t i = tid; i < nparts; i += kLlFinish) {
+    tr = tr + part[i].tr;
+    li = li + part[i].in;
+    st |= part[i].st;
+  }
+  s_tr[tid] = tr; s_in[tid] = li; s_st[tid] = st;
+  __syncthreads();
+#pragma unroll
+  for (int off = kLlFinish / 2; off > 0; off >>= 1) {
+    if (tid < off) {
+      s_tr[tid] = s_tr[tid] + s_tr[tid + off];
+      s_in[tid] = s_in[tid] + s_in[tid + off];
+      s_st[tid] |= s_st[tid + off];
+    }
+    __syncthreads();
+  }
+  if (tid != 0) return;
+  if (transition) *transition = s_tr[0];
+  if (innovations) *innovations = s_in[0];
+  bool finite = true;
+  for (int k = 0; k < n; ++k) {
+    finite = finite && isfinite(last[k]);
+    if (m_last) m_last[k] = last[k];
+  }
+  if (C_last)
+    for (int k = 0; k < n * n; ++k) C_last[k] = last[n + k];
+  if (status) *status = s_st[0] | (finite ? 0 : BDLM_ST_NONFINITE);
 }
 
 // ---- apply, backward: sequential (textbook) RTS recursion from the scanned successor state
@@ -1037,6 +1185,36 @@ static bool dense_aligned(const View &v, int64_t K) {
   return !v.ptr || (v.sk == 1 && v.sr == K && (reinterpret_cast<uintptr_t>(v.ptr) & 31) == 0);
 }
 
+// The model's level-1 table, rebuilt on the host and uploaded when the model changed since the
+// context last built it.
+template <int N>
+cudaError_t fwd_table_upload(const ScanArgs &a, const ScanModel<N> &md, cudaStream_t stream) {
+  if (!a.table_upload) return cudaSuccess;
+  static_assert(sizeof(FwdTable<N>) <= kScanTableBytes, "table buffer too small");
+  FwdTable<N> host;
+  build_fwd_table<N>(md, host);
+  // pageable source: staged by the driver before the call returns
+  return cudaMemcpyAsync(a.table, &host, sizeof(host), cudaMemcpyHostToDevice, stream);
+}
+
+// Level 1 + level 2 of the forward pass: X[0, M] = inclusive prefixes of (slot 0, aggregates) with
+// the top level's block prefixes left in scratch (defer_top).  identity: slot 0 is the identity
+// (chunk aggregate only), else the state st0 before the first observation.
+template <int N>
+cudaError_t fwd_prefixes(const ScanArgs &a, const ScanModel<N> &md, int64_t M, FElem<N> *X,
+                         FElem<N> *scratch, const StateArg<N> &st0, bool identity, int sub,
+                         cudaStream_t stream, int64_t *launches) {
+  const FwdTable<N> *tb = reinterpret_cast<const FwdTable<N> *>(a.table);
+  const unsigned blocks = (unsigned)((M + 127) / 128);
+  if ((reinterpret_cast<uintptr_t>(a.y) & 31) == 0)
+    fwd_reduce_kernel<N, true><<<blocks, 128, 0, stream>>>(md, tb, a.y, a.T, M, a.keep_init, X, st0, identity, sub);
+  else
+    fwd_reduce_kernel<N, false><<<blocks, 128, 0, stream>>>(md, tb, a.y, a.T, M, a.keep_init, X, st0, identity, sub);
+  ++*launches;
+  CK(cudaGetLastError());
+  return device_scan<FElem<N>, false, false>(X, M + 1, scratch, stream, launches, /*defer_top=*/true);
+}
+
 template <int N>
 cudaError_t scan_forward(const ScanArgs &a, cudaStream_t stream, int64_t *launches) {
   const ScanModel<N> md = make_model<N>(a);
@@ -1046,27 +1224,14 @@ cudaError_t scan_forward(const ScanArgs &a, cudaStream_t stream, int64_t *launch
   FElem<N> *scratch = X + (M + 1);                                // block totals
   const unsigned blocks = (unsigned)((M + 127) / 128);
   const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);  // level-2 blocks over X
-  FwdTable<N> *tb = reinterpret_cast<FwdTable<N> *>(a.table);
-  if (a.table_upload) {  // model changed since the context last built it
-    static_assert(sizeof(FwdTable<N>) <= kScanTableBytes, "table buffer too small");
-    FwdTable<N> host;
-    build_fwd_table<N>(md, host);
-    // pageable source: staged by the driver before the call returns
-    CK(cudaMemcpyAsync(tb, &host, sizeof(host), cudaMemcpyHostToDevice, stream));
-  }
+  CK(fwd_table_upload<N>(a, md, stream));
   const bool local = a.phase == kScanDistLocal, finish = a.phase == kScanDistFinish;
   FElem<N> *carry = reinterpret_cast<FElem<N> *>(scratch + (M + 1) / kScanBlock * 2 + 8);
   if (!finish) {
     // dist local: chunk aggregate only (identity start); apply: prefix of
     // (start (x) aggregates), a.start = host (m, C) of the state before t = 0
     const StateArg<N> st0 = state_arg<N>(local ? nullptr : a.start);
-    if ((reinterpret_cast<uintptr_t>(a.y) & 31) == 0)
-      fwd_reduce_kernel<N, true><<<blocks, 128, 0, stream>>>(md, tb, a.y, T, M, a.keep_init, X, st0, local, sub);
-    else
-      fwd_reduce_kernel<N, false><<<blocks, 128, 0, stream>>>(md, tb, a.y, T, M, a.keep_init, X, st0, local, sub);
-    ++*launches;
-    CK(cudaGetLastError());
-    CK((device_scan<FElem<N>, false, false>(X, M + 1, scratch, stream, launches, /*defer_top=*/true)));
+    CK(fwd_prefixes<N>(a, md, M, X, scratch, st0, local, sub, stream, launches));
     // the whole chunk: last element of a one-block scan, else the last scanned block total
     const FElem<N> *whole = nb > 1 ? scratch + (nb - 1) : X + M;
     if (local) {
@@ -1103,6 +1268,39 @@ cudaError_t scan_forward(const ScanArgs &a, cudaStream_t stream, int64_t *launch
   else if (sagg) BDLM_FWD_APPLY(false, true);
   else BDLM_FWD_APPLY(false, false);
 #undef BDLM_FWD_APPLY
+  ++*launches;
+  return cudaGetLastError();
+}
+
+// Log-likelihoods + last filtered state of the whole series (keep_init = 1): reduce, level-2 scan,
+// the store-free sweep and the fixed-order sum of its block partials.
+template <int N>
+cudaError_t scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream, int64_t *launches) {
+  if (a.keep_init != 1 || a.phase != kScanApply) return cudaErrorInvalidValue;
+  const ScanModel<N> md = make_model<N>(a);
+  const int sub = scan_rows_per_thread(a.n, a.T);
+  const int64_t T = a.T, M = (T + 1 + sub - 1) / sub;
+  FElem<N> *X = reinterpret_cast<FElem<N> *>(a.workspace);
+  FElem<N> *scratch = X + (M + 1);
+  const unsigned blocks = (unsigned)((M + kLlBlock - 1) / kLlBlock);
+  const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);
+  LoglikPart *part = reinterpret_cast<LoglikPart *>(o.parts);
+  double *last = reinterpret_cast<double *>(part + blocks);
+  CK(fwd_table_upload<N>(a, md, stream));
+  CK(fwd_prefixes<N>(a, md, M, X, scratch, state_arg<N>(a.start), false, sub, stream, launches));
+  const FElem<N> *tot = nb > 1 ? scratch : nullptr;
+  const bool vec = (reinterpret_cast<uintptr_t>(a.y) & 31) == 0, tr = o.transition != nullptr;
+#define BDLM_LL_SWEEP(VEC_, TR_) \
+  fwd_loglik_kernel<N, VEC_, TR_><<<blocks, kLlBlock, 0, stream>>>(md, a.y, T, M, X, tot, sub, part, last)
+  if (vec && tr) BDLM_LL_SWEEP(true, true);
+  else if (vec) BDLM_LL_SWEEP(true, false);
+  else if (tr) BDLM_LL_SWEEP(false, true);
+  else BDLM_LL_SWEEP(false, false);
+#undef BDLM_LL_SWEEP
+  ++*launches;
+  CK(cudaGetLastError());
+  loglik_finish_kernel<<<1, kLlFinish, 0, stream>>>(part, blocks, last, N, o.transition, o.innovations,
+                                                     o.m_last, o.C_last, o.status);
   ++*launches;
   return cudaGetLastError();
 }
@@ -1191,6 +1389,23 @@ cudaError_t launch_scan(const ScanArgs &a, cudaStream_t stream, int64_t *launche
     BDLM_SCAN_CASE(3)
     BDLM_SCAN_CASE(4)
 #undef BDLM_SCAN_CASE
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+size_t scan_loglik_bytes(int n, int64_t T) {
+  const int sub = scan_rows_per_thread(n, T);
+  const int64_t M = (T + 1 + sub - 1) / sub, blocks = (M + kLlBlock - 1) / kLlBlock;
+  return sizeof(LoglikPart) * (size_t)blocks + sizeof(double) * (size_t)(n + n * n) + 256;
+}
+
+cudaError_t launch_scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream,
+                               int64_t *launches) {
+  switch (a.n) {
+    case 1: return scan_loglik<1>(a, o, stream, launches);
+    case 2: return scan_loglik<2>(a, o, stream, launches);
+    case 3: return scan_loglik<3>(a, o, stream, launches);
+    case 4: return scan_loglik<4>(a, o, stream, launches);
     default: return cudaErrorInvalidValue;
   }
 }

@@ -2,7 +2,8 @@
 
 Not in the reference (strictly sequential recursion, Filter.scala:41-62); temporal
 parallelisation by associative scan (Sarkka & Garcia-Fernandez 2021), kernels in csrc/scan.cu.
-``scan_filter_smooth`` is the single-GPU call; ``DistScan`` runs one rank's time chunk of a
+``scan_filter_smooth`` is the single-GPU call, ``scan_loglik`` the log-likelihoods and last
+filtered state by the forward pass alone; ``DistScan`` runs one rank's time chunk of a
 sharded series with the device-side phases (one all-gather of a 3n^2+2n-double aggregate per rank
 for the filter, 2n^2+n for the smoother).
 """
@@ -56,6 +57,31 @@ def scan_filter_smooth(eng: Engine, model: Model, params: Dict, y, *, keep_init=
     out, ko, so = _outputs(y, model.T + int(keep_init), model.n, want)
     st = torch.zeros((1,), dtype=torch.int32, device=y.device)
     eng.ctx.check(capi.load().bdlm_scan_filter_smooth(eng.ctx.handle, pr, ko, so, st.data_ptr()))
+    out["status"] = st
+    return out
+
+
+def scan_loglik(eng: Engine, model: Model, params: Dict, y, *, transition=True, innovations=True,
+                last=False):
+    """Both log-likelihoods (as ``Engine.loglik``) and, with ``last``, the final filtered state
+    (as ``Engine.filter_last``) of ONE long series by the scan's forward pass (bdlm_scan_loglik).
+    y: CUDA tensor [T] (or [T, 1]).  Returns [1] / [n] / [n*n] device tensors + int32 status [1]."""
+    import torch
+    with bound_engine(eng):
+        pr, keep = _problem(model, params, y, True)
+    n = model.n
+    z = lambda k: torch.empty((k,), dtype=torch.float64, device=y.device)  # noqa: E731
+    out = {}
+    if transition:
+        out["transition"] = z(1)
+    if innovations:
+        out["innovations"] = z(1)
+    if last:
+        out["m"], out["C"] = z(n), z(n * n)
+    ptr = lambda k: out[k].data_ptr() if k in out else None  # noqa: E731
+    st = torch.zeros((1,), dtype=torch.int32, device=y.device)
+    eng.ctx.check(capi.load().bdlm_scan_loglik(eng.ctx.handle, pr, ptr("m"), ptr("C"), ptr("transition"),
+                                               ptr("innovations"), st.data_ptr()))
     out["status"] = st
     return out
 

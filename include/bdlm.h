@@ -93,13 +93,18 @@ enum {
   BDLM_TEXTBOOK_SMOOTHER = 1, /* S = C - B (R-S) B^T instead of Smoothing.scala:44's ... B */
   BDLM_SVD_CONSISTENT_W = 2,  /* SVD time update stacks W^{1/2} sqrt(dt) (DlmFsv.scala:213-217)
                                  instead of the raw W the filterDlm/ffbsDlm/Gibbs closures hold */
-  BDLM_PARALLEL_IN_TIME = 4   /* bdlm_kf_filter_smooth may run ONE long series (B = 1, T >= 4096,
-                                 p = 1, n <= 4, regular grid, time-invariant model, shared
-                                 parameters; n = 1 or BDLM_TEXTBOOK_SMOOTHER) through the
-                                 associative-scan kernels: T dependent steps of ~0.3 us each become a
-                                 few hundred microseconds, at 1e-9 relative instead of bit-for-bit
-                                 agreement with the sequential recursion -- hence opt-in.  Ignored
-                                 (sequential kernel) when the problem is not eligible. */
+  BDLM_PARALLEL_IN_TIME = 4   /* ONE long series may run through the associative-scan kernels
+                                 instead of T dependent steps of ~0.3 us each, at 1e-9 relative
+                                 instead of bit-for-bit agreement with the sequential recursion --
+                                 hence opt-in.  Eligible: B = 1, T >= 4096, p = 1, n <= 4, regular
+                                 grid, time-invariant model (no f_tv, g_tv, v_tv, w_tv), shared
+                                 parameters, device or host buffers; then
+                                   bdlm_kf_filter_smooth  runs bdlm_scan_filter_smooth when also
+                                                          n = 1 or BDLM_TEXTBOOK_SMOOTHER;
+                                   bdlm_loglik,
+                                   bdlm_kf_filter_last    run bdlm_scan_loglik (any n <= 4).
+                                 Ignored (sequential kernel, bit for bit) when the problem is not
+                                 eligible. */
 };
 
 /* which params are per series (bit mask for bdlm_problem.per_series) */
@@ -319,6 +324,15 @@ BDLM_API int bdlm_gibbs_suffstats(bdlm_ctx *ctx, const bdlm_problem *prob, const
 BDLM_API int bdlm_scan_filter_smooth(bdlm_ctx *ctx, const bdlm_problem *prob,
                                      const bdlm_kf_out *kf, const bdlm_smooth_out *sm,
                                      int32_t *status);
+/* Log-likelihoods and last filtered state of ONE long series by the scan's forward pass alone:
+ * arguments as bdlm_kf_filter_last (any output may be NULL, not all; status int32[1]), same
+ * restrictions as bdlm_scan_filter_smooth, any T >= 1, keep_init ignored (the state (m0, C0) sits
+ * before the first observation, as in bdlm_loglik).  Nothing is stored per time step; the sums are
+ * reduced in a fixed order (same bits on every call) and agree with bdlm_loglik to 1e-9 of
+ * sum_t |term_t|.  Enqueue-only: no host synchronisation. */
+BDLM_API int bdlm_scan_loglik(bdlm_ctx *ctx, const bdlm_problem *prob, double *m_last,
+                              double *C_last, double *transition, double *innovations,
+                              int32_t *status);
 BDLM_API int bdlm_scan_elem_doubles(int32_t n, int32_t backward);
 BDLM_API int bdlm_scan_dist_forward_local(bdlm_ctx *ctx, const bdlm_problem *prob, int32_t rank,
                                           int32_t world, double *agg_dev);
