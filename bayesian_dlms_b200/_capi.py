@@ -30,7 +30,7 @@ SYMBOLS = [
     "bdlm_rts_smooth", "bdlm_kf_filter_smooth", "bdlm_loglik", "bdlm_kf_filter_last", "bdlm_ffbs",
     "bdlm_svd_filter", "bdlm_svd_ffbs", "bdlm_gibbs_suffstats", "bdlm_wave_series",
     "bdlm_fp64_peak_tflops", "bdlm_scan_filter_smooth", "bdlm_scan_loglik", "bdlm_scan_elem_doubles",
-    "bdlm_scan_combine",
+    "bdlm_scan_combine", "bdlm_scan_ffbs",
     "bdlm_scan_dist_forward_local", "bdlm_scan_dist_forward_finish",
     "bdlm_scan_dist_backward_local", "bdlm_scan_dist_backward_finish",
     "bdlm_ar_filter", "bdlm_ar_ffbs", "bdlm_conjugate_filter", "bdlm_gibbs_draw",
@@ -145,6 +145,8 @@ def load():
                                             C.POINTER(SmoothOut), C.c_void_p]
     lib.bdlm_scan_loglik.argtypes = [C.c_void_p, PP, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_void_p]
+    lib.bdlm_scan_ffbs.argtypes = [C.c_void_p, PP, C.c_void_p, C.c_void_p, C.POINTER(KfOut),
+                                   C.POINTER(GibbsStats), C.c_void_p]
     lib.bdlm_scan_elem_doubles.argtypes = [C.c_int32, C.c_int32]
     lib.bdlm_scan_combine.argtypes = [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.bdlm_scan_dist_forward_local.argtypes = [C.c_void_p, PP, C.c_int32, C.c_int32, C.c_void_p]

@@ -411,9 +411,12 @@ class Engine:
 
     @_on_engine_stream
     def ffbs(self, model: Model, params: Dict, y, z, *, layout=TIME_MAJOR, want_kf=(),
-             stats=False, status=True, svd=False, consistent_w=False, pinned=False):
+             stats=False, status=True, svd=False, consistent_w=False, pinned=False,
+             parallel_in_time=False):
         """Smoothing.ffbsDlm (Smoothing.scala:173-180) or, with svd=True, SvdSampler.ffbsDlm
-        (SvdSampler.scala:79-82), batched over chains, with injected normals z."""
+        (SvdSampler.scala:79-82), batched over chains, with injected normals z.
+        ``parallel_in_time``: ONE long eligible series may run through the scan's sampler (same
+        normals, path within 1e-9 instead of bit-for-bit; include/bdlm.h BDLM_PARALLEL_IN_TIME)."""
         mem, _ = _mem_and_ptr(y)
         B = self._batch_of(model, y, layout)
         rows = model.T + 1
@@ -422,6 +425,8 @@ class Engine:
             (z.shape, rows, model.n)
         zptr = None if z is None else _mem_and_ptr(z)[1]
         compat = capi.SVD_CONSISTENT_W if (svd and consistent_w) else 0
+        if parallel_in_time and not svd:
+            compat |= capi.PARALLEL_IN_TIME
         pr, keep = self._problem(model, params, y, layout, True, compat, B, mem)
         theta = self._alloc(y, self._shape(layout, B, rows, model.n), pinned=pinned)
         out = dict(theta=theta)

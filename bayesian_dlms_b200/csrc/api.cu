@@ -1173,12 +1173,56 @@ int bdlm_kf_filter_last(bdlm_ctx *c, const bdlm_problem *p, double *m_last, doub
   return dispatch(c, d);
 }
 
+// BDLM_PARALLEL_IN_TIME on bdlm_ffbs: bdlm_scan_ffbs, with host buffers staged through pit_buf
+// ([y | z | theta | m | C | a | R | f | Q | ssy | ny | ssw | scatter | status]).
+static int pit_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *theta,
+                    const bdlm_kf_out *kf, const bdlm_gibbs_stats *stats, int32_t *status) {
+  bdlm_problem q = *p;
+  q.compat &= ~BDLM_PARALLEL_IN_TIME;
+  if (p->mem == BDLM_DEVICE) return bdlm_scan_ffbs(c, &q, z, theta, kf, stats, status);
+  const int64_t n = p->n, R = rows_of(*p);
+  // outputs: theta, kf fields, statistics (rows x k, or k for a statistic)
+  const int64_t ks[11] = {R * n, R * n, R * n * n, R * n, R * n * n, R, R, 1, 1, n, n * n};
+  double *host[11] = {theta,
+                      kf ? kf->m : nullptr, kf ? kf->C : nullptr, kf ? kf->a : nullptr, kf ? kf->R : nullptr,
+                      kf ? kf->f : nullptr, kf ? kf->Q : nullptr,
+                      stats ? stats->ssy : nullptr, stats ? stats->ny : nullptr,
+                      stats ? stats->ssw : nullptr, stats ? stats->scatter : nullptr};
+  size_t pos = align_up(sizeof(double) * (size_t)p->T);
+  const size_t z_off = pos;
+  if (z) pos = align_up(pos + sizeof(double) * (size_t)(R * n));
+  size_t off[12];
+  for (int i = 0; i < 11; ++i) { off[i] = pos; if (host[i]) pos = align_up(pos + sizeof(double) * (size_t)ks[i]); }
+  off[11] = pos; pos += 256;
+  int rc = pit_stage_y(c, p, pos);
+  if (rc) return rc;
+  if (z) CU(cudaMemcpyAsync(c->pit_buf + z_off, z, sizeof(double) * (size_t)(R * n), cudaMemcpyHostToDevice,
+                            c->stream));
+  q.mem = BDLM_DEVICE;
+  q.y = reinterpret_cast<const double *>(c->pit_buf);
+  double *dev[11];
+  for (int i = 0; i < 11; ++i) dev[i] = host[i] ? reinterpret_cast<double *>(c->pit_buf + off[i]) : nullptr;
+  bdlm_kf_out dk = {dev[1], dev[2], dev[3], dev[4], dev[5], dev[6]};
+  bdlm_gibbs_stats ds = {dev[7], dev[8], dev[9], dev[10]};
+  int32_t *dst = status ? reinterpret_cast<int32_t *>(c->pit_buf + off[11]) : nullptr;
+  rc = bdlm_scan_ffbs(c, &q, z ? reinterpret_cast<const double *>(c->pit_buf + z_off) : nullptr, dev[0],
+                      kf ? &dk : nullptr, stats ? &ds : nullptr, dst);
+  if (rc) return rc;
+  for (int i = 0; i < 11; ++i)
+    if (host[i])
+      CU(cudaMemcpyAsync(host[i], dev[i], sizeof(double) * (size_t)ks[i], cudaMemcpyDeviceToHost, c->stream));
+  if (status) CU(cudaMemcpyAsync(status, dst, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return 0;
+}
+
 int bdlm_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *theta,
               const bdlm_kf_out *kf, const bdlm_gibbs_stats *stats, int32_t *status) {
   NvtxRange nvtx_("bdlm_ffbs");
   int rc = validate(c, A_FFBS, p);
   if (rc) return rc;
   if (!theta) return fail(c, BDLM_E_ARG, "null theta");  // z == NULL: on-device Philox normals
+  if (pit_eligible_forward(p) && p->keep_init) return pit_ffbs(c, p, z, theta, kf, stats, status);
   DevCall d{}; d.op = A_FFBS; d.pr = *p; d.z = z; d.theta = theta;
   if (kf) d.kf = *kf;
   if (stats) d.stats = *stats;
@@ -1246,8 +1290,11 @@ static int scan_fill(bdlm_ctx *c, const bdlm_problem *p, ScanArgs &a, bool forwa
 // launch_scan for a forward pass: the table key is committed only once the upload is enqueued, so
 // a failed launch (or a finish phase without its local phase) can never leave a stale table that
 // a later call would trust.
-static int scan_launch_fwd(bdlm_ctx *c, ScanArgs &a, const ScanLoglikOut *ll = nullptr) {
-  CU(ll ? launch_scan_loglik(a, *ll, c->stream, &c->launches) : launch_scan(a, c->stream, &c->launches));
+static int scan_launch_fwd(bdlm_ctx *c, ScanArgs &a, const ScanLoglikOut *ll = nullptr,
+                           const ScanFfbsOut *fb = nullptr) {
+  CU(ll   ? launch_scan_loglik(a, *ll, c->stream, &c->launches)
+     : fb ? launch_scan_ffbs(a, *fb, c->stream, &c->launches)
+          : launch_scan(a, c->stream, &c->launches));
   if (a.table_upload) c->scan_key.swap(c->scan_key_pending);
   c->scan_key_pending.clear();
   return 0;
@@ -1341,6 +1388,53 @@ int bdlm_scan_loglik(bdlm_ctx *c, const bdlm_problem *p, double *m_last, double 
   a.phase = kScanApply; a.start = prior.data(); a.workspace = c->arena;
   const ScanLoglikOut o{transition, innovations, m_last, C_last, status, c->arena + ws};
   return scan_launch_fwd(c, a, &o);
+}
+
+int bdlm_scan_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *theta,
+                   const bdlm_kf_out *kf, const bdlm_gibbs_stats *stats, int32_t *status) {
+  NvtxRange nvtx_("bdlm_scan_ffbs");
+  int rc = scan_validate(c, p);
+  if (rc) return rc;
+  if (p->v_tv || p->w_tv) return fail(c, BDLM_E_ARG, "scan path: time-invariant model (v_tv = w_tv = 0)");
+  if (!p->keep_init) return fail(c, BDLM_E_ARG, "scan FFBS: keep_init = 1");
+  if (!theta) return fail(c, BDLM_E_ARG, "null theta");  // z == NULL: on-device Philox normals
+  CU(cudaSetDevice(c->device));
+  const int64_t n = p->n, R = rows_of(*p);
+  bdlm_kf_out k{};
+  if (kf) k = *kf;
+  // arena: [forward scan workspace | sampler scan workspace | statistics partials | (m, C) spill
+  // when not wanted]
+  const size_t ws = align_up(scan_workspace_bytes(p->n, p->T) + 4096);
+  const size_t parts = align_up(scan_ffbs_parts_bytes(p->n, p->T));
+  const size_t need = 2 * ws + parts + (k.m ? 0 : align_up(sizeof(double) * R * n)) +
+                      (k.C ? 0 : align_up(sizeof(double) * R * n * n)) + 4096;
+  rc = ensure_arena(c, need);
+  if (rc) return rc;
+  Bump bump{c->arena, 2 * ws + parts, c->arena_bytes};
+  if (!k.m) k.m = bump.take<double>((size_t)R * n);
+  if (!k.C) k.C = bump.take<double>((size_t)R * n * n);
+  std::vector<double> prior((size_t)n + n * n);
+  std::copy(p->m0, p->m0 + n, prior.begin());
+  std::copy(p->C0, p->C0 + n * n, prior.begin() + n);
+  ScanArgs a;
+  rc = scan_fill(c, p, a, true);
+  if (rc) return rc;
+  a.phase = kScanApply; a.start = prior.data(); a.workspace = c->arena;
+  a.kf = scan_kf_views(p, &k); a.status = status;
+  ScanFfbsOut o{};
+  o.z = mk_cview(z, p->layout, 0, 1, R, n);
+  o.theta = mk_view(theta, p->layout, 0, 1, R, n);
+  if (stats) {
+    o.stats.ssy = mk_rowview(stats->ssy, p->layout, 0, 1, 1);
+    o.stats.ny = mk_rowview(stats->ny, p->layout, 0, 1, 1);
+    o.stats.ssw = mk_rowview(stats->ssw, p->layout, 0, 1, n);
+    o.stats.scatter = mk_rowview(stats->scatter, p->layout, 0, 1, n * n);
+  }
+  o.rng_seed = c->rng_seed; o.rng_sweep = c->rng_sweep; o.rng_base = c->rng_first;
+  o.workspace = c->arena + ws;
+  o.parts = reinterpret_cast<double *>(c->arena + 2 * ws);
+  if (status) CU(cudaMemsetAsync(status, 0, sizeof(int32_t), c->stream));
+  return scan_launch_fwd(c, a, nullptr, &o);
 }
 
 // ---- device-side multi-GPU protocol for the scan (no host round trip) --------------------

@@ -17,124 +17,12 @@
 #include "launch.h"
 #include "rng.cuh"
 #include "small_steps.cuh"
-#include "warp_linalg.cuh"  // rr_partner, sym_rot
 
 namespace bdlm {
 
 namespace {
 
 using namespace small;
-
-// eigSym restatement (oracle jacobi_eigsym): one-sided Jacobi on the columns of U = A (lower
-// triangle of Ain read) with V accumulated from I; lam_j = sign(v_j . u_j) |u_j| ascending, Vout
-// columns = sign-normalised eigenvectors.  All indices are compile-time after unrolling.
-template <int N>
-__device__ __forceinline__ int jacobi_eigsym_small(const double (&Ain)[N * N], double (&lam)[N],
-                                                   double (&Vout)[N * N]) {
-  double A[N * N], V[N * N];
-#pragma unroll
-  for (int j = 0; j < N; ++j)
-#pragma unroll
-    for (int i = 0; i < N; ++i) {
-      A[i + j * N] = (i >= j) ? Ain[i + j * N] : Ain[j + i * N];
-      V[i + j * N] = (i == j) ? 1.0 : 0.0;
-    }
-  constexpr int M = (N + 1) & ~1;
-  int st = (N == 1) ? 0 : BDLM_ST_NOTCONVERGED;
-  for (int sweep = 0; sweep < kJacobiMaxSweeps && N > 1; ++sweep) {
-    bool rotated = false;
-#pragma unroll
-    for (int round = 0; round < M - 1; ++round) {
-#pragma unroll
-      for (int p = 0; p < N; ++p) {
-        const int q = rr_partner(N, round, p);
-        if (q < 0 || q < p) continue;   // compile-time after unrolling
-        double alpha = 0.0, beta = 0.0, gamma = 0.0;
-#pragma unroll
-        for (int i = 0; i < N; ++i) {
-          const double up = A[i + p * N], uq = A[i + q * N];
-          const double pp = up * up, qq = uq * uq, pq = up * uq;
-          alpha = (i == 0) ? pp : alpha + pp;
-          beta = (i == 0) ? qq : beta + qq;
-          gamma = (i == 0) ? pq : gamma + pq;
-        }
-        if (gamma * gamma > kJacobiThr2 * (alpha * beta)) {
-          rotated = true;
-          double c, s;
-          sym_rot(alpha, beta, gamma, c, s);
-#pragma unroll
-          for (int i = 0; i < N; ++i) {
-            const double up = A[i + p * N], uq = A[i + q * N];
-            A[i + p * N] = c * up - s * uq;
-            A[i + q * N] = s * up + c * uq;
-            const double vp = V[i + p * N], vq = V[i + q * N];
-            V[i + p * N] = c * vp - s * vq;
-            V[i + q * N] = s * vp + c * vq;
-          }
-        }
-      }
-    }
-    if (!rotated) { st = 0; break; }
-  }
-  double d[N];
-#pragma unroll
-  for (int j = 0; j < N; ++j) {
-    double nn = 0.0, dot = 0.0;
-#pragma unroll
-    for (int i = 0; i < N; ++i) {
-      const double u = A[i + j * N];
-      const double sq = u * u, vu = V[i + j * N] * u;
-      nn = (i == 0) ? sq : nn + sq;
-      dot = (i == 0) ? vu : dot + vu;
-    }
-    const double nrm = sqrt(nn);
-    d[j] = (dot < 0.0) ? -nrm : nrm;
-  }
-  // eigenvalues ascending (stable), sign rule: largest-|component| (first such) positive
-#pragma unroll
-  for (int k = 0; k < N; ++k) {
-    int rank = 0;
-#pragma unroll
-    for (int j = 0; j < N; ++j) rank += ((d[j] < d[k]) || (d[j] == d[k] && j < k)) ? 1 : 0;
-    int im = 0;
-    double best = fabs(V[0 + k * N]);
-#pragma unroll
-    for (int i = 1; i < N; ++i) {
-      const double a = fabs(V[i + k * N]);
-      if (a > best) { best = a; im = i; }
-    }
-    double vim = V[0 + k * N];
-#pragma unroll
-    for (int i = 1; i < N; ++i) vim = (im == i) ? V[i + k * N] : vim;
-    const bool flip = vim < 0.0;
-#pragma unroll
-    for (int r = 0; r < N; ++r)
-      if (rank == r) {
-        lam[r] = d[k];
-#pragma unroll
-        for (int i = 0; i < N; ++i) Vout[i + r * N] = flip ? -V[i + k * N] : V[i + k * N];
-      }
-  }
-  return st;
-}
-
-// MultivariateGaussianSvd(mu, cov).draw with injected normals z (oracle mvn_eig_draw)
-template <int N>
-__device__ __forceinline__ int eig_draw_small(const double (&mu)[N], const double (&cov)[N * N],
-                                              const double (&z)[N], double (&out)[N]) {
-  double lam[N], V[N * N], Mx[N * N], x[N];
-  const int st = jacobi_eigsym_small<N>(cov, lam, V);
-#pragma unroll
-  for (int j = 0; j < N; ++j) {
-    const double sq = sqrt(lam[j]);
-#pragma unroll
-    for (int i = 0; i < N; ++i) Mx[i + j * N] = V[i + j * N] * sq;
-  }
-  smm<N, N, 1, false, false>(Mx, z, x);
-#pragma unroll
-  for (int i = 0; i < N; ++i) out[i] = mu[i] + x[i];
-  return st;
-}
 
 template <int N>
 struct FfbsModel {

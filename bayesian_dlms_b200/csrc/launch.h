@@ -137,6 +137,20 @@ struct ScanLoglikOut {
 size_t scan_loglik_bytes(int n, int64_t T);
 cudaError_t launch_scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream,
                                int64_t *launches);
+// FFBS + Gibbs statistics of one series: a = a forward kScanApply pass with keep_init = 1 whose a.kf
+// has (m, C) (the caller's arrays or workspace) and any of a, R, f, Q; a.status is OR-ed (the caller
+// zeroes it).  Statistics pointers may be null.
+struct ScanFfbsOut {
+  CView z;             // injected normals, rows x n, or ptr == nullptr (Philox)
+  unsigned long long rng_seed, rng_sweep;
+  long long rng_base;
+  View theta;          // rows x n
+  StatViews stats;
+  void *workspace;     // device, scan_workspace_bytes(n, T): the sampler's level-2 elements
+  double *parts;       // device, scan_ffbs_parts_bytes(n, T): block partials of the statistics
+};
+size_t scan_ffbs_parts_bytes(int n, int64_t T);
+cudaError_t launch_scan_ffbs(const ScanArgs &a, const ScanFfbsOut &o, cudaStream_t stream, int64_t *launches);
 void scan_combine_host(int n, bool backward, const double *ei, const double *ej, double *out);
 
 // scalar_filters.cu: scalar AR(1) / OU filter + backward sampler (FilterAr.scala, FilterOu.scala)

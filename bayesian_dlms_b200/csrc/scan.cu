@@ -16,6 +16,8 @@
 //            writing the KfState outputs.  The smoother repeats this backwards with the
 //            elements (E, g, L); its apply phase is the sequential RTS step in textbook mode.
 // Elements are never materialised per time point: HBM traffic is y twice + outputs once.
+// The backward sampler of FFBS (bdlm_scan_ffbs) is a third scan of the same shape, over the affine
+// maps theta_r = B_r theta_{r+1} + c_r, with the Gibbs statistics summed in its apply sweep.
 //
 // Multi-GPU: a rank's chunk aggregate (3n^2+2n doubles forward, 2n^2+n backward) is all
 // that crosses the fabric (one all-gather per pass); the carry is folded on the host.
@@ -28,6 +30,7 @@
 
 #include "common.cuh"
 #include "launch.h"
+#include "rng.cuh"
 #include "small_steps.cuh"
 
 namespace bdlm {
@@ -1010,6 +1013,330 @@ bwd_apply_kernel(const ScanModel<N> md, View fm, View fC, int64_t nrows, int64_t
   if (status && st) atomicOr(status, st);
 }
 
+// ---- backward sampler + Gibbs statistics (bdlm_scan_ffbs) ------------------------------------
+// On the regular grid Smoothing.step's draw (ffbs_small.cu) is affine in the successor draw:
+//   theta_r = B_r theta_{r+1} + c_r,   c_r = m_r - B_r a_{r+1} + M_r z_r    (r < T)
+//   theta_T = m_T + M_T z_T
+// with B_r = C_r G^T R_{r+1}^-1 and M_r = V diag(sqrt(lam)) from jacobi_eigsym_small of the same
+// symmetrised Joseph-form covariance H_r the sequential kernel forms.  The eigen basis is part of
+// the contract: any other square root of H_r is an equally valid draw, but gives another path for
+// the same z.  Elements (B_r, c_r) compose as the (E, g) part of SElem; a type of their own saves
+// SElem's E L E^T (2 n^3 multiply-adds per combine) and a third of the level-2 shared memory.
+template <int N>
+struct BElem {
+  double E[N * N], g[N];
+};
+
+// out = ei (x) ej, ei earlier:  E = E_i E_j ; g = E_i g_j + g_i
+template <int N>
+__host__ __device__ __forceinline__ void b_combine(const BElem<N> &ei, const BElem<N> &ej, BElem<N> &out) {
+  double v[N];
+  smm<N, N, N, false, false>(ei.E, ej.E, out.E);
+  smm<N, N, 1, false, false>(ei.E, ej.g, v);
+#pragma unroll
+  for (int k = 0; k < N; ++k) out.g[k] = v[k] + ei.g[k];
+}
+template <int N>
+struct Op<BElem<N>> {
+  __device__ static void apply(const BElem<N> &earlier, const BElem<N> &later, BElem<N> &o) {
+    b_combine<N>(earlier, later, o);
+  }
+};
+
+// Philox key of the on-device normals (z == NULL), as ffbs_small_kernel's
+struct FfbsRng {
+  unsigned long long seed, sweep;
+  long long base;  // subsequence of the series
+};
+
+// The n normals consumed for theta[row]: injected, or Philox exactly as the sequential kernel
+template <int N>
+__device__ __forceinline__ void ffbs_normals(const CView &z, const FfbsRng &rng, int64_t rows, int64_t row,
+                                             double (&zr)[N]) {
+  if (z.ptr) {
+#pragma unroll
+    for (int k = 0; k < N; ++k) zr[k] = ld_stream(z.ptr + row * z.sr + k * z.sk);
+  } else {
+    const RngKey key{rng.seed, rng.sweep};
+#pragma unroll
+    for (int k = 0; k < N; ++k) zr[k] = philox_normal(key, rng.base, (int)rows, (int)row, N, k);
+  }
+}
+
+// RTS gain of row r from its filtered (m, C): B = C G^T R1^-1 (one inverse, as bwd_step), and a1.
+template <int N>
+__device__ __forceinline__ void ffbs_gain(const ScanModel<N> &md, const double (&W)[N * N], const double (&m)[N],
+                                          const double (&C)[N * N], double (&a1)[N], double (&Bg)[N * N],
+                                          int &st) {
+  double R1[N * N], CGt[N * N], Rinv[N * N];
+  advance<N, true>(md.G, W, 1.0, m, C, a1, R1);
+  smm<N, N, N, false, true>(C, md.G, CGt);
+  st |= small_inverse<N>(R1, Rinv);
+  smm<N, N, N, false, false>(CGt, Rinv, Bg);
+}
+
+// Element (B_r, c_r) of a row with a successor.  H_r = (I - B G) C (I - B G)^T + B W B^T,
+// symmetrised, as Smoothing.step (:93-95) and ffbs_small_kernel form it.
+template <int N>
+__device__ __forceinline__ void ffbs_element(const ScanModel<N> &md, const double (&W)[N * N], const double (&m)[N],
+                                             const double (&C)[N * N], const double (&z)[N], double (&Bg)[N * N],
+                                             double (&cr)[N], int &st) {
+  double a1[N], v[N], g[N], D[N * N], t1[N * N], t2[N * N], Hm[N * N], Hs[N * N];
+  ffbs_gain<N>(md, W, m, C, a1, Bg, st);
+  smm<N, N, 1, false, false>(Bg, a1, v);
+#pragma unroll
+  for (int i = 0; i < N; ++i) g[i] = m[i] - v[i];
+  smm<N, N, N, false, false>(Bg, md.G, D);
+#pragma unroll
+  for (int j = 0; j < N; ++j)
+#pragma unroll
+    for (int i = 0; i < N; ++i) D[i + j * N] = ((i == j) ? 1.0 : 0.0) - D[i + j * N];
+  smm<N, N, N, false, false>(D, C, t1);
+  smm<N, N, N, false, true>(t1, D, Hm);
+  smm<N, N, N, false, false>(Bg, W, t1);
+  smm<N, N, N, false, true>(t1, Bg, t2);
+#pragma unroll
+  for (int k = 0; k < N * N; ++k) Hm[k] = Hm[k] + t2[k];
+#pragma unroll
+  for (int j = 0; j < N; ++j)
+#pragma unroll
+    for (int i = 0; i < N; ++i) Hs[i + j * N] = (Hm[i + j * N] + Hm[j + i * N]) / 2.0;
+  st |= eig_draw_small<N>(g, Hs, z, cr);
+}
+
+// Level 1 of the sampler: thread c owns rows [c*sub, min((c+1)*sub, T)) -- the smoother's row
+// ownership -- and folds their elements in descending order.  c_r goes to theta's own row r as
+// scratch, so the apply sweep reads it back instead of repeating the eigen-decomposition.  The
+// thread that owns row T - 1 also draws theta_T and writes the terminal element (0, theta_T).
+template <int N, bool VEC>
+__global__ void __launch_bounds__(128)
+ffbs_reduce_kernel(const ScanModel<N> md, View fm, View fC, int64_t T, int64_t M, CView z, FfbsRng rng,
+                   View th, BElem<N> *agg /* [M + 1], slot M = terminal */, int32_t *status, int sub) {
+  const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (c >= M) return;
+  const int64_t r0 = c * (int64_t)sub, r1 = (r0 + sub < T) ? r0 + sub : T;
+  double W[N * N];
+#pragma unroll
+  for (int k = 0; k < N * N; ++k) W[k] = md.W[k];
+  int st = 0;
+  if (r1 == T) {  // Smoothing.initialise: theta_T ~ N(m_T, C_T)
+    double m[N], C[N * N], zr[N], tT[N];
+    load_row<N, false>(fm, T, m);
+    load_row<N * N, false>(fC, T, C);
+    ffbs_normals<N>(z, rng, T + 1, T, zr);
+    st |= eig_draw_small<N>(m, C, zr, tT);
+    store_row_scalar<N>(th, T, tT);
+    BElem<N> e;
+#pragma unroll
+    for (int k = 0; k < N * N; ++k) e.E[k] = 0.0;
+#pragma unroll
+    for (int k = 0; k < N; ++k) e.g[k] = tT[k];
+    agg[M] = e;
+  }
+  BElem<N> acc;
+  bool have = false;
+  auto fold = [&](int64_t r, double (&cr)[N]) {
+    double m[N], C[N * N], zr[N];
+    BElem<N> e, o;
+    load_row<N, VEC>(fm, r, m);
+    load_row<N * N, VEC>(fC, r, C);
+    ffbs_normals<N>(z, rng, T + 1, r, zr);
+    ffbs_element<N>(md, W, m, C, zr, e.E, e.g, st);
+#pragma unroll
+    for (int k = 0; k < N; ++k) cr[k] = e.g[k];
+    if (have) { b_combine<N>(e, acc, o); acc = o; }
+    else { acc = e; have = true; }
+  };
+  // Whole-sector group stores for n <= 3 (a row of n = 4 is one sector already): four inlined
+  // eigen-decompositions of n = 4 would spill.
+  constexpr bool kGroupStore = VEC && N <= 3;
+  int64_t r = r1;
+  const int64_t aligned_top = kGroupStore ? r0 + (r1 - r0) / kGrp * kGrp : r1;
+  auto scalar_row = [&](int64_t row) {
+    double cr[N];
+    fold(row, cr);
+    store_row_scalar<N>(th, row, cr);
+  };
+  if constexpr (kGroupStore) {
+    for (; r > aligned_top; --r) scalar_row(r - 1);
+    for (; r - kGrp >= r0; r -= kGrp) {
+      const int64_t g0 = r - kGrp;
+      GroupBuf<N> gc;
+#define BDLM_FFBS_FOLD(I)                               \
+  {                                                     \
+    double cr[N];                                       \
+    fold(g0 + I, cr);                                   \
+    gc.template put<I, false>(th.ptr + g0 * N, cr);     \
+  }
+      BDLM_FFBS_FOLD(3) BDLM_FFBS_FOLD(2) BDLM_FFBS_FOLD(1) BDLM_FFBS_FOLD(0)
+#undef BDLM_FFBS_FOLD
+    }
+  }
+  for (; r > r0; --r) scalar_row(r - 1);
+  agg[c] = acc;
+  if (status && st) atomicOr(status, st);
+}
+
+// Gibbs statistics of one path (ffbs_small_kernel / oracle_gibbs_stats), dt = 1:
+// [ssy, ny, ssw[N], scatter[N*N]]
+template <int N>
+struct FfbsStats {
+  static constexpr int kD = 2 + N + N * N;
+  double v[kD];
+  __device__ __forceinline__ void zero() {
+#pragma unroll
+    for (int k = 0; k < kD; ++k) v[k] = 0.0;
+  }
+  // step t: theta_{t+1} = cur, theta_t = prev, observation y_t
+  __device__ __forceinline__ void add(const ScanModel<N> &md, const double (&cur)[N], const double (&prev)[N],
+                                      double yt) {
+    double ft, gx[N], diff[N];
+    smm<1, N, 1, true, false>(md.F, cur, &ft);
+    if (!isnan(yt)) {
+      v[0] = v[0] + (yt - ft) * (yt - ft);
+      v[1] = v[1] + 1.0;
+    }
+    smm<N, N, 1, false, false>(md.G, prev, gx);
+#pragma unroll
+    for (int i = 0; i < N; ++i) diff[i] = cur[i] - gx[i];
+#pragma unroll
+    for (int i = 0; i < N; ++i) v[2 + i] = v[2 + i] + diff[i] * diff[i];
+#pragma unroll
+    for (int j = 0; j < N; ++j)
+#pragma unroll
+      for (int i = 0; i < N; ++i) v[2 + N + i + j * N] = v[2 + N + i + j * N] + diff[i] * diff[j];
+  }
+};
+constexpr int kFbBlock = 128, kFbFinish = 256;
+
+// Apply: thread c takes its successor theta_{r1} (the scanned suffix composed with the deferred
+// top-level block total, as bwd_apply_kernel) and walks theta_r = B_r theta_{r+1} + c_r down its
+// rows, c_r read back from theta's row r.  STATS: it adds the terms of steps r0 .. r1 - 1 (step t
+// pairs theta_{t+1} with theta_t and y_t, so every step is counted by exactly one thread); the
+// block's sums go through a fixed-order shared-memory tree to one partial per block.
+template <int N, bool VEC, bool STATS>
+__global__ void __launch_bounds__(kFbBlock, 1)
+ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restrict__ y, int64_t T, int64_t M,
+                  const BElem<N> *suf /* [M+1] suffix-inclusive scan, slot M = terminal */,
+                  const BElem<N> *tot /* scanned level-2 block totals (scan order) `suf` still lacks, or nullptr */,
+                  View th, int32_t *status, int sub, double *part /* [kD][gridDim.x] */) {
+  constexpr int kD = FfbsStats<N>::kD;
+  __shared__ double s_part[STATS ? kD * kFbBlock : 1];
+  const int tid = threadIdx.x;
+  const int64_t c = blockIdx.x * (int64_t)blockDim.x + tid;
+  FfbsStats<N> acc;
+  acc.zero();
+  if (c < M) {
+    const int64_t r0 = c * (int64_t)sub, r1 = (r0 + sub < T) ? r0 + sub : T;
+    double W[N * N], t[N];
+    int st = 0;
+    const int64_t blk = (M - (c + 1)) / (kScanBlock * kPer);  // suffix scan: position = M - index
+    if (tot && blk > 0) {
+      BElem<N> o;
+      b_combine<N>(suf[c + 1], tot[blk - 1], o);
+#pragma unroll
+      for (int k = 0; k < N; ++k) t[k] = o.g[k];
+    } else {
+#pragma unroll
+      for (int k = 0; k < N; ++k) t[k] = suf[c + 1].g[k];
+    }
+#pragma unroll
+    for (int k = 0; k < N * N; ++k) W[k] = md.W[k];
+    // theta_r from theta_{r+1} = t and c_r; t becomes theta_r
+    auto step = [&](int64_t r, const double (&cr)[N], double yr) {
+      double m[N], C[N * N], a1[N], Bg[N * N], v[N], nt[N];
+      load_row<N, VEC>(fm, r, m);
+      load_row<N * N, VEC>(fC, r, C);
+      ffbs_gain<N>(md, W, m, C, a1, Bg, st);
+      smm<N, N, 1, false, false>(Bg, t, v);
+#pragma unroll
+      for (int k = 0; k < N; ++k) nt[k] = v[k] + cr[k];
+      if (STATS) acc.add(md, t, nt, yr);
+#pragma unroll
+      for (int k = 0; k < N; ++k) t[k] = nt[k];
+    };
+    int64_t r = r1;
+    const int64_t aligned_top = VEC ? r0 + (r1 - r0) / kGrp * kGrp : r1;
+    auto scalar_row = [&](int64_t row) {
+      double cr[N];
+      load_row<N, false>(th, row, cr);
+      step(row, cr, STATS ? y[row] : 0.0);
+      store_row_scalar<N>(th, row, t);
+    };
+    if (VEC) {
+      for (; r > aligned_top; --r) scalar_row(r - 1);
+      for (; r - kGrp >= r0; r -= kGrp) {
+        const int64_t g0 = r - kGrp;
+        double cg[kGrp * N], yg[kGrp];
+        load_group<N>(th, g0, cg);  // every c of the group before the first store into it
+        if (STATS) ld_v4(y + g0, yg);
+        GroupBuf<N> gt;
+#define BDLM_FFBS_APPLY(I)                                 \
+  {                                                        \
+    double cr[N];                                          \
+    for (int k = 0; k < N; ++k) cr[k] = cg[I * N + k];     \
+    step(g0 + I, cr, STATS ? yg[I] : 0.0);                 \
+    gt.template put<I, false>(th.ptr + g0 * N, t);         \
+  }
+        BDLM_FFBS_APPLY(3) BDLM_FFBS_APPLY(2) BDLM_FFBS_APPLY(1) BDLM_FFBS_APPLY(0)
+#undef BDLM_FFBS_APPLY
+      }
+    }
+    for (; r > r0; --r) scalar_row(r - 1);
+    // t is theta_{r0}; for thread 0 the final state of the sequential sampler, flagged likewise
+    if (c == 0) {
+      bool finite = true;
+#pragma unroll
+      for (int k = 0; k < N; ++k) finite = finite && isfinite(t[k]);
+      if (!finite) st |= BDLM_ST_NONFINITE;
+    }
+    if (status && st) atomicOr(status, st);
+  }
+  if constexpr (STATS) {
+#pragma unroll
+    for (int k = 0; k < kD; ++k) s_part[k * kFbBlock + tid] = acc.v[k];
+    __syncthreads();
+#pragma unroll
+    for (int off = kFbBlock / 2; off > 0; off >>= 1) {
+      if (tid < off) {
+#pragma unroll
+        for (int k = 0; k < kD; ++k)
+          s_part[k * kFbBlock + tid] = s_part[k * kFbBlock + tid] + s_part[k * kFbBlock + tid + off];
+      }
+      __syncthreads();
+    }
+    if (tid < kD) part[(int64_t)tid * gridDim.x + blockIdx.x] = s_part[tid * kFbBlock];
+  }
+}
+
+// One block: thread i sums partials i, i + kFbFinish, ... of each statistic in order, then the
+// same fixed-order tree; no atomics, so a call gives the same bits on any stream or context.
+template <int N>
+__global__ void __launch_bounds__(kFbFinish)
+ffbs_stats_finish_kernel(const double *part, int64_t nparts, StatViews sv) {
+  constexpr int kD = FfbsStats<N>::kD;
+  __shared__ double s[kFbFinish];
+  const int tid = threadIdx.x;
+  for (int k = 0; k < kD; ++k) {
+    double x = 0.0;
+    for (int64_t i = tid; i < nparts; i += kFbFinish) x = x + part[(int64_t)k * nparts + i];
+    s[tid] = x;
+    __syncthreads();
+    for (int off = kFbFinish / 2; off > 0; off >>= 1) {
+      if (tid < off) s[tid] = s[tid] + s[tid + off];
+      __syncthreads();
+    }
+    if (tid == 0) {
+      const double v = s[0];
+      if (k == 0) { if (sv.ssy.ptr) sv.ssy.ptr[0] = v; }
+      else if (k == 1) { if (sv.ny.ptr) sv.ny.ptr[0] = v; }
+      else if (k < 2 + N) { if (sv.ssw.ptr) sv.ssw.ptr[(k - 2) * sv.ssw.sk] = v; }
+      else if (sv.scatter.ptr) sv.scatter.ptr[(k - 2 - N) * sv.scatter.sk] = v;
+    }
+    __syncthreads();
+  }
+}
+
 // terminal slot of a chunk that others follow: the identity, so that the chunk's aggregate leaves
 // them out (the finish phase brings them in through the carry)
 template <int N>
@@ -1305,6 +1632,52 @@ cudaError_t scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t 
   return cudaGetLastError();
 }
 
+// FFBS of the whole series (keep_init = 1): the forward pass writes (m, C) (+ whatever of a, R, f, Q
+// a.kf asks for), then the sampler's level 1, its level-2 suffix scan, the apply sweep and, with
+// statistics, the fixed-order sum of the apply's block partials.
+template <int N>
+cudaError_t scan_ffbs(const ScanArgs &a, const ScanFfbsOut &o, cudaStream_t stream, int64_t *launches) {
+  if (a.keep_init != 1 || a.phase != kScanApply || a.fuse_sagg) return cudaErrorInvalidValue;
+  CK(scan_forward<N>(a, stream, launches));
+  const ScanModel<N> md = make_model<N>(a);
+  const int sub = scan_rows_per_thread(a.n, a.T);
+  const int64_t T = a.T, M = (T + sub - 1) / sub;  // rows 0 .. T-1 have a successor
+  BElem<N> *X = reinterpret_cast<BElem<N> *>(o.workspace);  // [M + 1]
+  BElem<N> *scratch = X + (M + 1);
+  const unsigned blocks = (unsigned)((M + kFbBlock - 1) / kFbBlock);
+  const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);
+  const bool vec = dense_aligned(a.kf.m, N) && dense_aligned(a.kf.C, N * N) && dense_aligned(o.theta, N) &&
+                   (reinterpret_cast<uintptr_t>(a.y) & 31) == 0;
+  const FfbsRng rng{o.rng_seed, o.rng_sweep, o.rng_base};
+  if (vec)
+    ffbs_reduce_kernel<N, true><<<blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, T, M, o.z, rng, o.theta, X,
+                                                                  a.status, sub);
+  else
+    ffbs_reduce_kernel<N, false><<<blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, T, M, o.z, rng, o.theta, X,
+                                                                   a.status, sub);
+  ++*launches;
+  CK(cudaGetLastError());
+  CK((device_scan<BElem<N>, true, true>(X, M + 1, scratch, stream, launches, /*defer_top=*/true)));
+  const BElem<N> *tot = nb > 1 ? scratch : nullptr;
+  const StatViews &sv = o.stats;
+  const bool stats = sv.ssy.ptr || sv.ny.ptr || sv.ssw.ptr || sv.scatter.ptr;
+#define BDLM_FFBS_SWEEP(VEC_, STATS_)                                                                    \
+  ffbs_apply_kernel<N, VEC_, STATS_><<<blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, a.y, T, M, X, tot, \
+                                                                      o.theta, a.status, sub, o.parts)
+  if (vec && stats) BDLM_FFBS_SWEEP(true, true);
+  else if (vec) BDLM_FFBS_SWEEP(true, false);
+  else if (stats) BDLM_FFBS_SWEEP(false, true);
+  else BDLM_FFBS_SWEEP(false, false);
+#undef BDLM_FFBS_SWEEP
+  ++*launches;
+  CK(cudaGetLastError());
+  if (stats) {
+    ffbs_stats_finish_kernel<N><<<1, kFbFinish, 0, stream>>>(o.parts, blocks, sv);
+    ++*launches;
+  }
+  return cudaGetLastError();
+}
+
 template <int N>
 cudaError_t scan_backward(const ScanArgs &a, cudaStream_t stream, int64_t *launches) {
   const ScanModel<N> md = make_model<N>(a);
@@ -1406,6 +1779,22 @@ cudaError_t launch_scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaSt
     case 2: return scan_loglik<2>(a, o, stream, launches);
     case 3: return scan_loglik<3>(a, o, stream, launches);
     case 4: return scan_loglik<4>(a, o, stream, launches);
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+size_t scan_ffbs_parts_bytes(int n, int64_t T) {
+  const int sub = scan_rows_per_thread(n, T);
+  const int64_t M = (T + sub - 1) / sub, blocks = (M + kFbBlock - 1) / kFbBlock;
+  return sizeof(double) * (size_t)(2 + n + n * n) * (size_t)blocks + 256;
+}
+
+cudaError_t launch_scan_ffbs(const ScanArgs &a, const ScanFfbsOut &o, cudaStream_t stream, int64_t *launches) {
+  switch (a.n) {
+    case 1: return scan_ffbs<1>(a, o, stream, launches);
+    case 2: return scan_ffbs<2>(a, o, stream, launches);
+    case 3: return scan_ffbs<3>(a, o, stream, launches);
+    case 4: return scan_ffbs<4>(a, o, stream, launches);
     default: return cudaErrorInvalidValue;
   }
 }

@@ -17,7 +17,7 @@ from .batch import Engine, Model, TIME_MAJOR
 
 def sample(eng: Engine, model: Model, y, prior: Dict, init: Dict, n_iters: int, *, seed: int = 0,
            layout=TIME_MAJOR, svd: bool = False, record: bool = True,
-           z: Optional[object] = None, first_series: int = 0) -> Dict:
+           z: Optional[object] = None, first_series: int = 0, parallel_in_time: bool = False) -> Dict:
     """Run ``n_iters`` Gibbs sweeps for every chain of the batch.
 
     y       CUDA tensor, (T, p, B) time-major or (B, T, p) series-major; NaN = missing
@@ -26,6 +26,12 @@ def sample(eng: Engine, model: Model, y, prior: Dict, init: Dict, n_iters: int, 
     z       optional pre-drawn normals (n_iters, *theta-shape) for bit-exact comparisons;
             default: the FFBS kernels draw their own (Philox keyed by (seed, sweep)), so no
             normals are materialised in HBM at all
+    parallel_in_time
+            ONE long series (B = 1) may draw its path with the scan's sampler (include/bdlm.h
+            BDLM_PARALLEL_IN_TIME; ignored where the problem is not eligible).  The scan builds
+            its model table on the host from shared parameters, so each sweep hands the drawn
+            V and W to the next FFBS as host arrays: p*p + n*n doubles copied back and one host
+            synchronisation per sweep, instead of the device-resident per-series parameters
     Returns dict(V=(iters, p, B) diagonals, W=(iters, n or n*n, B), theta=last path, status=...)
     in time-major orientation regardless of ``layout`` for the recorded chains.
     """
@@ -40,17 +46,23 @@ def sample(eng: Engine, model: Model, y, prior: Dict, init: Dict, n_iters: int, 
     bad = torch.zeros((B,), dtype=torch.int32, device=y.device)
     draw_out = None
     out = None
+    pit = parallel_in_time and B == 1 and not svd
     vdiag = torch.arange(p, device=y.device) * (p + 1)
     wdiag = torch.arange(n, device=y.device) * (n + 1)
     for it in range(n_iters):
         zi = z[it] if z is not None else None
         eng.ctx.set_rng(seed, it, first_series)  # ranks sharding the chains pass their offset
-        out = eng.ffbs(model, params, y, zi, layout=layout, stats=True, status=True, svd=svd)
+        out = eng.ffbs(model, params, y, zi, layout=layout, stats=True, status=True, svd=svd,
+                       parallel_in_time=pit)
         draw_out = eng.gibbs_draw(n, p, T, out, prior, layout=layout, seed=seed, sweep=it,
                                   out=draw_out)
         bad |= out["status"] | draw_out["status"]
-        params = dict(V=draw_out["V"], W=draw_out["W"], m0=init["m0"], C0=init["C0"],
-                      per_series=("V", "W"))
+        if pit:  # shared host parameters: the scan's model table is built from them
+            params = dict(V=draw_out["V"].reshape(p, p).T.cpu().numpy(),
+                          W=draw_out["W"].reshape(n, n).T.cpu().numpy(), m0=init["m0"], C0=init["C0"])
+        else:
+            params = dict(V=draw_out["V"], W=draw_out["W"], m0=init["m0"], C0=init["C0"],
+                          per_series=("V", "W"))
         if record:
             V = draw_out["V"] if layout == TIME_MAJOR else draw_out["V"].t()
             W = draw_out["W"] if layout == TIME_MAJOR else draw_out["W"].t()

@@ -3,7 +3,8 @@
 Not in the reference (strictly sequential recursion, Filter.scala:41-62); temporal
 parallelisation by associative scan (Sarkka & Garcia-Fernandez 2021), kernels in csrc/scan.cu.
 ``scan_filter_smooth`` is the single-GPU call, ``scan_loglik`` the log-likelihoods and last
-filtered state by the forward pass alone; ``DistScan`` runs one rank's time chunk of a
+filtered state by the forward pass alone, ``scan_ffbs`` a backward-sampled path with its Gibbs
+statistics; ``DistScan`` runs one rank's time chunk of a
 sharded series with the device-side phases (one all-gather of a 3n^2+2n-double aggregate per rank
 for the filter, 2n^2+n for the smoother).
 """
@@ -82,6 +83,31 @@ def scan_loglik(eng: Engine, model: Model, params: Dict, y, *, transition=True, 
     st = torch.zeros((1,), dtype=torch.int32, device=y.device)
     eng.ctx.check(capi.load().bdlm_scan_loglik(eng.ctx.handle, pr, ptr("m"), ptr("C"), ptr("transition"),
                                                ptr("innovations"), st.data_ptr()))
+    out["status"] = st
+    return out
+
+
+def scan_ffbs(eng: Engine, model: Model, params: Dict, y, z=None, *, stats=True, want_kf=()):
+    """Smoothing.ffbsDlm of ONE long series by the scan (bdlm_scan_ffbs): the path theta [T+1, n],
+    with ``stats`` the Gibbs statistics ssy [1], ny [1], ssw [n], scatter [n*n] of it, and the
+    filter fields named in ``want_kf`` [T+1, k].  y: CUDA tensor [T] (or [T, 1]); z: CUDA tensor
+    [T+1, n] of injected normals, or None for the Philox normals of ``eng.ctx.set_rng`` (the values
+    the sequential ``Engine.ffbs`` consumes).  Adds the int32 status [1]."""
+    import torch
+    with bound_engine(eng):
+        pr, keep = _problem(model, params, y, True)
+    n, rows = model.n, model.T + 1
+    assert z is None or (tuple(z.shape) == (rows, n) and _mem_and_ptr(z)[0] == capi.DEVICE), z.shape
+    out, ko, _ = _outputs(y, rows, n, want_kf)
+    out["theta"] = torch.empty((rows, n), dtype=torch.float64, device=y.device)
+    gs = capi.GibbsStats()
+    if stats:
+        for k, d in (("ssy", 1), ("ny", 1), ("ssw", n), ("scatter", n * n)):
+            out[k] = torch.empty((d,), dtype=torch.float64, device=y.device)
+            setattr(gs, k, out[k].data_ptr())
+    st = torch.zeros((1,), dtype=torch.int32, device=y.device)
+    eng.ctx.check(capi.load().bdlm_scan_ffbs(eng.ctx.handle, pr, None if z is None else z.data_ptr(),
+                                             out["theta"].data_ptr(), ko, gs if stats else None, st.data_ptr()))
     out["status"] = st
     return out
 

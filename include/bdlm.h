@@ -102,7 +102,11 @@ enum {
                                    bdlm_kf_filter_smooth  runs bdlm_scan_filter_smooth when also
                                                           n = 1 or BDLM_TEXTBOOK_SMOOTHER;
                                    bdlm_loglik,
-                                   bdlm_kf_filter_last    run bdlm_scan_loglik (any n <= 4).
+                                   bdlm_kf_filter_last    run bdlm_scan_loglik (any n <= 4);
+                                   bdlm_ffbs              runs bdlm_scan_ffbs when also
+                                                          keep_init = 1 (any n <= 4; same
+                                                          normals as the sequential kernel for
+                                                          the same z or bdlm_set_rng).
                                  Ignored (sequential kernel, bit for bit) when the problem is not
                                  eligible. */
 };
@@ -333,6 +337,16 @@ BDLM_API int bdlm_scan_filter_smooth(bdlm_ctx *ctx, const bdlm_problem *prob,
 BDLM_API int bdlm_scan_loglik(bdlm_ctx *ctx, const bdlm_problem *prob, double *m_last,
                               double *C_last, double *transition, double *innovations,
                               int32_t *status);
+/* FFBS of ONE long series by the associative scan: forward pass, then the backward sampler as a
+ * scan of the affine maps theta_r = B_r theta_{r+1} + c_r, with the Gibbs statistics of the drawn
+ * path summed in the same sweep.  Arguments as bdlm_ffbs (z NULL = Philox normals of
+ * bdlm_set_rng, the same values the sequential kernel consumes; kf, stats and any of their fields
+ * may be NULL; status int32[1]); same restrictions as bdlm_scan_filter_smooth plus keep_init = 1,
+ * any T >= 1.  Each draw uses the eigen basis of the sequential kernel (same z, same path to 1e-9
+ * of each row's largest entry where H_r's eigenvalues are well separated); the statistics are
+ * reduced in a fixed order (same bits on every call).  Enqueue-only: no host synchronisation. */
+BDLM_API int bdlm_scan_ffbs(bdlm_ctx *ctx, const bdlm_problem *prob, const double *z, double *theta,
+                            const bdlm_kf_out *kf, const bdlm_gibbs_stats *stats, int32_t *status);
 BDLM_API int bdlm_scan_elem_doubles(int32_t n, int32_t backward);
 BDLM_API int bdlm_scan_dist_forward_local(bdlm_ctx *ctx, const bdlm_problem *prob, int32_t rank,
                                           int32_t world, double *agg_dev);
