@@ -32,15 +32,19 @@ SYMBOLS = [
     "bdlm_fp64_peak_tflops", "bdlm_scan_filter_smooth", "bdlm_scan_loglik", "bdlm_scan_elem_doubles",
     "bdlm_scan_combine", "bdlm_scan_ffbs",
     "bdlm_scan_dist_forward_local", "bdlm_scan_dist_forward_finish",
-    "bdlm_scan_dist_backward_local", "bdlm_scan_dist_backward_finish",
+    "bdlm_scan_dist_backward_local", "bdlm_scan_dist_backward_finish", "bdlm_scan_dist_doubles",
+    "bdlm_scan_dist_loglik_partial", "bdlm_scan_dist_loglik_finish", "bdlm_scan_dist_ffbs_local",
+    "bdlm_scan_dist_ffbs_finish", "bdlm_scan_dist_ffbs_stats_finish",
     "bdlm_ar_filter", "bdlm_ar_ffbs", "bdlm_conjugate_filter", "bdlm_gibbs_draw",
     # multi-GPU communicator
     "bdlm_comm_unique_id", "bdlm_comm_create", "bdlm_comm_destroy", "bdlm_comm_last_error",
     "bdlm_comm_size", "bdlm_comm_local_size", "bdlm_comm_ctx", "bdlm_comm_sync",
     "bdlm_comm_uses_peer_exchange", "bdlm_comm_allreduce_sum", "bdlm_comm_allreduce_sum_device",
     "bdlm_comm_kf_filter", "bdlm_comm_svd_filter", "bdlm_comm_kf_filter_smooth", "bdlm_comm_loglik", "bdlm_comm_ffbs", "bdlm_comm_svd_ffbs",
-    "bdlm_comm_scan_filter_smooth",
+    "bdlm_comm_scan_filter_smooth", "bdlm_comm_scan_loglik", "bdlm_comm_scan_ffbs",
 ]
+# bdlm_scan_dist_doubles(n, what)
+SCAN_DIST_SAMPLER_ELEM, SCAN_DIST_LOGLIK_PART, SCAN_DIST_FFBS_PART = 0, 1, 2
 COMM_ID_BYTES = 128
 AR1, OU = 0, 1
 V_SCALAR, V_PER_STEP, V_PER_SERIES_STEP = 0, 1, 2
@@ -156,6 +160,18 @@ def load():
                                                   C.POINTER(KfOut), C.POINTER(SmoothOut), C.c_void_p]
     lib.bdlm_scan_dist_backward_finish.argtypes = [C.c_void_p, PP, C.c_int32, C.c_int32, C.c_void_p,
                                                    C.POINTER(KfOut), C.POINTER(SmoothOut), C.c_void_p]
+    lib.bdlm_scan_dist_doubles.argtypes = [C.c_int32, C.c_int32]
+    lib.bdlm_scan_dist_loglik_partial.argtypes = [C.c_void_p, PP, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                                  C.c_void_p, C.c_void_p]
+    lib.bdlm_scan_dist_loglik_finish.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p]
+    lib.bdlm_scan_dist_ffbs_local.argtypes = [C.c_void_p, PP, C.c_int32, C.c_int32, C.c_int64, C.c_int64,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(KfOut), C.c_void_p,
+                                              C.c_void_p]
+    lib.bdlm_scan_dist_ffbs_finish.argtypes = [C.c_void_p, PP, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                               C.POINTER(KfOut), C.c_void_p, C.c_void_p]
+    lib.bdlm_scan_dist_ffbs_stats_finish.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p,
+                                                     C.POINTER(GibbsStats), C.c_void_p]
     lib.bdlm_ar_filter.argtypes = [C.c_void_p, C.POINTER(ArProblem), C.POINTER(ArOut)]
     lib.bdlm_ar_ffbs.argtypes = [C.c_void_p, C.POINTER(ArProblem), C.c_void_p, C.c_void_p,
                                  C.POINTER(ArOut)]
@@ -189,6 +205,10 @@ def load():
                                        C.POINTER(GibbsStats), C.c_void_p, C.POINTER(GibbsStats)]
     lib.bdlm_comm_scan_filter_smooth.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(KfOut),
                                                  C.POINTER(SmoothOut), C.POINTER(C.c_void_p)]
+    VP = C.POINTER(C.c_void_p)
+    lib.bdlm_comm_scan_loglik.argtypes = [C.c_void_p, PP, VP, VP, VP, VP, VP]
+    lib.bdlm_comm_scan_ffbs.argtypes = [C.c_void_p, PP, C.POINTER(C.c_int64), C.c_int64, VP, VP,
+                                        C.POINTER(KfOut), C.POINTER(GibbsStats), VP]
     _lib = lib
     return lib
 

@@ -230,3 +230,49 @@ class Comm:
         self._ck(capi.load().bdlm_comm_scan_filter_smooth(self._h, h["probs"], h["kfs"], h["sms"],
                                                           h["sts"]))
         return h["outs"]
+
+    def scan_loglik(self, h):
+        """Enqueue the log-likelihoods and last filtered state of the series of ``scan_setup``
+        (``bdlm_comm_scan_loglik``).  Per local device: transition [1], innovations [1], status [1]
+        (the whole series', same bits on every rank) and, on global rank world - 1, m [n] / C [n*n]."""
+        import torch
+        nl = len(self.engines)
+        outs, arrs = [], {k: (C.c_void_p * nl)() for k in ("m", "C", "transition", "innovations", "status")}
+        for i, (kp, model, y) in enumerate(h["keep"]):
+            n = model.n
+            z = lambda k: torch.zeros(k, dtype=torch.float64, device=y.device)  # noqa: E731
+            o = dict(transition=z(1), innovations=z(1), m=z(n), C=z(n * n),
+                     status=torch.zeros(1, dtype=torch.int32, device=y.device))
+            for k in arrs:
+                arrs[k][i] = o[k].data_ptr()
+            outs.append(o)
+        self._ck(capi.load().bdlm_comm_scan_loglik(self._h, h["probs"], arrs["m"], arrs["C"], arrs["transition"],
+                                                   arrs["innovations"], arrs["status"]))
+        return outs
+
+    def scan_ffbs(self, h, first_rows: Sequence[int], total_T: int, z: Optional[Sequence] = None):
+        """Enqueue FFBS + Gibbs statistics of the series of ``scan_setup`` (``bdlm_comm_scan_ffbs``):
+        the filter fields go to ``scan_setup``'s outputs, theta [rows, n] and ssy, ny, ssw, scatter,
+        status (the whole series', same bits on every rank) to the returned per-device dicts.
+        first_rows: global row of each local chunk's first row (``sharding.time_chunk``); z: per
+        local device a CUDA tensor [rows, n] of injected normals, or None for Philox."""
+        import torch
+        nl = len(self.engines)
+        theta, zs, sts = (C.c_void_p * nl)(), (C.c_void_p * nl)(), (C.c_void_p * nl)()
+        gs = (capi.GibbsStats * nl)()
+        outs = []
+        for i, (kp, model, y) in enumerate(h["keep"]):
+            n, rows = model.n, h["outs"][i]["m"].shape[0]
+            o = dict(theta=torch.empty((rows, n), dtype=torch.float64, device=y.device),
+                     status=torch.zeros(1, dtype=torch.int32, device=y.device))
+            for k, d in (("ssy", 1), ("ny", 1), ("ssw", n), ("scatter", n * n)):
+                o[k] = torch.zeros(d, dtype=torch.float64, device=y.device)
+                setattr(gs[i], k, o[k].data_ptr())
+            theta[i], sts[i] = o["theta"].data_ptr(), o["status"].data_ptr()
+            if z is not None:
+                zs[i] = z[i].data_ptr()
+            outs.append(o)
+        fr = (C.c_int64 * nl)(*[int(f) for f in first_rows])
+        self._ck(capi.load().bdlm_comm_scan_ffbs(self._h, h["probs"], fr, int(total_T), None if z is None else zs,
+                                                 theta, h["kfs"], gs, sts))
+        return outs

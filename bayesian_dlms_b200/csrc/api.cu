@@ -1431,6 +1431,7 @@ int bdlm_scan_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *
     o.stats.scatter = mk_rowview(stats->scatter, p->layout, 0, 1, n * n);
   }
   o.rng_seed = c->rng_seed; o.rng_sweep = c->rng_sweep; o.rng_base = c->rng_first;
+  o.total_rows = R; o.first_row = 0;
   o.workspace = c->arena + ws;
   o.parts = reinterpret_cast<double *>(c->arena + 2 * ws);
   if (status) CU(cudaMemsetAsync(status, 0, sizeof(int32_t), c->stream));
@@ -1438,8 +1439,9 @@ int bdlm_scan_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *
 }
 
 // ---- device-side multi-GPU protocol for the scan (no host round trip) --------------------
-// arena: [forward scan workspace | backward scan workspace]; it must survive from the local to
-// the finish phase, so all four calls size it identically.
+// arena: [forward scan workspace | backward (or sampler) scan workspace | sampler block partials |
+// status slot]; it must survive from the local to the finish phase, so every phase sizes it
+// identically.
 
 static int scan_dist_common(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *kf, int rank,
                             int world, size_t *ws_out) {
@@ -1451,7 +1453,7 @@ static int scan_dist_common(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_ou
   if (kf && (!kf->m || !kf->C)) return fail(c, BDLM_E_ARG, "time-sharded scan needs kf->m and kf->C");
   CU(cudaSetDevice(c->device));
   const size_t ws = align_up(scan_workspace_bytes(p->n, p->T) + 4096);
-  rc = ensure_arena(c, 2 * ws + 4096);
+  rc = ensure_arena(c, 2 * ws + align_up(scan_ffbs_parts_bytes(p->n, p->T)) + 256 + 4096);
   if (rc) return rc;
   *ws_out = ws;
   return 0;
@@ -1538,6 +1540,169 @@ int bdlm_scan_dist_backward_finish(bdlm_ctx *c, const bdlm_problem *p, int32_t r
   a.aggs_dev = aggs_dev; a.rank = rank; a.world = world; a.status = status;
   a.workspace = c->arena + ws; a.peers = c->scan_peers; a.epoch_dev = c->scan_epoch;
   CU(launch_scan(a, c->stream, &c->launches));
+  return 0;
+}
+
+// ---- time-sharded log-likelihoods and FFBS ---------------------------------------------------
+// Argument checks that need no device (they run before the context is looked at, so a misuse is
+// reported with its own message even on a null context).
+static int scan_dist_args(bdlm_ctx *c, const bdlm_problem *p, int rank, int world) {
+  if (!p) return fail(c, BDLM_E_ARG, "null problem");
+  if (world < 1 || rank < 0 || rank >= world) return fail(c, BDLM_E_ARG, "bad rank / world");
+  if ((p->keep_init != 0) != (rank == 0))
+    return fail(c, BDLM_E_ARG, "time-sharded scan: keep_init = 1 on rank 0 only");
+  if (p->n < 1 || p->n > 4) return fail(c, BDLM_E_ARG, "scan path: n <= 4");
+  if (p->v_tv || p->w_tv) return fail(c, BDLM_E_ARG, "scan path: time-invariant model (v_tv = w_tv = 0)");
+  return 0;
+}
+
+// The chunk's global rows [first_row, first_row + T + keep_init) within the T_total + 1 of the series.
+static int scan_dist_rows(bdlm_ctx *c, const bdlm_problem *p, int rank, int64_t first_row, int64_t total_T) {
+  if (total_T < 1 || total_T >= INT32_MAX || first_row < 0)
+    return fail(c, BDLM_E_ARG, "time-sharded FFBS: 1 <= total_T < 2^31 - 1 and first_row >= 0");
+  if ((first_row == 0) != (rank == 0)) return fail(c, BDLM_E_ARG, "time-sharded FFBS: first_row = 0 on rank 0 only");
+  if (first_row + p->T + (p->keep_init ? 1 : 0) > total_T + 1)
+    return fail(c, BDLM_E_ARG, "time-sharded FFBS: first_row + rows > total_T + 1");
+  return 0;
+}
+
+static std::vector<double> scan_prior(const bdlm_problem *p) {
+  std::vector<double> prior((size_t)p->n + p->n * p->n);
+  std::copy(p->m0, p->m0 + p->n, prior.begin());
+  std::copy(p->C0, p->C0 + p->n * p->n, prior.begin() + p->n);
+  return prior;
+}
+
+// the status the sampler's phases OR into: the caller's, or the arena's own slot
+static int32_t *scan_dist_status(bdlm_ctx *c, size_t ws, const bdlm_problem *p, int32_t *status) {
+  if (status) return status;
+  return reinterpret_cast<int32_t *>(c->arena + 2 * ws + align_up(scan_ffbs_parts_bytes(p->n, p->T)));
+}
+
+int bdlm_scan_dist_doubles(int32_t n, int32_t what) {
+  if (n < 1 || n > 4) return BDLM_E_ARG;
+  switch (what) {
+    case BDLM_SCAN_DIST_SAMPLER_ELEM: return scan_sampler_elem_doubles(n);
+    case BDLM_SCAN_DIST_LOGLIK_PART: return 3;
+    case BDLM_SCAN_DIST_FFBS_PART: return 2 + n + n * n + 1;
+    default: return BDLM_E_ARG;
+  }
+}
+
+int bdlm_scan_dist_loglik_partial(bdlm_ctx *c, const bdlm_problem *p, int32_t rank, int32_t world,
+                                  const double *aggs_dev, double *m_last, double *C_last, double *part_dev) {
+  NvtxRange nvtx_("bdlm_scan_dist_loglik_partial");
+  int rc = scan_dist_args(c, p, rank, world);
+  if (rc) return rc;
+  size_t ws;
+  rc = scan_dist_common(c, p, nullptr, rank, world, &ws);
+  if (rc) return rc;
+  if (!aggs_dev || !part_dev) return fail(c, BDLM_E_ARG, "null aggregates or partial-vector pointer");
+  const std::vector<double> prior = scan_prior(p);
+  ScanArgs a;
+  rc = scan_fill(c, p, a);
+  if (rc) return rc;
+  a.phase = kScanDistFinish; a.aggs_dev = aggs_dev; a.rank = rank; a.world = world;
+  a.start = prior.data(); a.workspace = c->arena;
+  ScanLoglikOut o{};
+  o.m_last = m_last; o.C_last = C_last; o.parts = c->arena + ws; o.part_vec = part_dev;
+  CU(launch_scan_dist_loglik(a, o, c->stream, &c->launches));
+  return 0;
+}
+
+int bdlm_scan_dist_loglik_finish(bdlm_ctx *c, int32_t world, const double *parts_dev, double *transition,
+                                 double *innovations, int32_t *status) {
+  NvtxRange nvtx_("bdlm_scan_dist_loglik_finish");
+  if (!c) return fail(nullptr, BDLM_E_ARG, "null context");
+  if (world < 1 || !parts_dev) return fail(c, BDLM_E_ARG, "bad world or null partial vectors");
+  if (!transition && !innovations && !status) return fail(c, BDLM_E_ARG, "nothing requested");
+  CU(cudaSetDevice(c->device));
+  CU(launch_scan_dist_loglik_finish(parts_dev, world, transition, innovations, status, c->stream, &c->launches));
+  return 0;
+}
+
+// Arguments of both sampler phases: the forward finish phase's, with (m, C) into kf and no smoother fold.
+static int scan_dist_ffbs_fill(bdlm_ctx *c, const bdlm_problem *p, int rank, int world, const bdlm_kf_out *kf,
+                               double *theta, size_t ws, int32_t *status, const std::vector<double> &prior,
+                               bool forward, ScanArgs &a, ScanFfbsOut &o) {
+  int rc = scan_fill(c, p, a, forward);
+  if (rc) return rc;
+  a.phase = kScanDistFinish; a.rank = rank; a.world = world; a.has_successor = rank < world - 1;
+  a.start = prior.data(); a.kf = scan_kf_views(p, kf); a.status = status; a.workspace = c->arena;
+  const int64_t n = p->n, R = rows_of(*p);
+  o = ScanFfbsOut{};
+  o.theta = mk_view(theta, p->layout, 0, 1, R, n);
+  o.rng_seed = c->rng_seed; o.rng_sweep = c->rng_sweep; o.rng_base = c->rng_first;
+  o.workspace = c->arena + ws;
+  o.parts = reinterpret_cast<double *>(c->arena + 2 * ws);
+  return 0;
+}
+
+int bdlm_scan_dist_ffbs_local(bdlm_ctx *c, const bdlm_problem *p, int32_t rank, int32_t world, int64_t first_row,
+                              int64_t total_T, const double *aggs_dev, const double *z, double *theta,
+                              const bdlm_kf_out *kf, double *agg_dev, int32_t *status) {
+  NvtxRange nvtx_("bdlm_scan_dist_ffbs_local");
+  int rc = scan_dist_args(c, p, rank, world);
+  if (!rc) rc = scan_dist_rows(c, p, rank, first_row, total_T);
+  if (rc) return rc;
+  if (!kf || !kf->m || !kf->C) return fail(c, BDLM_E_ARG, "time-sharded FFBS needs kf->m and kf->C");
+  size_t ws;
+  rc = scan_dist_common(c, p, kf, rank, world, &ws);
+  if (rc) return rc;
+  if (!aggs_dev || !agg_dev || !theta) return fail(c, BDLM_E_ARG, "null aggregate pointer or theta");
+  int32_t *st = scan_dist_status(c, ws, p, status);
+  const std::vector<double> prior = scan_prior(p);
+  ScanArgs a;
+  ScanFfbsOut o;
+  rc = scan_dist_ffbs_fill(c, p, rank, world, kf, theta, ws, st, prior, true, a, o);
+  if (rc) return rc;
+  a.aggs_dev = aggs_dev;
+  o.z = mk_cview(z, p->layout, 0, 1, rows_of(*p), p->n);
+  o.total_rows = total_T + 1; o.first_row = first_row;
+  o.agg_dev = agg_dev;
+  CU(cudaMemsetAsync(st, 0, sizeof(int32_t), c->stream));
+  CU(launch_scan_dist_ffbs(a, o, false, c->stream, &c->launches));
+  if (a.table_upload) c->scan_key.swap(c->scan_key_pending);
+  c->scan_key_pending.clear();
+  return 0;
+}
+
+int bdlm_scan_dist_ffbs_finish(bdlm_ctx *c, const bdlm_problem *p, int32_t rank, int32_t world,
+                               const double *aggs_dev, double *theta, const bdlm_kf_out *kf, double *part_dev,
+                               int32_t *status) {
+  NvtxRange nvtx_("bdlm_scan_dist_ffbs_finish");
+  int rc = scan_dist_args(c, p, rank, world);
+  if (rc) return rc;
+  if (!kf || !kf->m || !kf->C) return fail(c, BDLM_E_ARG, "time-sharded FFBS needs kf->m and kf->C");
+  size_t ws;
+  rc = scan_dist_common(c, p, kf, rank, world, &ws);
+  if (rc) return rc;
+  if (!aggs_dev || !part_dev || !theta) return fail(c, BDLM_E_ARG, "null aggregates, partial vector or theta");
+  int32_t *st = scan_dist_status(c, ws, p, status);
+  const std::vector<double> prior = scan_prior(p);
+  ScanArgs a;
+  ScanFfbsOut o;
+  rc = scan_dist_ffbs_fill(c, p, rank, world, kf, theta, ws, st, prior, false, a, o);  // no table needed
+  if (rc) return rc;
+  o.aggs_dev = aggs_dev; o.part_vec = part_dev;
+  CU(launch_scan_dist_ffbs(a, o, true, c->stream, &c->launches));
+  return 0;
+}
+
+int bdlm_scan_dist_ffbs_stats_finish(bdlm_ctx *c, int32_t n, int32_t world, const double *parts_dev,
+                                     const bdlm_gibbs_stats *stats, int32_t *status) {
+  NvtxRange nvtx_("bdlm_scan_dist_ffbs_stats_finish");
+  if (!c) return fail(nullptr, BDLM_E_ARG, "null context");
+  if (n < 1 || n > 4 || world < 1 || !parts_dev) return fail(c, BDLM_E_ARG, "bad n or world, or null partial vectors");
+  CU(cudaSetDevice(c->device));
+  StatViews sv{};
+  if (stats) {
+    sv.ssy = mk_rowview(stats->ssy, BDLM_SERIES_MAJOR, 0, 1, 1);
+    sv.ny = mk_rowview(stats->ny, BDLM_SERIES_MAJOR, 0, 1, 1);
+    sv.ssw = mk_rowview(stats->ssw, BDLM_SERIES_MAJOR, 0, 1, n);
+    sv.scatter = mk_rowview(stats->scatter, BDLM_SERIES_MAJOR, 0, 1, n * n);
+  }
+  CU(launch_scan_dist_ffbs_stats_finish(n, parts_dev, world, sv, status, c->stream, &c->launches));
   return 0;
 }
 

@@ -100,7 +100,13 @@ struct Local {
   double *agg = nullptr;     // device [2][kMaxElem]: this rank's scan aggregates (fwd, bwd)
   double *aggs = nullptr;    // device [2][world][kMaxElem]: gathered aggregates / peer mailbox
   unsigned long long *flags = nullptr;  // device [2][world] mailbox flags, then [1]: this rank's call counter
+  // device [kXch][kMaxElem] send slots, then [kXch][world][kMaxElem] gathered: the NCCL exchanges of
+  // the time-sharded log-likelihoods and FFBS.  Not agg / aggs: on a mailbox communicator those are
+  // the peers' store targets, and a peer that already runs the next filter + smoother could publish
+  // into a slot this rank's all-gather is still writing.
+  double *xch = nullptr;
 };
+constexpr int kXch = 3;  // exchanges of one call at most (FFBS: forward aggregates, sampler aggregates, partials)
 
 // One persistent host thread per local device: a single thread enqueuing ~20 launches per device
 // is the bottleneck of a multi-GPU call (measured at 8 GPUs: 0.64 ms of host enqueue for 0.2 ms of
@@ -296,6 +302,40 @@ int check_sharded(bdlm_comm *m, const bdlm_problem *p) {
   return 0;
 }
 
+// ---- helpers of the time-sharded log-likelihoods and FFBS (bdlm_comm_scan_loglik / _ffbs)
+
+// Checks every local chunk before any device work: a rank that failed after its peers had entered
+// an all-gather would leave them waiting.
+int check_scan_chunks(bdlm_comm *m, const bdlm_problem *probs, const int64_t *first_row, int64_t total_T) {
+  if (!m) return cfail(nullptr, BDLM_E_ARG, "null communicator");
+  if (!probs) return cfail(m, BDLM_E_ARG, "null problem array");
+  const int n = probs[0].n;
+  if (n < 1 || n > 4) return cfail(m, BDLM_E_ARG, "scan path: n <= 4");
+  for (size_t i = 0; i < m->loc.size(); ++i) {
+    const bdlm_problem &p = probs[i];
+    const int rank = m->loc[i].rank;
+    if (p.n != n) return cfail(m, BDLM_E_ARG, "time-sharded scan: every chunk describes the same model (n differs)");
+    if ((p.keep_init != 0) != (rank == 0)) return cfail(m, BDLM_E_ARG, "time-sharded scan: keep_init = 1 on rank 0 only");
+    if (p.T < 1) return cfail(m, BDLM_E_ARG, "time-sharded scan: every chunk holds at least one observation");
+    if (first_row && ((first_row[i] == 0) != (rank == 0) || first_row[i] < 0 ||
+                      first_row[i] + p.T + p.keep_init > total_T + 1))
+      return cfail(m, BDLM_E_ARG, "time-sharded FFBS: first_row = 0 on rank 0 only, first_row + rows <= total_T + 1");
+  }
+  return 0;
+}
+
+double *xch_send(const Local &L, int k) { return L.xch + (size_t)k * kMaxElem; }
+double *xch_recv(const Local &L, int world, int k) { return L.xch + (size_t)kXch * kMaxElem + (size_t)k * world * kMaxElem; }
+
+template <class P>
+P entry(P const *arr, int i) { return arr ? arr[i] : nullptr; }
+
+// ncclAllGather of `count` doubles from send slot k into the gathered slot k, on the context's stream
+int xch_gather(const Local &L, int world, int k, int count) {
+  return nccl()->AllGather(xch_send(L, k), xch_recv(L, world, k), (size_t)count, kNcclFloat64, L.nc,
+                           ctx_stream(L.ctx)) == 0 ? 0 : BDLM_E_NCCL;
+}
+
 }  // namespace
 
 extern "C" {
@@ -322,6 +362,7 @@ void bdlm_comm_destroy(bdlm_comm *m) {
     if (L.agg) cudaFree(L.agg);
     if (L.aggs) cudaFree(L.aggs);
     if (L.flags) cudaFree(L.flags);
+    if (L.xch) cudaFree(L.xch);
     if (L.ctx) bdlm_destroy(L.ctx);
   }
   delete m;
@@ -360,6 +401,7 @@ int bdlm_comm_create(const int32_t *devices, int32_t n_local, int32_t first_rank
     if (e == cudaSuccess) e = cudaMalloc(&L.aggs, sizeof(double) * 2 * world * kMaxElem);
     if (e == cudaSuccess) e = cudaMalloc(&L.flags, sizeof(unsigned long long) * (2 * world + 1));
     if (e == cudaSuccess) e = cudaMemset(L.flags, 0, sizeof(unsigned long long) * (2 * world + 1));
+    if (e == cudaSuccess) e = cudaMalloc(&L.xch, sizeof(double) * kXch * (world + 1) * kMaxElem);
     if (e != cudaSuccess) return bail(BDLM_E_CUDA, std::string("communicator buffers: ") + cudaGetErrorString(e));
   }
   if (!id) {
@@ -594,6 +636,54 @@ int bdlm_comm_scan_filter_smooth(bdlm_comm *m, const bdlm_problem *probs, const 
     return 0;
   };
   return for_each_local(m, enqueue);
+}
+
+
+// ---- the same long series' log-likelihoods and FFBS, cut along time over the ranks ---------------
+int bdlm_comm_scan_loglik(bdlm_comm *m, const bdlm_problem *probs, double *const *m_last, double *const *C_last,
+                          double *const *transition, double *const *innovations, int32_t *const *status) {
+  int rc = check_scan_chunks(m, probs, nullptr, 0);
+  if (rc) return rc;
+  const int W = m->world, n = probs[0].n;
+  const int ef = bdlm_scan_elem_doubles(n, 0), lp = bdlm_scan_dist_doubles(n, BDLM_SCAN_DIST_LOGLIK_PART);
+  return for_each_local(m, [&](int i) -> int {
+    const Local &L = m->loc[i];
+    if (cudaSetDevice(L.device) != cudaSuccess) return BDLM_E_CUDA;  // worker threads start on device 0
+    int r = bdlm_scan_dist_forward_local(L.ctx, &probs[i], L.rank, W, xch_send(L, 0));
+    if (!r) r = xch_gather(L, W, 0, ef);
+    if (!r) r = bdlm_scan_dist_loglik_partial(L.ctx, &probs[i], L.rank, W, xch_recv(L, W, 0), entry(m_last, i),
+                                              entry(C_last, i), xch_send(L, 1));
+    if (!r) r = xch_gather(L, W, 1, lp);
+    if (!r) r = bdlm_scan_dist_loglik_finish(L.ctx, W, xch_recv(L, W, 1), entry(transition, i),
+                                             entry(innovations, i), entry(status, i));
+    return r;
+  });
+}
+
+int bdlm_comm_scan_ffbs(bdlm_comm *m, const bdlm_problem *probs, const int64_t *first_row, int64_t total_T,
+                        const double *const *z, double *const *theta, const bdlm_kf_out *kfs,
+                        const bdlm_gibbs_stats *stats, int32_t *const *status) {
+  if (m && (!first_row || !theta || !kfs)) return cfail(m, BDLM_E_ARG, "null first_row, theta or kfs array");
+  int rc = check_scan_chunks(m, probs, first_row, total_T);
+  if (rc) return rc;
+  const int W = m->world, n = probs[0].n;
+  const int ef = bdlm_scan_elem_doubles(n, 0), es = bdlm_scan_dist_doubles(n, BDLM_SCAN_DIST_SAMPLER_ELEM);
+  const int fp = bdlm_scan_dist_doubles(n, BDLM_SCAN_DIST_FFBS_PART);
+  return for_each_local(m, [&](int i) -> int {
+    const Local &L = m->loc[i];
+    if (cudaSetDevice(L.device) != cudaSuccess) return BDLM_E_CUDA;
+    int32_t *st = entry(status, i);
+    int r = bdlm_scan_dist_forward_local(L.ctx, &probs[i], L.rank, W, xch_send(L, 0));
+    if (!r) r = xch_gather(L, W, 0, ef);
+    if (!r) r = bdlm_scan_dist_ffbs_local(L.ctx, &probs[i], L.rank, W, first_row[i], total_T, xch_recv(L, W, 0),
+                                          entry(z, i), theta[i], &kfs[i], xch_send(L, 1), st);
+    if (!r) r = xch_gather(L, W, 1, es);
+    if (!r) r = bdlm_scan_dist_ffbs_finish(L.ctx, &probs[i], L.rank, W, xch_recv(L, W, 1), theta[i], &kfs[i],
+                                           xch_send(L, 2), st);
+    if (!r) r = xch_gather(L, W, 2, fp);
+    if (!r) r = bdlm_scan_dist_ffbs_stats_finish(L.ctx, n, W, xch_recv(L, W, 2), stats ? &stats[i] : nullptr, st);
+    return r;
+  });
 }
 
 int bdlm_comm_sync(bdlm_comm *m) {

@@ -133,10 +133,19 @@ struct ScanLoglikOut {
   double *m_last, *C_last;           // [n], [n*n]
   int32_t *status;
   void *parts;                       // device, scan_loglik_bytes(n, T): block partials
+  double *part_vec;                  // time-sharded: the rank's [transition, innovations, status] (out)
 };
 size_t scan_loglik_bytes(int n, int64_t T);
 cudaError_t launch_scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream,
                                int64_t *launches);
+// Time-sharded log-likelihoods, one rank's chunk after the all-gather of the forward aggregates:
+// a = the forward finish phase's arguments (aggs_dev, rank, world, start = the prior, workspace =
+// that of the local phase); o.transition / o.innovations / o.status unused, o.m_last / o.C_last
+// written on rank world - 1.  Then the rank-order sum of the gathered partial vectors [world][3].
+cudaError_t launch_scan_dist_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream,
+                                    int64_t *launches);
+cudaError_t launch_scan_dist_loglik_finish(const double *parts, int world, double *transition, double *innovations,
+                                           int32_t *status, cudaStream_t stream, int64_t *launches);
 // FFBS + Gibbs statistics of one series: a = a forward kScanApply pass with keep_init = 1 whose a.kf
 // has (m, C) (the caller's arrays or workspace) and any of a, R, f, Q; a.status is OR-ed (the caller
 // zeroes it).  Statistics pointers may be null.
@@ -148,9 +157,21 @@ struct ScanFfbsOut {
   StatViews stats;
   void *workspace;     // device, scan_workspace_bytes(n, T): the sampler's level-2 elements
   double *parts;       // device, scan_ffbs_parts_bytes(n, T): block partials of the statistics
+  long long total_rows, first_row;  // Philox offsets: rows of the whole series (T + 1), global row of row 0
+  double *agg_dev;           // time-sharded local: this rank's sampler aggregate (out)
+  const double *aggs_dev;    // time-sharded finish: [world][n*n + n] gathered aggregates
+  double *part_vec;          // time-sharded finish: [ssy, ny, ssw, scatter, status] of the chunk (out)
 };
 size_t scan_ffbs_parts_bytes(int n, int64_t T);
 cudaError_t launch_scan_ffbs(const ScanArgs &a, const ScanFfbsOut &o, cudaStream_t stream, int64_t *launches);
+// Time-sharded FFBS, one rank's chunk: a = the forward finish phase's arguments with a.kf (m, C)
+// required and fuse_sagg = nullptr, has_successor = rank < world - 1.  finish = false: forward finish
+// + the sampler's level 1 and 2, aggregate into o.agg_dev; finish = true: carry, apply, partial vector.
+cudaError_t launch_scan_dist_ffbs(const ScanArgs &a, const ScanFfbsOut &o, bool finish, cudaStream_t stream,
+                                  int64_t *launches);
+cudaError_t launch_scan_dist_ffbs_stats_finish(int n, const double *parts, int world, const StatViews &sv,
+                                               int32_t *status, cudaStream_t stream, int64_t *launches);
+int scan_sampler_elem_doubles(int n);
 void scan_combine_host(int n, bool backward, const double *ei, const double *ej, double *out);
 
 // scalar_filters.cu: scalar AR(1) / OU filter + backward sampler (FilterAr.scala, FilterOu.scala)

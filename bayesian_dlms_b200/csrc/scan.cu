@@ -19,8 +19,9 @@
 // The backward sampler of FFBS (bdlm_scan_ffbs) is a third scan of the same shape, over the affine
 // maps theta_r = B_r theta_{r+1} + c_r, with the Gibbs statistics summed in its apply sweep.
 //
-// Multi-GPU: a rank's chunk aggregate (3n^2+2n doubles forward, 2n^2+n backward) is all
-// that crosses the fabric (one all-gather per pass); the carry is folded on the host.
+// Multi-GPU: a rank's chunk aggregate (3n^2+2n doubles forward, 2n^2+n backward, n^2+n for the
+// sampler) is all that crosses the fabric (one all-gather per pass), plus one all-gather of the
+// rank's partial sums for the log-likelihoods and the Gibbs statistics; the carry is folded on the device.
 //
 // Parity: equals the sequential kernel in textbook-smoother mode to 1e-9 relative (for n = 1
 // that is the reference itself); the apply phases reuse the sequential step code, so the
@@ -778,23 +779,45 @@ struct LoglikPart {
 };
 constexpr int kLlBlock = 128, kLlFinish = 256;
 
-template <int N, bool VEC, bool TR>
+// DIST: one rank's chunk of a time-sharded series (bdlm_scan_dist_loglik_partial).  Its scan ran with
+// an identity start, so every thread composes `carry` (the prior and every earlier chunk, i.e. the
+// filtered state at the end of the previous chunk) in front of its prefix, as fwd_apply_kernel does;
+// keep_init = 0 on every rank but the first, where row r then holds step t = r.
+template <int N, bool VEC, bool TR, bool DIST>
 __global__ void __launch_bounds__(kLlBlock)
 fwd_loglik_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T, int64_t M,
                   const FElem<N> *pre /* [M+1] inclusive scan with slot 0 = the prior */,
                   const FElem<N> *tot /* scanned level-2 block totals `pre` still lacks, or nullptr */,
-                  int sub, LoglikPart *part /* [gridDim.x] */, double *last /* [N + N*N]: (m_T, C_T) */) {
+                  int sub, LoglikPart *part /* [gridDim.x] */, double *last /* [N + N*N]: (m_T, C_T) */,
+                  int keep_init /* DIST */, const FElem<N> *carry /* DIST */) {
   __shared__ double s_tr[kLlBlock], s_in[kLlBlock];
   __shared__ int s_st[kLlBlock];
   const int tid = threadIdx.x;
   const int64_t c = blockIdx.x * (int64_t)blockDim.x + tid;
+  const int ki = DIST ? keep_init : 1;
   double tr = 0.0, li = 0.0;
   int st = 0;
   if (c < M) {
-    const int64_t rows = T + 1;
+    const int64_t rows = T + ki;
     const int64_t r0 = c * (int64_t)sub, r1 = (r0 + sub < rows) ? r0 + sub : rows;
     double m[N], C[N * N], W[N * N], an[N], Rn[N * N];
-    fwd_start_state<N>(pre, c, tot, m, C);
+    if constexpr (DIST) {
+      const int64_t blk = c / (kScanBlock * kPer);
+      FElem<N> o;  // only (b, C) is live
+      if (tot && blk > 0) {
+        FElem<N> left;
+        f_combine<N>(*carry, tot[blk - 1], left);
+        f_combine<N>(left, pre[c], o);
+      } else {
+        f_combine<N>(*carry, pre[c], o);
+      }
+#pragma unroll
+      for (int k = 0; k < N; ++k) m[k] = o.b[k];
+#pragma unroll
+      for (int k = 0; k < N * N; ++k) C[k] = o.C[k];
+    } else {
+      fwd_start_state<N>(pre, c, tot, m, C);
+    }
 #pragma unroll
     for (int k = 0; k < N * N; ++k) W[k] = md.W[k];
     MvnPrepared<N> mvn;  // S = W * 1.0 at every step: factorised once per thread
@@ -807,8 +830,9 @@ fwd_loglik_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T
     bool shave = false;
     auto row = [&](int64_t r, double yv) {
       FwdRow<N> o;
-      fwd_row<N, false>(md, W, r == 0, yv, m, C, an, Rn, o, st, false, sacc, shave);
-      if (r == 0) return;
+      const bool init = ki && r == 0;
+      fwd_row<N, false>(md, W, init, yv, m, C, an, Rn, o, st, false, sacc, shave);
+      if (init) return;
       if (TR) tr += mvn.eval(o.m, o.a);
       if (!isnan(yv)) {
         const double sd = sqrt(o.Q);
@@ -819,15 +843,15 @@ fwd_loglik_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T
     int64_t r = r0;
     if (VEC) {
       YGroup<true> yg;
-      yg.start(y, r0, 1);
+      yg.start(y, r0, ki);
       for (; r + kGrp <= r1; r += kGrp) {
         double yv[kGrp];
-        yg.load(y, r, T, 1, yv);
+        yg.load(y, r, T, ki, yv);
 #pragma unroll
         for (int i = 0; i < kGrp; ++i) row(r + i, yv[i]);
       }
     }
-    for (; r < r1; ++r) row(r, r > 0 ? y[r - 1] : 0.0);
+    for (; r < r1; ++r) row(r, r >= ki ? y[r - ki] : 0.0);
     if (r1 == rows) {  // this thread owns row T: its state is the final filtered state
 #pragma unroll
       for (int k = 0; k < N; ++k) last[k] = m[k];
@@ -851,10 +875,11 @@ fwd_loglik_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T
 
 // One block: thread i sums parts i, i + kLlFinish, ... in order, then the same fixed-order tree.
 // Status as the sequential kernel: the bits the sweep raised, plus BDLM_ST_NONFINITE when the final
-// filtered mean is not finite (C is not checked).
+// filtered mean is not finite (C is not checked).  A chunk of a time-sharded series that does not
+// hold row T passes last = nullptr; st_out receives the status as a double (the rank's partial vector).
 __global__ void __launch_bounds__(kLlFinish)
 loglik_finish_kernel(const LoglikPart *part, int64_t nparts, const double *last, int n, double *transition,
-                     double *innovations, double *m_last, double *C_last, int32_t *status) {
+                     double *innovations, double *m_last, double *C_last, int32_t *status, double *st_out) {
   __shared__ double s_tr[kLlFinish], s_in[kLlFinish];
   __shared__ int s_st[kLlFinish];
   const int tid = threadIdx.x;
@@ -880,13 +905,33 @@ loglik_finish_kernel(const LoglikPart *part, int64_t nparts, const double *last,
   if (transition) *transition = s_tr[0];
   if (innovations) *innovations = s_in[0];
   bool finite = true;
-  for (int k = 0; k < n; ++k) {
-    finite = finite && isfinite(last[k]);
-    if (m_last) m_last[k] = last[k];
+  if (last) {
+    for (int k = 0; k < n; ++k) {
+      finite = finite && isfinite(last[k]);
+      if (m_last) m_last[k] = last[k];
+    }
+    if (C_last)
+      for (int k = 0; k < n * n; ++k) C_last[k] = last[n + k];
   }
-  if (C_last)
-    for (int k = 0; k < n * n; ++k) C_last[k] = last[n + k];
-  if (status) *status = s_st[0] | (finite ? 0 : BDLM_ST_NONFINITE);
+  const int bits = s_st[0] | (finite ? 0 : BDLM_ST_NONFINITE);
+  if (status) *status = bits;
+  if (st_out) *st_out = (double)bits;
+}
+
+// bdlm_scan_dist_loglik_finish: every rank's [transition, innovations, status] partial vector, added
+// in rank order by one thread, so every rank writes the same bits.
+__global__ void dist_loglik_finish_kernel(const double *parts, int world, double *transition,
+                                          double *innovations, int32_t *status) {
+  double tr = 0.0, li = 0.0;
+  int st = 0;
+  for (int r = 0; r < world; ++r) {
+    tr = tr + parts[3 * r];
+    li = li + parts[3 * r + 1];
+    st |= (int)parts[3 * r + 2];
+  }
+  if (transition) *transition = tr;
+  if (innovations) *innovations = li;
+  if (status) *status = st;
 }
 
 // ---- apply, backward: sequential (textbook) RTS recursion from the scanned successor state
@@ -1037,29 +1082,38 @@ __host__ __device__ __forceinline__ void b_combine(const BElem<N> &ei, const BEl
   for (int k = 0; k < N; ++k) out.g[k] = v[k] + ei.g[k];
 }
 template <int N>
+__host__ __device__ __forceinline__ void b_identity(BElem<N> &e) {
+#pragma unroll
+  for (int k = 0; k < N * N; ++k) e.E[k] = (k % (N + 1) == 0) ? 1.0 : 0.0;
+#pragma unroll
+  for (int k = 0; k < N; ++k) e.g[k] = 0.0;
+}
+template <int N>
 struct Op<BElem<N>> {
   __device__ static void apply(const BElem<N> &earlier, const BElem<N> &later, BElem<N> &o) {
     b_combine<N>(earlier, later, o);
   }
 };
 
-// Philox key of the on-device normals (z == NULL), as ffbs_small_kernel's
+// Philox key of the on-device normals (z == NULL), as ffbs_small_kernel's.  The offset depends on the
+// GLOBAL row and row count, so a chunk of a time-sharded series draws the normals the whole series
+// would: local row r is global row first + r of rows.
 struct FfbsRng {
   unsigned long long seed, sweep;
-  long long base;  // subsequence of the series
+  long long base;         // subsequence of the series
+  long long rows, first;  // global row count (T + 1) and global index of the chunk's row 0
 };
 
-// The n normals consumed for theta[row]: injected, or Philox exactly as the sequential kernel
+// The n normals consumed for theta[row] (local row): injected, or Philox exactly as the sequential kernel
 template <int N>
-__device__ __forceinline__ void ffbs_normals(const CView &z, const FfbsRng &rng, int64_t rows, int64_t row,
-                                             double (&zr)[N]) {
+__device__ __forceinline__ void ffbs_normals(const CView &z, const FfbsRng &rng, int64_t row, double (&zr)[N]) {
   if (z.ptr) {
 #pragma unroll
     for (int k = 0; k < N; ++k) zr[k] = ld_stream(z.ptr + row * z.sr + k * z.sk);
   } else {
     const RngKey key{rng.seed, rng.sweep};
 #pragma unroll
-    for (int k = 0; k < N; ++k) zr[k] = philox_normal(key, rng.base, (int)rows, (int)row, N, k);
+    for (int k = 0; k < N; ++k) zr[k] = philox_normal(key, rng.base, (int)rng.rows, (int)(rng.first + row), N, k);
   }
 }
 
@@ -1107,11 +1161,14 @@ __device__ __forceinline__ void ffbs_element(const ScanModel<N> &md, const doubl
 // Level 1 of the sampler: thread c owns rows [c*sub, min((c+1)*sub, T)) -- the smoother's row
 // ownership -- and folds their elements in descending order.  c_r goes to theta's own row r as
 // scratch, so the apply sweep reads it back instead of repeating the eigen-decomposition.  The
-// thread that owns row T - 1 also draws theta_T and writes the terminal element (0, theta_T).
+// thread that owns row T - 1 also draws theta_T and writes the terminal element (0, theta_T) when
+// row T is the series' last (term = T; a chunk of a time-sharded series that others follow passes
+// term = -1 and its caller sets the terminal slot to the identity).
 template <int N, bool VEC>
 __global__ void __launch_bounds__(128)
 ffbs_reduce_kernel(const ScanModel<N> md, View fm, View fC, int64_t T, int64_t M, CView z, FfbsRng rng,
-                   View th, BElem<N> *agg /* [M + 1], slot M = terminal */, int32_t *status, int sub) {
+                   View th, BElem<N> *agg /* [M + 1], slot M = terminal */, int32_t *status, int sub,
+                   int64_t term) {
   const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (c >= M) return;
   const int64_t r0 = c * (int64_t)sub, r1 = (r0 + sub < T) ? r0 + sub : T;
@@ -1119,11 +1176,11 @@ ffbs_reduce_kernel(const ScanModel<N> md, View fm, View fC, int64_t T, int64_t M
 #pragma unroll
   for (int k = 0; k < N * N; ++k) W[k] = md.W[k];
   int st = 0;
-  if (r1 == T) {  // Smoothing.initialise: theta_T ~ N(m_T, C_T)
+  if (r1 == term) {  // Smoothing.initialise: theta_T ~ N(m_T, C_T)
     double m[N], C[N * N], zr[N], tT[N];
     load_row<N, false>(fm, T, m);
     load_row<N * N, false>(fC, T, C);
-    ffbs_normals<N>(z, rng, T + 1, T, zr);
+    ffbs_normals<N>(z, rng, T, zr);
     st |= eig_draw_small<N>(m, C, zr, tT);
     store_row_scalar<N>(th, T, tT);
     BElem<N> e;
@@ -1140,7 +1197,7 @@ ffbs_reduce_kernel(const ScanModel<N> md, View fm, View fC, int64_t T, int64_t M
     BElem<N> e, o;
     load_row<N, VEC>(fm, r, m);
     load_row<N * N, VEC>(fC, r, C);
-    ffbs_normals<N>(z, rng, T + 1, r, zr);
+    ffbs_normals<N>(z, rng, r, zr);
     ffbs_element<N>(md, W, m, C, zr, e.E, e.g, st);
 #pragma unroll
     for (int k = 0; k < N; ++k) cr[k] = e.g[k];
@@ -1187,15 +1244,18 @@ struct FfbsStats {
 #pragma unroll
     for (int k = 0; k < kD; ++k) v[k] = 0.0;
   }
-  // step t: theta_{t+1} = cur, theta_t = prev, observation y_t
-  __device__ __forceinline__ void add(const ScanModel<N> &md, const double (&cur)[N], const double (&prev)[N],
-                                      double yt) {
-    double ft, gx[N], diff[N];
+  // step t: theta_{t+1} = cur, theta_t = prev, observation y_t.  The observation term needs theta_{t+1}
+  // alone, the transition term both: a time-sharded chunk counts them on different rows.
+  __device__ __forceinline__ void add_obs(const ScanModel<N> &md, const double (&cur)[N], double yt) {
+    double ft;
     smm<1, N, 1, true, false>(md.F, cur, &ft);
     if (!isnan(yt)) {
       v[0] = v[0] + (yt - ft) * (yt - ft);
       v[1] = v[1] + 1.0;
     }
+  }
+  __device__ __forceinline__ void add_trans(const ScanModel<N> &md, const double (&cur)[N], const double (&prev)[N]) {
+    double gx[N], diff[N];
     smm<N, N, 1, false, false>(md.G, prev, gx);
 #pragma unroll
     for (int i = 0; i < N; ++i) diff[i] = cur[i] - gx[i];
@@ -1210,16 +1270,23 @@ struct FfbsStats {
 constexpr int kFbBlock = 128, kFbFinish = 256;
 
 // Apply: thread c takes its successor theta_{r1} (the scanned suffix composed with the deferred
-// top-level block total, as bwd_apply_kernel) and walks theta_r = B_r theta_{r+1} + c_r down its
-// rows, c_r read back from theta's row r.  STATS: it adds the terms of steps r0 .. r1 - 1 (step t
-// pairs theta_{t+1} with theta_t and y_t, so every step is counted by exactly one thread); the
-// block's sums go through a fixed-order shared-memory tree to one partial per block.
+// top-level block total and, on a chunk of a time-sharded series that others follow, the carry of
+// the later chunks, as bwd_apply_kernel) and walks theta_r = B_r theta_{r+1} + c_r down its rows,
+// c_r read back from theta's row r.  STATS: every row r it produces adds the transition term of the
+// step theta_r -> theta_{r+1} (the last row of a chunk pairs with the carry's theta) and one
+// observation term: with keep_init (the whole series, or rank 0) that of row r + 1, y[r], which
+// belongs to the next chunk when r is the chunk's last row (y[r] does not exist: skipped); without
+// it (ranks > 0) that of row r itself, y[r], plus that of the terminal row on the last chunk.  So
+// every step and every observation is counted once across threads and ranks.  The block's sums go
+// through a fixed-order shared-memory tree to one partial per block.
 template <int N, bool VEC, bool STATS>
 __global__ void __launch_bounds__(kFbBlock, 1)
 ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restrict__ y, int64_t T, int64_t M,
                   const BElem<N> *suf /* [M+1] suffix-inclusive scan, slot M = terminal */,
                   const BElem<N> *tot /* scanned level-2 block totals (scan order) `suf` still lacks, or nullptr */,
-                  View th, int32_t *status, int sub, double *part /* [kD][gridDim.x] */) {
+                  View th, int32_t *status, int sub, double *part /* [kD][gridDim.x] */,
+                  const BElem<N> *carry /* multi-GPU: everything after this chunk, or nullptr */,
+                  int keep_init, int64_t ny /* observations in y */, bool terminal) {
   constexpr int kD = FfbsStats<N>::kD;
   __shared__ double s_part[STATS ? kD * kFbBlock : 1];
   const int tid = threadIdx.x;
@@ -1231,9 +1298,16 @@ ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restr
     double W[N * N], t[N];
     int st = 0;
     const int64_t blk = (M - (c + 1)) / (kScanBlock * kPer);  // suffix scan: position = M - index
-    if (tot && blk > 0) {
+    const bool use_tot = tot && blk > 0;
+    if (carry || use_tot) {
       BElem<N> o;
-      b_combine<N>(suf[c + 1], tot[blk - 1], o);
+      if (carry && use_tot) {
+        BElem<N> mid;
+        b_combine<N>(suf[c + 1], tot[blk - 1], mid);  // later blocks of this chunk
+        b_combine<N>(mid, *carry, o);                  // later chunks
+      } else {
+        b_combine<N>(suf[c + 1], carry ? *carry : tot[blk - 1], o);
+      }
 #pragma unroll
       for (int k = 0; k < N; ++k) t[k] = o.g[k];
     } else {
@@ -1242,6 +1316,7 @@ ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restr
     }
 #pragma unroll
     for (int k = 0; k < N * N; ++k) W[k] = md.W[k];
+    if (STATS && !keep_init && terminal && r1 == T) acc.add_obs(md, t, y[T]);  // t = theta of the terminal row
     // theta_r from theta_{r+1} = t and c_r; t becomes theta_r
     auto step = [&](int64_t r, const double (&cr)[N], double yr) {
       double m[N], C[N * N], a1[N], Bg[N * N], v[N], nt[N];
@@ -1251,16 +1326,22 @@ ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restr
       smm<N, N, 1, false, false>(Bg, t, v);
 #pragma unroll
       for (int k = 0; k < N; ++k) nt[k] = v[k] + cr[k];
-      if (STATS) acc.add(md, t, nt, yr);
+      if (STATS) {
+        if (keep_init) acc.add_obs(md, t, yr);
+        else acc.add_obs(md, nt, yr);
+        acc.add_trans(md, t, nt);
+      }
 #pragma unroll
       for (int k = 0; k < N; ++k) t[k] = nt[k];
     };
     int64_t r = r1;
-    const int64_t aligned_top = VEC ? r0 + (r1 - r0) / kGrp * kGrp : r1;
+    // group loads of y need y[g0 .. g0 + kGrp) to exist: rows at or above ny go the scalar way
+    const int64_t vtop = (STATS && r1 > ny) ? ny : r1;
+    const int64_t aligned_top = VEC ? r0 + (vtop - r0) / kGrp * kGrp : r1;
     auto scalar_row = [&](int64_t row) {
       double cr[N];
       load_row<N, false>(th, row, cr);
-      step(row, cr, STATS ? y[row] : 0.0);
+      step(row, cr, STATS ? (row < ny ? y[row] : __longlong_as_double(0x7ff8000000000000LL)) : 0.0);
       store_row_scalar<N>(th, row, t);
     };
     if (VEC) {
@@ -1283,8 +1364,9 @@ ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restr
       }
     }
     for (; r > r0; --r) scalar_row(r - 1);
-    // t is theta_{r0}; for thread 0 the final state of the sequential sampler, flagged likewise
-    if (c == 0) {
+    // t is theta_{r0}; for thread 0 of the series' first chunk the final state of the sequential
+    // sampler, flagged likewise
+    if (c == 0 && keep_init) {
       bool finite = true;
 #pragma unroll
       for (int k = 0; k < N; ++k) finite = finite && isfinite(t[k]);
@@ -1311,9 +1393,11 @@ ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restr
 
 // One block: thread i sums partials i, i + kFbFinish, ... of each statistic in order, then the
 // same fixed-order tree; no atomics, so a call gives the same bits on any stream or context.
+// vec (a chunk of a time-sharded series): the sums and then the chunk's status bits go to the rank's
+// partial vector [kD + 1] instead of sv.
 template <int N>
 __global__ void __launch_bounds__(kFbFinish)
-ffbs_stats_finish_kernel(const double *part, int64_t nparts, StatViews sv) {
+ffbs_stats_finish_kernel(const double *part, int64_t nparts, StatViews sv, double *vec, const int32_t *status) {
   constexpr int kD = FfbsStats<N>::kD;
   __shared__ double s[kFbFinish];
   const int tid = threadIdx.x;
@@ -1328,13 +1412,33 @@ ffbs_stats_finish_kernel(const double *part, int64_t nparts, StatViews sv) {
     }
     if (tid == 0) {
       const double v = s[0];
-      if (k == 0) { if (sv.ssy.ptr) sv.ssy.ptr[0] = v; }
+      if (vec) vec[k] = v;
+      else if (k == 0) { if (sv.ssy.ptr) sv.ssy.ptr[0] = v; }
       else if (k == 1) { if (sv.ny.ptr) sv.ny.ptr[0] = v; }
       else if (k < 2 + N) { if (sv.ssw.ptr) sv.ssw.ptr[(k - 2) * sv.ssw.sk] = v; }
       else if (sv.scatter.ptr) sv.scatter.ptr[(k - 2 - N) * sv.scatter.sk] = v;
     }
     __syncthreads();
   }
+  if (vec && tid == 0) vec[kD] = status ? (double)*status : 0.0;
+}
+
+// bdlm_scan_dist_ffbs_stats_finish: every rank's partial vector [ssy, ny, ssw, scatter, status],
+// added in rank order by one thread, so every rank writes the same bits.
+template <int N>
+__global__ void dist_ffbs_stats_finish_kernel(const double *parts, int world, StatViews sv, int32_t *status) {
+  constexpr int kD = FfbsStats<N>::kD;
+  int st = 0;
+  for (int r = 0; r < world; ++r) st |= (int)parts[r * (kD + 1) + kD];
+  for (int k = 0; k < kD; ++k) {
+    double v = 0.0;
+    for (int r = 0; r < world; ++r) v = v + parts[r * (kD + 1) + k];
+    if (k == 0) { if (sv.ssy.ptr) sv.ssy.ptr[0] = v; }
+    else if (k == 1) { if (sv.ny.ptr) sv.ny.ptr[0] = v; }
+    else if (k < 2 + N) { if (sv.ssw.ptr) sv.ssw.ptr[(k - 2) * sv.ssw.sk] = v; }
+    else if (sv.scatter.ptr) sv.scatter.ptr[(k - 2 - N) * sv.scatter.sk] = v;
+  }
+  if (status) *status = st;
 }
 
 // terminal slot of a chunk that others follow: the identity, so that the chunk's aggregate leaves
@@ -1343,6 +1447,12 @@ template <int N>
 __global__ void set_s_identity(SElem<N> *slot) {
   SElem<N> e;
   s_identity<N>(e);
+  *slot = e;
+}
+template <int N>
+__global__ void set_b_identity(BElem<N> *slot) {
+  BElem<N> e;
+  b_identity<N>(e);
   *slot = e;
 }
 // last chunk: s_T = m_T, S_T = C_T go to the outputs and become the terminal element of the scan.
@@ -1443,6 +1553,16 @@ __global__ void fold_backward_kernel(const SElem<N> *aggs, int rank, int world, 
     if (ok) { s_combine<N>(in, e, t); e = t; }
   }
   if (!ok && status) atomicOr(status, BDLM_ST_TIMEOUT);
+  *carry = e;
+}
+
+// carry of rank r for the sampler: agg_{r+1} (x) ... (x) agg_{world-1} (rank < world - 1).  The last
+// rank's aggregate ends in its terminal element (0, theta_T), so E = 0 and g is theta at the first row
+// of chunk r + 1.
+template <int N>
+__global__ void fold_sampler_kernel(const BElem<N> *aggs, int rank, int world, BElem<N> *carry) {
+  BElem<N> e = aggs[world - 1], t;
+  for (int r = world - 2; r > rank; --r) { b_combine<N>(aggs[r], e, t); e = t; }
   *carry = e;
 }
 
@@ -1617,8 +1737,9 @@ cudaError_t scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t 
   CK(fwd_prefixes<N>(a, md, M, X, scratch, state_arg<N>(a.start), false, sub, stream, launches));
   const FElem<N> *tot = nb > 1 ? scratch : nullptr;
   const bool vec = (reinterpret_cast<uintptr_t>(a.y) & 31) == 0, tr = o.transition != nullptr;
-#define BDLM_LL_SWEEP(VEC_, TR_) \
-  fwd_loglik_kernel<N, VEC_, TR_><<<blocks, kLlBlock, 0, stream>>>(md, a.y, T, M, X, tot, sub, part, last)
+#define BDLM_LL_SWEEP(VEC_, TR_)                                                                    \
+  fwd_loglik_kernel<N, VEC_, TR_, false><<<blocks, kLlBlock, 0, stream>>>(md, a.y, T, M, X, tot, sub, part, \
+                                                                          last, 1, nullptr)
   if (vec && tr) BDLM_LL_SWEEP(true, true);
   else if (vec) BDLM_LL_SWEEP(true, false);
   else if (tr) BDLM_LL_SWEEP(false, true);
@@ -1627,8 +1748,127 @@ cudaError_t scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t 
   ++*launches;
   CK(cudaGetLastError());
   loglik_finish_kernel<<<1, kLlFinish, 0, stream>>>(part, blocks, last, N, o.transition, o.innovations,
-                                                     o.m_last, o.C_last, o.status);
+                                                     o.m_last, o.C_last, o.status, nullptr);
   ++*launches;
+  return cudaGetLastError();
+}
+
+// One rank's chunk of a time-sharded series after the all-gather of the forward aggregates: fold the
+// carry (as the forward finish phase), sweep the chunk from it with both terms, and sum the block
+// partials into the rank's [transition, innovations, status] vector o.part_vec.  X still holds the
+// chunk's scanned prefixes from bdlm_scan_dist_forward_local.  The rank holding row T also writes
+// (m_T, C_T) and flags a non-finite m_T in its status.
+template <int N>
+cudaError_t scan_dist_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream, int64_t *launches) {
+  if (a.phase != kScanDistFinish) return cudaErrorInvalidValue;
+  const ScanModel<N> md = make_model<N>(a);
+  const int sub = scan_rows_per_thread(a.n, a.T);
+  const int64_t T = a.T, M = (T + a.keep_init + sub - 1) / sub;  // as the local phase
+  FElem<N> *X = reinterpret_cast<FElem<N> *>(a.workspace);
+  FElem<N> *scratch = X + (M + 1);
+  FElem<N> *carry = reinterpret_cast<FElem<N> *>(scratch + (M + 1) / kScanBlock * 2 + 8);
+  const unsigned blocks = (unsigned)((M + kLlBlock - 1) / kLlBlock);
+  const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);
+  LoglikPart *part = reinterpret_cast<LoglikPart *>(o.parts);
+  double *last = reinterpret_cast<double *>(part + blocks);
+  const bool holds_last = a.rank == a.world - 1;
+  fold_forward_kernel<N><<<1, 1, 0, stream>>>(reinterpret_cast<const FElem<N> *>(a.aggs_dev), a.rank,
+                                              state_arg<N>(a.start), carry, ScanPeers{}, nullptr, nullptr);
+  ++*launches;
+  CK(cudaGetLastError());
+  const FElem<N> *tot = nb > 1 ? scratch : nullptr;
+  if ((reinterpret_cast<uintptr_t>(a.y) & 31) == 0)
+    fwd_loglik_kernel<N, true, true, true><<<blocks, kLlBlock, 0, stream>>>(md, a.y, T, M, X, tot, sub, part, last,
+                                                                            a.keep_init, carry);
+  else
+    fwd_loglik_kernel<N, false, true, true><<<blocks, kLlBlock, 0, stream>>>(md, a.y, T, M, X, tot, sub, part,
+                                                                             last, a.keep_init, carry);
+  ++*launches;
+  CK(cudaGetLastError());
+  loglik_finish_kernel<<<1, kLlFinish, 0, stream>>>(part, blocks, holds_last ? last : nullptr, N, o.part_vec,
+                                                     o.part_vec + 1, o.m_last, o.C_last, nullptr, o.part_vec + 2);
+  ++*launches;
+  return cudaGetLastError();
+}
+
+// Rows of the sampler on a chunk: rows 0 .. nsucc-1 have a successor (all of them when another chunk
+// follows), row nsucc is the series' last when `terminal`.  At least one thread: the last chunk may
+// hold a single row.
+struct SamplerShape {
+  int sub;
+  int64_t nsucc, M, nb;
+  unsigned blocks;
+  bool terminal;
+};
+SamplerShape sampler_shape(const ScanArgs &a) {
+  SamplerShape s;
+  s.sub = scan_rows_per_thread(a.n, a.T);
+  s.terminal = !a.has_successor;
+  s.nsucc = a.T + a.keep_init - (s.terminal ? 1 : 0);
+  s.M = (s.nsucc + s.sub - 1) / s.sub;
+  if (s.M < 1) s.M = 1;
+  s.blocks = (unsigned)((s.M + kFbBlock - 1) / kFbBlock);
+  s.nb = (s.M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);
+  return s;
+}
+
+template <int N>
+bool sampler_vec(const ScanArgs &a, const ScanFfbsOut &o) {
+  return dense_aligned(a.kf.m, N) && dense_aligned(a.kf.C, N * N) && dense_aligned(o.theta, N) &&
+         (reinterpret_cast<uintptr_t>(a.y) & 31) == 0;
+}
+
+// The sampler's level 1 (elements, c_r into theta, the terminal slot) and its level-2 suffix scan.
+template <int N>
+cudaError_t sampler_prefixes(const ScanArgs &a, const ScanFfbsOut &o, const SamplerShape &s, cudaStream_t stream,
+                             int64_t *launches) {
+  const ScanModel<N> md = make_model<N>(a);
+  BElem<N> *X = reinterpret_cast<BElem<N> *>(o.workspace);  // [M + 1]
+  BElem<N> *scratch = X + (s.M + 1);
+  const FfbsRng rng{o.rng_seed, o.rng_sweep, o.rng_base, o.total_rows, o.first_row};
+  const int64_t term = s.terminal ? s.nsucc : -1;
+  if (sampler_vec<N>(a, o))
+    ffbs_reduce_kernel<N, true><<<s.blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, s.nsucc, s.M, o.z, rng,
+                                                                    o.theta, X, a.status, s.sub, term);
+  else
+    ffbs_reduce_kernel<N, false><<<s.blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, s.nsucc, s.M, o.z, rng,
+                                                                     o.theta, X, a.status, s.sub, term);
+  ++*launches;
+  CK(cudaGetLastError());
+  // a chunk that others follow: the terminal slot is the identity, so its aggregate leaves the later
+  // chunks to the carry; a last chunk of one row: its one thread folded no row
+  if (!s.terminal || s.nsucc == 0) {
+    set_b_identity<N><<<1, 1, 0, stream>>>(s.terminal ? X : X + s.M);
+    ++*launches;
+    CK(cudaGetLastError());
+  }
+  return device_scan<BElem<N>, true, true>(X, s.M + 1, scratch, stream, launches, /*defer_top=*/true);
+}
+
+// The apply sweep from the scanned suffixes (and the carry of later chunks), then, with statistics,
+// the fixed-order sum of its block partials into `stats` or into the rank's partial vector `vec`.
+template <int N>
+cudaError_t sampler_apply(const ScanArgs &a, const ScanFfbsOut &o, const SamplerShape &s, const BElem<N> *carry,
+                          bool stats, double *vec, cudaStream_t stream, int64_t *launches) {
+  const ScanModel<N> md = make_model<N>(a);
+  const BElem<N> *X = reinterpret_cast<const BElem<N> *>(o.workspace);
+  const BElem<N> *tot = s.nb > 1 ? X + (s.M + 1) : nullptr;
+  const bool vec_io = sampler_vec<N>(a, o);
+#define BDLM_FFBS_SWEEP(VEC_, STATS_)                                                                         \
+  ffbs_apply_kernel<N, VEC_, STATS_><<<s.blocks, kFbBlock, 0, stream>>>(                                      \
+      md, a.kf.m, a.kf.C, a.y, s.nsucc, s.M, X, tot, o.theta, a.status, s.sub, o.parts, carry, a.keep_init, a.T, \
+      s.terminal)
+  if (vec_io && stats) BDLM_FFBS_SWEEP(true, true);
+  else if (vec_io) BDLM_FFBS_SWEEP(true, false);
+  else if (stats) BDLM_FFBS_SWEEP(false, true);
+  else BDLM_FFBS_SWEEP(false, false);
+#undef BDLM_FFBS_SWEEP
+  ++*launches;
+  CK(cudaGetLastError());
+  if (stats) {
+    ffbs_stats_finish_kernel<N><<<1, kFbFinish, 0, stream>>>(o.parts, s.blocks, o.stats, vec, a.status);
+    ++*launches;
+  }
   return cudaGetLastError();
 }
 
@@ -1637,45 +1877,40 @@ cudaError_t scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t 
 // statistics, the fixed-order sum of the apply's block partials.
 template <int N>
 cudaError_t scan_ffbs(const ScanArgs &a, const ScanFfbsOut &o, cudaStream_t stream, int64_t *launches) {
-  if (a.keep_init != 1 || a.phase != kScanApply || a.fuse_sagg) return cudaErrorInvalidValue;
+  if (a.keep_init != 1 || a.phase != kScanApply || a.fuse_sagg || a.has_successor) return cudaErrorInvalidValue;
   CK(scan_forward<N>(a, stream, launches));
-  const ScanModel<N> md = make_model<N>(a);
-  const int sub = scan_rows_per_thread(a.n, a.T);
-  const int64_t T = a.T, M = (T + sub - 1) / sub;  // rows 0 .. T-1 have a successor
-  BElem<N> *X = reinterpret_cast<BElem<N> *>(o.workspace);  // [M + 1]
-  BElem<N> *scratch = X + (M + 1);
-  const unsigned blocks = (unsigned)((M + kFbBlock - 1) / kFbBlock);
-  const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);
-  const bool vec = dense_aligned(a.kf.m, N) && dense_aligned(a.kf.C, N * N) && dense_aligned(o.theta, N) &&
-                   (reinterpret_cast<uintptr_t>(a.y) & 31) == 0;
-  const FfbsRng rng{o.rng_seed, o.rng_sweep, o.rng_base};
-  if (vec)
-    ffbs_reduce_kernel<N, true><<<blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, T, M, o.z, rng, o.theta, X,
-                                                                  a.status, sub);
-  else
-    ffbs_reduce_kernel<N, false><<<blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, T, M, o.z, rng, o.theta, X,
-                                                                   a.status, sub);
-  ++*launches;
-  CK(cudaGetLastError());
-  CK((device_scan<BElem<N>, true, true>(X, M + 1, scratch, stream, launches, /*defer_top=*/true)));
-  const BElem<N> *tot = nb > 1 ? scratch : nullptr;
+  const SamplerShape s = sampler_shape(a);
+  CK(sampler_prefixes<N>(a, o, s, stream, launches));
   const StatViews &sv = o.stats;
   const bool stats = sv.ssy.ptr || sv.ny.ptr || sv.ssw.ptr || sv.scatter.ptr;
-#define BDLM_FFBS_SWEEP(VEC_, STATS_)                                                                    \
-  ffbs_apply_kernel<N, VEC_, STATS_><<<blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, a.y, T, M, X, tot, \
-                                                                      o.theta, a.status, sub, o.parts)
-  if (vec && stats) BDLM_FFBS_SWEEP(true, true);
-  else if (vec) BDLM_FFBS_SWEEP(true, false);
-  else if (stats) BDLM_FFBS_SWEEP(false, true);
-  else BDLM_FFBS_SWEEP(false, false);
-#undef BDLM_FFBS_SWEEP
-  ++*launches;
-  CK(cudaGetLastError());
-  if (stats) {
-    ffbs_stats_finish_kernel<N><<<1, kFbFinish, 0, stream>>>(o.parts, blocks, sv);
-    ++*launches;
+  return sampler_apply<N>(a, o, s, nullptr, stats, nullptr, stream, launches);
+}
+
+// One rank's chunk of a time-sharded FFBS.  Local (a.phase = kScanDistFinish of the forward pass): the
+// forward finish with (m, C) into a.kf and no smoother fold, then the sampler's level 1 + level 2 and
+// the chunk's aggregate into o.agg_dev for the all-gather.  Finish: fold the carry of the later
+// chunks from o.aggs_dev, apply, and sum the statistics and status into the partial vector o.part_vec.
+template <int N>
+cudaError_t scan_dist_ffbs(const ScanArgs &a, const ScanFfbsOut &o, bool finish, cudaStream_t stream,
+                           int64_t *launches) {
+  if (a.phase != kScanDistFinish || a.fuse_sagg) return cudaErrorInvalidValue;
+  const SamplerShape s = sampler_shape(a);
+  BElem<N> *X = reinterpret_cast<BElem<N> *>(o.workspace);
+  BElem<N> *scratch = X + (s.M + 1);
+  BElem<N> *carry = scratch + (s.M + 1) / kScanBlock * 2 + 8;
+  if (!finish) {
+    CK(scan_forward<N>(a, stream, launches));
+    CK(sampler_prefixes<N>(a, o, s, stream, launches));
+    const BElem<N> *whole = s.nb > 1 ? scratch + (s.nb - 1) : X;  // suffix scan ends at index 0
+    return cudaMemcpyAsync(o.agg_dev, whole, sizeof(BElem<N>), cudaMemcpyDeviceToDevice, stream);
   }
-  return cudaGetLastError();
+  if (a.has_successor) {
+    fold_sampler_kernel<N><<<1, 1, 0, stream>>>(reinterpret_cast<const BElem<N> *>(o.aggs_dev), a.rank, a.world,
+                                                carry);
+    ++*launches;
+    CK(cudaGetLastError());
+  }
+  return sampler_apply<N>(a, o, s, a.has_successor ? carry : nullptr, true, o.part_vec, stream, launches);
 }
 
 template <int N>
@@ -1785,7 +2020,7 @@ cudaError_t launch_scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaSt
 
 size_t scan_ffbs_parts_bytes(int n, int64_t T) {
   const int sub = scan_rows_per_thread(n, T);
-  const int64_t M = (T + sub - 1) / sub, blocks = (M + kFbBlock - 1) / kFbBlock;
+  const int64_t M = (T + 1 + sub - 1) / sub, blocks = (M + kFbBlock - 1) / kFbBlock;  // any chunk of T
   return sizeof(double) * (size_t)(2 + n + n * n) * (size_t)blocks + 256;
 }
 
@@ -1798,6 +2033,53 @@ cudaError_t launch_scan_ffbs(const ScanArgs &a, const ScanFfbsOut &o, cudaStream
     default: return cudaErrorInvalidValue;
   }
 }
+
+cudaError_t launch_scan_dist_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream,
+                                    int64_t *launches) {
+  switch (a.n) {
+    case 1: return scan_dist_loglik<1>(a, o, stream, launches);
+    case 2: return scan_dist_loglik<2>(a, o, stream, launches);
+    case 3: return scan_dist_loglik<3>(a, o, stream, launches);
+    case 4: return scan_dist_loglik<4>(a, o, stream, launches);
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+cudaError_t launch_scan_dist_loglik_finish(const double *parts, int world, double *transition, double *innovations,
+                                           int32_t *status, cudaStream_t stream, int64_t *launches) {
+  dist_loglik_finish_kernel<<<1, 1, 0, stream>>>(parts, world, transition, innovations, status);
+  ++*launches;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_scan_dist_ffbs(const ScanArgs &a, const ScanFfbsOut &o, bool finish, cudaStream_t stream,
+                                  int64_t *launches) {
+  switch (a.n) {
+    case 1: return scan_dist_ffbs<1>(a, o, finish, stream, launches);
+    case 2: return scan_dist_ffbs<2>(a, o, finish, stream, launches);
+    case 3: return scan_dist_ffbs<3>(a, o, finish, stream, launches);
+    case 4: return scan_dist_ffbs<4>(a, o, finish, stream, launches);
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+cudaError_t launch_scan_dist_ffbs_stats_finish(int n, const double *parts, int world, const StatViews &sv,
+                                               int32_t *status, cudaStream_t stream, int64_t *launches) {
+  switch (n) {
+#define BDLM_STATS_CASE(N_) \
+  case N_: dist_ffbs_stats_finish_kernel<N_><<<1, 1, 0, stream>>>(parts, world, sv, status); break;
+    BDLM_STATS_CASE(1)
+    BDLM_STATS_CASE(2)
+    BDLM_STATS_CASE(3)
+    BDLM_STATS_CASE(4)
+#undef BDLM_STATS_CASE
+    default: return cudaErrorInvalidValue;
+  }
+  ++*launches;
+  return cudaGetLastError();
+}
+
+int scan_sampler_elem_doubles(int n) { return n * n + n; }
 
 // Host build of the combine the kernels inline: out = ei (x) ej (ei earlier in time).
 void scan_combine_host(int n, bool backward, const double *ei, const double *ej, double *out) {

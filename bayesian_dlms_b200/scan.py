@@ -6,7 +6,8 @@ parallelisation by associative scan (Sarkka & Garcia-Fernandez 2021), kernels in
 filtered state by the forward pass alone, ``scan_ffbs`` a backward-sampled path with its Gibbs
 statistics; ``DistScan`` runs one rank's time chunk of a
 sharded series with the device-side phases (one all-gather of a 3n^2+2n-double aggregate per rank
-for the filter, 2n^2+n for the smoother).
+for the filter, 2n^2+n for the smoother), ``DistLoglik`` and ``DistFfbs`` the log-likelihoods and
+FFBS of such a chunk (``sharding.time_chunk`` gives each rank its observations and first row).
 """
 from __future__ import annotations
 
@@ -171,4 +172,131 @@ class DistScan:
         self.backward_local()
         all_gather_into(self.aggs_b, self.agg_b)
         self.backward_finish()
+        return self.out
+
+
+def dist_doubles(n: int, what: int) -> int:
+    """Sizes of the time-sharded loglik / FFBS exchanges (capi.SCAN_DIST_*)."""
+    return int(capi.load().bdlm_scan_dist_doubles(n, what))
+
+
+class _DistChunk:
+    """One rank's chunk of a time-sharded series: the problem struct, the forward local phase and
+    the exchange buffers [size] -> [world * size] of the phases that follow it."""
+
+    def __init__(self, eng: Engine, model: Model, params: Dict, y_chunk, rank: int, world: int):
+        self.eng, self.rank, self.world, self.n = eng, rank, world, model.n
+        self.model, self.y = model, y_chunk   # the problem struct points into model.F / model.G
+        self.keep_init = rank == 0
+        self.rows = model.T + int(self.keep_init)
+        with bound_engine(eng):
+            self.pr, self._keep = _problem(model, params, y_chunk, self.keep_init)
+        self.agg_f, self.aggs_f = self._xch(elem_doubles(self.n, False))
+
+    def _xch(self, size):
+        import torch
+        z = lambda k: torch.zeros(k, dtype=torch.float64, device=self.y.device)  # noqa: E731
+        return z(size), z(self.world * size)
+
+    def _ck(self, rc):
+        self.eng.ctx.check(rc)
+
+    def forward_local(self):
+        self._ck(capi.load().bdlm_scan_dist_forward_local(self.eng.ctx.handle, self.pr, self.rank,
+                                                          self.world, self.agg_f.data_ptr()))
+
+    @staticmethod
+    def _gather(all_gather_into):
+        if all_gather_into is None:
+            import torch.distributed as dist
+            all_gather_into = dist.all_gather_into_tensor
+        return all_gather_into
+
+
+class DistLoglik(_DistChunk):
+    """Log-likelihoods of a time-sharded series (``bdlm_scan_dist_loglik_*``): every rank ends with
+    the sums and status of ``scan_loglik`` on the whole series, bit-identical across ranks; the rank
+    holding the series' last observation also has its final filtered state (m, C).  ``run`` takes
+    the same injectable all-gather as ``DistScan``."""
+
+    def __init__(self, eng: Engine, model: Model, params: Dict, y_chunk, rank: int, world: int):
+        import torch
+        super().__init__(eng, model, params, y_chunk, rank, world)
+        self.part, self.parts = self._xch(dist_doubles(self.n, capi.SCAN_DIST_LOGLIK_PART))
+        z = lambda k: torch.zeros(k, dtype=torch.float64, device=y_chunk.device)  # noqa: E731
+        self.out = dict(transition=z(1), innovations=z(1), m=z(self.n), C=z(self.n * self.n),
+                        status=torch.zeros(1, dtype=torch.int32, device=y_chunk.device))
+
+    def partial(self):
+        self._ck(capi.load().bdlm_scan_dist_loglik_partial(
+            self.eng.ctx.handle, self.pr, self.rank, self.world, self.aggs_f.data_ptr(),
+            self.out["m"].data_ptr(), self.out["C"].data_ptr(), self.part.data_ptr()))
+
+    def finish(self):
+        o = self.out
+        self._ck(capi.load().bdlm_scan_dist_loglik_finish(
+            self.eng.ctx.handle, self.world, self.parts.data_ptr(), o["transition"].data_ptr(),
+            o["innovations"].data_ptr(), o["status"].data_ptr()))
+
+    def run(self, all_gather_into=None):
+        gather = self._gather(all_gather_into)
+        self.forward_local()
+        gather(self.aggs_f, self.agg_f)
+        self.partial()
+        gather(self.parts, self.part)
+        self.finish()
+        return self.out
+
+
+class DistFfbs(_DistChunk):
+    """FFBS + Gibbs statistics of a time-sharded series (``bdlm_scan_dist_ffbs_*``): theta of the
+    chunk's rows (concatenated over ranks: ``scan_ffbs``'s path of the whole series), the filter
+    fields in ``want_kf`` (m and C are always kept: the sampler reads them), and the statistics and
+    status of the whole series, bit-identical on every rank.  ``first_row`` / ``total_T`` place the
+    chunk in the series (``sharding.time_chunk``); z: CUDA tensor [rows, n] of the chunk's injected
+    normals, or None for the Philox normals of ``eng.ctx.set_rng`` at the global rows."""
+
+    def __init__(self, eng: Engine, model: Model, params: Dict, y_chunk, rank: int, world: int,
+                 first_row: int, total_T: int, z=None, want_kf=()):
+        import torch
+        super().__init__(eng, model, params, y_chunk, rank, world)
+        n = self.n
+        assert z is None or (tuple(z.shape) == (self.rows, n) and _mem_and_ptr(z)[0] == capi.DEVICE)
+        self.first_row, self.total_T, self.z = int(first_row), int(total_T), z
+        self.out, self.ko, _ = _outputs(y_chunk, self.rows, n, tuple(dict.fromkeys(("m", "C") + tuple(want_kf))))
+        dev = y_chunk.device
+        self.out["theta"] = torch.empty((self.rows, n), dtype=torch.float64, device=dev)
+        self.gs = capi.GibbsStats()
+        for k, d in (("ssy", 1), ("ny", 1), ("ssw", n), ("scatter", n * n)):
+            self.out[k] = torch.zeros((d,), dtype=torch.float64, device=dev)
+            setattr(self.gs, k, self.out[k].data_ptr())
+        self.out["status"] = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.agg_s, self.aggs_s = self._xch(dist_doubles(n, capi.SCAN_DIST_SAMPLER_ELEM))
+        self.part, self.parts = self._xch(dist_doubles(n, capi.SCAN_DIST_FFBS_PART))
+
+    def local(self):
+        self._ck(capi.load().bdlm_scan_dist_ffbs_local(
+            self.eng.ctx.handle, self.pr, self.rank, self.world, self.first_row, self.total_T,
+            self.aggs_f.data_ptr(), None if self.z is None else self.z.data_ptr(),
+            self.out["theta"].data_ptr(), self.ko, self.agg_s.data_ptr(), self.out["status"].data_ptr()))
+
+    def finish(self):
+        self._ck(capi.load().bdlm_scan_dist_ffbs_finish(
+            self.eng.ctx.handle, self.pr, self.rank, self.world, self.aggs_s.data_ptr(),
+            self.out["theta"].data_ptr(), self.ko, self.part.data_ptr(), self.out["status"].data_ptr()))
+
+    def stats_finish(self):
+        self._ck(capi.load().bdlm_scan_dist_ffbs_stats_finish(
+            self.eng.ctx.handle, self.n, self.world, self.parts.data_ptr(), self.gs,
+            self.out["status"].data_ptr()))
+
+    def run(self, all_gather_into=None):
+        gather = self._gather(all_gather_into)
+        self.forward_local()
+        gather(self.aggs_f, self.agg_f)
+        self.local()
+        gather(self.aggs_s, self.agg_s)
+        self.finish()
+        gather(self.parts, self.part)
+        self.stats_finish()
         return self.out

@@ -20,6 +20,17 @@ def shard_range(total: int, rank: int, world: int) -> Tuple[int, int]:
     return lo, lo + base + (1 if rank < extra else 0)
 
 
+def time_chunk(total_T: int, rank: int, world: int) -> Tuple[int, int, int]:
+    """Rank's chunk of ONE series of ``total_T`` observations cut along time (the time-sharded scan):
+    observations y[lo:hi] and ``first_row``, the global row of the chunk's first row.  Rank 0 also holds
+    row 0, the prior (keep_init = 1), so its rows are 0 .. hi and every later rank's first row is
+    1 + lo.  Every chunk holds at least one observation: world <= total_T."""
+    if int(world) > int(total_T):
+        raise ValueError(f"{world} ranks for {total_T} observations: every chunk needs one")
+    lo, hi = shard_range(total_T, rank, world)
+    return lo, hi, 0 if rank == 0 else lo + 1
+
+
 def wave_aligned_slabs(lo: int, hi: int, wave: int, waves_per_launch: int):
     """Split a rank's block into launches of whole GPU waves (last one takes the remainder)."""
     per = max(1, int(wave) * max(1, int(waves_per_launch)))

@@ -360,6 +360,60 @@ BDLM_API int bdlm_scan_dist_backward_finish(bdlm_ctx *ctx, const bdlm_problem *p
                                             int32_t world, const double *aggs_dev,
                                             const bdlm_kf_out *filt, const bdlm_smooth_out *sm,
                                             int32_t *status);
+/* Time-sharded log-likelihoods (bdlm_scan_loglik of the whole series) and FFBS (bdlm_scan_ffbs of
+ * the whole series) for hosts that bring their own transport; bdlm_comm_scan_loglik /
+ * bdlm_comm_scan_ffbs run the same phases over a communicator.  prob describes the rank's chunk as
+ * in the bdlm_scan_dist_* filter + smoother phases (keep_init = 1 on rank 0 only, any chunk of at
+ * least one observation), with the bdlm_scan_loglik / bdlm_scan_ffbs restrictions.  Every call is
+ * enqueue-only; the "all-gather" steps are the caller's, on the context's stream, into
+ * [world][size] doubles in rank order.  Sizes: bdlm_scan_dist_doubles(n, what).
+ *
+ * Log-likelihoods, per rank:
+ *   bdlm_scan_dist_forward_local(agg) -> all-gather -> bdlm_scan_dist_loglik_partial(aggs, part)
+ *   -> all-gather -> bdlm_scan_dist_loglik_finish(parts).
+ * loglik_partial folds the carry (the prior and every earlier chunk) and sweeps the chunk from it;
+ * the first observation's transition term uses G m of the previous chunk's last filtered state.
+ * part_dev receives [transition, innovations, status bits] of the chunk; m_last / C_last (either may
+ * be NULL) are written by rank world - 1 only, which also flags a non-finite m_T.  loglik_finish adds
+ * the world partials in rank order, so every rank writes the same bits: the sums and the status of
+ * bdlm_scan_loglik on the whole series (to 1e-9 of sum_t |term_t|).  The context's workspace must
+ * not be used by other calls between forward_local and loglik_partial.
+ *
+ * FFBS, per rank (first_row = global index of the chunk's first row: 0 on rank 0, 1 + the
+ * observations of the earlier ranks elsewhere; total_T = observations of the whole series):
+ *   bdlm_scan_dist_forward_local(agg) -> all-gather -> bdlm_scan_dist_ffbs_local(aggs, sagg)
+ *   -> all-gather -> bdlm_scan_dist_ffbs_finish(saggs, part) -> all-gather
+ *   -> bdlm_scan_dist_ffbs_stats_finish(parts).
+ * ffbs_local runs the forward finish (kf->m and kf->C required, any of a, R, f, Q written), the
+ * sampler's level 1 and 2, and writes the chunk's sampler aggregate [E | g] (n*n + n doubles).  z
+ * holds the normals of the chunk's own rows (same row split as theta) or is NULL: Philox normals of
+ * bdlm_set_rng at the GLOBAL row, the ones bdlm_scan_ffbs of the whole series consumes.
+ * ffbs_finish composes the carry of the later chunks (its g is theta at the next chunk's first row),
+ * draws theta for the chunk's rows and writes part_dev = [ssy, ny, ssw[n], scatter[n*n], status
+ * bits] of the chunk: every observation term and every transition term of the series is counted by
+ * exactly one rank (a step across a chunk boundary by the rank before it).  ffbs_stats_finish adds
+ * the world partials in rank order and writes the statistics (any field may be NULL) and the status
+ * of the whole series on every rank, with the same bits on every rank, so bdlm_gibbs_draw with the
+ * same rng draws the same V and W everywhere.  status (int32[1], may be NULL in the local and finish
+ * phases) must be the same pointer in both; the context's workspace must not be used by other
+ * calls between forward_local and ffbs_finish. */
+enum { BDLM_SCAN_DIST_SAMPLER_ELEM = 0, BDLM_SCAN_DIST_LOGLIK_PART = 1, BDLM_SCAN_DIST_FFBS_PART = 2 };
+BDLM_API int bdlm_scan_dist_doubles(int32_t n, int32_t what);
+BDLM_API int bdlm_scan_dist_loglik_partial(bdlm_ctx *ctx, const bdlm_problem *prob, int32_t rank,
+                                           int32_t world, const double *aggs_dev, double *m_last,
+                                           double *C_last, double *part_dev);
+BDLM_API int bdlm_scan_dist_loglik_finish(bdlm_ctx *ctx, int32_t world, const double *parts_dev,
+                                          double *transition, double *innovations, int32_t *status);
+BDLM_API int bdlm_scan_dist_ffbs_local(bdlm_ctx *ctx, const bdlm_problem *prob, int32_t rank,
+                                       int32_t world, int64_t first_row, int64_t total_T,
+                                       const double *aggs_dev, const double *z, double *theta,
+                                       const bdlm_kf_out *kf, double *agg_dev, int32_t *status);
+BDLM_API int bdlm_scan_dist_ffbs_finish(bdlm_ctx *ctx, const bdlm_problem *prob, int32_t rank,
+                                        int32_t world, const double *aggs_dev, double *theta,
+                                        const bdlm_kf_out *kf, double *part_dev, int32_t *status);
+BDLM_API int bdlm_scan_dist_ffbs_stats_finish(bdlm_ctx *ctx, int32_t n, int32_t world,
+                                              const double *parts_dev, const bdlm_gibbs_stats *stats,
+                                              int32_t *status);
 /* out = earlier (x) later on the host: the host build of the combine the scan kernels inline. */
 BDLM_API int bdlm_scan_combine(int32_t n, int32_t backward, const double *earlier,
                                const double *later, double *out);
@@ -431,6 +485,25 @@ BDLM_API int bdlm_comm_svd_ffbs(bdlm_comm *comm, const bdlm_problem *prob, const
 BDLM_API int bdlm_comm_scan_filter_smooth(bdlm_comm *comm, const bdlm_problem *probs,
                                           const bdlm_kf_out *kfs, const bdlm_smooth_out *sms,
                                           int32_t *const *status);
+/* The same series' log-likelihoods and last filtered state (bdlm_scan_loglik of the whole series):
+ * the bdlm_scan_dist_* loglik phases behind one call, with NCCL all-gathers on every communicator
+ * (also those that use peer mailboxes for the filter + smoother, whose epochs these calls leave
+ * alone).  Arrays have one entry per LOCAL device and may be NULL, as may their entries;
+ * m_last / C_last are written on global rank world - 1 only.  Every rank ends with the same bits
+ * in transition, innovations and status.  Enqueue-only (bdlm_comm_sync). */
+BDLM_API int bdlm_comm_scan_loglik(bdlm_comm *comm, const bdlm_problem *probs, double *const *m_last,
+                                   double *const *C_last, double *const *transition,
+                                   double *const *innovations, int32_t *const *status);
+/* FFBS + Gibbs statistics of the same series (bdlm_scan_ffbs of the whole series), the
+ * bdlm_scan_dist_* FFBS phases behind one call.  first_row[i]: global index of local device i's
+ * first row; total_T: observations of the whole series; z: NULL (Philox, the same bdlm_set_rng on
+ * every context) or one entry per local device (its chunk's rows); theta and kfs (m and C
+ * required) per local device; stats and status per local device or NULL.  Every rank ends with
+ * the same bits in its statistics and status.  Enqueue-only (bdlm_comm_sync). */
+BDLM_API int bdlm_comm_scan_ffbs(bdlm_comm *comm, const bdlm_problem *probs, const int64_t *first_row,
+                                 int64_t total_T, const double *const *z, double *const *theta,
+                                 const bdlm_kf_out *kfs, const bdlm_gibbs_stats *stats,
+                                 int32_t *const *status);
 
 /* ======================================================================================
  * "Next" rows (SURVEY.md section 8f): the callers and neighbours of the hot path.
