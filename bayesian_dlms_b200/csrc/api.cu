@@ -12,6 +12,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -1044,60 +1045,95 @@ int bdlm_rts_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *filt,
   return dispatch(c, d);
 }
 
+// The problems the associative scan computes; needs no context, so the time-sharded phases report
+// a misuse with its reason even on a null one.
+static const char kScanShapes[] =
+    "scan path: B = 1, p = 1, n <= 4, regular grid, time-invariant model (f_tv = g_tv = v_tv = w_tv = 0), "
+    "shared parameters";
+static bool scan_supported(const bdlm_problem *p) {
+  return p->B == 1 && p->p == 1 && p->n >= 1 && p->n <= 4 && !p->times && !p->f_tv && !p->g_tv && !p->v_tv &&
+         !p->w_tv && !p->per_series;
+}
+
 // BDLM_PARALLEL_IN_TIME: one long eligible series goes to the associative-scan kernels.  The
 // forward pass alone (log-likelihoods, last state) runs any n <= 4; the smoother needs n = 1 or the
 // textbook smoother, which is what its backward sweep computes.
 static bool pit_eligible_forward(const bdlm_problem *p) {
-  return (p->compat & BDLM_PARALLEL_IN_TIME) && p->B == 1 && p->T >= 4096 && p->p == 1 && p->n <= 4 &&
-         !p->times && !p->f_tv && !p->g_tv && !p->per_series && !p->v_tv && !p->w_tv;
+  return (p->compat & BDLM_PARALLEL_IN_TIME) && p->T >= 4096 && scan_supported(p);
 }
 static bool pit_eligible(const bdlm_problem *p) {
   return pit_eligible_forward(p) && (p->n == 1 || (p->compat & BDLM_TEXTBOOK_SMOOTHER));
 }
 
-// Staging buffer of the host-buffer BDLM_PARALLEL_IN_TIME calls (the scan owns the arena); y is
-// copied to its start.
-static int pit_stage_y(bdlm_ctx *c, const bdlm_problem *p, size_t bytes) {
+// One field of a host-buffer BDLM_PARALLEL_IN_TIME call: `in` is copied to the device before the
+// call, `out` back after it; both null when the field is not requested.
+struct PitField {
+  const double *in;
+  double *out;
+  size_t doubles;
+};
+
+// Runs call(q, dev, status) with q = *p on device memory: y and the fields are laid out in pit_buf
+// ([y | fields | status]; the scan owns the arena), y and the inputs copied in, dev[i] the device
+// copy of field i; then the outputs and status are copied back and the stream synchronised once.
+static int pit_staged(bdlm_ctx *c, const bdlm_problem *p, const std::vector<PitField> &fields, int32_t *status,
+                      const std::function<int(const bdlm_problem &, double *const *, int32_t *)> &call) {
+  std::vector<size_t> off(fields.size());
+  size_t pos = align_up(sizeof(double) * (size_t)p->T);
+  for (size_t i = 0; i < fields.size(); ++i) {
+    off[i] = pos;
+    if (fields[i].in || fields[i].out) pos = align_up(pos + sizeof(double) * fields[i].doubles);
+  }
+  const size_t st_off = pos;
+  pos += 256;
   CU(cudaSetDevice(c->device));
-  if (bytes > c->pit_bytes) {
+  if (pos > c->pit_bytes) {
     CU(cudaStreamSynchronize(c->stream));
     if (c->pit_buf) CU(cudaFree(c->pit_buf));
     c->pit_buf = nullptr; c->pit_bytes = 0;
-    CU(cudaMalloc(&c->pit_buf, bytes));
-    c->pit_bytes = bytes;
+    CU(cudaMalloc(&c->pit_buf, pos));
+    c->pit_bytes = pos;
   }
   CU(cudaMemcpyAsync(c->pit_buf, p->y, sizeof(double) * (size_t)p->T, cudaMemcpyHostToDevice, c->stream));
-  return 0;
-}
-
-static int pit_host(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *kf,
-                    const bdlm_smooth_out *sm, int32_t *status) {
-  // stage y in, every requested field out, through a buffer of its own (the scan owns the arena)
-  const int64_t n = p->n, R = rows_of(*p);
-  const int64_t ks[8] = {n, n * n, n, n * n, 1, 1, n, n * n};
-  double *host[8] = {kf ? kf->m : nullptr, kf ? kf->C : nullptr, kf ? kf->a : nullptr, kf ? kf->R : nullptr,
-                     kf ? kf->f : nullptr, kf ? kf->Q : nullptr, sm->s, sm->S};
-  size_t off[9], pos = align_up(sizeof(double) * (size_t)p->T);
-  for (int i = 0; i < 8; ++i) { off[i] = pos; if (host[i]) pos = align_up(pos + sizeof(double) * (size_t)R * ks[i]); }
-  off[8] = pos; pos += 256;
-  int rc0 = pit_stage_y(c, p, pos);
-  if (rc0) return rc0;
+  std::vector<double *> dev(fields.size());
+  for (size_t i = 0; i < fields.size(); ++i) {
+    const PitField &f = fields[i];
+    dev[i] = f.in || f.out ? reinterpret_cast<double *>(c->pit_buf + off[i]) : nullptr;
+    if (f.in) CU(cudaMemcpyAsync(dev[i], f.in, sizeof(double) * f.doubles, cudaMemcpyHostToDevice, c->stream));
+  }
   bdlm_problem q = *p;
   q.mem = BDLM_DEVICE;
   q.y = reinterpret_cast<const double *>(c->pit_buf);
-  double *dev[8];
-  for (int i = 0; i < 8; ++i) dev[i] = host[i] ? reinterpret_cast<double *>(c->pit_buf + off[i]) : nullptr;
-  bdlm_kf_out dk = {dev[0], dev[1], dev[2], dev[3], dev[4], dev[5]};
-  bdlm_smooth_out ds = {dev[6], dev[7]};
-  int32_t *dst = status ? reinterpret_cast<int32_t *>(c->pit_buf + off[8]) : nullptr;
-  int rc = bdlm_scan_filter_smooth(c, &q, &dk, &ds, dst);
+  int32_t *dst = status ? reinterpret_cast<int32_t *>(c->pit_buf + st_off) : nullptr;
+  int rc = call(q, dev.data(), dst);
   if (rc) return rc;
-  for (int i = 0; i < 8; ++i)
-    if (host[i])
-      CU(cudaMemcpyAsync(host[i], dev[i], sizeof(double) * (size_t)R * ks[i], cudaMemcpyDeviceToHost, c->stream));
+  for (size_t i = 0; i < fields.size(); ++i)
+    if (fields[i].out)
+      CU(cudaMemcpyAsync(fields[i].out, dev[i], sizeof(double) * fields[i].doubles, cudaMemcpyDeviceToHost,
+                         c->stream));
   if (status) CU(cudaMemcpyAsync(status, dst, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
   return 0;
+}
+
+// BDLM_PARALLEL_IN_TIME on bdlm_kf_filter_smooth: bdlm_scan_filter_smooth.
+static int pit_filter_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *kf,
+                             const bdlm_smooth_out *sm, int32_t *status) {
+  bdlm_problem q = *p;
+  q.compat &= ~BDLM_PARALLEL_IN_TIME;
+  if (p->mem == BDLM_DEVICE) return bdlm_scan_filter_smooth(c, &q, kf, sm, status);
+  const size_t n = p->n, R = rows_of(*p);
+  bdlm_kf_out k{};
+  if (kf) k = *kf;
+  return pit_staged(c, &q,
+                    {{nullptr, k.m, R * n}, {nullptr, k.C, R * n * n}, {nullptr, k.a, R * n},
+                     {nullptr, k.R, R * n * n}, {nullptr, k.f, R}, {nullptr, k.Q, R}, {nullptr, sm->s, R * n},
+                     {nullptr, sm->S, R * n * n}},
+                    status, [&](const bdlm_problem &d, double *const *v, int32_t *st) {
+                      const bdlm_kf_out dk = {v[0], v[1], v[2], v[3], v[4], v[5]};
+                      const bdlm_smooth_out ds = {v[6], v[7]};
+                      return bdlm_scan_filter_smooth(c, &d, &dk, &ds, st);
+                    });
 }
 
 int bdlm_kf_filter_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *kf,
@@ -1106,45 +1142,24 @@ int bdlm_kf_filter_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out 
   int rc = validate(c, A_FILTER_SMOOTH, p);
   if (rc) return rc;
   if (!sm) return fail(c, BDLM_E_ARG, "null smoother output struct");
-  if (pit_eligible(p) && (sm->s || sm->S)) {
-    bdlm_problem q = *p;
-    q.compat &= ~BDLM_PARALLEL_IN_TIME;
-    return p->mem == BDLM_DEVICE ? bdlm_scan_filter_smooth(c, &q, kf, sm, status)
-                                 : pit_host(c, &q, kf, sm, status);
-  }
+  if (pit_eligible(p) && (sm->s || sm->S)) return pit_filter_smooth(c, p, kf, sm, status);
   DevCall d{}; d.op = A_FILTER_SMOOTH; d.pr = *p; if (kf) d.kf = *kf; d.sm = *sm;
   d.status = status;
   return dispatch(c, d);
 }
 
-// BDLM_PARALLEL_IN_TIME on bdlm_loglik / bdlm_kf_filter_last: bdlm_scan_loglik, with host buffers
-// staged through pit_buf ([y | m_last | C_last | transition | innovations | status]).
+// BDLM_PARALLEL_IN_TIME on bdlm_loglik / bdlm_kf_filter_last: bdlm_scan_loglik.
 static int pit_loglik(bdlm_ctx *c, const bdlm_problem *p, double *m_last, double *C_last,
                       double *transition, double *innovations, int32_t *status) {
   bdlm_problem q = *p;
   q.compat &= ~BDLM_PARALLEL_IN_TIME;
   if (p->mem == BDLM_DEVICE) return bdlm_scan_loglik(c, &q, m_last, C_last, transition, innovations, status);
-  const int64_t n = p->n;
-  const int64_t ks[4] = {n, n * n, 1, 1};
-  double *host[4] = {m_last, C_last, transition, innovations};
-  size_t off[5], pos = align_up(sizeof(double) * (size_t)p->T);
-  for (int i = 0; i < 4; ++i) { off[i] = pos; if (host[i]) pos = align_up(pos + sizeof(double) * (size_t)ks[i]); }
-  off[4] = pos; pos += 256;
-  int rc = pit_stage_y(c, p, pos);
-  if (rc) return rc;
-  q.mem = BDLM_DEVICE;
-  q.y = reinterpret_cast<const double *>(c->pit_buf);
-  double *dev[4];
-  for (int i = 0; i < 4; ++i) dev[i] = host[i] ? reinterpret_cast<double *>(c->pit_buf + off[i]) : nullptr;
-  int32_t *dst = status ? reinterpret_cast<int32_t *>(c->pit_buf + off[4]) : nullptr;
-  rc = bdlm_scan_loglik(c, &q, dev[0], dev[1], dev[2], dev[3], dst);
-  if (rc) return rc;
-  for (int i = 0; i < 4; ++i)
-    if (host[i])
-      CU(cudaMemcpyAsync(host[i], dev[i], sizeof(double) * (size_t)ks[i], cudaMemcpyDeviceToHost, c->stream));
-  if (status) CU(cudaMemcpyAsync(status, dst, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
-  return 0;
+  const size_t n = p->n;
+  return pit_staged(c, &q, {{nullptr, m_last, n}, {nullptr, C_last, n * n}, {nullptr, transition, 1},
+                            {nullptr, innovations, 1}},
+                    status, [&](const bdlm_problem &d, double *const *v, int32_t *st) {
+                      return bdlm_scan_loglik(c, &d, v[0], v[1], v[2], v[3], st);
+                    });
 }
 
 int bdlm_loglik(bdlm_ctx *c, const bdlm_problem *p, double *transition, double *innovations,
@@ -1173,47 +1188,27 @@ int bdlm_kf_filter_last(bdlm_ctx *c, const bdlm_problem *p, double *m_last, doub
   return dispatch(c, d);
 }
 
-// BDLM_PARALLEL_IN_TIME on bdlm_ffbs: bdlm_scan_ffbs, with host buffers staged through pit_buf
-// ([y | z | theta | m | C | a | R | f | Q | ssy | ny | ssw | scatter | status]).
+// BDLM_PARALLEL_IN_TIME on bdlm_ffbs: bdlm_scan_ffbs.
 static int pit_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *theta,
                     const bdlm_kf_out *kf, const bdlm_gibbs_stats *stats, int32_t *status) {
   bdlm_problem q = *p;
   q.compat &= ~BDLM_PARALLEL_IN_TIME;
   if (p->mem == BDLM_DEVICE) return bdlm_scan_ffbs(c, &q, z, theta, kf, stats, status);
-  const int64_t n = p->n, R = rows_of(*p);
-  // outputs: theta, kf fields, statistics (rows x k, or k for a statistic)
-  const int64_t ks[11] = {R * n, R * n, R * n * n, R * n, R * n * n, R, R, 1, 1, n, n * n};
-  double *host[11] = {theta,
-                      kf ? kf->m : nullptr, kf ? kf->C : nullptr, kf ? kf->a : nullptr, kf ? kf->R : nullptr,
-                      kf ? kf->f : nullptr, kf ? kf->Q : nullptr,
-                      stats ? stats->ssy : nullptr, stats ? stats->ny : nullptr,
-                      stats ? stats->ssw : nullptr, stats ? stats->scatter : nullptr};
-  size_t pos = align_up(sizeof(double) * (size_t)p->T);
-  const size_t z_off = pos;
-  if (z) pos = align_up(pos + sizeof(double) * (size_t)(R * n));
-  size_t off[12];
-  for (int i = 0; i < 11; ++i) { off[i] = pos; if (host[i]) pos = align_up(pos + sizeof(double) * (size_t)ks[i]); }
-  off[11] = pos; pos += 256;
-  int rc = pit_stage_y(c, p, pos);
-  if (rc) return rc;
-  if (z) CU(cudaMemcpyAsync(c->pit_buf + z_off, z, sizeof(double) * (size_t)(R * n), cudaMemcpyHostToDevice,
-                            c->stream));
-  q.mem = BDLM_DEVICE;
-  q.y = reinterpret_cast<const double *>(c->pit_buf);
-  double *dev[11];
-  for (int i = 0; i < 11; ++i) dev[i] = host[i] ? reinterpret_cast<double *>(c->pit_buf + off[i]) : nullptr;
-  bdlm_kf_out dk = {dev[1], dev[2], dev[3], dev[4], dev[5], dev[6]};
-  bdlm_gibbs_stats ds = {dev[7], dev[8], dev[9], dev[10]};
-  int32_t *dst = status ? reinterpret_cast<int32_t *>(c->pit_buf + off[11]) : nullptr;
-  rc = bdlm_scan_ffbs(c, &q, z ? reinterpret_cast<const double *>(c->pit_buf + z_off) : nullptr, dev[0],
-                      kf ? &dk : nullptr, stats ? &ds : nullptr, dst);
-  if (rc) return rc;
-  for (int i = 0; i < 11; ++i)
-    if (host[i])
-      CU(cudaMemcpyAsync(host[i], dev[i], sizeof(double) * (size_t)ks[i], cudaMemcpyDeviceToHost, c->stream));
-  if (status) CU(cudaMemcpyAsync(status, dst, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
-  return 0;
+  const size_t n = p->n, R = rows_of(*p);
+  bdlm_kf_out k{};
+  if (kf) k = *kf;
+  bdlm_gibbs_stats g{};
+  if (stats) g = *stats;
+  return pit_staged(c, &q,
+                    {{z, nullptr, R * n}, {nullptr, theta, R * n}, {nullptr, k.m, R * n},
+                     {nullptr, k.C, R * n * n}, {nullptr, k.a, R * n}, {nullptr, k.R, R * n * n},
+                     {nullptr, k.f, R}, {nullptr, k.Q, R}, {nullptr, g.ssy, 1}, {nullptr, g.ny, 1},
+                     {nullptr, g.ssw, n}, {nullptr, g.scatter, n * n}},
+                    status, [&](const bdlm_problem &d, double *const *v, int32_t *st) {
+                      const bdlm_kf_out dk = {v[2], v[3], v[4], v[5], v[6], v[7]};
+                      const bdlm_gibbs_stats ds = {v[8], v[9], v[10], v[11]};
+                      return bdlm_scan_ffbs(c, &d, v[0], v[1], kf ? &dk : nullptr, stats ? &ds : nullptr, st);
+                    });
 }
 
 int bdlm_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *theta,
@@ -1258,11 +1253,8 @@ int bdlm_svd_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *t
 static int scan_validate(bdlm_ctx *c, const bdlm_problem *p) {
   int rc = validate(c, A_FILTER, p);
   if (rc) return rc;
-  if (p->B != 1 || p->p != 1 || p->n > 4 || p->times || p->f_tv || p->g_tv || p->per_series ||
-      p->mem != BDLM_DEVICE)
-    return fail(c, BDLM_E_ARG,
-                "scan path: B = 1, p = 1, n <= 4, regular grid, time-invariant model, shared "
-                "parameters, device memory");
+  if (!scan_supported(p)) return fail(c, BDLM_E_ARG, kScanShapes);
+  if (p->mem != BDLM_DEVICE) return fail(c, BDLM_E_ARG, "scan path: device memory");
   return 0;
 }
 
@@ -1287,17 +1279,21 @@ static int scan_fill(bdlm_ctx *c, const bdlm_problem *p, ScanArgs &a, bool forwa
   return 0;
 }
 
-// launch_scan for a forward pass: the table key is committed only once the upload is enqueued, so
-// a failed launch (or a finish phase without its local phase) can never leave a stale table that
-// a later call would trust.
-static int scan_launch_fwd(bdlm_ctx *c, ScanArgs &a, const ScanLoglikOut *ll = nullptr,
-                           const ScanFfbsOut *fb = nullptr) {
-  CU(ll   ? launch_scan_loglik(a, *ll, c->stream, &c->launches)
-     : fb ? launch_scan_ffbs(a, *fb, c->stream, &c->launches)
-          : launch_scan(a, c->stream, &c->launches));
+// scan_launch: the result of enqueuing a forward pass filled by scan_fill(..., true).  The table key
+// is committed only once the upload is enqueued, so a failed launch (or a finish phase without its
+// local phase) can never leave a stale table that a later call would trust.
+static int scan_table_commit(bdlm_ctx *c, const ScanArgs &a, cudaError_t scan_launch) {
+  CU(scan_launch);
   if (a.table_upload) c->scan_key.swap(c->scan_key_pending);
   c->scan_key_pending.clear();
   return 0;
+}
+
+static std::vector<double> scan_prior(const bdlm_problem *p) {
+  std::vector<double> prior((size_t)p->n + p->n * p->n);
+  std::copy(p->m0, p->m0 + p->n, prior.begin());
+  std::copy(p->C0, p->C0 + p->n * p->n, prior.begin() + p->n);
+  return prior;
 }
 
 static KfViews scan_kf_views(const bdlm_problem *p, const bdlm_kf_out *kf) {
@@ -1308,6 +1304,42 @@ static KfViews scan_kf_views(const bdlm_problem *p, const bdlm_kf_out *kf) {
   v.a = mk_view(kf->a, p->layout, 0, 1, R, n); v.R = mk_view(kf->R, p->layout, 0, 1, R, n * n);
   v.f = mk_view(kf->f, p->layout, 0, 1, R, 1); v.Q = mk_view(kf->Q, p->layout, 0, 1, R, 1);
   return v;
+}
+
+// What a scan call keeps in the arena besides its forward workspace.  Every phase of a time-sharded
+// call is kScanCallDist, so a local phase and its finish phase lay the arena out identically.
+enum ScanCall { kScanCallFilterSmooth, kScanCallLoglik, kScanCallFfbs, kScanCallDist };
+
+// [forward workspace | second workspace (smoother or sampler) | block partials | (m, C) spill when
+// the caller does not want them | status slot]
+struct ScanArena {
+  char *ws, *ws2;
+  double *parts;    // of the log-likelihoods or of the sampler's statistics
+  double *m, *C;    // the caller's kf->m / kf->C, else the spill
+  int32_t *status;  // for the phases whose caller passed none
+};
+
+static int scan_arena(bdlm_ctx *c, const bdlm_problem *p, ScanCall call, const bdlm_kf_out *kf, ScanArena &ar) {
+  const size_t n = p->n, R = rows_of(*p);
+  const size_t ws = align_up(scan_workspace_bytes(p->n, p->T));
+  const size_t ll = scan_loglik_bytes(p->n, p->T), fb = scan_ffbs_parts_bytes(p->n, p->T);
+  const size_t parts = call == kScanCallLoglik ? ll : call == kScanCallFfbs ? fb
+                       : call == kScanCallDist ? std::max(ll, fb) : 0;
+  const bool spill = call == kScanCallFilterSmooth || call == kScanCallFfbs;
+  double *m = kf ? kf->m : nullptr, *C = kf ? kf->C : nullptr;
+  const size_t o_parts = (call == kScanCallLoglik ? 1 : 2) * ws;
+  const size_t o_m = o_parts + align_up(parts);
+  const size_t o_C = o_m + (spill && !m ? align_up(sizeof(double) * R * n) : 0);
+  const size_t o_st = o_C + (spill && !C ? align_up(sizeof(double) * R * n * n) : 0);
+  int rc = ensure_arena(c, o_st + 256);
+  if (rc) return rc;
+  ar.ws = c->arena;
+  ar.ws2 = call == kScanCallLoglik ? nullptr : c->arena + ws;
+  ar.parts = reinterpret_cast<double *>(c->arena + o_parts);
+  ar.m = spill && !m ? reinterpret_cast<double *>(c->arena + o_m) : m;
+  ar.C = spill && !C ? reinterpret_cast<double *>(c->arena + o_C) : C;
+  ar.status = reinterpret_cast<int32_t *>(c->arena + o_st);
+  return 0;
 }
 
 int bdlm_scan_elem_doubles(int32_t n, int32_t backward) {
@@ -1330,36 +1362,30 @@ int bdlm_scan_filter_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_ou
   if (!sm) return fail(c, BDLM_E_ARG, "null smoother output struct");
   CU(cudaSetDevice(c->device));
   const int64_t n = p->n, R = rows_of(*p);
+  ScanArena ar;
+  rc = scan_arena(c, p, kScanCallFilterSmooth, kf, ar);
+  if (rc) return rc;
   bdlm_kf_out k{};
   if (kf) k = *kf;
-  // arena: [forward scan workspace | backward scan workspace | (m, C) spill when not wanted]
-  const size_t ws = align_up(scan_workspace_bytes(p->n, p->T) + 4096);
-  const size_t need = 2 * ws + (k.m ? 0 : align_up(sizeof(double) * R * n)) +
-                      (k.C ? 0 : align_up(sizeof(double) * R * n * n)) + 4096;
-  rc = ensure_arena(c, need);
-  if (rc) return rc;
-  Bump bump{c->arena, 2 * ws, c->arena_bytes};
-  if (!k.m) k.m = bump.take<double>((size_t)R * n);
-  if (!k.C) k.C = bump.take<double>((size_t)R * n * n);
-  std::vector<double> prior((size_t)n + n * n);
-  std::copy(p->m0, p->m0 + n, prior.begin());
-  std::copy(p->C0, p->C0 + n * n, prior.begin() + n);
+  k.m = ar.m; k.C = ar.C;
+  const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
   rc = scan_fill(c, p, a, true);
   if (rc) return rc;
   // forward: filter outputs + the smoother's level-1 aggregates (fused into the apply sweep)
   a.phase = kScanApply; a.start = prior.data();
-  a.kf = scan_kf_views(p, &k); a.status = status; a.workspace = c->arena;
-  a.fuse_sagg = R > 1 ? c->arena + ws : nullptr;
+  a.kf = scan_kf_views(p, &k); a.status = status; a.workspace = ar.ws;
+  a.fuse_sagg = R > 1 ? ar.ws2 : nullptr;
   if (status) CU(cudaMemsetAsync(status, 0, sizeof(int32_t), c->stream));
-  { rc = scan_launch_fwd(c, a); if (rc) return rc; }
+  rc = scan_table_commit(c, a, launch_scan(a, c->stream, &c->launches));
+  if (rc) return rc;
   // backward: scan the aggregates, apply
   rc = scan_fill(c, p, a);
   if (rc) return rc;
   a.backward = 1; a.phase = kScanApply; a.has_successor = 0;
   a.kf = scan_kf_views(p, &k);
   a.s = mk_view(sm->s, p->layout, 0, 1, R, n); a.S = mk_view(sm->S, p->layout, 0, 1, R, n * n);
-  a.status = status; a.workspace = c->arena + ws;
+  a.status = status; a.workspace = ar.ws2;
   CU(launch_scan(a, c->stream, &c->launches));
   return 0;
 }
@@ -1369,25 +1395,20 @@ int bdlm_scan_loglik(bdlm_ctx *c, const bdlm_problem *p, double *m_last, double 
   NvtxRange nvtx_("bdlm_scan_loglik");
   int rc = scan_validate(c, p);
   if (rc) return rc;
-  if (p->v_tv || p->w_tv) return fail(c, BDLM_E_ARG, "scan path: time-invariant model (v_tv = w_tv = 0)");
   if (!m_last && !C_last && !transition && !innovations) return fail(c, BDLM_E_ARG, "nothing requested");
   CU(cudaSetDevice(c->device));
-  const int64_t n = p->n;
-  // arena: [forward scan workspace | block partials + last state]
-  const size_t ws = align_up(scan_workspace_bytes(p->n, p->T) + 4096);
-  rc = ensure_arena(c, ws + align_up(scan_loglik_bytes(p->n, p->T)) + 4096);
+  ScanArena ar;
+  rc = scan_arena(c, p, kScanCallLoglik, nullptr, ar);
   if (rc) return rc;
   bdlm_problem q = *p;
   q.keep_init = 1;  // as bdlm_loglik: the state (m0, C0) is row 0, every observation a step
-  std::vector<double> prior((size_t)n + n * n);
-  std::copy(p->m0, p->m0 + n, prior.begin());
-  std::copy(p->C0, p->C0 + n * n, prior.begin() + n);
+  const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
   rc = scan_fill(c, &q, a, true);
   if (rc) return rc;
-  a.phase = kScanApply; a.start = prior.data(); a.workspace = c->arena;
-  const ScanLoglikOut o{transition, innovations, m_last, C_last, status, c->arena + ws};
-  return scan_launch_fwd(c, a, &o);
+  a.phase = kScanApply; a.start = prior.data(); a.workspace = ar.ws;
+  const ScanLoglikOut o{transition, innovations, m_last, C_last, status, ar.parts};
+  return scan_table_commit(c, a, launch_scan_loglik(a, o, c->stream, &c->launches));
 }
 
 int bdlm_scan_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *theta,
@@ -1395,31 +1416,21 @@ int bdlm_scan_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *
   NvtxRange nvtx_("bdlm_scan_ffbs");
   int rc = scan_validate(c, p);
   if (rc) return rc;
-  if (p->v_tv || p->w_tv) return fail(c, BDLM_E_ARG, "scan path: time-invariant model (v_tv = w_tv = 0)");
   if (!p->keep_init) return fail(c, BDLM_E_ARG, "scan FFBS: keep_init = 1");
   if (!theta) return fail(c, BDLM_E_ARG, "null theta");  // z == NULL: on-device Philox normals
   CU(cudaSetDevice(c->device));
   const int64_t n = p->n, R = rows_of(*p);
+  ScanArena ar;
+  rc = scan_arena(c, p, kScanCallFfbs, kf, ar);
+  if (rc) return rc;
   bdlm_kf_out k{};
   if (kf) k = *kf;
-  // arena: [forward scan workspace | sampler scan workspace | statistics partials | (m, C) spill
-  // when not wanted]
-  const size_t ws = align_up(scan_workspace_bytes(p->n, p->T) + 4096);
-  const size_t parts = align_up(scan_ffbs_parts_bytes(p->n, p->T));
-  const size_t need = 2 * ws + parts + (k.m ? 0 : align_up(sizeof(double) * R * n)) +
-                      (k.C ? 0 : align_up(sizeof(double) * R * n * n)) + 4096;
-  rc = ensure_arena(c, need);
-  if (rc) return rc;
-  Bump bump{c->arena, 2 * ws + parts, c->arena_bytes};
-  if (!k.m) k.m = bump.take<double>((size_t)R * n);
-  if (!k.C) k.C = bump.take<double>((size_t)R * n * n);
-  std::vector<double> prior((size_t)n + n * n);
-  std::copy(p->m0, p->m0 + n, prior.begin());
-  std::copy(p->C0, p->C0 + n * n, prior.begin() + n);
+  k.m = ar.m; k.C = ar.C;
+  const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
   rc = scan_fill(c, p, a, true);
   if (rc) return rc;
-  a.phase = kScanApply; a.start = prior.data(); a.workspace = c->arena;
+  a.phase = kScanApply; a.start = prior.data(); a.workspace = ar.ws;
   a.kf = scan_kf_views(p, &k); a.status = status;
   ScanFfbsOut o{};
   o.z = mk_cview(z, p->layout, 0, 1, R, n);
@@ -1432,80 +1443,85 @@ int bdlm_scan_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *
   }
   o.rng_seed = c->rng_seed; o.rng_sweep = c->rng_sweep; o.rng_base = c->rng_first;
   o.total_rows = R; o.first_row = 0;
-  o.workspace = c->arena + ws;
-  o.parts = reinterpret_cast<double *>(c->arena + 2 * ws);
+  o.workspace = ar.ws2; o.parts = ar.parts;
   if (status) CU(cudaMemsetAsync(status, 0, sizeof(int32_t), c->stream));
-  return scan_launch_fwd(c, a, nullptr, &o);
+  return scan_table_commit(c, a, launch_scan_ffbs(a, o, c->stream, &c->launches));
 }
 
 // ---- device-side multi-GPU protocol for the scan (no host round trip) --------------------
-// arena: [forward scan workspace | backward (or sampler) scan workspace | sampler block partials |
-// status slot]; it must survive from the local to the finish phase, so every phase sizes it
-// identically.
 
-static int scan_dist_common(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *kf, int rank,
-                            int world, size_t *ws_out) {
-  int rc = scan_validate(c, p);
-  if (rc) return rc;
+// Argument checks that need no device (they run before the context is looked at, so a misuse is
+// reported with its own message even on a null context).
+static int scan_dist_args(bdlm_ctx *c, const bdlm_problem *p, int rank, int world) {
+  if (!p) return fail(c, BDLM_E_ARG, "null problem");
   if (world < 1 || rank < 0 || rank >= world) return fail(c, BDLM_E_ARG, "bad rank / world");
   if ((p->keep_init != 0) != (rank == 0))
     return fail(c, BDLM_E_ARG, "time-sharded scan: keep_init = 1 on rank 0 only");
-  if (kf && (!kf->m || !kf->C)) return fail(c, BDLM_E_ARG, "time-sharded scan needs kf->m and kf->C");
-  CU(cudaSetDevice(c->device));
-  const size_t ws = align_up(scan_workspace_bytes(p->n, p->T) + 4096);
-  rc = ensure_arena(c, 2 * ws + align_up(scan_ffbs_parts_bytes(p->n, p->T)) + 256 + 4096);
-  if (rc) return rc;
-  *ws_out = ws;
+  if (!scan_supported(p)) return fail(c, BDLM_E_ARG, kScanShapes);
   return 0;
+}
+
+// the filtered (m, C) that every phase after the forward local one writes or reads
+static int scan_dist_kf(bdlm_ctx *c, const bdlm_kf_out *kf) {
+  return kf && kf->m && kf->C ? 0 : fail(c, BDLM_E_ARG, "time-sharded scan needs kf->m and kf->C");
+}
+
+static int scan_dist_common(bdlm_ctx *c, const bdlm_problem *p, ScanArena &ar) {
+  int rc = scan_validate(c, p);
+  if (rc) return rc;
+  CU(cudaSetDevice(c->device));
+  return scan_arena(c, p, kScanCallDist, nullptr, ar);
 }
 
 int bdlm_scan_dist_forward_local(bdlm_ctx *c, const bdlm_problem *p, int32_t rank, int32_t world,
                                  double *agg_dev) {
   NvtxRange nvtx_("bdlm_scan_dist_forward_local");
-  size_t ws;
-  int rc = scan_dist_common(c, p, nullptr, rank, world, &ws);
+  int rc = scan_dist_args(c, p, rank, world);
+  if (rc) return rc;
+  ScanArena ar;
+  rc = scan_dist_common(c, p, ar);
   if (rc) return rc;
   if (!agg_dev) return fail(c, BDLM_E_ARG, "null aggregate pointer");
   ScanArgs a;
   rc = scan_fill(c, p, a, true);
   if (rc) return rc;
-  a.phase = kScanDistLocal; a.agg_dev = agg_dev; a.workspace = c->arena;
+  a.phase = kScanDistLocal; a.agg_dev = agg_dev; a.workspace = ar.ws;
   a.rank = rank; a.world = world; a.peers = c->scan_peers; a.epoch_dev = c->scan_epoch;
-  { rc = scan_launch_fwd(c, a); if (rc) return rc; }
-  return 0;
+  return scan_table_commit(c, a, launch_scan(a, c->stream, &c->launches));
 }
 
 int bdlm_scan_dist_forward_finish(bdlm_ctx *c, const bdlm_problem *p, int32_t rank, int32_t world,
                                   const double *aggs_dev, const bdlm_kf_out *kf, int32_t *status) {
   NvtxRange nvtx_("bdlm_scan_dist_forward_finish");
-  size_t ws;
-  if (!kf) return fail(c, BDLM_E_ARG, "null output struct");
-  int rc = scan_dist_common(c, p, kf, rank, world, &ws);
+  int rc = scan_dist_args(c, p, rank, world);
+  if (!rc) rc = scan_dist_kf(c, kf);
+  if (rc) return rc;
+  ScanArena ar;
+  rc = scan_dist_common(c, p, ar);
   if (rc) return rc;
   if (!aggs_dev) return fail(c, BDLM_E_ARG, "null aggregates pointer");
-  std::vector<double> prior((size_t)p->n + p->n * p->n);
-  std::copy(p->m0, p->m0 + p->n, prior.begin());
-  std::copy(p->C0, p->C0 + p->n * p->n, prior.begin() + p->n);
+  const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
   rc = scan_fill(c, p, a, true);
   if (rc) return rc;
   a.phase = kScanDistFinish; a.aggs_dev = aggs_dev; a.rank = rank; a.world = world;
   a.peers = c->scan_peers; a.epoch_dev = c->scan_epoch;
   a.start = prior.data(); a.has_successor = rank < world - 1;
-  a.kf = scan_kf_views(p, kf); a.status = status; a.workspace = c->arena;
-  a.fuse_sagg = c->arena + ws;  // smoother level-1 aggregates for the backward phases
+  a.kf = scan_kf_views(p, kf); a.status = status; a.workspace = ar.ws;
+  a.fuse_sagg = ar.ws2;  // smoother level-1 aggregates for the backward phases
   if (status) CU(cudaMemsetAsync(status, 0, sizeof(int32_t), c->stream));
-  { rc = scan_launch_fwd(c, a); if (rc) return rc; }
-  return 0;
+  return scan_table_commit(c, a, launch_scan(a, c->stream, &c->launches));
 }
 
 int bdlm_scan_dist_backward_local(bdlm_ctx *c, const bdlm_problem *p, int32_t rank, int32_t world,
                                   const bdlm_kf_out *filt, const bdlm_smooth_out *sm,
                                   double *agg_dev) {
   NvtxRange nvtx_("bdlm_scan_dist_backward_local");
-  size_t ws;
-  if (!filt) return fail(c, BDLM_E_ARG, "null filtered-state struct");
-  int rc = scan_dist_common(c, p, filt, rank, world, &ws);
+  int rc = scan_dist_args(c, p, rank, world);
+  if (!rc) rc = scan_dist_kf(c, filt);
+  if (rc) return rc;
+  ScanArena ar;
+  rc = scan_dist_common(c, p, ar);
   if (rc) return rc;
   if (!agg_dev || !sm) return fail(c, BDLM_E_ARG, "null aggregate pointer or output struct");
   const int64_t n = p->n, R = rows_of(*p);
@@ -1515,7 +1531,7 @@ int bdlm_scan_dist_backward_local(bdlm_ctx *c, const bdlm_problem *p, int32_t ra
   a.backward = 1; a.phase = kScanDistLocal; a.has_successor = rank < world - 1;
   a.kf = scan_kf_views(p, filt);
   a.s = mk_view(sm->s, p->layout, 0, 1, R, n); a.S = mk_view(sm->S, p->layout, 0, 1, R, n * n);
-  a.agg_dev = agg_dev; a.rank = rank; a.world = world; a.workspace = c->arena + ws;
+  a.agg_dev = agg_dev; a.rank = rank; a.world = world; a.workspace = ar.ws2;
   a.peers = c->scan_peers; a.epoch_dev = c->scan_epoch;
   CU(launch_scan(a, c->stream, &c->launches));
   return 0;
@@ -1525,9 +1541,11 @@ int bdlm_scan_dist_backward_finish(bdlm_ctx *c, const bdlm_problem *p, int32_t r
                                    const double *aggs_dev, const bdlm_kf_out *filt,
                                    const bdlm_smooth_out *sm, int32_t *status) {
   NvtxRange nvtx_("bdlm_scan_dist_backward_finish");
-  size_t ws;
-  if (!filt) return fail(c, BDLM_E_ARG, "null filtered-state struct");
-  int rc = scan_dist_common(c, p, filt, rank, world, &ws);
+  int rc = scan_dist_args(c, p, rank, world);
+  if (!rc) rc = scan_dist_kf(c, filt);
+  if (rc) return rc;
+  ScanArena ar;
+  rc = scan_dist_common(c, p, ar);
   if (rc) return rc;
   if (!aggs_dev || !sm) return fail(c, BDLM_E_ARG, "null aggregates pointer or output struct");
   const int64_t n = p->n, R = rows_of(*p);
@@ -1538,23 +1556,12 @@ int bdlm_scan_dist_backward_finish(bdlm_ctx *c, const bdlm_problem *p, int32_t r
   a.kf = scan_kf_views(p, filt);
   a.s = mk_view(sm->s, p->layout, 0, 1, R, n); a.S = mk_view(sm->S, p->layout, 0, 1, R, n * n);
   a.aggs_dev = aggs_dev; a.rank = rank; a.world = world; a.status = status;
-  a.workspace = c->arena + ws; a.peers = c->scan_peers; a.epoch_dev = c->scan_epoch;
+  a.workspace = ar.ws2; a.peers = c->scan_peers; a.epoch_dev = c->scan_epoch;
   CU(launch_scan(a, c->stream, &c->launches));
   return 0;
 }
 
 // ---- time-sharded log-likelihoods and FFBS ---------------------------------------------------
-// Argument checks that need no device (they run before the context is looked at, so a misuse is
-// reported with its own message even on a null context).
-static int scan_dist_args(bdlm_ctx *c, const bdlm_problem *p, int rank, int world) {
-  if (!p) return fail(c, BDLM_E_ARG, "null problem");
-  if (world < 1 || rank < 0 || rank >= world) return fail(c, BDLM_E_ARG, "bad rank / world");
-  if ((p->keep_init != 0) != (rank == 0))
-    return fail(c, BDLM_E_ARG, "time-sharded scan: keep_init = 1 on rank 0 only");
-  if (p->n < 1 || p->n > 4) return fail(c, BDLM_E_ARG, "scan path: n <= 4");
-  if (p->v_tv || p->w_tv) return fail(c, BDLM_E_ARG, "scan path: time-invariant model (v_tv = w_tv = 0)");
-  return 0;
-}
 
 // The chunk's global rows [first_row, first_row + T + keep_init) within the T_total + 1 of the series.
 static int scan_dist_rows(bdlm_ctx *c, const bdlm_problem *p, int rank, int64_t first_row, int64_t total_T) {
@@ -1564,19 +1571,6 @@ static int scan_dist_rows(bdlm_ctx *c, const bdlm_problem *p, int rank, int64_t 
   if (first_row + p->T + (p->keep_init ? 1 : 0) > total_T + 1)
     return fail(c, BDLM_E_ARG, "time-sharded FFBS: first_row + rows > total_T + 1");
   return 0;
-}
-
-static std::vector<double> scan_prior(const bdlm_problem *p) {
-  std::vector<double> prior((size_t)p->n + p->n * p->n);
-  std::copy(p->m0, p->m0 + p->n, prior.begin());
-  std::copy(p->C0, p->C0 + p->n * p->n, prior.begin() + p->n);
-  return prior;
-}
-
-// the status the sampler's phases OR into: the caller's, or the arena's own slot
-static int32_t *scan_dist_status(bdlm_ctx *c, size_t ws, const bdlm_problem *p, int32_t *status) {
-  if (status) return status;
-  return reinterpret_cast<int32_t *>(c->arena + 2 * ws + align_up(scan_ffbs_parts_bytes(p->n, p->T)));
 }
 
 int bdlm_scan_dist_doubles(int32_t n, int32_t what) {
@@ -1594,8 +1588,8 @@ int bdlm_scan_dist_loglik_partial(bdlm_ctx *c, const bdlm_problem *p, int32_t ra
   NvtxRange nvtx_("bdlm_scan_dist_loglik_partial");
   int rc = scan_dist_args(c, p, rank, world);
   if (rc) return rc;
-  size_t ws;
-  rc = scan_dist_common(c, p, nullptr, rank, world, &ws);
+  ScanArena ar;
+  rc = scan_dist_common(c, p, ar);
   if (rc) return rc;
   if (!aggs_dev || !part_dev) return fail(c, BDLM_E_ARG, "null aggregates or partial-vector pointer");
   const std::vector<double> prior = scan_prior(p);
@@ -1603,9 +1597,9 @@ int bdlm_scan_dist_loglik_partial(bdlm_ctx *c, const bdlm_problem *p, int32_t ra
   rc = scan_fill(c, p, a);
   if (rc) return rc;
   a.phase = kScanDistFinish; a.aggs_dev = aggs_dev; a.rank = rank; a.world = world;
-  a.start = prior.data(); a.workspace = c->arena;
+  a.start = prior.data(); a.workspace = ar.ws;
   ScanLoglikOut o{};
-  o.m_last = m_last; o.C_last = C_last; o.parts = c->arena + ws; o.part_vec = part_dev;
+  o.m_last = m_last; o.C_last = C_last; o.parts = ar.parts; o.part_vec = part_dev;
   CU(launch_scan_dist_loglik(a, o, c->stream, &c->launches));
   return 0;
 }
@@ -1623,18 +1617,18 @@ int bdlm_scan_dist_loglik_finish(bdlm_ctx *c, int32_t world, const double *parts
 
 // Arguments of both sampler phases: the forward finish phase's, with (m, C) into kf and no smoother fold.
 static int scan_dist_ffbs_fill(bdlm_ctx *c, const bdlm_problem *p, int rank, int world, const bdlm_kf_out *kf,
-                               double *theta, size_t ws, int32_t *status, const std::vector<double> &prior,
+                               double *theta, const ScanArena &ar, int32_t *status, const std::vector<double> &prior,
                                bool forward, ScanArgs &a, ScanFfbsOut &o) {
   int rc = scan_fill(c, p, a, forward);
   if (rc) return rc;
   a.phase = kScanDistFinish; a.rank = rank; a.world = world; a.has_successor = rank < world - 1;
-  a.start = prior.data(); a.kf = scan_kf_views(p, kf); a.status = status; a.workspace = c->arena;
+  a.start = prior.data(); a.kf = scan_kf_views(p, kf); a.status = status; a.workspace = ar.ws;
   const int64_t n = p->n, R = rows_of(*p);
   o = ScanFfbsOut{};
   o.theta = mk_view(theta, p->layout, 0, 1, R, n);
   o.rng_seed = c->rng_seed; o.rng_sweep = c->rng_sweep; o.rng_base = c->rng_first;
-  o.workspace = c->arena + ws;
-  o.parts = reinterpret_cast<double *>(c->arena + 2 * ws);
+  o.workspace = ar.ws2;
+  o.parts = ar.parts;
   return 0;
 }
 
@@ -1644,27 +1638,24 @@ int bdlm_scan_dist_ffbs_local(bdlm_ctx *c, const bdlm_problem *p, int32_t rank, 
   NvtxRange nvtx_("bdlm_scan_dist_ffbs_local");
   int rc = scan_dist_args(c, p, rank, world);
   if (!rc) rc = scan_dist_rows(c, p, rank, first_row, total_T);
+  if (!rc) rc = scan_dist_kf(c, kf);
   if (rc) return rc;
-  if (!kf || !kf->m || !kf->C) return fail(c, BDLM_E_ARG, "time-sharded FFBS needs kf->m and kf->C");
-  size_t ws;
-  rc = scan_dist_common(c, p, kf, rank, world, &ws);
+  ScanArena ar;
+  rc = scan_dist_common(c, p, ar);
   if (rc) return rc;
   if (!aggs_dev || !agg_dev || !theta) return fail(c, BDLM_E_ARG, "null aggregate pointer or theta");
-  int32_t *st = scan_dist_status(c, ws, p, status);
+  int32_t *st = status ? status : ar.status;
   const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
   ScanFfbsOut o;
-  rc = scan_dist_ffbs_fill(c, p, rank, world, kf, theta, ws, st, prior, true, a, o);
+  rc = scan_dist_ffbs_fill(c, p, rank, world, kf, theta, ar, st, prior, true, a, o);
   if (rc) return rc;
   a.aggs_dev = aggs_dev;
   o.z = mk_cview(z, p->layout, 0, 1, rows_of(*p), p->n);
   o.total_rows = total_T + 1; o.first_row = first_row;
   o.agg_dev = agg_dev;
   CU(cudaMemsetAsync(st, 0, sizeof(int32_t), c->stream));
-  CU(launch_scan_dist_ffbs(a, o, false, c->stream, &c->launches));
-  if (a.table_upload) c->scan_key.swap(c->scan_key_pending);
-  c->scan_key_pending.clear();
-  return 0;
+  return scan_table_commit(c, a, launch_scan_dist_ffbs(a, o, false, c->stream, &c->launches));
 }
 
 int bdlm_scan_dist_ffbs_finish(bdlm_ctx *c, const bdlm_problem *p, int32_t rank, int32_t world,
@@ -1672,17 +1663,17 @@ int bdlm_scan_dist_ffbs_finish(bdlm_ctx *c, const bdlm_problem *p, int32_t rank,
                                int32_t *status) {
   NvtxRange nvtx_("bdlm_scan_dist_ffbs_finish");
   int rc = scan_dist_args(c, p, rank, world);
+  if (!rc) rc = scan_dist_kf(c, kf);
   if (rc) return rc;
-  if (!kf || !kf->m || !kf->C) return fail(c, BDLM_E_ARG, "time-sharded FFBS needs kf->m and kf->C");
-  size_t ws;
-  rc = scan_dist_common(c, p, kf, rank, world, &ws);
+  ScanArena ar;
+  rc = scan_dist_common(c, p, ar);
   if (rc) return rc;
   if (!aggs_dev || !part_dev || !theta) return fail(c, BDLM_E_ARG, "null aggregates, partial vector or theta");
-  int32_t *st = scan_dist_status(c, ws, p, status);
+  int32_t *st = status ? status : ar.status;
   const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
   ScanFfbsOut o;
-  rc = scan_dist_ffbs_fill(c, p, rank, world, kf, theta, ws, st, prior, false, a, o);  // no table needed
+  rc = scan_dist_ffbs_fill(c, p, rank, world, kf, theta, ar, st, prior, false, a, o);  // no table needed
   if (rc) return rc;
   o.aggs_dev = aggs_dev; o.part_vec = part_dev;
   CU(launch_scan_dist_ffbs(a, o, true, c->stream, &c->launches));

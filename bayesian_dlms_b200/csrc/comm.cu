@@ -595,14 +595,12 @@ int bdlm_comm_svd_ffbs(bdlm_comm *m, const bdlm_problem *p, const double *z, dou
 // the contexts' streams; call bdlm_sync on the contexts (or bdlm_comm_sync) before reading.
 int bdlm_comm_scan_filter_smooth(bdlm_comm *m, const bdlm_problem *probs, const bdlm_kf_out *kfs,
                                  const bdlm_smooth_out *sms, int32_t *const *status) {
-  if (!m) return cfail(nullptr, BDLM_E_ARG, "null communicator");
-  if (!probs || !kfs || !sms) return cfail(m, BDLM_E_ARG, "null problem / output arrays");
+  int rc = check_scan_chunks(m, probs, nullptr, 0);
+  if (rc) return rc;
+  if (!kfs || !sms) return cfail(m, BDLM_E_ARG, "null output arrays");
   Nccl *nc = nccl();
   const int W = m->world;
   const int n = probs[0].n;
-  if (n < 1 || n > 4) return cfail(m, BDLM_E_ARG, "scan path: n <= 4");
-  for (size_t i = 1; i < m->loc.size(); ++i)
-    if (probs[i].n != n) return cfail(m, BDLM_E_ARG, "time-sharded scan: every chunk describes the same model (n differs)");
   const int ef = bdlm_scan_elem_doubles(n, 0), eb = bdlm_scan_elem_doubles(n, 1);
   // Every device's phases are enqueued by its own host thread: local scan -> exchange -> finish,
   // forwards then backwards.  With peer mailboxes nothing on the host couples the devices (the

@@ -27,6 +27,7 @@
 // that is the reference itself); the apply phases reuse the sequential step code, so the
 // only difference is the rounding of the scanned start states.
 #include <cmath>
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -1589,15 +1590,20 @@ int apply_slots() {
   return slots;
 }
 
-int scan_rows_per_thread(int n, int64_t T) {
-  int slots = 444;
+// f(std::integral_constant<int, N>{}) for the scan's state dimension n = N (1..4), else `none`.
+template <class R, class F>
+R with_n(int n, R none, F &&f) {
   switch (n) {
-    case 1: slots = apply_slots<1>(); break;
-    case 2: slots = apply_slots<2>(); break;
-    case 3: slots = apply_slots<3>(); break;
-    case 4: slots = apply_slots<4>(); break;
-    default: break;
+    case 1: return f(std::integral_constant<int, 1>{});
+    case 2: return f(std::integral_constant<int, 2>{});
+    case 3: return f(std::integral_constant<int, 3>{});
+    case 4: return f(std::integral_constant<int, 4>{});
+    default: return none;
   }
+}
+
+int scan_rows_per_thread(int n, int64_t T) {
+  const int slots = with_n(n, 444, [](auto N) { return apply_slots<N>(); });
   const double rows = (double)(T + 1);
   int best = kSub;
   double best_cost = 1e300;
@@ -1615,6 +1621,52 @@ int scan_rows_per_thread(int n, int64_t T) {
   }
   return best;
 }
+
+// ---- geometry and workspace layout of one pass over a chunk ------------------------------------
+enum ScanPass { kPassForward, kPassLoglik, kPassBackward, kPassSampler };
+
+// `sub` rows per thread over the `rows` the sweep walks, M level-1 threads (their elements X[0, M),
+// then the slot X[M]), the apply grid for the pass's block size and the level-2 blocks over
+// X[0, M].  A finish phase finds its local phase's prefixes where this puts them because both
+// derive the geometry here from the same chunk.
+struct ScanGeom {
+  int sub;
+  int64_t rows, M, nb;
+  unsigned blocks;
+};
+ScanGeom scan_geom(int n, int64_t T, int keep_init, bool has_successor, ScanPass pass) {
+  ScanGeom g;
+  g.sub = scan_rows_per_thread(n, T);
+  // the forward passes walk every row, the backward ones the rows with a successor in the chunk
+  const bool forward = pass == kPassForward || pass == kPassLoglik;
+  g.rows = T + keep_init - (forward || has_successor ? 0 : 1);
+  g.M = (g.rows + g.sub - 1) / g.sub;
+  if (pass == kPassSampler && g.M < 1) g.M = 1;  // the last chunk may hold a single row
+  const int block = pass == kPassLoglik ? kLlBlock : pass == kPassSampler ? kFbBlock : 128;
+  g.blocks = (unsigned)((g.M + block - 1) / block);
+  g.nb = (g.M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);
+  return g;
+}
+ScanGeom scan_geom(const ScanArgs &a, ScanPass pass) {
+  return scan_geom(a.n, a.T, a.keep_init, a.has_successor != 0, pass);
+}
+
+// Block totals device_scan leaves after the `count` elements it scans, over all its levels.
+int64_t level2_elems(int64_t count) {
+  constexpr int64_t per_block = kScanBlock * kPer;
+  int64_t s = 0;
+  for (int64_t nb = (count + per_block - 1) / per_block; nb > 1; nb = (nb + per_block - 1) / per_block) s += nb;
+  return s;
+}
+
+// Workspace of one pass: X [M + 1], the level-2 block totals, and the carry of the other chunks.
+template <class E>
+struct ScanLayout {
+  E *X, *scratch, *carry;
+  ScanLayout(const ScanGeom &g, void *base)
+      : X(reinterpret_cast<E *>(base)), scratch(X + (g.M + 1)), carry(scratch + level2_elems(g.M + 1)) {}
+  static size_t bytes(const ScanGeom &g) { return sizeof(E) * (size_t)(g.M + 2 + level2_elems(g.M + 1)); }
+};
 
 template <int N>
 ScanModel<N> make_model(const ScanArgs &a) {
@@ -1648,39 +1700,33 @@ cudaError_t fwd_table_upload(const ScanArgs &a, const ScanModel<N> &md, cudaStre
 // the top level's block prefixes left in scratch (defer_top).  identity: slot 0 is the identity
 // (chunk aggregate only), else the state st0 before the first observation.
 template <int N>
-cudaError_t fwd_prefixes(const ScanArgs &a, const ScanModel<N> &md, int64_t M, FElem<N> *X,
-                         FElem<N> *scratch, const StateArg<N> &st0, bool identity, int sub,
-                         cudaStream_t stream, int64_t *launches) {
+cudaError_t fwd_prefixes(const ScanArgs &a, const ScanModel<N> &md, const ScanGeom &g, const ScanLayout<FElem<N>> &w,
+                         const StateArg<N> &st0, bool identity, cudaStream_t stream, int64_t *launches) {
   const FwdTable<N> *tb = reinterpret_cast<const FwdTable<N> *>(a.table);
-  const unsigned blocks = (unsigned)((M + 127) / 128);
+  const unsigned blocks = (unsigned)((g.M + 127) / 128);
   if ((reinterpret_cast<uintptr_t>(a.y) & 31) == 0)
-    fwd_reduce_kernel<N, true><<<blocks, 128, 0, stream>>>(md, tb, a.y, a.T, M, a.keep_init, X, st0, identity, sub);
+    fwd_reduce_kernel<N, true><<<blocks, 128, 0, stream>>>(md, tb, a.y, a.T, g.M, a.keep_init, w.X, st0, identity, g.sub);
   else
-    fwd_reduce_kernel<N, false><<<blocks, 128, 0, stream>>>(md, tb, a.y, a.T, M, a.keep_init, X, st0, identity, sub);
+    fwd_reduce_kernel<N, false><<<blocks, 128, 0, stream>>>(md, tb, a.y, a.T, g.M, a.keep_init, w.X, st0, identity, g.sub);
   ++*launches;
   CK(cudaGetLastError());
-  return device_scan<FElem<N>, false, false>(X, M + 1, scratch, stream, launches, /*defer_top=*/true);
+  return device_scan<FElem<N>, false, false>(w.X, g.M + 1, w.scratch, stream, launches, /*defer_top=*/true);
 }
 
 template <int N>
 cudaError_t scan_forward(const ScanArgs &a, cudaStream_t stream, int64_t *launches) {
   const ScanModel<N> md = make_model<N>(a);
-  const int sub = scan_rows_per_thread(a.n, a.T);
-  const int64_t T = a.T, M = (T + a.keep_init + sub - 1) / sub;
-  FElem<N> *X = reinterpret_cast<FElem<N> *>(a.workspace);       // [M + 1]
-  FElem<N> *scratch = X + (M + 1);                                // block totals
-  const unsigned blocks = (unsigned)((M + 127) / 128);
-  const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);  // level-2 blocks over X
+  const ScanGeom g = scan_geom(a, kPassForward);
+  const ScanLayout<FElem<N>> w(g, a.workspace);
   CK(fwd_table_upload<N>(a, md, stream));
   const bool local = a.phase == kScanDistLocal, finish = a.phase == kScanDistFinish;
-  FElem<N> *carry = reinterpret_cast<FElem<N> *>(scratch + (M + 1) / kScanBlock * 2 + 8);
   if (!finish) {
     // dist local: chunk aggregate only (identity start); apply: prefix of
     // (start (x) aggregates), a.start = host (m, C) of the state before t = 0
     const StateArg<N> st0 = state_arg<N>(local ? nullptr : a.start);
-    CK(fwd_prefixes<N>(a, md, M, X, scratch, st0, local, sub, stream, launches));
+    CK(fwd_prefixes<N>(a, md, g, w, st0, local, stream, launches));
     // the whole chunk: last element of a one-block scan, else the last scanned block total
-    const FElem<N> *whole = nb > 1 ? scratch + (nb - 1) : X + M;
+    const FElem<N> *whole = g.nb > 1 ? w.scratch + (g.nb - 1) : w.X + g.M;
     if (local) {
       if (a.peers.world > 0) {  // straight into every peer's mailbox over NVLink
         publish_kernel<FElem<N>><<<a.peers.world, 64, 0, stream>>>(whole, a.peers, a.rank, a.epoch_dev);
@@ -1693,7 +1739,7 @@ cudaError_t scan_forward(const ScanArgs &a, cudaStream_t stream, int64_t *launch
   } else {
     // X still holds this rank's scanned prefixes from the local phase
     fold_forward_kernel<N><<<1, 1, 0, stream>>>(reinterpret_cast<const FElem<N> *>(a.aggs_dev),
-                                                a.rank, state_arg<N>(a.start), carry, a.peers,
+                                                a.rank, state_arg<N>(a.start), w.carry, a.peers,
                                                 a.epoch_dev, a.status);
     ++*launches;
   }
@@ -1704,12 +1750,12 @@ cudaError_t scan_forward(const ScanArgs &a, cudaStream_t stream, int64_t *launch
   // a.fuse_sagg: the caller runs the smoother next on the same rows: fold the smoothing
   // elements here so the backward pass starts from ready level-1 aggregates.
   SElem<N> *sagg = reinterpret_cast<SElem<N> *>(a.fuse_sagg);
-  const int64_t nrows = T + a.keep_init - (a.has_successor ? 0 : 1);
-  const FElem<N> *cr = finish ? carry : nullptr;
-  const FElem<N> *tot = nb > 1 ? scratch : nullptr;  // top-level block prefixes, composed by the sweep
-#define BDLM_FWD_APPLY(VEC_, FUSE_)                                                         \
-  fwd_apply_kernel<N, VEC_, FUSE_><<<blocks, 128, 0, stream>>>(md, a.y, T, M, X, a.keep_init, \
-                                                               a.kf, a.status, sagg, nrows, cr, tot, sub)
+  const int64_t nrows = scan_geom(a, kPassBackward).rows;  // the smoother's rows
+  const FElem<N> *cr = finish ? w.carry : nullptr;
+  const FElem<N> *tot = g.nb > 1 ? w.scratch : nullptr;  // top-level block prefixes, composed by the sweep
+#define BDLM_FWD_APPLY(VEC_, FUSE_)                                                                 \
+  fwd_apply_kernel<N, VEC_, FUSE_><<<g.blocks, 128, 0, stream>>>(md, a.y, a.T, g.M, w.X, a.keep_init, \
+                                                                 a.kf, a.status, sagg, nrows, cr, tot, g.sub)
   if (vec && sagg) BDLM_FWD_APPLY(true, true);
   else if (vec) BDLM_FWD_APPLY(true, false);
   else if (sagg) BDLM_FWD_APPLY(false, true);
@@ -1725,21 +1771,17 @@ template <int N>
 cudaError_t scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream, int64_t *launches) {
   if (a.keep_init != 1 || a.phase != kScanApply) return cudaErrorInvalidValue;
   const ScanModel<N> md = make_model<N>(a);
-  const int sub = scan_rows_per_thread(a.n, a.T);
-  const int64_t T = a.T, M = (T + 1 + sub - 1) / sub;
-  FElem<N> *X = reinterpret_cast<FElem<N> *>(a.workspace);
-  FElem<N> *scratch = X + (M + 1);
-  const unsigned blocks = (unsigned)((M + kLlBlock - 1) / kLlBlock);
-  const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);
+  const ScanGeom g = scan_geom(a, kPassLoglik);
+  const ScanLayout<FElem<N>> w(g, a.workspace);
   LoglikPart *part = reinterpret_cast<LoglikPart *>(o.parts);
-  double *last = reinterpret_cast<double *>(part + blocks);
+  double *last = reinterpret_cast<double *>(part + g.blocks);
   CK(fwd_table_upload<N>(a, md, stream));
-  CK(fwd_prefixes<N>(a, md, M, X, scratch, state_arg<N>(a.start), false, sub, stream, launches));
-  const FElem<N> *tot = nb > 1 ? scratch : nullptr;
+  CK(fwd_prefixes<N>(a, md, g, w, state_arg<N>(a.start), false, stream, launches));
+  const FElem<N> *tot = g.nb > 1 ? w.scratch : nullptr;
   const bool vec = (reinterpret_cast<uintptr_t>(a.y) & 31) == 0, tr = o.transition != nullptr;
 #define BDLM_LL_SWEEP(VEC_, TR_)                                                                    \
-  fwd_loglik_kernel<N, VEC_, TR_, false><<<blocks, kLlBlock, 0, stream>>>(md, a.y, T, M, X, tot, sub, part, \
-                                                                          last, 1, nullptr)
+  fwd_loglik_kernel<N, VEC_, TR_, false><<<g.blocks, kLlBlock, 0, stream>>>(md, a.y, a.T, g.M, w.X, tot, g.sub, \
+                                                                            part, last, 1, nullptr)
   if (vec && tr) BDLM_LL_SWEEP(true, true);
   else if (vec) BDLM_LL_SWEEP(true, false);
   else if (tr) BDLM_LL_SWEEP(false, true);
@@ -1747,7 +1789,7 @@ cudaError_t scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t 
 #undef BDLM_LL_SWEEP
   ++*launches;
   CK(cudaGetLastError());
-  loglik_finish_kernel<<<1, kLlFinish, 0, stream>>>(part, blocks, last, N, o.transition, o.innovations,
+  loglik_finish_kernel<<<1, kLlFinish, 0, stream>>>(part, g.blocks, last, N, o.transition, o.innovations,
                                                      o.m_last, o.C_last, o.status, nullptr);
   ++*launches;
   return cudaGetLastError();
@@ -1762,54 +1804,28 @@ template <int N>
 cudaError_t scan_dist_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream, int64_t *launches) {
   if (a.phase != kScanDistFinish) return cudaErrorInvalidValue;
   const ScanModel<N> md = make_model<N>(a);
-  const int sub = scan_rows_per_thread(a.n, a.T);
-  const int64_t T = a.T, M = (T + a.keep_init + sub - 1) / sub;  // as the local phase
-  FElem<N> *X = reinterpret_cast<FElem<N> *>(a.workspace);
-  FElem<N> *scratch = X + (M + 1);
-  FElem<N> *carry = reinterpret_cast<FElem<N> *>(scratch + (M + 1) / kScanBlock * 2 + 8);
-  const unsigned blocks = (unsigned)((M + kLlBlock - 1) / kLlBlock);
-  const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);
+  const ScanGeom g = scan_geom(a, kPassLoglik);
+  const ScanLayout<FElem<N>> w(g, a.workspace);
   LoglikPart *part = reinterpret_cast<LoglikPart *>(o.parts);
-  double *last = reinterpret_cast<double *>(part + blocks);
+  double *last = reinterpret_cast<double *>(part + g.blocks);
   const bool holds_last = a.rank == a.world - 1;
   fold_forward_kernel<N><<<1, 1, 0, stream>>>(reinterpret_cast<const FElem<N> *>(a.aggs_dev), a.rank,
-                                              state_arg<N>(a.start), carry, ScanPeers{}, nullptr, nullptr);
+                                              state_arg<N>(a.start), w.carry, ScanPeers{}, nullptr, nullptr);
   ++*launches;
   CK(cudaGetLastError());
-  const FElem<N> *tot = nb > 1 ? scratch : nullptr;
+  const FElem<N> *tot = g.nb > 1 ? w.scratch : nullptr;
   if ((reinterpret_cast<uintptr_t>(a.y) & 31) == 0)
-    fwd_loglik_kernel<N, true, true, true><<<blocks, kLlBlock, 0, stream>>>(md, a.y, T, M, X, tot, sub, part, last,
-                                                                            a.keep_init, carry);
+    fwd_loglik_kernel<N, true, true, true><<<g.blocks, kLlBlock, 0, stream>>>(md, a.y, a.T, g.M, w.X, tot, g.sub,
+                                                                              part, last, a.keep_init, w.carry);
   else
-    fwd_loglik_kernel<N, false, true, true><<<blocks, kLlBlock, 0, stream>>>(md, a.y, T, M, X, tot, sub, part,
-                                                                             last, a.keep_init, carry);
+    fwd_loglik_kernel<N, false, true, true><<<g.blocks, kLlBlock, 0, stream>>>(md, a.y, a.T, g.M, w.X, tot, g.sub,
+                                                                               part, last, a.keep_init, w.carry);
   ++*launches;
   CK(cudaGetLastError());
-  loglik_finish_kernel<<<1, kLlFinish, 0, stream>>>(part, blocks, holds_last ? last : nullptr, N, o.part_vec,
+  loglik_finish_kernel<<<1, kLlFinish, 0, stream>>>(part, g.blocks, holds_last ? last : nullptr, N, o.part_vec,
                                                      o.part_vec + 1, o.m_last, o.C_last, nullptr, o.part_vec + 2);
   ++*launches;
   return cudaGetLastError();
-}
-
-// Rows of the sampler on a chunk: rows 0 .. nsucc-1 have a successor (all of them when another chunk
-// follows), row nsucc is the series' last when `terminal`.  At least one thread: the last chunk may
-// hold a single row.
-struct SamplerShape {
-  int sub;
-  int64_t nsucc, M, nb;
-  unsigned blocks;
-  bool terminal;
-};
-SamplerShape sampler_shape(const ScanArgs &a) {
-  SamplerShape s;
-  s.sub = scan_rows_per_thread(a.n, a.T);
-  s.terminal = !a.has_successor;
-  s.nsucc = a.T + a.keep_init - (s.terminal ? 1 : 0);
-  s.M = (s.nsucc + s.sub - 1) / s.sub;
-  if (s.M < 1) s.M = 1;
-  s.blocks = (unsigned)((s.M + kFbBlock - 1) / kFbBlock);
-  s.nb = (s.M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);
-  return s;
 }
 
 template <int N>
@@ -1819,45 +1835,47 @@ bool sampler_vec(const ScanArgs &a, const ScanFfbsOut &o) {
 }
 
 // The sampler's level 1 (elements, c_r into theta, the terminal slot) and its level-2 suffix scan.
+// Rows 0 .. g.rows - 1 have a successor (all of them when another chunk follows); row g.rows is the
+// series' last when no chunk follows (`terminal`).
 template <int N>
-cudaError_t sampler_prefixes(const ScanArgs &a, const ScanFfbsOut &o, const SamplerShape &s, cudaStream_t stream,
+cudaError_t sampler_prefixes(const ScanArgs &a, const ScanFfbsOut &o, const ScanGeom &g, cudaStream_t stream,
                              int64_t *launches) {
   const ScanModel<N> md = make_model<N>(a);
-  BElem<N> *X = reinterpret_cast<BElem<N> *>(o.workspace);  // [M + 1]
-  BElem<N> *scratch = X + (s.M + 1);
+  const ScanLayout<BElem<N>> w(g, o.workspace);
   const FfbsRng rng{o.rng_seed, o.rng_sweep, o.rng_base, o.total_rows, o.first_row};
-  const int64_t term = s.terminal ? s.nsucc : -1;
+  const bool terminal = !a.has_successor;
+  const int64_t term = terminal ? g.rows : -1;
   if (sampler_vec<N>(a, o))
-    ffbs_reduce_kernel<N, true><<<s.blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, s.nsucc, s.M, o.z, rng,
-                                                                    o.theta, X, a.status, s.sub, term);
+    ffbs_reduce_kernel<N, true><<<g.blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, g.rows, g.M, o.z, rng,
+                                                                    o.theta, w.X, a.status, g.sub, term);
   else
-    ffbs_reduce_kernel<N, false><<<s.blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, s.nsucc, s.M, o.z, rng,
-                                                                     o.theta, X, a.status, s.sub, term);
+    ffbs_reduce_kernel<N, false><<<g.blocks, kFbBlock, 0, stream>>>(md, a.kf.m, a.kf.C, g.rows, g.M, o.z, rng,
+                                                                     o.theta, w.X, a.status, g.sub, term);
   ++*launches;
   CK(cudaGetLastError());
   // a chunk that others follow: the terminal slot is the identity, so its aggregate leaves the later
   // chunks to the carry; a last chunk of one row: its one thread folded no row
-  if (!s.terminal || s.nsucc == 0) {
-    set_b_identity<N><<<1, 1, 0, stream>>>(s.terminal ? X : X + s.M);
+  if (!terminal || g.rows == 0) {
+    set_b_identity<N><<<1, 1, 0, stream>>>(terminal ? w.X : w.X + g.M);
     ++*launches;
     CK(cudaGetLastError());
   }
-  return device_scan<BElem<N>, true, true>(X, s.M + 1, scratch, stream, launches, /*defer_top=*/true);
+  return device_scan<BElem<N>, true, true>(w.X, g.M + 1, w.scratch, stream, launches, /*defer_top=*/true);
 }
 
 // The apply sweep from the scanned suffixes (and the carry of later chunks), then, with statistics,
 // the fixed-order sum of its block partials into `stats` or into the rank's partial vector `vec`.
 template <int N>
-cudaError_t sampler_apply(const ScanArgs &a, const ScanFfbsOut &o, const SamplerShape &s, const BElem<N> *carry,
+cudaError_t sampler_apply(const ScanArgs &a, const ScanFfbsOut &o, const ScanGeom &g, const BElem<N> *carry,
                           bool stats, double *vec, cudaStream_t stream, int64_t *launches) {
   const ScanModel<N> md = make_model<N>(a);
-  const BElem<N> *X = reinterpret_cast<const BElem<N> *>(o.workspace);
-  const BElem<N> *tot = s.nb > 1 ? X + (s.M + 1) : nullptr;
-  const bool vec_io = sampler_vec<N>(a, o);
-#define BDLM_FFBS_SWEEP(VEC_, STATS_)                                                                         \
-  ffbs_apply_kernel<N, VEC_, STATS_><<<s.blocks, kFbBlock, 0, stream>>>(                                      \
-      md, a.kf.m, a.kf.C, a.y, s.nsucc, s.M, X, tot, o.theta, a.status, s.sub, o.parts, carry, a.keep_init, a.T, \
-      s.terminal)
+  const ScanLayout<BElem<N>> w(g, o.workspace);
+  const BElem<N> *tot = g.nb > 1 ? w.scratch : nullptr;
+  const bool vec_io = sampler_vec<N>(a, o), terminal = !a.has_successor;
+#define BDLM_FFBS_SWEEP(VEC_, STATS_)                                                                          \
+  ffbs_apply_kernel<N, VEC_, STATS_><<<g.blocks, kFbBlock, 0, stream>>>(                                       \
+      md, a.kf.m, a.kf.C, a.y, g.rows, g.M, w.X, tot, o.theta, a.status, g.sub, o.parts, carry, a.keep_init, a.T, \
+      terminal)
   if (vec_io && stats) BDLM_FFBS_SWEEP(true, true);
   else if (vec_io) BDLM_FFBS_SWEEP(true, false);
   else if (stats) BDLM_FFBS_SWEEP(false, true);
@@ -1866,7 +1884,7 @@ cudaError_t sampler_apply(const ScanArgs &a, const ScanFfbsOut &o, const Sampler
   ++*launches;
   CK(cudaGetLastError());
   if (stats) {
-    ffbs_stats_finish_kernel<N><<<1, kFbFinish, 0, stream>>>(o.parts, s.blocks, o.stats, vec, a.status);
+    ffbs_stats_finish_kernel<N><<<1, kFbFinish, 0, stream>>>(o.parts, g.blocks, o.stats, vec, a.status);
     ++*launches;
   }
   return cudaGetLastError();
@@ -1879,11 +1897,11 @@ template <int N>
 cudaError_t scan_ffbs(const ScanArgs &a, const ScanFfbsOut &o, cudaStream_t stream, int64_t *launches) {
   if (a.keep_init != 1 || a.phase != kScanApply || a.fuse_sagg || a.has_successor) return cudaErrorInvalidValue;
   CK(scan_forward<N>(a, stream, launches));
-  const SamplerShape s = sampler_shape(a);
-  CK(sampler_prefixes<N>(a, o, s, stream, launches));
+  const ScanGeom g = scan_geom(a, kPassSampler);
+  CK(sampler_prefixes<N>(a, o, g, stream, launches));
   const StatViews &sv = o.stats;
   const bool stats = sv.ssy.ptr || sv.ny.ptr || sv.ssw.ptr || sv.scatter.ptr;
-  return sampler_apply<N>(a, o, s, nullptr, stats, nullptr, stream, launches);
+  return sampler_apply<N>(a, o, g, nullptr, stats, nullptr, stream, launches);
 }
 
 // One rank's chunk of a time-sharded FFBS.  Local (a.phase = kScanDistFinish of the forward pass): the
@@ -1894,55 +1912,45 @@ template <int N>
 cudaError_t scan_dist_ffbs(const ScanArgs &a, const ScanFfbsOut &o, bool finish, cudaStream_t stream,
                            int64_t *launches) {
   if (a.phase != kScanDistFinish || a.fuse_sagg) return cudaErrorInvalidValue;
-  const SamplerShape s = sampler_shape(a);
-  BElem<N> *X = reinterpret_cast<BElem<N> *>(o.workspace);
-  BElem<N> *scratch = X + (s.M + 1);
-  BElem<N> *carry = scratch + (s.M + 1) / kScanBlock * 2 + 8;
+  const ScanGeom g = scan_geom(a, kPassSampler);
+  const ScanLayout<BElem<N>> w(g, o.workspace);
   if (!finish) {
     CK(scan_forward<N>(a, stream, launches));
-    CK(sampler_prefixes<N>(a, o, s, stream, launches));
-    const BElem<N> *whole = s.nb > 1 ? scratch + (s.nb - 1) : X;  // suffix scan ends at index 0
+    CK(sampler_prefixes<N>(a, o, g, stream, launches));
+    const BElem<N> *whole = g.nb > 1 ? w.scratch + (g.nb - 1) : w.X;  // suffix scan ends at index 0
     return cudaMemcpyAsync(o.agg_dev, whole, sizeof(BElem<N>), cudaMemcpyDeviceToDevice, stream);
   }
   if (a.has_successor) {
     fold_sampler_kernel<N><<<1, 1, 0, stream>>>(reinterpret_cast<const BElem<N> *>(o.aggs_dev), a.rank, a.world,
-                                                carry);
+                                                w.carry);
     ++*launches;
     CK(cudaGetLastError());
   }
-  return sampler_apply<N>(a, o, s, a.has_successor ? carry : nullptr, true, o.part_vec, stream, launches);
+  return sampler_apply<N>(a, o, g, a.has_successor ? w.carry : nullptr, true, o.part_vec, stream, launches);
 }
 
 template <int N>
 cudaError_t scan_backward(const ScanArgs &a, cudaStream_t stream, int64_t *launches) {
   const ScanModel<N> md = make_model<N>(a);
-  const int64_t rows = a.T + a.keep_init;
   // rows with a successor inside this chunk: all but the last, plus the last when the chunk
   // is followed by another one (has_successor)
-  const int64_t nrows = a.has_successor ? rows : rows - 1;
-  const int sub = scan_rows_per_thread(a.n, a.T);
-  const int64_t M = (nrows + sub - 1) / sub;
-  SElem<N> *X = reinterpret_cast<SElem<N> *>(a.workspace);  // [M + 1]
-  SElem<N> *scratch = X + (M + 1);
-  double *term_dev = reinterpret_cast<double *>(scratch + (M + 1) / kScanBlock * 2 + 8);
-  const unsigned blocks = (unsigned)((M + 127) / 128);
-  const int64_t nb = (M + 1 + kScanBlock * kPer - 1) / (kScanBlock * kPer);  // level-2 blocks over X
+  const ScanGeom g = scan_geom(a, kPassBackward);
+  const ScanLayout<SElem<N>> w(g, a.workspace);
   const bool local = a.phase == kScanDistLocal, finish = a.phase == kScanDistFinish;
   const bool vec = dense_aligned(a.kf.m, N) && dense_aligned(a.kf.C, N * N) &&
                    dense_aligned(a.s, N) && dense_aligned(a.S, N * N);
-  SElem<N> *carry = reinterpret_cast<SElem<N> *>(term_dev + 64);
   if (!finish) {
     // X[0, M) already holds the level-1 aggregates, written by the forward apply sweep (fuse_sagg)
     if (a.has_successor) {  // dist local of a chunk followed by others
-      set_s_identity<N><<<1, 1, 0, stream>>>(X + M);
-    } else {  // last chunk: s_T = m_T, S_T = C_T (Smoothing.scala:59-61)
-      terminal_from_last_row<N><<<1, 1, 0, stream>>>(a.kf.m, a.kf.C, rows - 1, a.s, a.S, X + M,
-                                                     M == 0 ? a.status : nullptr);
+      set_s_identity<N><<<1, 1, 0, stream>>>(w.X + g.M);
+    } else {  // last chunk: s_T = m_T, S_T = C_T at its last row, g.rows (Smoothing.scala:59-61)
+      terminal_from_last_row<N><<<1, 1, 0, stream>>>(a.kf.m, a.kf.C, g.rows, a.s, a.S, w.X + g.M,
+                                                     g.M == 0 ? a.status : nullptr);
     }
     ++*launches;
     CK(cudaGetLastError());
-    CK((device_scan<SElem<N>, true, true>(X, M + 1, scratch, stream, launches, /*defer_top=*/true)));
-    const SElem<N> *whole = nb > 1 ? scratch + (nb - 1) : X;  // the whole chunk (suffix scan ends at index 0)
+    CK((device_scan<SElem<N>, true, true>(w.X, g.M + 1, w.scratch, stream, launches, /*defer_top=*/true)));
+    const SElem<N> *whole = g.nb > 1 ? w.scratch + (g.nb - 1) : w.X;  // the whole chunk (suffix scan ends at index 0)
     if (local) {
       if (a.peers.world > 0) {
         publish_kernel<SElem<N>><<<a.peers.world, 64, 0, stream>>>(whole, a.peers, a.rank, a.epoch_dev);
@@ -1953,16 +1961,18 @@ cudaError_t scan_backward(const ScanArgs &a, cudaStream_t stream, int64_t *launc
     }
   } else if (a.has_successor) {
     fold_backward_kernel<N><<<1, 1, 0, stream>>>(reinterpret_cast<const SElem<N> *>(a.aggs_dev),
-                                                 a.rank, a.world, carry, a.peers, a.epoch_dev, a.status);
+                                                 a.rank, a.world, w.carry, a.peers, a.epoch_dev, a.status);
     ++*launches;
   }
-  const SElem<N> *cr = (finish && a.has_successor) ? carry : nullptr;
-  const SElem<N> *tot = nb > 1 ? scratch : nullptr;
-  if (M > 0) {
+  const SElem<N> *cr = (finish && a.has_successor) ? w.carry : nullptr;
+  const SElem<N> *tot = g.nb > 1 ? w.scratch : nullptr;
+  if (g.M > 0) {
     if (vec)
-      bwd_apply_kernel<N, true><<<blocks, 128, 0, stream>>>(md, a.kf.m, a.kf.C, nrows, M, X, a.s, a.S, a.status, cr, tot, sub);
+      bwd_apply_kernel<N, true><<<g.blocks, 128, 0, stream>>>(md, a.kf.m, a.kf.C, g.rows, g.M, w.X, a.s, a.S,
+                                                              a.status, cr, tot, g.sub);
     else
-      bwd_apply_kernel<N, false><<<blocks, 128, 0, stream>>>(md, a.kf.m, a.kf.C, nrows, M, X, a.s, a.S, a.status, cr, tot, sub);
+      bwd_apply_kernel<N, false><<<g.blocks, 128, 0, stream>>>(md, a.kf.m, a.kf.C, g.rows, g.M, w.X, a.s, a.S,
+                                                               a.status, cr, tot, g.sub);
     ++*launches;
   }
   return cudaGetLastError();
@@ -1970,11 +1980,11 @@ cudaError_t scan_backward(const ScanArgs &a, cudaStream_t stream, int64_t *launc
 
 }  // namespace
 
+// Every pass over a chunk of T observations fits the forward pass's layout with keep_init = 1: no
+// pass has more level-1 threads, and no element is larger than the forward one.
 size_t scan_workspace_bytes(int n, int64_t T) {
-  const int sub = scan_rows_per_thread(n, T);
-  const int64_t M = (T + 1 + sub - 1) / sub + 2;
-  const size_t elem = sizeof(double) * (3 * n * n + 2 * n);
-  return elem * (size_t)(M + 1 + (M + 1) / kScanBlock * 2 + 24) + 8192;
+  const ScanGeom g = scan_geom(n, T, 1, false, kPassForward);
+  return with_n(n, (size_t)0, [&](auto N) { return ScanLayout<FElem<N>>::bytes(g); });
 }
 
 __global__ void epoch_bump_kernel(unsigned long long *epoch_dev) { *epoch_dev = *epoch_dev + 1; }
@@ -1988,61 +1998,34 @@ int scan_forward_elem_doubles(int n) { return 3 * n * n + 2 * n; }
 int scan_backward_elem_doubles(int n) { return 2 * n * n + n; }
 
 cudaError_t launch_scan(const ScanArgs &a, cudaStream_t stream, int64_t *launches) {
-  switch (a.n) {
-#define BDLM_SCAN_CASE(N_)                                                         \
-  case N_:                                                                         \
-    return a.backward ? scan_backward<N_>(a, stream, launches) : scan_forward<N_>(a, stream, launches);
-    BDLM_SCAN_CASE(1)
-    BDLM_SCAN_CASE(2)
-    BDLM_SCAN_CASE(3)
-    BDLM_SCAN_CASE(4)
-#undef BDLM_SCAN_CASE
-    default: return cudaErrorInvalidValue;
-  }
+  return with_n(a.n, cudaErrorInvalidValue, [&](auto N) {
+    return a.backward ? scan_backward<N>(a, stream, launches) : scan_forward<N>(a, stream, launches);
+  });
 }
 
+// block partials, then the last state (n + n*n doubles); a chunk with keep_init = 0 has no more blocks
 size_t scan_loglik_bytes(int n, int64_t T) {
-  const int sub = scan_rows_per_thread(n, T);
-  const int64_t M = (T + 1 + sub - 1) / sub, blocks = (M + kLlBlock - 1) / kLlBlock;
-  return sizeof(LoglikPart) * (size_t)blocks + sizeof(double) * (size_t)(n + n * n) + 256;
+  return sizeof(LoglikPart) * (size_t)scan_geom(n, T, 1, false, kPassLoglik).blocks +
+         sizeof(double) * (size_t)(n + n * n);
 }
 
 cudaError_t launch_scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream,
                                int64_t *launches) {
-  switch (a.n) {
-    case 1: return scan_loglik<1>(a, o, stream, launches);
-    case 2: return scan_loglik<2>(a, o, stream, launches);
-    case 3: return scan_loglik<3>(a, o, stream, launches);
-    case 4: return scan_loglik<4>(a, o, stream, launches);
-    default: return cudaErrorInvalidValue;
-  }
+  return with_n(a.n, cudaErrorInvalidValue, [&](auto N) { return scan_loglik<N>(a, o, stream, launches); });
 }
 
+// 2 + n + n*n statistics per block of the sampler's sweep over any chunk of T observations
 size_t scan_ffbs_parts_bytes(int n, int64_t T) {
-  const int sub = scan_rows_per_thread(n, T);
-  const int64_t M = (T + 1 + sub - 1) / sub, blocks = (M + kFbBlock - 1) / kFbBlock;  // any chunk of T
-  return sizeof(double) * (size_t)(2 + n + n * n) * (size_t)blocks + 256;
+  return sizeof(double) * (size_t)(2 + n + n * n) * (size_t)scan_geom(n, T, 1, true, kPassSampler).blocks;
 }
 
 cudaError_t launch_scan_ffbs(const ScanArgs &a, const ScanFfbsOut &o, cudaStream_t stream, int64_t *launches) {
-  switch (a.n) {
-    case 1: return scan_ffbs<1>(a, o, stream, launches);
-    case 2: return scan_ffbs<2>(a, o, stream, launches);
-    case 3: return scan_ffbs<3>(a, o, stream, launches);
-    case 4: return scan_ffbs<4>(a, o, stream, launches);
-    default: return cudaErrorInvalidValue;
-  }
+  return with_n(a.n, cudaErrorInvalidValue, [&](auto N) { return scan_ffbs<N>(a, o, stream, launches); });
 }
 
 cudaError_t launch_scan_dist_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t stream,
                                     int64_t *launches) {
-  switch (a.n) {
-    case 1: return scan_dist_loglik<1>(a, o, stream, launches);
-    case 2: return scan_dist_loglik<2>(a, o, stream, launches);
-    case 3: return scan_dist_loglik<3>(a, o, stream, launches);
-    case 4: return scan_dist_loglik<4>(a, o, stream, launches);
-    default: return cudaErrorInvalidValue;
-  }
+  return with_n(a.n, cudaErrorInvalidValue, [&](auto N) { return scan_dist_loglik<N>(a, o, stream, launches); });
 }
 
 cudaError_t launch_scan_dist_loglik_finish(const double *parts, int world, double *transition, double *innovations,
@@ -2054,52 +2037,32 @@ cudaError_t launch_scan_dist_loglik_finish(const double *parts, int world, doubl
 
 cudaError_t launch_scan_dist_ffbs(const ScanArgs &a, const ScanFfbsOut &o, bool finish, cudaStream_t stream,
                                   int64_t *launches) {
-  switch (a.n) {
-    case 1: return scan_dist_ffbs<1>(a, o, finish, stream, launches);
-    case 2: return scan_dist_ffbs<2>(a, o, finish, stream, launches);
-    case 3: return scan_dist_ffbs<3>(a, o, finish, stream, launches);
-    case 4: return scan_dist_ffbs<4>(a, o, finish, stream, launches);
-    default: return cudaErrorInvalidValue;
-  }
+  return with_n(a.n, cudaErrorInvalidValue,
+                [&](auto N) { return scan_dist_ffbs<N>(a, o, finish, stream, launches); });
 }
 
 cudaError_t launch_scan_dist_ffbs_stats_finish(int n, const double *parts, int world, const StatViews &sv,
                                                int32_t *status, cudaStream_t stream, int64_t *launches) {
-  switch (n) {
-#define BDLM_STATS_CASE(N_) \
-  case N_: dist_ffbs_stats_finish_kernel<N_><<<1, 1, 0, stream>>>(parts, world, sv, status); break;
-    BDLM_STATS_CASE(1)
-    BDLM_STATS_CASE(2)
-    BDLM_STATS_CASE(3)
-    BDLM_STATS_CASE(4)
-#undef BDLM_STATS_CASE
-    default: return cudaErrorInvalidValue;
-  }
-  ++*launches;
-  return cudaGetLastError();
+  return with_n(n, cudaErrorInvalidValue, [&](auto N) {
+    dist_ffbs_stats_finish_kernel<N><<<1, 1, 0, stream>>>(parts, world, sv, status);
+    ++*launches;
+    return cudaGetLastError();
+  });
 }
 
 int scan_sampler_elem_doubles(int n) { return n * n + n; }
 
 // Host build of the combine the kernels inline: out = ei (x) ej (ei earlier in time).
 void scan_combine_host(int n, bool backward, const double *ei, const double *ej, double *out) {
-  switch (n) {
-#define BDLM_COMB_CASE(N_)                                                                  \
-  case N_:                                                                                  \
-    if (backward) s_combine<N_>(*reinterpret_cast<const SElem<N_> *>(ei),                   \
-                                *reinterpret_cast<const SElem<N_> *>(ej),                   \
-                                *reinterpret_cast<SElem<N_> *>(out));                       \
-    else f_combine<N_>(*reinterpret_cast<const FElem<N_> *>(ei),                            \
-                       *reinterpret_cast<const FElem<N_> *>(ej),                            \
-                       *reinterpret_cast<FElem<N_> *>(out));                                \
-    break;
-    BDLM_COMB_CASE(1)
-    BDLM_COMB_CASE(2)
-    BDLM_COMB_CASE(3)
-    BDLM_COMB_CASE(4)
-#undef BDLM_COMB_CASE
-    default: break;
-  }
+  with_n(n, 0, [&](auto N) {
+    if (backward)
+      s_combine<N>(*reinterpret_cast<const SElem<N> *>(ei), *reinterpret_cast<const SElem<N> *>(ej),
+                   *reinterpret_cast<SElem<N> *>(out));
+    else
+      f_combine<N>(*reinterpret_cast<const FElem<N> *>(ei), *reinterpret_cast<const FElem<N> *>(ej),
+                   *reinterpret_cast<FElem<N> *>(out));
+    return 0;
+  });
 }
 
 }  // namespace bdlm

@@ -117,64 +117,6 @@ def elem_doubles(n: int, backward: bool) -> int:
     return int(capi.load().bdlm_scan_elem_doubles(n, int(backward)))
 
 
-class DistScan:
-    """Time-sharded scan of ONE series over ``world`` GPUs with no host round trip
-    (``bdlm_scan_dist_*``): per pass one all-gather of a 3n^2+2n (filter) / 2n^2+n (smoother)
-    double aggregate per rank, issued on the engine's stream between the local and the finish
-    kernels.  ``all_gather_into(out, x)`` defaults to ``torch.distributed.all_gather_into_tensor``
-    (NCCL); tests pass their own to emulate several ranks on one GPU."""
-
-    def __init__(self, eng: Engine, model: Model, params: Dict, y_chunk, rank: int, world: int):
-        import torch
-        self.eng, self.rank, self.world, self.n = eng, rank, world, model.n
-        self.model, self.y = model, y_chunk   # the problem struct points into model.F / model.G
-        self.keep_init = rank == 0
-        self.rows = model.T + int(self.keep_init)
-        with bound_engine(eng):
-            self.pr, self._keep = _problem(model, params, y_chunk, self.keep_init)
-        n = self.n
-        self.out, self.ko, self.so = _outputs(y_chunk, self.rows, n)
-        ef, eb = elem_doubles(n, False), elem_doubles(n, True)
-        z = lambda k: torch.zeros(k, dtype=torch.float64, device=y_chunk.device)  # noqa: E731
-        self.agg_f, self.aggs_f = z(ef), z(world * ef)
-        self.agg_b, self.aggs_b = z(eb), z(world * eb)
-        self.status = torch.zeros(1, dtype=torch.int32, device=y_chunk.device)
-
-    def _ck(self, rc):
-        self.eng.ctx.check(rc)
-
-    def forward_local(self):
-        self._ck(capi.load().bdlm_scan_dist_forward_local(self.eng.ctx.handle, self.pr, self.rank,
-                                                          self.world, self.agg_f.data_ptr()))
-
-    def forward_finish(self):
-        self._ck(capi.load().bdlm_scan_dist_forward_finish(
-            self.eng.ctx.handle, self.pr, self.rank, self.world, self.aggs_f.data_ptr(), self.ko,
-            self.status.data_ptr()))
-
-    def backward_local(self):
-        self._ck(capi.load().bdlm_scan_dist_backward_local(
-            self.eng.ctx.handle, self.pr, self.rank, self.world, self.ko, self.so,
-            self.agg_b.data_ptr()))
-
-    def backward_finish(self):
-        self._ck(capi.load().bdlm_scan_dist_backward_finish(
-            self.eng.ctx.handle, self.pr, self.rank, self.world, self.aggs_b.data_ptr(), self.ko,
-            self.so, self.status.data_ptr()))
-
-    def run(self, all_gather_into=None):
-        if all_gather_into is None:
-            import torch.distributed as dist
-            all_gather_into = dist.all_gather_into_tensor
-        self.forward_local()
-        all_gather_into(self.aggs_f, self.agg_f)
-        self.forward_finish()
-        self.backward_local()
-        all_gather_into(self.aggs_b, self.agg_b)
-        self.backward_finish()
-        return self.out
-
-
 def dist_doubles(n: int, what: int) -> int:
     """Sizes of the time-sharded loglik / FFBS exchanges (capi.SCAN_DIST_*)."""
     return int(capi.load().bdlm_scan_dist_doubles(n, what))
@@ -211,6 +153,46 @@ class _DistChunk:
             import torch.distributed as dist
             all_gather_into = dist.all_gather_into_tensor
         return all_gather_into
+
+
+class DistScan(_DistChunk):
+    """Time-sharded scan of ONE series over ``world`` GPUs with no host round trip
+    (``bdlm_scan_dist_*``): per pass one all-gather of a 3n^2+2n (filter) / 2n^2+n (smoother)
+    double aggregate per rank, issued on the engine's stream between the local and the finish
+    kernels.  ``all_gather_into(out, x)`` defaults to ``torch.distributed.all_gather_into_tensor``
+    (NCCL); tests pass their own to emulate several ranks on one GPU."""
+
+    def __init__(self, eng: Engine, model: Model, params: Dict, y_chunk, rank: int, world: int):
+        import torch
+        super().__init__(eng, model, params, y_chunk, rank, world)
+        self.out, self.ko, self.so = _outputs(y_chunk, self.rows, self.n)
+        self.agg_b, self.aggs_b = self._xch(elem_doubles(self.n, True))
+        self.status = torch.zeros(1, dtype=torch.int32, device=y_chunk.device)
+
+    def forward_finish(self):
+        self._ck(capi.load().bdlm_scan_dist_forward_finish(
+            self.eng.ctx.handle, self.pr, self.rank, self.world, self.aggs_f.data_ptr(), self.ko,
+            self.status.data_ptr()))
+
+    def backward_local(self):
+        self._ck(capi.load().bdlm_scan_dist_backward_local(
+            self.eng.ctx.handle, self.pr, self.rank, self.world, self.ko, self.so,
+            self.agg_b.data_ptr()))
+
+    def backward_finish(self):
+        self._ck(capi.load().bdlm_scan_dist_backward_finish(
+            self.eng.ctx.handle, self.pr, self.rank, self.world, self.aggs_b.data_ptr(), self.ko,
+            self.so, self.status.data_ptr()))
+
+    def run(self, all_gather_into=None):
+        gather = self._gather(all_gather_into)
+        self.forward_local()
+        gather(self.aggs_f, self.agg_f)
+        self.forward_finish()
+        self.backward_local()
+        gather(self.aggs_b, self.agg_b)
+        self.backward_finish()
+        return self.out
 
 
 class DistLoglik(_DistChunk):

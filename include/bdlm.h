@@ -310,8 +310,8 @@ BDLM_API int bdlm_gibbs_suffstats(bdlm_ctx *ctx, const bdlm_problem *prob, const
 /* ---- parallel-in-time filter + smoother for ONE long series ---------------------------
  * Not in the reference (its recursion is strictly sequential, Filter.scala:41-62; BASELINE
  * config 5).  Temporal parallelisation by associative scan (Sarkka & Garcia-Fernandez 2021).
- * Restrictions: B = 1, p = 1, n <= 4, regular grid (times = NULL), time-invariant F and G,
- * shared parameters, mem = BDLM_DEVICE.  Results equal bdlm_kf_filter_smooth with
+ * Restrictions: B = 1, p = 1, n <= 4, regular grid (times = NULL), time-invariant F, G, V and W
+ * (f_tv = g_tv = v_tv = w_tv = 0), shared parameters, mem = BDLM_DEVICE.  Results equal bdlm_kf_filter_smooth with
  * BDLM_TEXTBOOK_SMOOTHER to 1e-9 relative (for n = 1 that is the reference itself).
  *
  * Single GPU: bdlm_scan_filter_smooth.  Several GPUs, each owning a contiguous time chunk:

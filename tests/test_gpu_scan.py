@@ -122,6 +122,36 @@ def test_scan_rejects_unsupported_shapes(eng):
         scan_filter_smooth(eng, model, dict(V=V, W=W, m0=m0, C0=C0), torch.zeros(10, dtype=torch.float64).cuda())
 
 
+def test_scan_rejects_per_step_v(eng):
+    """A per-step V is not a scan model: bdlm_scan_filter_smooth refuses it (rather than using step
+    0's V) and launches nothing; the opt-in routes leave such a problem to the sequential kernels."""
+    import torch
+    from bayesian_dlms_b200 import Model, _capi as capi
+    from bayesian_dlms_b200.scan import _outputs, _problem
+    mod, V, W, m0, C0 = _models()[1]
+    T = 5000
+    y = H.simulate(mod, V, W, m0, C0, np.arange(1, T + 1.0), np.random.default_rng(5), missing=0.02)[:, 0]
+    yd = torch.from_numpy(y).cuda()
+    model = Model.build(mod, T=T)
+    Vt = np.linspace(1.0, 3.0, T)
+    pr, keep = _problem(model, dict(V=V, W=W, m0=m0, C0=C0), yd, True)
+    pr.V, pr.v_tv = Vt.ctypes.data, 1
+    _, ko, so = _outputs(yd, T + 1, 1)
+    lib = capi.load()
+    n0 = eng.ctx.launch_count()
+    assert lib.bdlm_scan_filter_smooth(eng.ctx.handle, pr, ko, so, None) == capi.E_ARG
+    assert b"v_tv" in lib.bdlm_last_error(eng.ctx.handle)
+    assert eng.ctx.launch_count() == n0
+    params = dict(V=Vt.reshape(T, 1), W=W, m0=m0, C0=C0, v_tv=True)
+    yt = yd.reshape(T, 1, 1)
+    for call in (lambda pit: eng.filter_smooth(model, params, yt, textbook=True, parallel_in_time=pit),
+                 lambda pit: eng.loglik(model, params, yt, parallel_in_time=pit)):
+        seq, pit = call(False), call(True)
+        eng.sync()
+        for k in seq:
+            assert np.array_equal(seq[k].cpu().numpy(), pit[k].cpu().numpy(), equal_nan=True), k
+
+
 @pytest.mark.parametrize("n", [1, 2, 3])
 @pytest.mark.parametrize("world", [1, 2, 3, 5, 8])
 def test_device_side_protocol_emulated_ranks(n, world):

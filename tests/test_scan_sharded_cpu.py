@@ -49,6 +49,19 @@ def test_bad_arguments_are_codes_with_their_reason_even_without_a_context():
     assert "n <= 4" in _err()
     assert lib.bdlm_scan_dist_ffbs_local(None, _problem(n=5), 1, 2, 11, 20, d, None, d, kf, d, None) == capi.E_ARG
     assert "n <= 4" in _err()
+    # a per-step V or W is not a scan model: the filter / smoother phases refuse it too
+    sm = capi.SmoothOut(s=d, S=d)
+    for tv in ("v_tv", "w_tv"):
+        p = _problem(keep_init=1)
+        setattr(p, tv, 1)
+        assert lib.bdlm_scan_dist_forward_local(None, p, 0, 1, d) == capi.E_ARG
+        assert tv in _err()
+        assert lib.bdlm_scan_dist_forward_finish(None, p, 0, 1, d, kf, None) == capi.E_ARG
+        assert tv in _err()
+        assert lib.bdlm_scan_dist_backward_local(None, p, 0, 1, kf, sm, d) == capi.E_ARG
+        assert tv in _err()
+        assert lib.bdlm_scan_dist_backward_finish(None, p, 0, 1, d, kf, sm, None) == capi.E_ARG
+        assert tv in _err()
     # null problem / context; the well-formed call still needs a context
     assert lib.bdlm_scan_dist_loglik_partial(None, None, 0, 1, d, None, None, d) == capi.E_ARG
     assert lib.bdlm_scan_dist_ffbs_local(None, _problem(T=10), 1, 2, 11, 20, d, None, d, kf, d, None) == capi.E_ARG
