@@ -1048,11 +1048,11 @@ int bdlm_rts_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_out *filt,
 // The problems the associative scan computes; needs no context, so the time-sharded phases report
 // a misuse with its reason even on a null one.
 static const char kScanShapes[] =
-    "scan path: B = 1, p = 1, n <= 4, regular grid, time-invariant model (f_tv = g_tv = v_tv = w_tv = 0), "
-    "shared parameters";
+    "scan path: B = 1, p = 1, n <= 4, regular grid, time-invariant G, V, W (g_tv = v_tv = w_tv = 0), "
+    "shared parameters; F time-invariant or per step (f_tv = 1: host [T][n], or BDLM_PS_F alone on the device)";
 static bool scan_supported(const bdlm_problem *p) {
-  return p->B == 1 && p->p == 1 && p->n >= 1 && p->n <= 4 && !p->times && !p->f_tv && !p->g_tv && !p->v_tv &&
-         !p->w_tv && !p->per_series;
+  return p->B == 1 && p->p == 1 && p->n >= 1 && p->n <= 4 && !p->times && !p->g_tv && !p->v_tv && !p->w_tv &&
+         (p->per_series == 0 || (p->f_tv && p->per_series == BDLM_PS_F));
 }
 
 // BDLM_PARALLEL_IN_TIME: one long eligible series goes to the associative-scan kernels.  The
@@ -1073,13 +1073,16 @@ struct PitField {
   size_t doubles;
 };
 
-// Runs call(q, dev, status) with q = *p on device memory: y and the fields are laid out in pit_buf
-// ([y | fields | status]; the scan owns the arena), y and the inputs copied in, dev[i] the device
-// copy of field i; then the outputs and status are copied back and the stream synchronised once.
+// Runs call(q, dev, status) with q = *p on device memory: y, a per-series F and the fields are laid
+// out in pit_buf ([y | F | fields | status]; the scan owns the arena), y, F and the inputs copied in,
+// dev[i] the device copy of field i; then the outputs and status are copied back and the stream
+// synchronised once.
 static int pit_staged(bdlm_ctx *c, const bdlm_problem *p, const std::vector<PitField> &fields, int32_t *status,
                       const std::function<int(const bdlm_problem &, double *const *, int32_t *)> &call) {
   std::vector<size_t> off(fields.size());
-  size_t pos = align_up(sizeof(double) * (size_t)p->T);
+  const size_t F_off = align_up(sizeof(double) * (size_t)p->T);
+  const size_t F_bytes = (p->per_series & BDLM_PS_F) ? sizeof(double) * (size_t)p->T * p->n : 0;
+  size_t pos = align_up(F_off + F_bytes);
   for (size_t i = 0; i < fields.size(); ++i) {
     off[i] = pos;
     if (fields[i].in || fields[i].out) pos = align_up(pos + sizeof(double) * fields[i].doubles);
@@ -1095,6 +1098,7 @@ static int pit_staged(bdlm_ctx *c, const bdlm_problem *p, const std::vector<PitF
     c->pit_bytes = pos;
   }
   CU(cudaMemcpyAsync(c->pit_buf, p->y, sizeof(double) * (size_t)p->T, cudaMemcpyHostToDevice, c->stream));
+  if (F_bytes) CU(cudaMemcpyAsync(c->pit_buf + F_off, p->F, F_bytes, cudaMemcpyHostToDevice, c->stream));
   std::vector<double *> dev(fields.size());
   for (size_t i = 0; i < fields.size(); ++i) {
     const PitField &f = fields[i];
@@ -1104,6 +1108,7 @@ static int pit_staged(bdlm_ctx *c, const bdlm_problem *p, const std::vector<PitF
   bdlm_problem q = *p;
   q.mem = BDLM_DEVICE;
   q.y = reinterpret_cast<const double *>(c->pit_buf);
+  if (F_bytes) q.F = reinterpret_cast<const double *>(c->pit_buf + F_off);
   int32_t *dst = status ? reinterpret_cast<int32_t *>(c->pit_buf + st_off) : nullptr;
   int rc = call(q, dev.data(), dst);
   if (rc) return rc;
@@ -1258,13 +1263,18 @@ static int scan_validate(bdlm_ctx *c, const bdlm_problem *p) {
   return 0;
 }
 
-static int scan_fill(bdlm_ctx *c, const bdlm_problem *p, ScanArgs &a, bool forward = false) {
+// Fd: the device F of an f_tv problem (ScanArena::F), for the passes that read F.
+static int scan_fill(bdlm_ctx *c, const bdlm_problem *p, ScanArgs &a, bool forward = false,
+                     const double *Fd = nullptr) {
   a = ScanArgs{};
   a.n = p->n; a.T = p->T; a.keep_init = p->keep_init ? 1 : 0;
-  a.G = p->G; a.F = p->F; a.W = p->W; a.V = p->V[0]; a.y = p->y;
+  a.G = p->G; a.F = p->f_tv ? nullptr : p->F; a.W = p->W; a.V = p->V[0]; a.y = p->y;
+  a.Fd = p->f_tv ? Fd : nullptr;
   if (!forward) return 0;
   // The forward level-1 table depends on the model only: rebuild it when (n, G, F, W, V) change.
   if (!c->scan_table) CU(cudaMalloc(&c->scan_table, scan_table_bytes()));
+  a.table = c->scan_table;
+  if (p->f_tv) return 0;  // per-step F: no table, and the cached one stays valid for later calls
   const int n = p->n;
   std::vector<double> key;
   key.push_back(n);
@@ -1272,7 +1282,6 @@ static int scan_fill(bdlm_ctx *c, const bdlm_problem *p, ScanArgs &a, bool forwa
   key.insert(key.end(), p->F, p->F + n);
   key.insert(key.end(), p->W, p->W + n * n);
   key.push_back(p->V[0]);
-  a.table = c->scan_table;
   a.table_upload = (key.size() != c->scan_key.size() ||
                     std::memcmp(key.data(), c->scan_key.data(), key.size() * sizeof(double)) != 0);
   if (a.table_upload) { c->scan_key.clear(); c->scan_key_pending = key; }
@@ -1311,15 +1320,18 @@ static KfViews scan_kf_views(const bdlm_problem *p, const bdlm_kf_out *kf) {
 enum ScanCall { kScanCallFilterSmooth, kScanCallLoglik, kScanCallFfbs, kScanCallDist };
 
 // [forward workspace | second workspace (smoother or sampler) | block partials | (m, C) spill when
-// the caller does not want them | status slot]
+// the caller does not want them | status slot | device copy of a shared host F of an f_tv problem]
 struct ScanArena {
   char *ws, *ws2;
   double *parts;    // of the log-likelihoods or of the sampler's statistics
   double *m, *C;    // the caller's kf->m / kf->C, else the spill
   int32_t *status;  // for the phases whose caller passed none
+  const double *F;  // f_tv: the device F [T][n] (BDLM_PS_F: the caller's array), else nullptr
 };
 
-static int scan_arena(bdlm_ctx *c, const bdlm_problem *p, ScanCall call, const bdlm_kf_out *kf, ScanArena &ar) {
+// with_F: the call reads F (every pass but the smoother's), so an f_tv problem's host F is copied in.
+static int scan_arena(bdlm_ctx *c, const bdlm_problem *p, ScanCall call, const bdlm_kf_out *kf, ScanArena &ar,
+                      bool with_F = true) {
   const size_t n = p->n, R = rows_of(*p);
   const size_t ws = align_up(scan_workspace_bytes(p->n, p->T));
   const size_t ll = scan_loglik_bytes(p->n, p->T), fb = scan_ffbs_parts_bytes(p->n, p->T);
@@ -1331,7 +1343,9 @@ static int scan_arena(bdlm_ctx *c, const bdlm_problem *p, ScanCall call, const b
   const size_t o_m = o_parts + align_up(parts);
   const size_t o_C = o_m + (spill && !m ? align_up(sizeof(double) * R * n) : 0);
   const size_t o_st = o_C + (spill && !C ? align_up(sizeof(double) * R * n * n) : 0);
-  int rc = ensure_arena(c, o_st + 256);
+  const bool host_F = with_F && p->f_tv && !(p->per_series & BDLM_PS_F);
+  const size_t o_F = o_st + 256;
+  int rc = ensure_arena(c, o_F + (host_F ? sizeof(double) * (size_t)p->T * n : 0));
   if (rc) return rc;
   ar.ws = c->arena;
   ar.ws2 = call == kScanCallLoglik ? nullptr : c->arena + ws;
@@ -1339,6 +1353,10 @@ static int scan_arena(bdlm_ctx *c, const bdlm_problem *p, ScanCall call, const b
   ar.m = spill && !m ? reinterpret_cast<double *>(c->arena + o_m) : m;
   ar.C = spill && !C ? reinterpret_cast<double *>(c->arena + o_C) : C;
   ar.status = reinterpret_cast<int32_t *>(c->arena + o_st);
+  ar.F = !p->f_tv ? nullptr : host_F ? reinterpret_cast<const double *>(c->arena + o_F) : p->F;
+  // pageable source: staged by the driver before the call returns
+  if (host_F)
+    CU(cudaMemcpyAsync(c->arena + o_F, p->F, sizeof(double) * (size_t)p->T * n, cudaMemcpyHostToDevice, c->stream));
   return 0;
 }
 
@@ -1370,7 +1388,7 @@ int bdlm_scan_filter_smooth(bdlm_ctx *c, const bdlm_problem *p, const bdlm_kf_ou
   k.m = ar.m; k.C = ar.C;
   const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
-  rc = scan_fill(c, p, a, true);
+  rc = scan_fill(c, p, a, true, ar.F);
   if (rc) return rc;
   // forward: filter outputs + the smoother's level-1 aggregates (fused into the apply sweep)
   a.phase = kScanApply; a.start = prior.data();
@@ -1404,7 +1422,7 @@ int bdlm_scan_loglik(bdlm_ctx *c, const bdlm_problem *p, double *m_last, double 
   q.keep_init = 1;  // as bdlm_loglik: the state (m0, C0) is row 0, every observation a step
   const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
-  rc = scan_fill(c, &q, a, true);
+  rc = scan_fill(c, &q, a, true, ar.F);
   if (rc) return rc;
   a.phase = kScanApply; a.start = prior.data(); a.workspace = ar.ws;
   const ScanLoglikOut o{transition, innovations, m_last, C_last, status, ar.parts};
@@ -1428,7 +1446,7 @@ int bdlm_scan_ffbs(bdlm_ctx *c, const bdlm_problem *p, const double *z, double *
   k.m = ar.m; k.C = ar.C;
   const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
-  rc = scan_fill(c, p, a, true);
+  rc = scan_fill(c, p, a, true, ar.F);
   if (rc) return rc;
   a.phase = kScanApply; a.start = prior.data(); a.workspace = ar.ws;
   a.kf = scan_kf_views(p, &k); a.status = status;
@@ -1466,11 +1484,11 @@ static int scan_dist_kf(bdlm_ctx *c, const bdlm_kf_out *kf) {
   return kf && kf->m && kf->C ? 0 : fail(c, BDLM_E_ARG, "time-sharded scan needs kf->m and kf->C");
 }
 
-static int scan_dist_common(bdlm_ctx *c, const bdlm_problem *p, ScanArena &ar) {
+static int scan_dist_common(bdlm_ctx *c, const bdlm_problem *p, ScanArena &ar, bool with_F = true) {
   int rc = scan_validate(c, p);
   if (rc) return rc;
   CU(cudaSetDevice(c->device));
-  return scan_arena(c, p, kScanCallDist, nullptr, ar);
+  return scan_arena(c, p, kScanCallDist, nullptr, ar, with_F);
 }
 
 int bdlm_scan_dist_forward_local(bdlm_ctx *c, const bdlm_problem *p, int32_t rank, int32_t world,
@@ -1483,7 +1501,7 @@ int bdlm_scan_dist_forward_local(bdlm_ctx *c, const bdlm_problem *p, int32_t ran
   if (rc) return rc;
   if (!agg_dev) return fail(c, BDLM_E_ARG, "null aggregate pointer");
   ScanArgs a;
-  rc = scan_fill(c, p, a, true);
+  rc = scan_fill(c, p, a, true, ar.F);
   if (rc) return rc;
   a.phase = kScanDistLocal; a.agg_dev = agg_dev; a.workspace = ar.ws;
   a.rank = rank; a.world = world; a.peers = c->scan_peers; a.epoch_dev = c->scan_epoch;
@@ -1502,7 +1520,7 @@ int bdlm_scan_dist_forward_finish(bdlm_ctx *c, const bdlm_problem *p, int32_t ra
   if (!aggs_dev) return fail(c, BDLM_E_ARG, "null aggregates pointer");
   const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
-  rc = scan_fill(c, p, a, true);
+  rc = scan_fill(c, p, a, true, ar.F);
   if (rc) return rc;
   a.phase = kScanDistFinish; a.aggs_dev = aggs_dev; a.rank = rank; a.world = world;
   a.peers = c->scan_peers; a.epoch_dev = c->scan_epoch;
@@ -1521,7 +1539,7 @@ int bdlm_scan_dist_backward_local(bdlm_ctx *c, const bdlm_problem *p, int32_t ra
   if (!rc) rc = scan_dist_kf(c, filt);
   if (rc) return rc;
   ScanArena ar;
-  rc = scan_dist_common(c, p, ar);
+  rc = scan_dist_common(c, p, ar, false);
   if (rc) return rc;
   if (!agg_dev || !sm) return fail(c, BDLM_E_ARG, "null aggregate pointer or output struct");
   const int64_t n = p->n, R = rows_of(*p);
@@ -1545,7 +1563,7 @@ int bdlm_scan_dist_backward_finish(bdlm_ctx *c, const bdlm_problem *p, int32_t r
   if (!rc) rc = scan_dist_kf(c, filt);
   if (rc) return rc;
   ScanArena ar;
-  rc = scan_dist_common(c, p, ar);
+  rc = scan_dist_common(c, p, ar, false);
   if (rc) return rc;
   if (!aggs_dev || !sm) return fail(c, BDLM_E_ARG, "null aggregates pointer or output struct");
   const int64_t n = p->n, R = rows_of(*p);
@@ -1594,7 +1612,7 @@ int bdlm_scan_dist_loglik_partial(bdlm_ctx *c, const bdlm_problem *p, int32_t ra
   if (!aggs_dev || !part_dev) return fail(c, BDLM_E_ARG, "null aggregates or partial-vector pointer");
   const std::vector<double> prior = scan_prior(p);
   ScanArgs a;
-  rc = scan_fill(c, p, a);
+  rc = scan_fill(c, p, a, false, ar.F);
   if (rc) return rc;
   a.phase = kScanDistFinish; a.aggs_dev = aggs_dev; a.rank = rank; a.world = world;
   a.start = prior.data(); a.workspace = ar.ws;
@@ -1619,7 +1637,7 @@ int bdlm_scan_dist_loglik_finish(bdlm_ctx *c, int32_t world, const double *parts
 static int scan_dist_ffbs_fill(bdlm_ctx *c, const bdlm_problem *p, int rank, int world, const bdlm_kf_out *kf,
                                double *theta, const ScanArena &ar, int32_t *status, const std::vector<double> &prior,
                                bool forward, ScanArgs &a, ScanFfbsOut &o) {
-  int rc = scan_fill(c, p, a, forward);
+  int rc = scan_fill(c, p, a, forward, ar.F);
   if (rc) return rc;
   a.phase = kScanDistFinish; a.rank = rank; a.world = world; a.has_successor = rank < world - 1;
   a.start = prior.data(); a.kf = scan_kf_views(p, kf); a.status = status; a.workspace = ar.ws;

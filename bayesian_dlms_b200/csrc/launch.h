@@ -76,7 +76,7 @@ cudaError_t launch_dt_from_times(const double *times, int64_t tsb, int64_t tsr, 
                                  cudaStream_t stream);
 
 // scan.cu: parallel-in-time filter / smoother for one long series (n <= 4, p = 1, regular
-// grid, time-invariant model).
+// grid, time-invariant G, V, W; F time-invariant or given per step).
 enum { kScanApply = 0,
        // time-sharded run over several GPUs: local = level-1 + scan with an identity carry, chunk
        // aggregate left in DEVICE memory for the all-gather; finish = fold the gathered aggregates
@@ -100,9 +100,10 @@ struct ScanArgs {
   int backward;        // 0 = filter pass, 1 = smoother pass
   int phase;           // kScanApply: whole series on one GPU; kScanDist*: one rank's chunk
   int has_successor;   // backward: another chunk follows this one in time
-  const double *G, *F, *W;  // host, column-major
+  const double *G, *F, *W;  // host, column-major; F = nullptr with a per-step F (f_tv)
   double V;
   const double *y;     // device [T]
+  const double *Fd;    // f_tv: device [T][n], F of each observation of the chunk; else nullptr
   const double *start; // host [n + n*n]: the prior (m0, C0) of the series (forward apply / finish)
   KfViews kf;          // forward: outputs; backward: filtered (m, C) inputs
   View s, S;           // backward outputs

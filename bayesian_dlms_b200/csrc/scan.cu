@@ -305,6 +305,50 @@ struct YGroup {
   }
 };
 
+// Per-step observation vectors behind a group of kGrp rows (f_tv): F[t] = F + t*N, t = r - keep_init + i,
+// fetched like YGroup fetches y -- the N sectors of steps r .. r + kGrp - 1 at once, the last step's
+// vector carried to the next group when keep_init puts the rows one step ahead of the sectors.
+template <int N, bool VEC>
+struct FGroup {
+  double carry[N];
+  __device__ __forceinline__ void start(const double *F, int64_t r0, int keep_init) {
+#pragma unroll
+    for (int k = 0; k < N; ++k) carry[k] = (VEC && keep_init && r0 > 0) ? F[(r0 - 1) * N + k] : 0.0;
+  }
+  // precondition as YGroup::load; a row before the first step (the prior) gets zeros
+  __device__ __forceinline__ void load(const double *F, int64_t r, int64_t T, int keep_init,
+                                       double (&fv)[kGrp][N]) {
+    if (VEC) {
+      double v[kGrp * N];
+      if (r + kGrp <= T) {
+#pragma unroll
+        for (int k = 0; k < kGrp * N; k += 4) ld_v4(F + r * N + k, v + k);
+      } else {
+#pragma unroll
+        for (int k = 0; k < kGrp * N; ++k) v[k] = (r + k / N < T) ? F[r * N + k] : 0.0;
+      }
+#pragma unroll
+      for (int i = 0; i < kGrp; ++i)
+#pragma unroll
+        for (int k = 0; k < N; ++k) {
+          if (keep_init) fv[i][k] = i == 0 ? carry[k] : v[(i - 1) * N + k];
+          else fv[i][k] = v[i * N + k];
+        }
+      if (keep_init) {
+#pragma unroll
+        for (int k = 0; k < N; ++k) carry[k] = v[(kGrp - 1) * N + k];
+      }
+    } else {
+#pragma unroll
+      for (int i = 0; i < kGrp; ++i) {
+        const int64_t t = r + i - keep_init;
+#pragma unroll
+        for (int k = 0; k < N; ++k) fv[i][k] = t >= 0 ? F[t * N + k] : 0.0;
+      }
+    }
+  }
+};
+
 // kGrp consecutive rows of a dense field in one go (whole lines for K >= 4).
 template <int K>
 __device__ __forceinline__ void load_group(const View &v, int64_t row, double (&x)[kGrp * K]) {
@@ -405,12 +449,16 @@ StateArg<N> state_arg(const double *host) {
   return s;
 }
 
-template <int N, bool VEC>
+//
+// FTV (f_tv, per-step F[t] = Fd + t*N): no table -- the steps' (A, C, J) differ -- so every thread
+// composes its steps with the generic combine, reading F like y.
+template <int N, bool VEC, bool FTV = false>
 __global__ void __launch_bounds__(128)
 fwd_reduce_kernel(const ScanModel<N> md, const FwdTable<N> *__restrict__ tb,
                   const double *__restrict__ y, int64_t T, int64_t M, int keep_init,
                   FElem<N> *agg /* [M + 1], slot 0 = the start element */,
-                  const StateArg<N> start, bool identity_start, int sub) {
+                  const StateArg<N> start, bool identity_start, int sub,
+                  const double *__restrict__ Fd /* FTV: [T][N] */) {
   const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (c >= M) return;
   if (c == 0) {  // slot 0: the state before the chunk, or the identity (aggregate-only phases)
@@ -420,6 +468,32 @@ fwd_reduce_kernel(const ScanModel<N> md, const FwdTable<N> *__restrict__ tb,
   }
   const int64_t rows = T + keep_init;
   const int64_t r0 = c * (int64_t)sub, r1 = (r0 + sub < rows) ? r0 + sub : rows;
+  if constexpr (FTV) {
+    FElem<N> acc, e, tmp;
+    bool have = false;
+    auto fold = [&](const double *Ft, double yt) {
+      f_element<N>(md.G, Ft, md.W, md.V, yt, e);
+      if (have) { f_combine<N>(acc, e, tmp); acc = tmp; }
+      else { acc = e; have = true; }
+    };
+    YGroup<VEC> yg;
+    FGroup<N, VEC> fg;
+    yg.start(y, r0, keep_init);
+    fg.start(Fd, r0, keep_init);
+    int64_t r = r0;
+    for (; r + kGrp <= r1; r += kGrp) {
+      double yv[kGrp], fv[kGrp][N];
+      yg.load(y, r, T, keep_init, yv);
+      fg.load(Fd, r, T, keep_init, fv);
+#pragma unroll
+      for (int i = 0; i < kGrp; ++i)
+        if (r + i >= keep_init) fold(fv[i], yv[i]);
+    }
+    for (; r < r1; ++r)
+      if (r >= keep_init) fold(Fd + (r - keep_init) * N, y[r - keep_init]);
+    agg[c + 1] = acc;
+    return;
+  }
   const int64_t t0 = first_step(c, keep_init, sub), t1 = r1 - keep_init;
   double b[N], eta[N];
 #pragma unroll
@@ -633,7 +707,8 @@ struct FwdRow {  // everything KfState holds for one row
 // prediction into the next row.  FUSE: also fold this row's smoothing element into sacc when the
 // row has a successor (r < nrows), which saves the smoother's level-1 pass over (m, C).
 template <int N, bool FUSE>
-__device__ __forceinline__ void fwd_row(const ScanModel<N> &md, const double (&W)[N * N], bool init_row,
+__device__ __forceinline__ void fwd_row(const ScanModel<N> &md, const double *F /* this row's */,
+                                        const double (&W)[N * N], bool init_row,
                                         double yv, double (&m)[N], double (&C)[N * N],
                                         double (&an)[N], double (&Rn)[N * N], FwdRow<N> &o, int &st,
                                         bool has_succ, SElem<N> &sacc, bool &shave) {
@@ -649,7 +724,7 @@ __device__ __forceinline__ void fwd_row(const ScanModel<N> &md, const double (&W
     for (int k = 0; k < N; ++k) o.a[k] = an[k];
 #pragma unroll
     for (int k = 0; k < N * N; ++k) o.R[k] = Rn[k];
-    update<N, true>(md.F, md.V, yv, o.a, o.R, o.f, o.Q, m, C, st);
+    update<N, true>(F, md.V, yv, o.a, o.R, o.f, o.Q, m, C, st);
   }
 #pragma unroll
   for (int k = 0; k < N; ++k) o.m[k] = m[k];
@@ -689,7 +764,8 @@ __device__ __forceinline__ void fwd_start_state(const FElem<N> *pre, int64_t c, 
 
 // The two apply sweeps ask ptxas for one resident block per SM: asking for more makes them spill,
 // which costs more than the occupancy gains (profiles/r1_tuning.txt, "scan apply sweeps").
-template <int N, bool VEC, bool FUSE>
+// FTV: row r updates with F[t] = Fd + t*N, t = r - keep_init.
+template <int N, bool VEC, bool FUSE, bool FTV = false>
 __global__ void __launch_bounds__(128, 1)
 fwd_apply_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T, int64_t M,
                  const FElem<N> *pre /* [M+1] inclusive scan with slot 0 = start */,
@@ -697,7 +773,7 @@ fwd_apply_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T,
                  SElem<N> *sagg /* FUSE: smoother level-1 aggregates */, int64_t nrows,
                  const FElem<N> *carry /* multi-GPU: everything before this chunk, or nullptr */,
                  const FElem<N> *tot /* scanned level-2 block totals whose prefix `pre` still lacks, or nullptr */,
-                 int sub) {
+                 int sub, const double *__restrict__ Fd /* FTV: [T][N] */) {
   const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (c >= M) return;
   const int64_t rows = T + keep_init;
@@ -731,18 +807,21 @@ fwd_apply_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T,
   int64_t r = r0;
   if (VEC) {
     YGroup<true> yg;
+    FGroup<N, true> fg;
     yg.start(y, r0, keep_init);
+    if constexpr (FTV) fg.start(Fd, r0, keep_init);
     for (; r + kGrp <= r1; r += kGrp) {
-      double yv[kGrp];
+      double yv[kGrp], fv[kGrp][N];
       yg.load(y, r, T, keep_init, yv);
+      if constexpr (FTV) fg.load(Fd, r, T, keep_init, fv);
       GroupBuf<N> ga, gm;
       GroupBuf<N * N> gR, gC;
       GroupBuf<1> gf, gQ;
 #define BDLM_FWD_ROW(I)                                                          \
   {                                                                              \
     FwdRow<N> o;                                                                 \
-    fwd_row<N, FUSE>(md, W, keep_init && r + I == 0, yv[I], m, C, an, Rn, o, st, \
-                     r + I < nrows, sacc, shave);                                \
+    fwd_row<N, FUSE>(md, FTV ? fv[I] : md.F, W, keep_init && r + I == 0, yv[I],  \
+                     m, C, an, Rn, o, st, r + I < nrows, sacc, shave);           \
     if (kf.a.ptr) ga.template put<I, true>(kf.a.ptr + r * N, o.a);               \
     if (kf.R.ptr) gR.template put<I, true>(kf.R.ptr + r * (N * N), o.R);         \
     if (kf.f.ptr) gf.template put<I, true>(kf.f.ptr + r, &o.f);                  \
@@ -757,7 +836,8 @@ fwd_apply_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T,
   for (; r < r1; ++r) {  // ragged tail (or unaligned / strided outputs): scalar stores
     const int64_t t = r - keep_init;
     FwdRow<N> o;
-    fwd_row<N, FUSE>(md, W, t < 0, t >= 0 ? y[t] : 0.0, m, C, an, Rn, o, st, r < nrows, sacc, shave);
+    fwd_row<N, FUSE>(md, (FTV && t >= 0) ? Fd + t * N : md.F, W, t < 0, t >= 0 ? y[t] : 0.0, m, C, an, Rn, o,
+                     st, r < nrows, sacc, shave);
     store_row_scalar<N>(kf.a, r, o.a); store_row_scalar<N * N>(kf.R, r, o.R);
     store_row_scalar<1>(kf.f, r, &o.f); store_row_scalar<1>(kf.Q, r, &o.Q);
     store_row_scalar<N>(kf.m, r, o.m); store_row_scalar<N * N>(kf.C, r, o.C);
@@ -784,13 +864,15 @@ constexpr int kLlBlock = 128, kLlFinish = 256;
 // an identity start, so every thread composes `carry` (the prior and every earlier chunk, i.e. the
 // filtered state at the end of the previous chunk) in front of its prefix, as fwd_apply_kernel does;
 // keep_init = 0 on every rank but the first, where row r then holds step t = r.
-template <int N, bool VEC, bool TR, bool DIST>
+// FTV: row r updates with F[t] = Fd + t*N, as fwd_apply_kernel.
+template <int N, bool VEC, bool TR, bool DIST, bool FTV = false>
 __global__ void __launch_bounds__(kLlBlock)
 fwd_loglik_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T, int64_t M,
                   const FElem<N> *pre /* [M+1] inclusive scan with slot 0 = the prior */,
                   const FElem<N> *tot /* scanned level-2 block totals `pre` still lacks, or nullptr */,
                   int sub, LoglikPart *part /* [gridDim.x] */, double *last /* [N + N*N]: (m_T, C_T) */,
-                  int keep_init /* DIST */, const FElem<N> *carry /* DIST */) {
+                  int keep_init /* DIST */, const FElem<N> *carry /* DIST */,
+                  const double *__restrict__ Fd /* FTV: [T][N] */) {
   __shared__ double s_tr[kLlBlock], s_in[kLlBlock];
   __shared__ int s_st[kLlBlock];
   const int tid = threadIdx.x;
@@ -829,10 +911,10 @@ fwd_loglik_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T
     advance<N, true>(md.G, W, 1.0, m, C, an, Rn);
     SElem<N> sacc;  // unused (no smoother fold)
     bool shave = false;
-    auto row = [&](int64_t r, double yv) {
+    auto row = [&](int64_t r, double yv, const double *Ft) {
       FwdRow<N> o;
       const bool init = ki && r == 0;
-      fwd_row<N, false>(md, W, init, yv, m, C, an, Rn, o, st, false, sacc, shave);
+      fwd_row<N, false>(md, Ft, W, init, yv, m, C, an, Rn, o, st, false, sacc, shave);
       if (init) return;
       if (TR) tr += mvn.eval(o.m, o.a);
       if (!isnan(yv)) {
@@ -844,15 +926,18 @@ fwd_loglik_kernel(const ScanModel<N> md, const double *__restrict__ y, int64_t T
     int64_t r = r0;
     if (VEC) {
       YGroup<true> yg;
+      FGroup<N, true> fg;
       yg.start(y, r0, ki);
+      if constexpr (FTV) fg.start(Fd, r0, ki);
       for (; r + kGrp <= r1; r += kGrp) {
-        double yv[kGrp];
+        double yv[kGrp], fv[kGrp][N];
         yg.load(y, r, T, ki, yv);
+        if constexpr (FTV) fg.load(Fd, r, T, ki, fv);
 #pragma unroll
-        for (int i = 0; i < kGrp; ++i) row(r + i, yv[i]);
+        for (int i = 0; i < kGrp; ++i) row(r + i, yv[i], FTV ? fv[i] : md.F);
       }
     }
-    for (; r < r1; ++r) row(r, r >= ki ? y[r - ki] : 0.0);
+    for (; r < r1; ++r) row(r, r >= ki ? y[r - ki] : 0.0, (FTV && r >= ki) ? Fd + (r - ki) * N : md.F);
     if (r1 == rows) {  // this thread owns row T: its state is the final filtered state
 #pragma unroll
       for (int k = 0; k < N; ++k) last[k] = m[k];
@@ -1245,11 +1330,11 @@ struct FfbsStats {
 #pragma unroll
     for (int k = 0; k < kD; ++k) v[k] = 0.0;
   }
-  // step t: theta_{t+1} = cur, theta_t = prev, observation y_t.  The observation term needs theta_{t+1}
-  // alone, the transition term both: a time-sharded chunk counts them on different rows.
-  __device__ __forceinline__ void add_obs(const ScanModel<N> &md, const double (&cur)[N], double yt) {
+  // step t: theta_{t+1} = cur, theta_t = prev, observation y_t with F = F_t.  The observation term needs
+  // theta_{t+1} alone, the transition term both: a time-sharded chunk counts them on different rows.
+  __device__ __forceinline__ void add_obs(const double *F, const double (&cur)[N], double yt) {
     double ft;
-    smm<1, N, 1, true, false>(md.F, cur, &ft);
+    smm<1, N, 1, true, false>(F, cur, &ft);
     if (!isnan(yt)) {
       v[0] = v[0] + (yt - ft) * (yt - ft);
       v[1] = v[1] + 1.0;
@@ -1279,15 +1364,17 @@ constexpr int kFbBlock = 128, kFbFinish = 256;
 // belongs to the next chunk when r is the chunk's last row (y[r] does not exist: skipped); without
 // it (ranks > 0) that of row r itself, y[r], plus that of the terminal row on the last chunk.  So
 // every step and every observation is counted once across threads and ranks.  The block's sums go
-// through a fixed-order shared-memory tree to one partial per block.
-template <int N, bool VEC, bool STATS>
+// through a fixed-order shared-memory tree to one partial per block.  FTV: the observation term of
+// y[r] uses F[r] = Fd + r*N (F is indexed like y).
+template <int N, bool VEC, bool STATS, bool FTV = false>
 __global__ void __launch_bounds__(kFbBlock, 1)
 ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restrict__ y, int64_t T, int64_t M,
                   const BElem<N> *suf /* [M+1] suffix-inclusive scan, slot M = terminal */,
                   const BElem<N> *tot /* scanned level-2 block totals (scan order) `suf` still lacks, or nullptr */,
                   View th, int32_t *status, int sub, double *part /* [kD][gridDim.x] */,
                   const BElem<N> *carry /* multi-GPU: everything after this chunk, or nullptr */,
-                  int keep_init, int64_t ny /* observations in y */, bool terminal) {
+                  int keep_init, int64_t ny /* observations in y */, bool terminal,
+                  const double *__restrict__ Fd /* FTV: [ny][N] */) {
   constexpr int kD = FfbsStats<N>::kD;
   __shared__ double s_part[STATS ? kD * kFbBlock : 1];
   const int tid = threadIdx.x;
@@ -1317,9 +1404,10 @@ ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restr
     }
 #pragma unroll
     for (int k = 0; k < N * N; ++k) W[k] = md.W[k];
-    if (STATS && !keep_init && terminal && r1 == T) acc.add_obs(md, t, y[T]);  // t = theta of the terminal row
+    if (STATS && !keep_init && terminal && r1 == T)  // t = theta of the terminal row
+      acc.add_obs(FTV ? Fd + T * N : md.F, t, y[T]);
     // theta_r from theta_{r+1} = t and c_r; t becomes theta_r
-    auto step = [&](int64_t r, const double (&cr)[N], double yr) {
+    auto step = [&](int64_t r, const double (&cr)[N], double yr, const double *Fr) {
       double m[N], C[N * N], a1[N], Bg[N * N], v[N], nt[N];
       load_row<N, VEC>(fm, r, m);
       load_row<N * N, VEC>(fC, r, C);
@@ -1328,8 +1416,8 @@ ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restr
 #pragma unroll
       for (int k = 0; k < N; ++k) nt[k] = v[k] + cr[k];
       if (STATS) {
-        if (keep_init) acc.add_obs(md, t, yr);
-        else acc.add_obs(md, nt, yr);
+        if (keep_init) acc.add_obs(Fr, t, yr);
+        else acc.add_obs(Fr, nt, yr);
         acc.add_trans(md, t, nt);
       }
 #pragma unroll
@@ -1342,22 +1430,27 @@ ffbs_apply_kernel(const ScanModel<N> md, View fm, View fC, const double *__restr
     auto scalar_row = [&](int64_t row) {
       double cr[N];
       load_row<N, false>(th, row, cr);
-      step(row, cr, STATS ? (row < ny ? y[row] : __longlong_as_double(0x7ff8000000000000LL)) : 0.0);
+      step(row, cr, STATS ? (row < ny ? y[row] : __longlong_as_double(0x7ff8000000000000LL)) : 0.0,
+           (FTV && row < ny) ? Fd + row * N : md.F);
       store_row_scalar<N>(th, row, t);
     };
     if (VEC) {
       for (; r > aligned_top; --r) scalar_row(r - 1);
       for (; r - kGrp >= r0; r -= kGrp) {
         const int64_t g0 = r - kGrp;
-        double cg[kGrp * N], yg[kGrp];
+        double cg[kGrp * N], yg[kGrp], fg[kGrp * N];
         load_group<N>(th, g0, cg);  // every c of the group before the first store into it
         if (STATS) ld_v4(y + g0, yg);
+        if constexpr (STATS && FTV) {
+#pragma unroll
+          for (int k = 0; k < kGrp * N; k += 4) ld_v4(Fd + g0 * N + k, fg + k);
+        }
         GroupBuf<N> gt;
 #define BDLM_FFBS_APPLY(I)                                 \
   {                                                        \
     double cr[N];                                          \
     for (int k = 0; k < N; ++k) cr[k] = cg[I * N + k];     \
-    step(g0 + I, cr, STATS ? yg[I] : 0.0);                 \
+    step(g0 + I, cr, STATS ? yg[I] : 0.0, FTV ? fg + I * N : md.F); \
     gt.template put<I, false>(th.ptr + g0 * N, t);         \
   }
         BDLM_FFBS_APPLY(3) BDLM_FFBS_APPLY(2) BDLM_FFBS_APPLY(1) BDLM_FFBS_APPLY(0)
@@ -1602,6 +1695,15 @@ R with_n(int n, R none, F &&f) {
   }
 }
 
+// f(std::bool_constant<b>...) for the run-time flags b...: one kernel instance per combination.
+template <class F>
+void with_flags(F &&f) { f(); }
+template <class F, class... Bs>
+void with_flags(F &&f, bool b, Bs... bs) {
+  if (b) with_flags([&](auto... x) { f(std::true_type{}, x...); }, bs...);
+  else with_flags([&](auto... x) { f(std::false_type{}, x...); }, bs...);
+}
+
 int scan_rows_per_thread(int n, int64_t T) {
   const int slots = with_n(n, 444, [](auto N) { return apply_slots<N>(); });
   const double rows = (double)(T + 1);
@@ -1672,7 +1774,7 @@ template <int N>
 ScanModel<N> make_model(const ScanArgs &a) {
   ScanModel<N> md;
   for (int k = 0; k < N * N; ++k) { md.G[k] = a.G[k]; md.W[k] = a.W[k]; }
-  for (int k = 0; k < N; ++k) md.F[k] = a.F[k];
+  for (int k = 0; k < N; ++k) md.F[k] = a.F ? a.F[k] : 0.0;  // f_tv: the kernels read a.Fd
   md.V = a.V;
   return md;
 }
@@ -1682,6 +1784,11 @@ ScanModel<N> make_model(const ScanArgs &a) {
 // 256-bit path: dense rows (sk = 1, sr = K) on a 32-byte aligned base.
 static bool dense_aligned(const View &v, int64_t K) {
   return !v.ptr || (v.sk == 1 && v.sr == K && (reinterpret_cast<uintptr_t>(v.ptr) & 31) == 0);
+}
+
+// 256-bit loads of the streamed inputs: y and, with f_tv, F on 32-byte aligned bases.
+static bool inputs_aligned(const ScanArgs &a) {
+  return ((reinterpret_cast<uintptr_t>(a.y) | reinterpret_cast<uintptr_t>(a.Fd)) & 31) == 0;
 }
 
 // The model's level-1 table, rebuilt on the host and uploaded when the model changed since the
@@ -1704,10 +1811,10 @@ cudaError_t fwd_prefixes(const ScanArgs &a, const ScanModel<N> &md, const ScanGe
                          const StateArg<N> &st0, bool identity, cudaStream_t stream, int64_t *launches) {
   const FwdTable<N> *tb = reinterpret_cast<const FwdTable<N> *>(a.table);
   const unsigned blocks = (unsigned)((g.M + 127) / 128);
-  if ((reinterpret_cast<uintptr_t>(a.y) & 31) == 0)
-    fwd_reduce_kernel<N, true><<<blocks, 128, 0, stream>>>(md, tb, a.y, a.T, g.M, a.keep_init, w.X, st0, identity, g.sub);
-  else
-    fwd_reduce_kernel<N, false><<<blocks, 128, 0, stream>>>(md, tb, a.y, a.T, g.M, a.keep_init, w.X, st0, identity, g.sub);
+  with_flags([&](auto VEC_, auto FTV_) {
+    fwd_reduce_kernel<N, VEC_, FTV_><<<blocks, 128, 0, stream>>>(md, tb, a.y, a.T, g.M, a.keep_init, w.X, st0,
+                                                                 identity, g.sub, a.Fd);
+  }, inputs_aligned(a), a.Fd != nullptr);
   ++*launches;
   CK(cudaGetLastError());
   return device_scan<FElem<N>, false, false>(w.X, g.M + 1, w.scratch, stream, launches, /*defer_top=*/true);
@@ -1745,22 +1852,17 @@ cudaError_t scan_forward(const ScanArgs &a, cudaStream_t stream, int64_t *launch
   }
   const bool vec = dense_aligned(a.kf.m, N) && dense_aligned(a.kf.C, N * N) &&
                    dense_aligned(a.kf.a, N) && dense_aligned(a.kf.R, N * N) &&
-                   dense_aligned(a.kf.f, 1) && dense_aligned(a.kf.Q, 1) &&
-                   (reinterpret_cast<uintptr_t>(a.y) & 31) == 0;
+                   dense_aligned(a.kf.f, 1) && dense_aligned(a.kf.Q, 1) && inputs_aligned(a);
   // a.fuse_sagg: the caller runs the smoother next on the same rows: fold the smoothing
   // elements here so the backward pass starts from ready level-1 aggregates.
   SElem<N> *sagg = reinterpret_cast<SElem<N> *>(a.fuse_sagg);
   const int64_t nrows = scan_geom(a, kPassBackward).rows;  // the smoother's rows
   const FElem<N> *cr = finish ? w.carry : nullptr;
   const FElem<N> *tot = g.nb > 1 ? w.scratch : nullptr;  // top-level block prefixes, composed by the sweep
-#define BDLM_FWD_APPLY(VEC_, FUSE_)                                                                 \
-  fwd_apply_kernel<N, VEC_, FUSE_><<<g.blocks, 128, 0, stream>>>(md, a.y, a.T, g.M, w.X, a.keep_init, \
-                                                                 a.kf, a.status, sagg, nrows, cr, tot, g.sub)
-  if (vec && sagg) BDLM_FWD_APPLY(true, true);
-  else if (vec) BDLM_FWD_APPLY(true, false);
-  else if (sagg) BDLM_FWD_APPLY(false, true);
-  else BDLM_FWD_APPLY(false, false);
-#undef BDLM_FWD_APPLY
+  with_flags([&](auto VEC_, auto FUSE_, auto FTV_) {
+    fwd_apply_kernel<N, VEC_, FUSE_, FTV_><<<g.blocks, 128, 0, stream>>>(md, a.y, a.T, g.M, w.X, a.keep_init, a.kf,
+                                                                        a.status, sagg, nrows, cr, tot, g.sub, a.Fd);
+  }, vec, sagg != nullptr, a.Fd != nullptr);
   ++*launches;
   return cudaGetLastError();
 }
@@ -1778,15 +1880,10 @@ cudaError_t scan_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStream_t 
   CK(fwd_table_upload<N>(a, md, stream));
   CK(fwd_prefixes<N>(a, md, g, w, state_arg<N>(a.start), false, stream, launches));
   const FElem<N> *tot = g.nb > 1 ? w.scratch : nullptr;
-  const bool vec = (reinterpret_cast<uintptr_t>(a.y) & 31) == 0, tr = o.transition != nullptr;
-#define BDLM_LL_SWEEP(VEC_, TR_)                                                                    \
-  fwd_loglik_kernel<N, VEC_, TR_, false><<<g.blocks, kLlBlock, 0, stream>>>(md, a.y, a.T, g.M, w.X, tot, g.sub, \
-                                                                            part, last, 1, nullptr)
-  if (vec && tr) BDLM_LL_SWEEP(true, true);
-  else if (vec) BDLM_LL_SWEEP(true, false);
-  else if (tr) BDLM_LL_SWEEP(false, true);
-  else BDLM_LL_SWEEP(false, false);
-#undef BDLM_LL_SWEEP
+  with_flags([&](auto VEC_, auto TR_, auto FTV_) {
+    fwd_loglik_kernel<N, VEC_, TR_, false, FTV_><<<g.blocks, kLlBlock, 0, stream>>>(
+        md, a.y, a.T, g.M, w.X, tot, g.sub, part, last, 1, nullptr, a.Fd);
+  }, inputs_aligned(a), o.transition != nullptr, a.Fd != nullptr);
   ++*launches;
   CK(cudaGetLastError());
   loglik_finish_kernel<<<1, kLlFinish, 0, stream>>>(part, g.blocks, last, N, o.transition, o.innovations,
@@ -1814,12 +1911,10 @@ cudaError_t scan_dist_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStre
   ++*launches;
   CK(cudaGetLastError());
   const FElem<N> *tot = g.nb > 1 ? w.scratch : nullptr;
-  if ((reinterpret_cast<uintptr_t>(a.y) & 31) == 0)
-    fwd_loglik_kernel<N, true, true, true><<<g.blocks, kLlBlock, 0, stream>>>(md, a.y, a.T, g.M, w.X, tot, g.sub,
-                                                                              part, last, a.keep_init, w.carry);
-  else
-    fwd_loglik_kernel<N, false, true, true><<<g.blocks, kLlBlock, 0, stream>>>(md, a.y, a.T, g.M, w.X, tot, g.sub,
-                                                                               part, last, a.keep_init, w.carry);
+  with_flags([&](auto VEC_, auto FTV_) {
+    fwd_loglik_kernel<N, VEC_, true, true, FTV_><<<g.blocks, kLlBlock, 0, stream>>>(
+        md, a.y, a.T, g.M, w.X, tot, g.sub, part, last, a.keep_init, w.carry, a.Fd);
+  }, inputs_aligned(a), a.Fd != nullptr);
   ++*launches;
   CK(cudaGetLastError());
   loglik_finish_kernel<<<1, kLlFinish, 0, stream>>>(part, g.blocks, holds_last ? last : nullptr, N, o.part_vec,
@@ -1831,7 +1926,7 @@ cudaError_t scan_dist_loglik(const ScanArgs &a, const ScanLoglikOut &o, cudaStre
 template <int N>
 bool sampler_vec(const ScanArgs &a, const ScanFfbsOut &o) {
   return dense_aligned(a.kf.m, N) && dense_aligned(a.kf.C, N * N) && dense_aligned(o.theta, N) &&
-         (reinterpret_cast<uintptr_t>(a.y) & 31) == 0;
+         inputs_aligned(a);
 }
 
 // The sampler's level 1 (elements, c_r into theta, the terminal slot) and its level-2 suffix scan.
@@ -1872,15 +1967,12 @@ cudaError_t sampler_apply(const ScanArgs &a, const ScanFfbsOut &o, const ScanGeo
   const ScanLayout<BElem<N>> w(g, o.workspace);
   const BElem<N> *tot = g.nb > 1 ? w.scratch : nullptr;
   const bool vec_io = sampler_vec<N>(a, o), terminal = !a.has_successor;
-#define BDLM_FFBS_SWEEP(VEC_, STATS_)                                                                          \
-  ffbs_apply_kernel<N, VEC_, STATS_><<<g.blocks, kFbBlock, 0, stream>>>(                                       \
-      md, a.kf.m, a.kf.C, a.y, g.rows, g.M, w.X, tot, o.theta, a.status, g.sub, o.parts, carry, a.keep_init, a.T, \
-      terminal)
-  if (vec_io && stats) BDLM_FFBS_SWEEP(true, true);
-  else if (vec_io) BDLM_FFBS_SWEEP(true, false);
-  else if (stats) BDLM_FFBS_SWEEP(false, true);
-  else BDLM_FFBS_SWEEP(false, false);
-#undef BDLM_FFBS_SWEEP
+  // F enters the statistics only
+  with_flags([&](auto VEC_, auto STATS_, auto FTV_) {
+    ffbs_apply_kernel<N, VEC_, STATS_, FTV_ && STATS_><<<g.blocks, kFbBlock, 0, stream>>>(
+        md, a.kf.m, a.kf.C, a.y, g.rows, g.M, w.X, tot, o.theta, a.status, g.sub, o.parts, carry, a.keep_init, a.T,
+        terminal, a.Fd);
+  }, vec_io, stats, a.Fd != nullptr);
   ++*launches;
   CK(cudaGetLastError());
   if (stats) {

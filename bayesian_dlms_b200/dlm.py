@@ -94,12 +94,13 @@ def polynomial(order: int) -> Dlm:
 
 
 def regression(x: Sequence[np.ndarray]) -> Dlm:
-    """``Dlm.regression`` (Dlm.scala:159-169): F_t = (1, x_t), G = I_2."""
+    """``Dlm.regression`` (Dlm.scala:159-169): F_t = (1, x_t), G = I of size 1 + len(x_t)."""
     def f(t):
         idx = int(t) - 1
-        return np.concatenate([[1.0], np.asarray(x[idx], dtype=np.float64)]).reshape(-1, 1)
+        return np.concatenate([[1.0], np.asarray(x[idx], dtype=np.float64).ravel()]).reshape(-1, 1)
 
-    return Dlm(f, lambda dt: np.eye(2))
+    n = 1 + np.asarray(x[0], dtype=np.float64).size
+    return Dlm(f, lambda dt: np.eye(n))
 
 
 def autoregressive(*phi: float) -> Dlm:

@@ -8,6 +8,11 @@ statistics; ``DistScan`` runs one rank's time chunk of a
 sharded series with the device-side phases (one all-gather of a 3n^2+2n-double aggregate per rank
 for the filter, 2n^2+n for the smoother), ``DistLoglik`` and ``DistFfbs`` the log-likelihoods and
 FFBS of such a chunk (``sharding.time_chunk`` gives each rank its observations and first row).
+
+A model with a per-step F (``f_tv``: dynamic regression, F_t = (1, x_t)) runs on every one of these
+calls: ``model.F`` (T, n) on the host is copied to the device with each call, or, with
+``model.per_series = ("F",)``, a CUDA tensor of T * n doubles is read in place.  A chunk's model
+holds the F rows of its own observations.
 """
 from __future__ import annotations
 
@@ -21,16 +26,26 @@ from .batch import Engine, Model, SERIES_MAJOR, _mem_and_ptr, bound_engine
 
 
 def _problem(model: Model, params: Dict, y, keep_init: bool):
-    assert model.p == 1 and model.n <= 4 and model.times is None and not model.f_tv and not model.g_tv
+    assert model.p == 1 and model.n <= 4 and model.times is None and not model.g_tv
+    assert tuple(model.per_series) in ((), ("F",)) and (model.f_tv or not model.per_series)
     keep = [_dlm.cm(np.atleast_2d(np.asarray(params["V"], float))),
             _dlm.cm(np.atleast_2d(np.asarray(params["W"], float))),
             np.ascontiguousarray(np.asarray(params["m0"], float).ravel()),
             _dlm.cm(np.atleast_2d(np.asarray(params["C0"], float)))]
     mem, yptr = _mem_and_ptr(y)
     assert mem == capi.DEVICE, "scan path takes device-resident y"
+    F, per = model.F, 0
+    if model.per_series:  # device F [T][n], read in place
+        assert model.F.numel() == model.T * model.n, tuple(model.F.shape)
+        fmem, F = _mem_and_ptr(model.F)
+        assert fmem == capi.DEVICE, "per-series F lives with y on the device"
+        per = capi.PS_F
+    elif model.f_tv:  # host F [T][n]
+        F = np.ascontiguousarray(np.asarray(model.F, float).reshape(model.T, model.n))
+        keep.append(F)
     pr = capi.make_problem(B=1, T=model.T, n=model.n, p=1, layout=SERIES_MAJOR, mem=capi.DEVICE,
-                           keep_init=keep_init, F=model.F, G=model.G, times=None, V=keep[0],
-                           W=keep[1], m0=keep[2], C0=keep[3], y=yptr)
+                           keep_init=keep_init, F=F, G=model.G, times=None, V=keep[0],
+                           W=keep[1], m0=keep[2], C0=keep[3], y=yptr, per_series=per, f_tv=model.f_tv)
     return pr, keep
 
 

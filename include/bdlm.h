@@ -97,7 +97,8 @@ enum {
                                  instead of T dependent steps of ~0.3 us each, at 1e-9 relative
                                  instead of bit-for-bit agreement with the sequential recursion --
                                  hence opt-in.  Eligible: B = 1, T >= 4096, p = 1, n <= 4, regular
-                                 grid, time-invariant model (no f_tv, g_tv, v_tv, w_tv), shared
+                                 grid, time-invariant G, V, W (no g_tv, v_tv, w_tv), F time-invariant
+                                 or per step (f_tv, shared or BDLM_PS_F), otherwise shared
                                  parameters, device or host buffers; then
                                    bdlm_kf_filter_smooth  runs bdlm_scan_filter_smooth when also
                                                           n = 1 or BDLM_TEXTBOOK_SMOOTHER;
@@ -310,8 +311,13 @@ BDLM_API int bdlm_gibbs_suffstats(bdlm_ctx *ctx, const bdlm_problem *prob, const
 /* ---- parallel-in-time filter + smoother for ONE long series ---------------------------
  * Not in the reference (its recursion is strictly sequential, Filter.scala:41-62; BASELINE
  * config 5).  Temporal parallelisation by associative scan (Sarkka & Garcia-Fernandez 2021).
- * Restrictions: B = 1, p = 1, n <= 4, regular grid (times = NULL), time-invariant F, G, V and W
- * (f_tv = g_tv = v_tv = w_tv = 0), shared parameters, mem = BDLM_DEVICE.  Results equal bdlm_kf_filter_smooth with
+ * Restrictions: B = 1, p = 1, n <= 4, regular grid (times = NULL), time-invariant G, V and W
+ * (g_tv = v_tv = w_tv = 0), shared parameters, mem = BDLM_DEVICE.  F is time-invariant, or given
+ * per step with f_tv = 1 (dynamic regression, F_t = (1, x_t)): a host F[T][n] (per_series = 0;
+ * copied to the device with each call) or, with per_series = BDLM_PS_F and no other bit, a device
+ * array laid out like y with k = n, read in place.  A per-step F costs each forward pass 8n bytes
+ * per step next to y's 8, and its level 1 composes the steps generically (no model table).
+ * Results equal bdlm_kf_filter_smooth with
  * BDLM_TEXTBOOK_SMOOTHER to 1e-9 relative (for n = 1 that is the reference itself).
  *
  * Single GPU: bdlm_scan_filter_smooth.  Several GPUs, each owning a contiguous time chunk:
